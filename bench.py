@@ -13,6 +13,7 @@ field inside the timed region).
   python bench.py --gpus 1 --steps 5 --warmup 3
   python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
   python bench.py --impl reference ...      (CPU arm: the oracle on the host cores)
+  python bench.py ... --dump-outputs DIR    (results of the last timed step as DIR/<name>.npy)
 
 Prints ONE JSON line (rank 0).  Keys: see the contract in the task; extra objects
 `roofline` (FP64 FMA pipe of the solve kernel, peak measured live by a DFMA probe)
@@ -89,6 +90,25 @@ def clocks_sampler(stop, out, gpu_index):
         except Exception:
             pass
         stop.wait(0.2)
+
+
+DUMP_FIELDS = ("u", "y", "cost", "exit_status", "outer", "inner", "fpr", "f1", "f2", "pen", "pred")
+DUMP_LIMIT_BYTES = 64 * 1024 * 1024
+
+
+def dump_outputs(bufs, out_dir):
+    """Write the results of one device solve (the buffers run_device filled) as out_dir/<name>.npy in
+    float64, rows in batch order.  `evals` is left out: two of its columns are clock readings.  A batch
+    larger than 64 MB is cut to a fixed, seeded sample of scenes; scene_index.npy lists the rows kept."""
+    host = {k: bufs[k].double().cpu().numpy() for k in DUMP_FIELDS if bufs[k] is not None}
+    n = len(host["cost"])
+    per_scene = sum(a[0].nbytes for a in host.values()) + 8
+    keep = min(n, DUMP_LIMIT_BYTES // per_scene)
+    idx = np.arange(n) if keep == n else np.sort(np.random.default_rng(0).choice(n, keep, replace=False))
+    host["scene_index"] = idx.astype(np.float64)
+    os.makedirs(out_dir, exist_ok=True)
+    for k, a in host.items():
+        np.save(os.path.join(out_dir, k + ".npy"), a if k == "scene_index" else a[idx])
 
 
 def summarize_clocks(samples):
@@ -200,6 +220,10 @@ def main():
                     help="host calls in flight in the e2e leg (0 = the same number as --depth; measured on one B200 with "
                          "20 steps, tools/e2e_ab.py: 5 calls 552 k, 6 calls 537 k, 7 calls 530 k, 8 calls 527 k solves/s)")
     ap.add_argument("--quick", action="store_true", help="sweep rows: skip the sequential / pageable / one-scene legs")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the results of the last timed step (rank 0) as DIR/<name>.npy, float64, at most "
+                         "64 MB (a fixed, seeded sample of scenes beyond that): two builds run with the same "
+                         "arguments solve the same inputs and can be compared output for output")
     args = ap.parse_args()
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else max(args.warmup, 1)
 
@@ -324,6 +348,8 @@ def main():
     barrier()
     t_wall = time.perf_counter() - t_wall0
     stop.set()
+    if args.dump_outputs and rank == 0:  # before the buffers are reused below
+        dump_outputs(bufs_ring[(warm + args.steps - 1) % D], args.dump_outputs)
     total_ms = ev_a.elapsed_time(ev_b)
     stats = solver.read_stats(reset=True)
     local_ms = total_ms / args.steps

@@ -37,10 +37,7 @@ def test_reference_arm_other_ranks_do_no_work():
 
 
 def test_product_arm_has_no_cpu_path():
-    import torch
-    if torch.cuda.is_available():
-        import pytest
-        pytest.skip("a GPU is present: the product arm would run")
+    # the GPU is hidden from the child process, so this holds on a machine with a GPU as well
     r = run_bench("--steps", "1", "--warmup", "1", env={"CUDA_VISIBLE_DEVICES": ""})
     assert r.returncode != 0
     assert "no CPU path" in (r.stderr + r.stdout)
@@ -65,6 +62,43 @@ def test_workload_parsing_and_common_config():
     _, q0, _ = bench.build_workload("static4096", 0, 8, 2)
     import numpy as np
     assert np.array_equal(p0, p5) and not np.array_equal(p0, q0)
+
+
+def test_dump_outputs_writes_float64_and_samples_large_batches(tmp_path):
+    """--dump-outputs: every result field as <name>.npy in float64, rows in batch order; a batch over
+    the 64 MB cap becomes the same seeded sample of scenes every time."""
+    sys.path.insert(0, ROOT)
+    import bench
+    import numpy as np
+    import torch
+
+    def bufs(n, N=20):
+        g = torch.Generator().manual_seed(n)
+        f = lambda *s: torch.rand(*s, generator=g, dtype=torch.float64)
+        i = lambda *s: torch.randint(0, 4, s, generator=g, dtype=torch.int32)
+        return dict(u=f(n, 2 * N), y=f(n, 2 * N), cost=f(n), exit_status=i(n), outer=i(n), inner=i(n),
+                    fpr=f(n), f1=f(n), f2=f(n), pen=f(n), pred=f(n, N, 3),
+                    evals=torch.zeros(n, 4, dtype=torch.int64))
+
+    small = bufs(64)
+    bench.dump_outputs(small, str(tmp_path / "small"))
+    names = sorted(p.stem for p in (tmp_path / "small").iterdir())
+    assert names == sorted(list(bench.DUMP_FIELDS) + ["scene_index"])
+    for k in bench.DUMP_FIELDS:
+        a = np.load(tmp_path / "small" / f"{k}.npy")
+        assert a.dtype == np.float64 and np.array_equal(a, small[k].double().numpy())
+    assert np.array_equal(np.load(tmp_path / "small" / "scene_index.npy"), np.arange(64))
+
+    big = bufs(70000)   # ~1.2 kB of results per scene: more than 64 MB in all
+    for d in ("a", "b"):
+        bench.dump_outputs(big, str(tmp_path / d))
+    total = sum(p.stat().st_size for p in (tmp_path / "a").iterdir())
+    assert total <= bench.DUMP_LIMIT_BYTES + 256 * len(names)   # + the .npy headers
+    idx = np.load(tmp_path / "a" / "scene_index.npy").astype(np.int64)
+    assert 0 < len(idx) < 70000 and np.all(np.diff(idx) > 0)
+    assert np.array_equal(np.load(tmp_path / "a" / "u.npy"), big["u"].numpy()[idx])
+    for k in list(bench.DUMP_FIELDS) + ["scene_index"]:
+        assert np.array_equal(np.load(tmp_path / "a" / f"{k}.npy"), np.load(tmp_path / "b" / f"{k}.npy"))
 
 
 def test_default_depth_divides_the_step_count():
