@@ -94,20 +94,6 @@ def test_solve_parity_with_terminal_weights_and_changing_penalties(cfg, solver):
     assert_parity(sol, ref, n)
 
 
-def test_split_kernel_parity_with_oracle(cfg, solver, monkeypatch):
-    """The experimental cluster kernel (solver CTA + evaluator CTA over DSMEM, TTMPC_SPLIT=1)
-    must produce the same bits as the default kernel and the oracle."""
-    monkeypatch.setenv("TTMPC_SPLIT", "1")
-    n = 160
-    p = t.scenes.make_scenes(n, cfg, seed=12, n_static=4, n_dynamic=3, blocking_fraction=0.2)
-    sol = solver.run(p)
-    ref = O.solve_batch(cfg, p, threads=os.cpu_count(), warp=True)
-    assert_parity(sol, ref, n)
-    monkeypatch.setenv("TTMPC_SPLIT", "0")
-    sol0 = solver.run(p)
-    assert np.array_equal(sol0.solution, sol.solution) and np.array_equal(sol0.cost, sol.cost)
-
-
 def test_solve_parity_reference_order_easy_scenes(cfg, solver):
     """Against the oracle in the REFERENCE's operation order (libm, sequential sums):
     the two orders differ by rounding, which PANOC amplifies (DESIGN.md

@@ -339,16 +339,6 @@ static int solve_device_impl(const ttmpc_config *cfg, int n_scenes, const double
                              int use_y0, const double *d_c0, const ttmpc_result *res,
                              cudaStream_t st, Slot *host_slot, bool gated);
 
-// warps per CTA of the split kernel: as many scene regions as fit the 227 KB of one SM (<= 12)
-static int split_warps(const DevCfg &g) {
-  const int w = (int)(232448 / (size_t)g.smem_per_warp);
-  return w > 12 ? 12 : w;
-}
-static bool use_split(const DevCfg &g) {
-  const char *e = std::getenv("TTMPC_SPLIT");
-  return e && e[0] == '1' && split_warps(g) >= 1;
-}
-
 extern "C" int ttmpc_solve_batch_device(const ttmpc_config *cfg, int n_scenes, const double *d_p,
                                         int use_u0, int use_y0, const double *d_c0,
                                         const ttmpc_result *res, void *stream) {
@@ -371,8 +361,6 @@ static int solve_device_impl(const ttmpc_config *cfg, int n_scenes, const double
   Slot *sl = host_slot;
   const int *d_ready = (host_slot && gated) ? host_slot->ready : nullptr;
   int grid;
-  DevCfg gs = g;  // split kernel: clusters of (solver CTA, evaluator CTA)
-  int clusters = 0;
   bool want_order = false;
   {
     std::lock_guard<std::mutex> lk(g_mu);
@@ -384,20 +372,12 @@ static int solve_device_impl(const ttmpc_config *cfg, int n_scenes, const double
     rc = grid_for(w, g, n_scenes, &grid);
     if (rc) return rc;
     const size_t table = (size_t)DYN_FIELDS * g.Ndyn * g.N * sizeof(double);
-    if (use_split(g)) {
-      gs.warps_per_block = split_warps(g);
-      const long long want = ((long long)n_scenes + gs.warps_per_block - 1) / gs.warps_per_block;
-      clusters = (int)std::min<long long>(std::max(1, w->sm_count / 2), want);
-    }
-    rc = ensure_dyn(sl, (table ? table : 8) * std::max((size_t)grid * g.warps_per_block,
-                                                       (size_t)clusters * gs.warps_per_block));
+    rc = ensure_dyn(sl, (table ? table : 8) * (size_t)grid * g.warps_per_block);
     if (rc) return rc;
     // more scenes than resident warps: dispatch the likely-long ones first.  Not on the streamed
     // host path (scenes become available in index order there).  TTMPC_NO_ORDER=1 disables it.
     const char *no = std::getenv("TTMPC_NO_ORDER");
-    const long long resident = clusters > 0 ? (long long)clusters * gs.warps_per_block
-                                            : (long long)grid * g.warps_per_block;
-    want_order = !d_ready && n_scenes > resident && !(no && no[0] == '1');
+    want_order = !d_ready && n_scenes > (long long)grid * g.warps_per_block && !(no && no[0] == '1');
     if (want_order) {
       rc = ensure_order(sl, 2 * (size_t)n_scenes + 64);
       if (rc) return rc;
@@ -432,8 +412,7 @@ static int solve_device_impl(const ttmpc_config *cfg, int n_scenes, const double
     if (e[0] == 's') small_code = true;
     else if (e[0] == 'u') small_code = false;
   }
-  if (clusters > 0) CUDA_TRY(launch_solve_split(gs, A, clusters, st));
-  else if (small_code) CUDA_TRY(launch_solve_small(g, A, grid, st));
+  if (small_code) CUDA_TRY(launch_solve_small(g, A, grid, st));
   else CUDA_TRY(launch_solve(g, A, grid, st));
   return TTMPC_OK;
 }

@@ -27,64 +27,11 @@
 
 // Unroll policy of the hot loops.  The kernel is bound by instruction-cache refills (DESIGN.md
 // section 6), so every unroll factor is a trade between dependent-issue latency and code bytes;
-// -DTTMPC_SMALL_CODE builds the variant with every hot loop rolled.
-// Round-2 experiment (off by default, the default build is unchanged): -DTTMPC_COLD_OUTLINE keeps
-// the per-scene code (staging, helper service loop) out of the kernel body so that the
-// per-iteration code is contiguous; measure with tools/variants_r2.sh.  First measurement (end of
-// round 1): bit-identical, in-flight rate 428 k against 435 k solves/s -- no gain.
-#ifdef TTMPC_COLD_OUTLINE
-#define TT_COLD_INLINE static __noinline__
-#define TT_COLD_TPL __noinline__
-#else
-#define TT_COLD_INLINE inline
-#define TT_COLD_TPL
-#endif
+// -DTTMPC_SMALL_CODE builds the variant with the static-obstacle loop rolled.
 #ifdef TTMPC_SMALL_CODE
-#define TT_UNROLL_SCAN _Pragma("unroll 1")
-// the reference-path loop (10 trips, the largest dynamic block of an evaluation) is unrolled by 2
-// in the bulk build as well: two independent distance chains per trip, +4 % (measured, r2)
-#ifndef TT_SMALL_UNROLL_REFPATH
-#define TT_SMALL_UNROLL_REFPATH 2
-#endif
-#define TT_PRAGMA_(x) _Pragma(#x)
-#define TT_PRAGMA(x) TT_PRAGMA_(x)
-#define TT_UNROLL_2 TT_PRAGMA(unroll TT_SMALL_UNROLL_REFPATH)
-#ifdef TT_SMALL_UNROLL_STATIC    // experiment: static-obstacle loop unrolled by 2 in the bulk build
-#define TT_UNROLL_4 _Pragma("unroll 2")
-#else
 #define TT_UNROLL_4 _Pragma("unroll 1")
-#endif
 #else
-#define TT_UNROLL_SCAN _Pragma("unroll")
-#define TT_UNROLL_2 _Pragma("unroll 2")
 #define TT_UNROLL_4 _Pragma("unroll 4")
-#endif
-
-// Code-factoring switches (round 2).  The solve kernel is bound by instruction-cache refills: 8-12
-// warps per SM walk a ~39 KB hot loop out of phase through a 32 KB cache.  Each bit moves one
-// family of repeated code out of line into ONE shared copy (a few call instructions instead of an
-// inlined body per use): fewer distinct cache lines at the price of call overhead and less
-// interleaving.  Same operations in the same order either way (bit-identical results); the
-// default is what measured fastest on the B200 (profiles/r2_*, DESIGN.md section 6).
-//   1 sincos   2 scans   4 divisions / square roots   16 literal (UMOV) sincos constants
-#ifndef TT_FACTOR
-#define TT_FACTOR 4
-#endif
-// Scalar-work switches (round 2, third session; bit-identical either way, tools/r2_ab4.sh / r2_ab5.sh):
-//   1 zero numerators of the envelope divisions bypass the IEEE division (its slow path otherwise)
-//   2 sigma is formed when gamma changes, not in every iteration
-//   4 so is the coefficient of the Lipschitz check (kept in the warp's shared-memory context)
-//   8 the sum over the penalty rows when only the static obstacles contribute is unrolled by 5
-//  16 1 / max(c, 1) is cached per penalty value in the warp's context (eval_psi)
-//  32 the terminal-cost block is skipped when both of its weights are zero (eval_psi; oracle mirrors it)
-//  64 the butterflies of the L-BFGS two-loop recursion are inlined (ttmpc_solve.cu lbfgs_apply)
-// Measured on static4096 (driver protocol): 0 -> 609 k solves/s, 15 -> 661 k (icc hit rate 86.6 -> 90.2 %:
-// the slow path of the division alone was 1.5 KB of hot code), 63 -> 655 k with 9 % fewer executed
-// instructions than 0 (2.22 G against 2.45 G per batch) -- below ~660 k the kernel no longer responds to the
-// instruction count, only to the layout of the hot lines and to the length of the dependent chain of an
-// iteration (127: 658.5 -> 666.7 k).
-#ifndef TT_OPT
-#define TT_OPT 127
 #endif
 namespace ttmpc {
 
@@ -174,24 +121,11 @@ __device__ __forceinline__ void tt_sincos_c(double x, double *s, double *c) {
   *s = so; *c = co;
 }
 
-#if TT_FACTOR & 1
-struct SC2 { double s, c; };
-static __device__ __noinline__ SC2 tt_sincos_call(double x) { SC2 r; tt_sincos_c(x, &r.s, &r.c); return r; }
-__device__ __forceinline__ void tt_sincos_hot(double x, double *s, double *c) { const SC2 r = tt_sincos_call(x); *s = r.s; *c = r.c; }
-#elif TT_FACTOR & 16
-__device__ __forceinline__ void tt_sincos_hot(double x, double *s, double *c) { tt_sincos(x, s, c); }
-#else
-__device__ __forceinline__ void tt_sincos_hot(double x, double *s, double *c) { tt_sincos_c(x, s, c); }
-#endif
 // IEEE division / square root: ~15 inlined instructions per use (MUFU seed, Newton steps, range
-// check, slow-path call); the PANOC step has a dozen of them
-#if TT_FACTOR & 4
+// check, slow-path call) and the PANOC step has a dozen of them, so they are out of line: one
+// shared copy keeps the hot loop inside the instruction cache (DESIGN.md section 6)
 static __device__ __noinline__ double tt_div(double a, double b) { return a / b; }
 static __device__ __noinline__ double tt_sqrt(double a) { return sqrt(a); }
-#else
-__device__ __forceinline__ double tt_div(double a, double b) { return a / b; }
-__device__ __forceinline__ double tt_sqrt(double a) { return sqrt(a); }
-#endif
 
 // ---------------------------------------------------------------- warp utils
 // Hand-written shuffle primitives.  Round 1 left these to the compiler as rolled loops in
@@ -225,82 +159,24 @@ __device__ __forceinline__ void down_add(double &v) {  // v += v[lane + O] on la
                "@p add.rn.f64 %0, %0, t;\n\t}"
                : "+d"(v) : "n"(O));
 }
-#if TT_FACTOR & 2
-#define TT_SCAN_FN static __device__ __noinline__
-#else
-#define TT_SCAN_FN __device__ __forceinline__
-#endif
-// The same scan levels with the offset in a register: a rolled loop of five trips (TT_SCAN_ROLLED, off).
-// One level is the same 9 instructions, the loop adds 3 per trip -- more executed instructions in the scans
-// for 1/4 of their code bytes (the six scans of an evaluation are 3.4 KB unrolled).  Measured (r2_ab5, both
-// scan directions rolled): instruction-cache hit rate 87.7 -> 90.0 %, `no_instruction` 0.65 -> 0.44 per
-// issue, but `wait` 2.14 -> 2.30 and `short_scoreboard` 1.04 -> 1.13: 644-648 k solves/s against 641-667 k.
-__device__ __forceinline__ void up_add_r(double &v, int o) {
-  asm volatile("{\n\t.reg .pred p;\n\t.reg .b32 lo, hi, tl, th;\n\t.reg .f64 t;\n\t"
-               "mov.b64 {lo, hi}, %0;\n\t"
-               "shfl.sync.up.b32 tl|p, lo, %1, 0, 0xffffffff;\n\t"
-               "shfl.sync.up.b32 th, hi, %1, 0, 0xffffffff;\n\t"
-               "mov.b64 t, {tl, th};\n\t"
-               "@p add.rn.f64 %0, %0, t;\n\t}"
-               : "+d"(v) : "r"(o));
-}
-__device__ __forceinline__ void down_add_r(double &v, int o) {
-  asm volatile("{\n\t.reg .pred p;\n\t.reg .b32 lo, hi, tl, th;\n\t.reg .f64 t;\n\t"
-               "mov.b64 {lo, hi}, %0;\n\t"
-               "shfl.sync.down.b32 tl|p, lo, %1, 31, 0xffffffff;\n\t"
-               "shfl.sync.down.b32 th, hi, %1, 31, 0xffffffff;\n\t"
-               "mov.b64 t, {tl, th};\n\t"
-               "@p add.rn.f64 %0, %0, t;\n\t}"
-               : "+d"(v) : "r"(o));
-}
-#ifndef TT_SCAN_ROLLED   // bit 0: prefix scans (rollout)  bit 1: suffix scans (adjoint)
-#define TT_SCAN_ROLLED 0
-#endif
-struct D2 { double a, b; };
 // inclusive prefix sum over lanes (Kogge-Stone)
-TT_SCAN_FN double wscan(double v, int) {
-#if TT_SCAN_ROLLED & 1
-#pragma unroll 1
-  for (int o = 1; o < 32; o <<= 1) up_add_r(v, o);
-#else
+__device__ __forceinline__ double wscan(double v, int) {
   up_add<1>(v); up_add<2>(v); up_add<4>(v); up_add<8>(v); up_add<16>(v);
-#endif
   return v;
 }
-TT_SCAN_FN D2 wscan2v(double a, double b) {  // two scans, interleaved
-#if TT_SCAN_ROLLED & 1
-#pragma unroll 1
-  for (int o = 1; o < 32; o <<= 1) { up_add_r(a, o); up_add_r(b, o); }
-#else
+__device__ __forceinline__ void wscan2(double &a, double &b) {  // two scans, interleaved
   up_add<1>(a); up_add<1>(b); up_add<2>(a); up_add<2>(b); up_add<4>(a); up_add<4>(b);
   up_add<8>(a); up_add<8>(b); up_add<16>(a); up_add<16>(b);
-#endif
-  D2 r; r.a = a; r.b = b;
-  return r;
 }
-__device__ __forceinline__ void wscan2(double &a, double &b) { const D2 r = wscan2v(a, b); a = r.a; b = r.b; }
 // inclusive suffix sum over lanes
-TT_SCAN_FN double wsuffix(double v, int) {
-#if TT_SCAN_ROLLED & 2
-#pragma unroll 1
-  for (int o = 1; o < 32; o <<= 1) down_add_r(v, o);
-#else
+__device__ __forceinline__ double wsuffix(double v, int) {
   down_add<1>(v); down_add<2>(v); down_add<4>(v); down_add<8>(v); down_add<16>(v);
-#endif
   return v;
 }
-TT_SCAN_FN D2 wsuffix2v(double a, double b) {
-#if TT_SCAN_ROLLED & 2
-#pragma unroll 1
-  for (int o = 1; o < 32; o <<= 1) { down_add_r(a, o); down_add_r(b, o); }
-#else
+__device__ __forceinline__ void wsuffix2(double &a, double &b) {
   down_add<1>(a); down_add<1>(b); down_add<2>(a); down_add<2>(b); down_add<4>(a); down_add<4>(b);
   down_add<8>(a); down_add<8>(b); down_add<16>(a); down_add<16>(b);
-#endif
-  D2 r; r.a = a; r.b = b;
-  return r;
 }
-__device__ __forceinline__ void wsuffix2(double &a, double &b) { const D2 r = wsuffix2v(a, b); a = r.a; b = r.b; }
 // v + v[lane ^ O] (the 64-bit shuffle intrinsic costs two extra moves per use)
 template <int O>
 __device__ __forceinline__ double xor_get(double v) {
@@ -403,8 +279,8 @@ struct WarpCtx {
   double box_half;
   unsigned long long dyn_live;       // bit j: dynamic obstacle j can matter inside the box
   unsigned fleet_live;               // bit j: other robot j can matter inside the box
-  double lipc;                       // PANOC: GAMMA_L_COEFF / (2 gamma) of the current gamma (TT_OPT & 4)
-  double icm_c, icm;                 // 1 / max(c, 1) of the last penalty c this warp evaluated with (TT_OPT & 16)
+  double lipc;                       // PANOC: GAMMA_L_COEFF / (2 gamma) of the current gamma
+  double icm_c, icm;                 // 1 / max(c, 1) of the last penalty c this warp evaluated with
 #ifdef TTMPC_PROFILE
   long long prof[8];                 // cycles per phase (diagnostic build only)
   long long eprof[10];               // cycles per section of eval_psi
@@ -432,11 +308,8 @@ struct WarpSmem {
   struct HelpHdr *hhdr;
 };
 struct HelpHdr {
-  unsigned long long bar;  // split kernel: mbarrier the peer CTA arrives on when a message is complete
   int state;        // 0 idle, 1 request posted, 2 result ready
   int grad;         // request: gradient wanted
-  int cmd, scene;   // split kernel: what the evaluator warp is asked to do / scene to stage
-  double *st_out;   // split kernel: predicted states of this evaluation go here (or null)
   double c, gamma_ls;
   double psi, f, f2sq, S, dd, g2;  // result
 };
@@ -700,7 +573,7 @@ __device__ inline void stage_part2(const DevCfg &g, const WarpSmem &sm, const do
 // ~35 us per scene, 1 % of an average solve: measured with -DTTMPC_PROFILE_STAGE, tools/stage_profile.py).
 // A cp.async.bulk landing zone in the (then empty) L-BFGS ring was tried and dropped: part 2 is
 // bound by its 300 sincos + 1200 divisions, not by the loads, and its 14.4 KB block does not fit the ring.
-__device__ TT_COLD_INLINE void stage_scene(const DevCfg &g, const WarpSmem &sm, const double *p,
+__device__ inline void stage_scene(const DevCfg &g, const WarpSmem &sm, const double *p,
                                    double *dyn_scratch, int lane) {
 #ifdef TTMPC_PROFILE_STAGE
   const long long td0 = clock64();
@@ -786,7 +659,6 @@ __device__ __noinline__ EvalOut eval_psi(const DevCfg *gp, unsigned char *smem_b
   //      chain (theta scan -> sincos -> position scan); in the same basic block these ~60 independent
   //      instructions fill its bubbles (+3 % solves/s, round 2).  They are ADDED to the cost at their
   //      original places below, so every accumulation keeps its order and the bits do not change.
-#if TT_OPT & 16
   // 1 / max(c, 1): c changes once per outer iteration, the division (an out-of-line call, with the NaN-aware
   // fmax ~55 executed instructions, 4 % of an evaluation) ran in every evaluation.  The warp that owns the
   // scene keeps the last (c, 1 / max(c, 1)) pair in its context; a helper evaluating on another warp's
@@ -794,9 +666,6 @@ __device__ __noinline__ EvalOut eval_psi(const DevCfg *gp, unsigned char *smem_b
   // The miss path is a function of its own: inlined it sat in the middle of the hot instruction stream
   // (0.5 KB the sequential prefetch fetched for nothing: icc hit rate 90.2 -> 87.7 %, -3 % solves/s).
   const double icm = __builtin_expect(!Dalt && c == cx->icm_c, 1) ? cx->icm : icm_miss(c, sm.ctx, Dalt == nullptr);
-#else
-  const double icm = tt_div(1.0, fmax(c, 1.0));  // an out-of-line call: first, so that what follows is ONE block
-#endif
   const double vr = sm.vref[lk];
   double t_vel, t_ctl, t_acc;
   double aa, aw, ea, ew, alm;
@@ -823,8 +692,8 @@ __device__ __noinline__ EvalOut eval_psi(const DevCfg *gp, unsigned char *smem_b
   const double tha = cx->th0 + th_ex;
   const double thb = fma(0.5, tw, tha), thc = tha + tw;
   double sa, ca, sb, cb, sc, cc;
-  tt_sincos_hot(tha, &sa, &ca);
-  tt_sincos_hot(thb, &sb, &cb);
+  tt_sincos_c(tha, &sa, &ca);
+  tt_sincos_c(thb, &sb, &cb);
   // heading at the end of step k = heading at the start of step k + 1 (lane k + 1 holds its sine
   // and cosine; lane N exists and carries w = 0 when N < 32): two sincos per evaluation, not three.
   // The two values differ by the rounding of (th0 + scan_{k-1}) + ts w_k against th0 + scan_k;
@@ -832,7 +701,7 @@ __device__ __noinline__ EvalOut eval_psi(const DevCfg *gp, unsigned char *smem_b
   if (N < 32) {
     sc = __shfl_down_sync(FULL, sa, 1); cc = __shfl_down_sync(FULL, ca, 1);
   } else {
-    tt_sincos_hot(thc, &sc, &cc);
+    tt_sincos_c(thc, &sc, &cc);
   }
   const double Cs = fma(4.0, cb, ca) + cc, Ss = fma(4.0, sb, sa) + sc;
   const double hv = g.h6 * v;
@@ -905,7 +774,8 @@ __device__ __noinline__ EvalOut eval_psi(const DevCfg *gp, unsigned char *smem_b
     const int trips = (nh >= N) ? (N + 1) / 2 : max((N + 1) / 2, N - nh);
     double dmin = INFINITY; int jmin = lo;
     const double2 *segv = reinterpret_cast<const double2 *>(sm.seg);
-TT_UNROLL_2
+    // unrolled by 2 in both builds: two independent distance chains per trip
+#pragma unroll 2
     for (int t = 0; t < trips; t++) {
       const int j = min(lo + t, N - 1);
       const double2 s1 = segv[3 * j], sd = segv[3 * j + 1];
@@ -1073,13 +943,9 @@ TT_UNROLL_2
   EPROF(3)
   // ---- terminal cost (l.242)
   double gt = 0.0;
-#if TT_OPT & 32
   // both terminal weights zero (config/mpc_default.yaml): every term below is a signed zero; the block is
   // a divergent branch of ~25 instructions run by one lane while 31 wait.  Mirrored in the oracle's WARP order.
   if (lane == N - 1 && (cx->qN != 0.0 || cx->qthetaN != 0.0)) {
-#else
-  if (lane == N - 1) {
-#endif
     const double dxg = X - cx->xg, dyg = Y - cx->yg, dtg = TH - cx->thg;
     cost += fma(cx->qthetaN, dtg * dtg, cx->qN * fma(dyg, dyg, dxg * dxg));
     if (GRAD) {
@@ -1116,11 +982,7 @@ TT_UNROLL_4
   } else if (__builtin_expect(S != 0.0, 0)) {  // every D_j is zero: F2_j = S + 0.0 = S (same operations, no loads)
     // taken by every second evaluation of the static workload (a robot inside a polygon): two dependent
     // chains of Ndyn links; unrolled by 5 the 15 trips cost 39 instructions instead of 75
-#if TT_OPT & 8
 #pragma unroll 5
-#else
-#pragma unroll 1
-#endif
     for (int j = 0; j < Ndyn; j++) {
       f2sq = fma(S, S, f2sq);
       sumF2 += S;

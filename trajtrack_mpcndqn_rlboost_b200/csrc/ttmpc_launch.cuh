@@ -38,7 +38,6 @@ struct EvalArgs {
 cudaError_t launch_solve(const DevCfg &g, const SolveArgs &A, int grid, cudaStream_t st);
 // the rolled-loop build of the same kernel (ttmpc_solve_small.cu): bulk batches
 cudaError_t launch_solve_small(const DevCfg &g, const SolveArgs &A, int grid, cudaStream_t st);
-cudaError_t launch_solve_split(const DevCfg &g, const SolveArgs &A, int clusters, cudaStream_t st);
 cudaError_t launch_rank_scenes(const DevCfg &g, const double *p, int n, int *scratch, int *order,
                                cudaStream_t st);
 cudaError_t launch_eval(const DevCfg &g, const EvalArgs &A, int grid, cudaStream_t st);

@@ -11,7 +11,6 @@
 // butterfly all-reduces.
 #include "ttmpc_device.cuh"
 #include "ttmpc_launch.cuh"
-#include <cooperative_groups.h>
 #include <algorithm>
 #include <cstdlib>
 #include <map>
@@ -86,32 +85,21 @@ __device__ __forceinline__ void project(const DevCfg &g, double a0, double a1, d
 // (The coefficient of the check lives in the warp's shared-memory context: a 256th register does
 // not exist and a spill costs more than the broadcast load.)
 __device__ __forceinline__ void set_lip_coeff(const Uni &U, const WarpSmem &sm) {
-#if TT_OPT & 4
   const double lc = tt_div(GAMMA_L_COEFF, 2.0 * U.gamma);
   __syncwarp();
   if ((threadIdx.x & 31) == 0) sm.ctx->lipc = lc;
   __syncwarp();
-#endif
 }
 __device__ __forceinline__ void set_gamma_terms(Uni &U, const WarpSmem &sm) {
   U.sigma = tt_div(1.0 - GAMMA_L_COEFF, 4.0 * U.gamma);
   set_lip_coeff(U, sm);
-}
-__device__ __forceinline__ double lip_coeff(const Uni &U, const WarpSmem &sm) {
-#if TT_OPT & 4
-  return sm.ctx->lipc;
-#else
-  return tt_div(GAMMA_L_COEFF, 2.0 * U.gamma);
-#endif
 }
 // x / gamma for the forward-backward envelope.  x = |gradient step - half step|^2 / 2 is exactly zero
 // whenever no box bound is active, and a zero numerator sends the IEEE division down its slow path
 // (~60 instructions and 1.5 KB of otherwise cold code in the instruction cache, taken by 11 % of all
 // divisions of a static4096 batch).  0 / y = 0 with the sign of x for every y > 0: same bits.
 __device__ __forceinline__ double div_env(double x, double y) {
-#if TT_OPT & 1
   if (x == 0.0 && y > 0.0) return x;
-#endif
   return tt_div(x, y);
 }
 
@@ -162,16 +150,10 @@ __device__ __forceinline__ void lbfgs_update(const DevCfg &g, const WarpSmem &sm
   __syncwarp();
 }
 
-// The 2 m inner products of the recursion are one dependent chain (each needs the vector the previous one
-// left), and with two warps per scheduler the solve follows the length of its dependent chains: their
-// butterfly is inlined (TT_OPT & 64: no call, no argument / result moves on that chain) at the price of
-// ~0.5 KB of hot code.  658.5 -> 666.7 k solves/s (two interleaved runs each, tools/r2_ab5.sh ab11).
-#if TT_OPT & 64
-#define TT_LBFGS_WSUM wsum_inl
-#else
-#define TT_LBFGS_WSUM wsum
-#endif
-// lbfgs::apply_hessian on the direction
+// lbfgs::apply_hessian on the direction.  The 2 m inner products of the recursion are one dependent chain
+// (each needs the vector the previous one left), and with two warps per scheduler the solve follows the
+// length of its dependent chains: their butterfly is inlined (no call, no argument / result moves on that
+// chain) at the price of ~0.5 KB of hot code (DESIGN.md section 6).
 template <class DM>
 __device__ __forceinline__ void lbfgs_apply(const DevCfg &g, const WarpSmem &sm, Lane &z,
                                             const Uni &U, int lane) {
@@ -185,7 +167,7 @@ __device__ __forceinline__ void lbfgs_apply(const DevCfg &g, const WarpSmem &sm,
 #pragma unroll 1
   for (int i = 0; i < m; i++) {  // newest to oldest
     const double2 s = sm.lbs[k * NP + lk], y = sm.lby[k * NP + lk];
-    const double a = sm.rho[k] * TT_LBFGS_WSUM(act ? pdot(s.x, s.y, q0, q1) : 0.0);
+    const double a = sm.rho[k] * wsum_inl(act ? pdot(s.x, s.y, q0, q1) : 0.0);
     if (lane == i) a_me = a;
     q0 = fma(-a, y.x, q0); q1 = fma(-a, y.y, q1);
     k = (k + 1 == M1) ? 0 : k + 1;
@@ -195,7 +177,7 @@ __device__ __forceinline__ void lbfgs_apply(const DevCfg &g, const WarpSmem &sm,
   for (int i = m - 1; i >= 0; i--) {  // oldest to newest
     k = (k == 0) ? M1 - 1 : k - 1;
     const double2 s = sm.lbs[k * NP + lk], y = sm.lby[k * NP + lk];
-    const double beta = sm.rho[k] * TT_LBFGS_WSUM(act ? pdot(y.x, y.y, q0, q1) : 0.0);
+    const double beta = sm.rho[k] * wsum_inl(act ? pdot(y.x, y.y, q0, q1) : 0.0);
     const double cf = __shfl_sync(FULL, a_me, i) - beta;
     q0 = fma(cf, s.x, q0); q1 = fma(cf, s.y, q1);
   }
@@ -235,96 +217,17 @@ struct HelpCtl {
                              // before the scene tables are re-staged (see solve_kernel)
   volatile int *slot;        // &cta->helper[me]
   bool pending;              // a posted request has not been collected yet
-  // split kernel (solver CTA): this warp's evaluator mailbox in the peer CTA's shared memory
-  double2 *r_hreq, *r_yrow;
-  HelpHdr *r_hdr;
-  unsigned phase, peer_rank; // parity of the next answer on sm.hhdr->bar; rank of the evaluator CTA
-  int *fail;                 // set when the evaluator did not answer (host re-runs the batch)
 };
-enum { CMD_EVAL = 0, CMD_STAGE = 1, CMD_EXIT = 2 };
-
-__device__ __forceinline__ void fence_cluster() { asm volatile("fence.acq_rel.cluster;" ::: "memory"); }
-// mbarrier helpers of the split kernel: a waiting warp sleeps in hardware instead of polling
-__device__ __forceinline__ unsigned smem_u32(const void *p) { return (unsigned)__cvta_generic_to_shared(p); }
-__device__ __forceinline__ void mbar_init(void *bar, int count) {
-  asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(smem_u32(bar)), "r"(count) : "memory");
-}
-// arrive on the barrier at the same offset in CTA `peer_rank` of the cluster
-__device__ __forceinline__ void mbar_arrive_peer(const void *local_bar, unsigned peer_rank) {
-  unsigned raddr;
-  asm volatile("mapa.shared::cluster.u32 %0, %1, %2;" : "=r"(raddr) : "r"(smem_u32(local_bar)), "r"(peer_rank));
-  asm volatile("mbarrier.arrive.release.cluster.shared::cluster.b64 _, [%0];" ::"r"(raddr) : "memory");
-}
-__device__ __forceinline__ bool mbar_try_wait(void *bar, unsigned parity) {
-  unsigned ok;
-  const unsigned hint_ns = 100000;  // the warp may stay suspended this long before try_wait gives up
-  asm volatile(
-      "{ .reg .pred p; mbarrier.try_wait.parity.acquire.cluster.shared::cta.b64 p, [%1], %2, %3; selp.u32 %0, 1, 0, p; }"
-      : "=r"(ok) : "r"(smem_u32(bar)), "r"(parity), "r"(hint_ns) : "memory");
-  return ok != 0;
-}
-// false = nothing arrived within `limit_ns`
-__device__ __forceinline__ bool mbar_wait(void *bar, unsigned parity, unsigned long long limit_ns) {
-  if (mbar_try_wait(bar, parity)) return true;
-  const unsigned long long t0 = globaltimer_ns();
-  int n = 0;
-  while (!mbar_try_wait(bar, parity))
-    if (((++n) & 63) == 0 && globaltimer_ns() - t0 > limit_ns) return false;
-  return true;
-}
-// SP = split kernel: requests go to the evaluator warp in the peer CTA (always there)
 // HELP = false: the instantiation of panoc_step without any request path (see solve_scene)
-template <bool SP, bool HELP = true>
+template <bool HELP>
 __device__ __forceinline__ bool help_available(const HelpCtl &hc) {
-  if constexpr (SP) return hc.enabled;
-  else if constexpr (!HELP) return false;
+  if constexpr (!HELP) return false;
   else return hc.enabled && *hc.slot >= 0;
 }
-template <bool SP>
-__device__ __forceinline__ bool help_wait(HelpCtl &hc, const WarpSmem &sm, int lane, int N, EvalOut &e);
-// The mailbox lives in the owner's shared-memory region (request row, answer row, header);
-// in the split kernel the request half is in the evaluator's region, the answer half here.
-template <bool SP>
-__device__ __forceinline__ void help_post(HelpCtl &hc, const WarpSmem &sm, int lane, int N, double v,
-                                          double w, double c, int grad, double gamma_ls,
-                                          int cmd = CMD_EVAL, int scene = 0, double *st_out = nullptr) {
-  if (hc.pending) {  // a speculative evaluation nobody needed: let it finish first
-    EvalOut tmp;
-    if (!help_wait<SP>(hc, sm, lane, N, tmp)) return;
-  }
-  if constexpr (SP) {
-    if (!hc.enabled) return;
-    // every lane stores its share of the message and then arrives (release) on the evaluator's
-    // barrier: no fence, no cross-lane ordering needed
-    if (lane < N) hc.r_hreq[lane] = make_double2(v, w);
-    {
-      HelpHdr *h = hc.r_hdr;
-      if (lane == 31) h->c = c;
-      if (lane == 30) h->gamma_ls = gamma_ls;
-      if (lane == 29) { h->grad = grad; h->cmd = cmd; }
-      if (lane == 28) h->scene = scene;
-      if (lane == 27) h->st_out = st_out;
-    }
-    mbar_arrive_peer(&sm.hhdr->bar, hc.peer_rank);
-  } else {
-    if (lane < N) sm.hreq[lane] = make_double2(v, w);
-    if (lane == 0) { sm.hhdr->c = c; sm.hhdr->gamma_ls = gamma_ls; sm.hhdr->grad = grad; }
-    __threadfence_block();
-    __syncwarp();
-    if (lane == 0) *reinterpret_cast<volatile int *>(&sm.hhdr->state) = 1;
-  }
-  hc.pending = true;
-}
 // Collect the posted evaluation.  false = the helper did not answer in time (treated as gone).
-template <bool SP>
 __device__ __forceinline__ bool help_wait(HelpCtl &hc, const WarpSmem &sm, int lane, int N, EvalOut &e) {
-  if (SP && !hc.pending) return false;
   int ok = 1;
-  if constexpr (SP) {
-    ok = mbar_wait(&sm.hhdr->bar, hc.phase, 2000000000ull) ? 1 : 0;  // acquire, every lane
-    ok = __all_sync(FULL, ok);
-    hc.phase ^= 1u;
-  } else if (lane == 0) {
+  if (lane == 0) {
     const volatile int *st = reinterpret_cast<volatile int *>(&sm.hhdr->state);
     const unsigned long long t0 = globaltimer_ns();
     int spins = 0;
@@ -332,15 +235,14 @@ __device__ __forceinline__ bool help_wait(HelpCtl &hc, const WarpSmem &sm, int l
       if (((++spins) & 1023) == 0 && globaltimer_ns() - t0 > 50000000ull) { ok = 0; break; }
     }
   }
-  if (!SP) ok = __shfl_sync(FULL, ok, 0);
+  ok = __shfl_sync(FULL, ok, 0);
   hc.pending = false;
   if (!ok) {
     hc.enabled = false;
     hc.timed_out = true;
-    if (SP && lane == 0 && hc.fail) atomicExch(hc.fail, 1);
     return false;
   }
-  if constexpr (!SP) __threadfence_block();
+  __threadfence_block();
   const volatile HelpHdr *h = sm.hhdr;
   e.psi = h->psi; e.f = h->f; e.f2sq = h->f2sq; e.S = h->S; e.dd = h->dd; e.g2 = h->g2;
   {
@@ -351,69 +253,48 @@ __device__ __forceinline__ bool help_wait(HelpCtl &hc, const WarpSmem &sm, int l
   e.any_hard = false;
   e.h0 = e.h1 = 0.0;
   __syncwarp();
-  if (!SP && lane == 0) *reinterpret_cast<volatile int *>(&sm.hhdr->state) = 0;
+  if (lane == 0) *reinterpret_cast<volatile int *>(&sm.hhdr->state) = 0;
   return true;
 }
-template <bool SP>
-__device__ __forceinline__ void help_drain(HelpCtl &hc, const WarpSmem &sm, int lane, int N) {
-  if (hc.pending) { EvalOut tmp; help_wait<SP>(hc, sm, lane, N, tmp); }
-}
-// split kernel: an evaluation is a request to the evaluator warp
-__device__ __forceinline__ EvalOut remote_eval(HelpCtl &hc, const WarpSmem &sm, int lane, int N, double v,
-                                               double w, double c, int grad, double gamma_ls,
-                                               double *st_out = nullptr) {
-  EvalOut e;
-  help_post<true>(hc, sm, lane, N, v, w, c, grad, gamma_ls, CMD_EVAL, 0, st_out);
-  if (!help_wait<true>(hc, sm, lane, N, e)) {
-    e.psi = e.f = e.f2sq = e.S = e.dd = e.g2 = e.gv = e.gw = NAN;
-    e.h0 = e.h1 = NAN; e.any_hard = false;
+// The mailbox lives in the owner's shared-memory region (request row, answer row, header).
+__device__ __forceinline__ void help_post(HelpCtl &hc, const WarpSmem &sm, int lane, int N, double v,
+                                          double w, double c, int grad, double gamma_ls) {
+  if (hc.pending) {  // a speculative evaluation nobody needed: let it finish first
+    EvalOut tmp;
+    if (!help_wait(hc, sm, lane, N, tmp)) return;
   }
-  return e;
+  if (lane < N) sm.hreq[lane] = make_double2(v, w);
+  if (lane == 0) { sm.hhdr->c = c; sm.hhdr->gamma_ls = gamma_ls; sm.hhdr->grad = grad; }
+  __threadfence_block();
+  __syncwarp();
+  if (lane == 0) *reinterpret_cast<volatile int *>(&sm.hhdr->state) = 1;
+  hc.pending = true;
+}
+__device__ __forceinline__ void help_drain(HelpCtl &hc, const WarpSmem &sm, int lane, int N) {
+  if (hc.pending) { EvalOut tmp; help_wait(hc, sm, lane, N, tmp); }
 }
 
 struct Problem {  // what eval needs besides the point
   double c, ya, yw;
 };
 
-template <class DM, bool SP>
+template <class DM>
 __device__ __forceinline__ double eval_cost(const DevCfg &g, const WarpSmem &sm, int lane,
                                             const Problem &pb, double a0, double a1, HelpCtl &hc) {
-  if constexpr (SP) {
-    PROF_BEGIN(t0)
-    const EvalOut e = remote_eval(hc, sm, lane, DM::N(g), a0, a1, pb.c, 0, 0.0);
-    PROF_END(t0, 0)
-    if (lane == 0) sm.ctx->n_cost++;
-    return e.psi;
-  } else {
-    PROF_BEGIN(t0)
-    EvalOut e = eval_psi<DM>(&g, reinterpret_cast<unsigned char *>(sm.ctx), a0, a1, pb.c, pb.ya,
-                             pb.yw, nullptr, false, 0.0);
-    PROF_END(t0, 0)
-#ifdef TTMPC_PROFILE_DOUBLE
-    {  // I-cache experiment: the same evaluation again, timed separately (slot 4)
-      PROF_BEGIN(t1)
-      EvalOut e2 = eval_psi<DM>(&g, reinterpret_cast<unsigned char *>(sm.ctx), a0, a1, pb.c, pb.ya,
-                                pb.yw, nullptr, false, 0.0);
-      PROF_END(t1, 4)
-      if (e2.psi != e.psi) __trap();
-    }
-#endif
-    if (lane == 0) sm.ctx->n_cost++;
-    return e.psi;
-  }
+  PROF_BEGIN(t0)
+  EvalOut e = eval_psi<DM>(&g, reinterpret_cast<unsigned char *>(sm.ctx), a0, a1, pb.c, pb.ya,
+                           pb.yw, nullptr, false, 0.0);
+  PROF_END(t0, 0)
+  if (lane == 0) sm.ctx->n_cost++;
+  return e.psi;
 }
-template <class DM, bool SP>
+template <class DM>
 __device__ __forceinline__ double eval_grad(const DevCfg &g, const WarpSmem &sm, int lane,
                                             const Problem &pb, double a0, double a1, double &o0,
                                             double &o1, HelpCtl &hc) {
   PROF_BEGIN(t0)
-  EvalOut e;
-  if constexpr (SP) {
-    e = remote_eval(hc, sm, lane, DM::N(g), a0, a1, pb.c, 1, 0.0);
-  } else {
-    e = eval_psi<DM>(&g, reinterpret_cast<unsigned char *>(sm.ctx), a0, a1, pb.c, pb.ya, pb.yw,
-                     nullptr, true, 0.0);
-  }
+  EvalOut e = eval_psi<DM>(&g, reinterpret_cast<unsigned char *>(sm.ctx), a0, a1, pb.c, pb.ya, pb.yw,
+                           nullptr, true, 0.0);
   PROF_END(t0, 1)
   if (lane == 0) sm.ctx->n_grad++;
   o0 = e.gv; o1 = e.gw;
@@ -446,7 +327,7 @@ __device__ __forceinline__ void gradient_and_half_step(const DevCfg &g, Lane &z,
 // Serve owner m (helper slot already taken) until its current scene ends.
 // false = nothing happened for 3 s (the caller gives up helping).
 template <class DM>
-__device__ TT_COLD_TPL bool serve_owner(const DevCfg &g, CtaHelp *cta, unsigned char *smem_raw, int m, int epoch_m,
+__device__ bool serve_owner(const DevCfg &g, CtaHelp *cta, unsigned char *smem_raw, int m, int epoch_m,
                             const WarpSmem &mine, int lane) {
   unsigned char *base_m = smem_raw + (size_t)m * g.smem_per_warp;
   const WarpSmem own = carve<DM>(base_m, g);
@@ -567,7 +448,7 @@ __device__ bool help_long_running_mate(const DevCfg &g, const SolveArgs &A, CtaH
 }
 
 // PANOCEngine::step.  Returns true to continue.
-template <class DM, bool SP, bool HELP>
+template <class DM, bool HELP>
 __device__ __forceinline__ bool panoc_step(const DevCfg &g, const WarpSmem &sm, int lane, const Problem &pb,
                            Lane &z, Uni &U, double tolerance, HelpCtl &hc) {
   PROF_BEGIN(t_step)
@@ -588,23 +469,19 @@ __device__ __forceinline__ bool panoc_step(const DevCfg &g, const WarpSmem &sm, 
   bool lbfgs_done = false;
   {
     double cost_half = 0.0;
-    const bool spec = __builtin_expect(help_available<SP, HELP>(hc), SP ? 1 : 0);
+    const bool spec = __builtin_expect(help_available<HELP>(hc), 0);
     int s_first = 0, s_head = 0, s_active = 0;
     double s_gamma = 0.0, s_os0 = 0.0, s_os1 = 0.0, s_og0 = 0.0, s_og1 = 0.0;
     if (spec) {
       PROF_BEGIN(tp)
-      help_post<SP>(hc, sm, lane, DM::N(g), z.h0, z.h1, pb.c, 0, 0.0);
+      help_post(hc, sm, lane, DM::N(g), z.h0, z.h1, pb.c, 0, 0.0);
       PROF_END(tp, 4)  // helper timeline: post
       s_first = U.lb_first; s_head = U.lb_head; s_active = U.lb_active;
       s_gamma = U.lb_gamma; s_os0 = z.os0; s_os1 = z.os1; s_og0 = z.og0; s_og1 = z.og1;
     }
 #pragma unroll 1
     for (int pass = 0; pass < 2; pass++) {
-#ifdef TT_EXPERIMENT_NO_LBFGS  // i-cache experiment only (wrong algorithm: gradient direction)
-      if (false) {
-#else
       if (pass == 0 ? spec : !lbfgs_done) {
-#endif
         PROF_BEGIN(tl)
         {
           PROF_BEGIN(t0)
@@ -624,17 +501,17 @@ __device__ __forceinline__ bool panoc_step(const DevCfg &g, const WarpSmem &sm, 
       if (spec) {
         EvalOut r;
         PROF_BEGIN(tw)
-        got = hc.pending && help_wait<SP>(hc, sm, lane, DM::N(g), r);
+        got = hc.pending && help_wait(hc, sm, lane, DM::N(g), r);
         PROF_END(tw, 6)  // waiting for the helper's psi(u_half)
         if (got) {
           cost_half = r.psi;
           if (lane == 0) sm.ctx->n_cost++;
         }
       }
-      if (!got) cost_half = eval_cost<DM, SP>(g, sm, lane, pb, z.h0, z.h1, hc);
+      if (!got) cost_half = eval_cost<DM>(g, sm, lane, pb, z.h0, z.h1, hc);
       if (spec) {
         const double rhs0 = U.cost + LIPSCHITZ_UPDATE_EPSILON * fabs(U.cost) - U.ip +
-                            lip_coeff(U, sm) * (U.norm_fpr * U.norm_fpr);
+                            sm.ctx->lipc * (U.norm_fpr * U.norm_fpr);
         if (cost_half > rhs0 && U.L < MAX_LIPSCHITZ_CONSTANT) {  // speculation lost
           U.lb_first = s_first; U.lb_head = s_head; U.lb_active = s_active; U.lb_gamma = s_gamma;
           z.os0 = s_os0; z.os1 = s_os1; z.og0 = s_og0; z.og1 = s_og1;
@@ -645,7 +522,7 @@ __device__ __forceinline__ bool panoc_step(const DevCfg &g, const WarpSmem &sm, 
       int it = 0;
       while (true) {
         const double rhs = U.cost + LIPSCHITZ_UPDATE_EPSILON * fabs(U.cost) - U.ip +
-                           lip_coeff(U, sm) * (U.norm_fpr * U.norm_fpr);
+                           sm.ctx->lipc * (U.norm_fpr * U.norm_fpr);
         if (!(cost_half > rhs && it < MAX_LIPSCHITZ_UPDATE_ITERATIONS &&
               U.L < MAX_LIPSCHITZ_CONSTANT))
           break;
@@ -654,23 +531,19 @@ __device__ __forceinline__ bool panoc_step(const DevCfg &g, const WarpSmem &sm, 
         U.gamma /= 2.0;
         set_lip_coeff(U, sm);
         gradient_and_half_step<false>(g, z, U, z.u0, z.u1);
-        cost_half = eval_cost<DM, SP>(g, sm, lane, pb, z.h0, z.h1, hc);
+        cost_half = eval_cost<DM>(g, sm, lane, pb, z.h0, z.h1, hc);
         compute_fpr(z, U);
         it++;
       }
       // gamma moved: the envelope scalars of the new gradient step / half step (iteration 0 takes its own step below)
       if (it > 0 && U.iteration > 0) gradient_and_half_step<true>(g, z, U, z.u0, z.u1);
-#if TT_OPT & 2
       if (it > 0) U.sigma = tt_div(1.0 - GAMMA_L_COEFF, 4.0 * U.gamma);  // gamma moved
-#else
-      U.sigma = tt_div(1.0 - GAMMA_L_COEFF, 4.0 * U.gamma);
-#endif
     }
   }
   if (U.iteration == 0) {
     // update_no_linesearch
     z.u0 = z.h0; z.u1 = z.h1;
-    U.cost = eval_grad<DM, SP>(g, sm, lane, pb, z.u0, z.u1, z.g0, z.g1, hc);
+    U.cost = eval_grad<DM>(g, sm, lane, pb, z.u0, z.u1, z.g0, z.g1, hc);
     gradient_and_half_step<true>(g, z, U, z.u0, z.u1);
   } else {
     // linesearch on the forward-backward envelope
@@ -684,30 +557,14 @@ __device__ __forceinline__ bool panoc_step(const DevCfg &g, const WarpSmem &sm, 
       const double one_m = 1.0 - U.tau;
       p0 = fma(-U.tau, z.d0, fma(-one_m, z.f0, z.u0));
       p1 = fma(-U.tau, z.d1, fma(-one_m, z.f1, z.u1));
-      if constexpr (SP) {
-        // split kernel: the evaluation runs on the evaluator warp; the gradient step and the
-        // half step are formed here from the returned gradient (same operations)
-        PROF_BEGIN(t0)
-        const EvalOut e = remote_eval(hc, sm, lane, DM::N(g), p0, p1, pb.c, 1, U.gamma);
-        PROF_END(t0, 1)
-        if (lane == 0) sm.ctx->n_grad++;
-        U.cost = e.psi;
-        z.g0 = e.gv; z.g1 = e.gw;
-        gradient_and_half_step<false>(g, z, U, p0, p1);
-        const double lhs_ls = U.cost - 0.5 * U.gamma * e.g2 + div_env(0.5 * e.dd, U.gamma);
-        U.env_dd = e.dd; U.env_g2 = e.g2;
-        if (!(lhs_ls > rhs_ls && nls < MAX_LINESEARCH_ITERATIONS)) break;
-        U.tau /= 2.0;
-        nls++;
-      } else {
       // with a helper: the next candidate (tau/2) is evaluated speculatively at the same time
       bool posted = false;
       double n0 = 0.0, n1 = 0.0;
-      if (__builtin_expect(nls < MAX_LINESEARCH_ITERATIONS && help_available<SP, HELP>(hc), 0)) {
+      if (__builtin_expect(nls < MAX_LINESEARCH_ITERATIONS && help_available<HELP>(hc), 0)) {
         const double tau2 = U.tau / 2.0, one_m2 = 1.0 - tau2;
         n0 = fma(-tau2, z.d0, fma(-one_m2, z.f0, z.u0));
         n1 = fma(-tau2, z.d1, fma(-one_m2, z.f1, z.u1));
-        help_post<SP>(hc, sm, lane, DM::N(g), n0, n1, pb.c, 1, U.gamma);
+        help_post(hc, sm, lane, DM::N(g), n0, n1, pb.c, 1, U.gamma);
         posted = hc.pending;
       }
       // cost, gradient, gradient step, half step and both envelope scalars in one evaluation
@@ -723,7 +580,7 @@ __device__ __forceinline__ bool panoc_step(const DevCfg &g, const WarpSmem &sm, 
       if (!(lhs_ls > rhs_ls && nls < MAX_LINESEARCH_ITERATIONS)) break;
       U.tau /= 2.0;
       nls++;
-      if (posted && help_wait<SP>(hc, sm, lane, DM::N(g), e)) {  // the helper's evaluation is the one at this tau
+      if (posted && help_wait(hc, sm, lane, DM::N(g), e)) {  // the helper's evaluation is the one at this tau
         if (lane == 0) sm.ctx->n_grad++;
         p0 = n0; p1 = n1;
         U.cost = e.psi;
@@ -734,7 +591,6 @@ __device__ __forceinline__ bool panoc_step(const DevCfg &g, const WarpSmem &sm, 
         if (!(lhs_ls > rhs_ls && nls < MAX_LINESEARCH_ITERATIONS)) break;
         U.tau /= 2.0;
         nls++;
-      }
       }
     }
     z.u0 = p0; z.u1 = p1;
@@ -750,7 +606,7 @@ __device__ __forceinline__ void panoc_reset(Uni &U) {
 }
 
 // One scene, start to finish.
-template <class DM, bool SP>
+template <class DM>
 __device__ void solve_scene(const DevCfg &g, const WarpSmem &sm, const SolveArgs &A, int scene,
                             int lane, unsigned long long *wstats, HelpCtl &hc) {
   const int N = g.N;
@@ -798,15 +654,15 @@ __device__ void solve_scene(const DevCfg &g, const WarpSmem &sm, const SolveArgs
     num_outer++;
     pb.ya = clipd(pb.ya, -1e12, 1e12);
     pb.yw = clipd(pb.yw, -1e12, 1e12);
-    help_drain<SP>(hc, sm, lane, N);
-    if (act) (SP ? hc.r_yrow : sm.yrow)[lane] = make_double2(pb.ya, pb.yw);  // what a helper evaluates with
+    help_drain(hc, sm, lane, N);
+    if (act) sm.yrow[lane] = make_double2(pb.ya, pb.yw);  // what a helper evaluates with
     __syncwarp();
     // ---------------- inner problem: PANOCOptimizer::solve
     int inner_status;
     {
       panoc_reset(U);
       // init: cost, gradient, local Lipschitz estimate
-      U.cost = eval_grad<DM, SP>(g, sm, lane, pb, z.u0, z.u1, z.g0, z.g1, hc);
+      U.cost = eval_grad<DM>(g, sm, lane, pb, z.u0, z.u1, z.g0, z.g1, hc);
       if (lane == 0) sm.ctx->n_cost++;  // the reference evaluates cost and gradient separately
       {
         double h0 = 0.0, h1 = 0.0;
@@ -815,7 +671,7 @@ __device__ void solve_scene(const DevCfg &g, const WarpSmem &sm, const SolveArgs
           h1 = (EPSILON_LIPSCHITZ * z.u1 > DELTA_LIPSCHITZ) ? EPSILON_LIPSCHITZ * z.u1 : DELTA_LIPSCHITZ;
         }
         double t0, t1;
-        eval_grad<DM, SP>(g, sm, lane, pb, z.u0 + h0, z.u1 + h1, t0, t1, hc);
+        eval_grad<DM>(g, sm, lane, pb, z.u0 + h0, z.u1 + h1, t0, t1, hc);
         const double e0 = t0 - z.g0, e1 = t1 - z.g1;
         double nh = pdot(h0, h1, h0, h1);
         double nd = pdot(e0, e1, e0, e1);
@@ -836,14 +692,10 @@ __device__ void solve_scene(const DevCfg &g, const WarpSmem &sm, const SolveArgs
         // helper-aware one takes over the moment a helper attaches (tail of a batch, one scene
         // alone).  Same arithmetic: results do not depend on which one ran.
         bool flag;
-        if constexpr (SP) {
-          flag = panoc_step<DM, true, true>(g, sm, lane, pb, z, U, g.tol, hc);
-        } else {
-          if (__builtin_expect(hc.enabled && *hc.slot >= 0, 0))
-            flag = panoc_step<DM, false, true>(g, sm, lane, pb, z, U, g.tol, hc);
-          else
-            flag = panoc_step<DM, false, false>(g, sm, lane, pb, z, U, g.tol, hc);
-        }
+        if (__builtin_expect(hc.enabled && *hc.slot >= 0, 0))
+          flag = panoc_step<DM, true>(g, sm, lane, pb, z, U, g.tol, hc);
+        else
+          flag = panoc_step<DM, false>(g, sm, lane, pb, z, U, g.tol, hc);
         if (!(flag && cont && in_time)) break;
         num_iter++;
         cont = num_iter < g.max_inner;
@@ -878,10 +730,9 @@ __device__ void solve_scene(const DevCfg &g, const WarpSmem &sm, const SolveArgs
       if (!act) { yp_a = 0.0; yp_w = 0.0; }
     }
     {
-      EvalOut e;
-      if constexpr (SP) e = remote_eval(hc, sm, lane, N, z.u0, z.u1, 0.0, 0, 0.0);  // c = 0: the multipliers do not enter f, F2
-      else e = eval_psi<DM>(&g, reinterpret_cast<unsigned char *>(sm.ctx), z.u0, z.u1, 0.0, 0.0,
-                            0.0, nullptr, false, 0.0);
+      // c = 0: the multipliers do not enter f, F2
+      const EvalOut e = eval_psi<DM>(&g, reinterpret_cast<unsigned char *>(sm.ctx), z.u0, z.u1, 0.0, 0.0,
+                                     0.0, nullptr, false, 0.0);
       if (lane == 0) sm.ctx->n_cost++;
       f2_norm_plus = sqrt(e.f2sq);
       f_final = e.f;
@@ -909,7 +760,7 @@ __device__ void solve_scene(const DevCfg &g, const WarpSmem &sm, const SolveArgs
   if (exit_status != TTMPC_NOT_FINITE && in_time && num_outer == g.max_outer)
     exit_status = TTMPC_NOT_CONVERGED_ITERATIONS;
 
-  help_drain<SP>(hc, sm, lane, N);  // no evaluation on this scene's tables may still be in flight
+  help_drain(hc, sm, lane, N);  // no evaluation on this scene's tables may still be in flight
   // ---------------- results
   if (act) {
     A.u[(size_t)scene * 2 * N + 2 * lane] = z.u0;
@@ -919,11 +770,9 @@ __device__ void solve_scene(const DevCfg &g, const WarpSmem &sm, const SolveArgs
       A.y[(size_t)scene * 2 * N + N + lane] = pb.yw;
     }
   }
-  if (A.pred_states) {
-    if constexpr (SP) remote_eval(hc, sm, lane, N, z.u0, z.u1, 0.0, 0, 0.0, A.pred_states + (size_t)scene * N * 3);
-    else eval_psi<DM>(&g, reinterpret_cast<unsigned char *>(sm.ctx), z.u0, z.u1, 0.0, 0.0, 0.0,
-                      A.pred_states + (size_t)scene * N * 3, false, 0.0);
-  }
+  if (A.pred_states)
+    eval_psi<DM>(&g, reinterpret_cast<unsigned char *>(sm.ctx), z.u0, z.u1, 0.0, 0.0, 0.0,
+                 A.pred_states + (size_t)scene * N * 3, false, 0.0);
   if (lane == 0) {
     if (A.cost) A.cost[scene] = f_final;
     if (A.exit_status) A.exit_status[scene] = exit_status;
@@ -945,9 +794,6 @@ __device__ void solve_scene(const DevCfg &g, const WarpSmem &sm, const SolveArgs
 #ifdef TTMPC_PROFILE
     // 4: cost evals, 5: grad evals, 6: lbfgs update + apply, 7: whole solve (cycles)
     wstats[4] += sm.ctx->prof[0]; wstats[5] += sm.ctx->prof[1];
-#ifdef TTMPC_PROFILE_DOUBLE
-    wstats[5] = wstats[5] - sm.ctx->prof[1] + sm.ctx->prof[4];  // slot 5 := repeated cost evals
-#endif
     wstats[6] += sm.ctx->prof[2] + sm.ctx->prof[3];
     wstats[7] += clock64() - t_clk0;
 #ifndef TTMPC_PROFILE_STAGE
@@ -980,7 +826,6 @@ __global__ void __launch_bounds__(TTMPC_MAX_THREADS, TTMPC_MIN_BLOCKS) solve_ker
   hc.timed_out = false;
   hc.slot = &cta->helper[warp];
   hc.pending = false;
-  hc.r_hreq = nullptr; hc.r_yrow = nullptr; hc.r_hdr = nullptr; hc.fail = nullptr; hc.phase = 0; hc.peer_rank = 0;
   if (lane == 0) sm.hhdr->state = 0;
   unsigned long long wstats[8] = {0, 0, 0, 0, 0, 0, 0, 0};
   bool had_scene = false;
@@ -1043,7 +888,7 @@ __global__ void __launch_bounds__(TTMPC_MAX_THREADS, TTMPC_MIN_BLOCKS) solve_ker
     if (lane == 0 && A.eprof) atomicAdd(A.eprof + 9, (unsigned long long)(clock64() - t_stage0));  // staging cycles (slot of the apply timer)
 #endif
     hc.enabled = A.helpers != 0 && !hc.timed_out;
-    solve_scene<DM, false>(g, sm, A, scene, lane, wstats, hc);
+    solve_scene<DM>(g, sm, A, scene, lane, wstats, hc);
     if (lane == 0) {
       *reinterpret_cast<volatile int *>(&cta->busy[warp]) = 0;
       if (A.run_stats) {
@@ -1114,150 +959,6 @@ __global__ void __launch_bounds__(256) order_scenes_kernel(int n, const int *__r
   int base = 0;
   for (int k = RANK_CLASSES - 1; k > c; k--) base += hist[k];
   order[base + atomicAdd(cursor + c, 1)] = scene;
-}
-
-// ------------------------------------------------------------------ split kernel
-// The hot loop of solve_kernel is ~47 KB of SASS per PANOC iteration against a 32 KB
-// instruction cache: with all resident warps at different places in it the SM is bound by
-// instruction-cache refills (a warp runs 3x slower than alone; the same code run in phase by
-// all warps only 1.3x, see tools/probe.py).  Here a cluster of two CTAs splits the work by
-// CODE: the solver CTA (rank 0) runs PANOC / L-BFGS / ALM and owns the L-BFGS history, the
-// evaluator CTA (rank 1) holds the scene tables and runs stage_scene + eval_psi.  Warp w of
-// the solver is paired with warp w of the evaluator; they talk through mailboxes in each
-// other's shared memory (DSMEM, ~215 cycles): request row + header in the evaluator's region,
-// gradient row + header in the solver's.  Each SM now loops over < 32 KB of code.  The
-// Lipschitz check psi(u_half) overlaps with the L-BFGS update/apply on every iteration
-// (the speculative path the tail helpers use).  Arithmetic is unchanged: results are
-// bit-identical to solve_kernel.
-template <class DM>
-__device__ void evaluator_loop(const DevCfg &g, const SolveArgs &A, unsigned char *my_base,
-                               const WarpSmem &peer, double *dyn, int lane, unsigned long long *wstats) {
-  const WarpSmem mine = carve<DM>(my_base, g);
-  const int N = g.N;
-  bool staged = false;
-  unsigned phase = 0;
-  const unsigned solver_rank = 0;
-  while (true) {
-    // sleep on the mailbox barrier until the solver warp has posted a message
-    if (!__all_sync(FULL, mbar_wait(&mine.hhdr->bar, phase, 5000000000ull))) break;  // never hang the GPU
-    phase ^= 1u;
-    const volatile HelpHdr *h = mine.hhdr;
-    const int cmd = h->cmd, scene = h->scene, grad = h->grad;
-    const double c = h->c, gamma_ls = h->gamma_ls;
-    double *st_out = h->st_out;
-    double2 pt = make_double2(0.0, 0.0), yv = make_double2(0.0, 0.0);
-    if (lane < N) {
-      const volatile double *rq = reinterpret_cast<const volatile double *>(mine.hreq);
-      const volatile double *yr = reinterpret_cast<const volatile double *>(mine.yrow);
-      pt.x = rq[2 * lane]; pt.y = rq[2 * lane + 1];
-      yv.x = yr[2 * lane]; yv.y = yr[2 * lane + 1];
-    }
-    __syncwarp();
-    if (cmd == CMD_EXIT) break;
-    if (cmd == CMD_STAGE) {
-      if (staged) wstats[2] += mine.ctx->n_body;
-      __syncwarp();
-      stage_scene(g, mine, A.p + (size_t)scene * g.np, dyn, lane);
-      staged = true;
-    } else {
-#ifdef TTMPC_PROFILE
-      const long long tp0 = clock64();
-#endif
-      const EvalOut e = eval_psi<DM>(&g, my_base, pt.x, pt.y, c, yv.x, yv.y, st_out, grad != 0, gamma_ls);
-#ifdef TTMPC_PROFILE
-      wstats[6] += clock64() - tp0;  // evaluator-side cycles (reported in the L-BFGS slot)
-#endif
-      if (lane < N) peer.hres[lane] = make_double2(e.gv, e.gw);
-      {
-        HelpHdr *r = peer.hhdr;
-        if (lane == 31) r->psi = e.psi;
-        if (lane == 30) r->f = e.f;
-        if (lane == 29) r->f2sq = e.f2sq;
-        if (lane == 28) r->S = e.S;
-        if (lane == 27) r->dd = e.dd;
-        if (lane == 26) r->g2 = e.g2;
-      }
-    }
-    mbar_arrive_peer(&mine.hhdr->bar, solver_rank);  // every lane: its stores, then release-arrive
-  }
-  if (staged) wstats[2] += mine.ctx->n_body;
-}
-
-template <class DM>
-__global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(384, 1)
-    solve_split_kernel(const __grid_constant__ DevCfg g, const __grid_constant__ SolveArgs A) {
-  namespace cg = cooperative_groups;
-  cg::cluster_group cluster = cg::this_cluster();
-  extern __shared__ __align__(16) unsigned char smem_raw[];
-  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-  const unsigned rank = cluster.block_rank();
-  unsigned char *my_base = smem_raw + (size_t)warp * g.smem_per_warp;
-  const WarpSmem sm = carve<DM>(my_base, g);
-  const WarpSmem peer = carve<DM>(cluster.map_shared_rank(my_base, rank ^ 1u), g);
-  if (lane == 0) {
-    sm.hhdr->state = 0;
-    mbar_init(&sm.hhdr->bar, 32);
-    asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-  }
-  cluster.sync();
-  unsigned long long wstats[8] = {0, 0, 0, 0, 0, 0, 0, 0};
-  if (rank == 0) {
-    HelpCtl hc;
-    hc.enabled = true; hc.timed_out = false; hc.slot = nullptr; hc.pending = false; hc.phase = 0; hc.peer_rank = 1;
-    hc.r_hreq = peer.hreq; hc.r_yrow = peer.yrow; hc.r_hdr = peer.hhdr; hc.fail = A.timeout_flag;
-    const int N = g.N;
-    while (true) {
-      int scene = 0;
-      if (lane == 0) scene = atomicAdd(A.work_counter, 1);
-      scene = __shfl_sync(FULL, scene, 0);
-      if (scene >= A.n_scenes) break;
-      if (A.order) scene = A.order[scene];
-      if (A.ready) {  // parameters of this scene may still be on their way from the host
-        int ok = 1;
-        if (lane == 0) {
-          const volatile int *rdy = A.ready;
-          const unsigned long long t0 = globaltimer_ns();
-          while (*rdy <= scene) {
-            __nanosleep(200);
-            if (globaltimer_ns() - t0 > 2000000000ull) {
-              ok = 0; if (A.timeout_flag) atomicExch(A.timeout_flag, 1); break;
-            }
-          }
-        }
-        ok = __shfl_sync(FULL, ok, 0);
-        if (!ok) break;
-        __threadfence();
-      }
-      // the evaluator builds the scene tables; this side only needs the initial controls
-      help_post<true>(hc, sm, lane, N, 0.0, 0.0, 0.0, 0, 0.0, CMD_STAGE, scene, nullptr);
-      if (lane == 0) {
-        const double *s = A.p + (size_t)scene * g.np + g.off_s;
-        WarpCtx *c = sm.ctx;
-        c->v_init = s[6]; c->w_init = s[7];
-        c->n_cost = 0; c->n_grad = 0; c->n_body = 0;
-#ifdef TTMPC_PROFILE
-        for (int i = 0; i < 8; i++) c->prof[i] = 0;
-        for (int i = 0; i < 10; i++) c->eprof[i] = 0;
-#endif
-      }
-      __syncwarp();
-      { EvalOut ack; help_wait<true>(hc, sm, lane, N, ack); }
-      solve_scene<DM, true>(g, sm, A, scene, lane, wstats, hc);
-      __syncwarp();
-    }
-    hc.enabled = true;  // the evaluator warp must always be released
-    help_drain<true>(hc, sm, lane, N);
-    help_post<true>(hc, sm, lane, N, 0.0, 0.0, 0.0, 0, 0.0, CMD_EXIT, 0, nullptr);
-  } else {
-    const int W = blockDim.x >> 5;
-    double *dyn = A.dyn_scratch + ((size_t)(blockIdx.x >> 1) * W + warp) * DYN_FIELDS * g.Ndyn * g.N;
-    evaluator_loop<DM>(g, A, my_base, peer, dyn, lane, wstats);
-  }
-  if (lane == 0 && A.stats) {
-    for (int i = 0; i < 8; i++)
-      if (wstats[i]) atomicAdd(A.stats + i, wstats[i]);
-  }
-  cluster.sync();  // nobody leaves while its shared memory may still be written by the peer
 }
 
 // ------------------------------------------------------------------ batched evaluation
@@ -1468,19 +1169,6 @@ cudaError_t solve_occupancy_impl(const DevCfg &g, int *blocks_per_sm) {
   });
 }
 #ifndef TTMPC_SMALL_CODE
-// clusters of (solver CTA, evaluator CTA); g.warps_per_block warps each
-cudaError_t launch_solve_split(const DevCfg &g, const SolveArgs &A, int clusters, cudaStream_t st) {
-  const size_t smem = (size_t)g.smem_per_warp * g.warps_per_block;
-  cudaError_t e;
-  if (is_default_dims(g)) {
-    if ((e = set_smem(solve_split_kernel<DimsDefault>, smem)) != cudaSuccess) return e;
-    solve_split_kernel<DimsDefault><<<2 * clusters, g.warps_per_block * 32, smem, st>>>(g, A);
-  } else {
-    if ((e = set_smem(solve_split_kernel<DimsRuntime>, smem)) != cudaSuccess) return e;
-    solve_split_kernel<DimsRuntime><<<2 * clusters, g.warps_per_block * 32, smem, st>>>(g, A);
-  }
-  return cudaGetLastError();
-}
 // scratch: cls[n] | hist[16] | cursor[16]   (ints; hist and cursor zeroed here)
 cudaError_t launch_rank_scenes(const DevCfg &g, const double *p, int n, int *scratch, int *order,
                                cudaStream_t st) {
