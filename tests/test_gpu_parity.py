@@ -282,6 +282,32 @@ def test_both_builds_of_the_solve_kernel_match_the_oracle(cfg, solver, monkeypat
     assert_parity(sol, ref, 160)
 
 
+@pytest.mark.parametrize("n", [300, 2500])
+def test_tail_helpers_change_no_result(cfg, solver, monkeypatch, n):
+    """A warp whose scenes are done helps a mate that is still solving (DESIGN.md section 3.1): the
+    solve is the same bit for bit with the helpers off (TTMPC_NO_HELPERS=1).  300 scenes fit the
+    resident warps: the unrolled build, and every CTA has a mate that finishes first and attaches as a
+    tail helper.  2500 scenes queue behind them: the rolled build, the dispatch order (device path)
+    and the early helpers.  Every field but `evals`: its columns 2-3 are clock readings, and its
+    columns 0-1 count evaluations that a helper may run speculatively."""
+    import dataclasses
+    import torch
+    p = t.scenes.make_scenes(n, cfg, seed=95, n_static=4, n_dynamic=3, blocking_fraction=0.2)
+    dp = torch.from_numpy(p).cuda()
+
+    def solve():
+        sol = solver.run_device(dp, solver.alloc_device(n))
+        torch.cuda.synchronize()
+        return {f.name: getattr(sol, f.name).cpu().numpy() for f in dataclasses.fields(sol)
+                if f.name not in ("evals", "solve_time_ms")}
+
+    helped = solve()
+    monkeypatch.setenv("TTMPC_NO_HELPERS", "1")
+    alone = solve()
+    for name, a in helped.items():
+        assert np.array_equal(a, alone[name]), name
+
+
 def test_batches_in_flight_on_several_streams_and_host_threads(cfg, solver):
     """Consecutive batches may overlap on the GPU (one scene queue per stream / per host call):
     every batch still gets exactly the results of a solve that had the GPU to itself."""

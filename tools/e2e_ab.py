@@ -1,8 +1,8 @@
-"""A/B of host-path settings inside one process (the library reads its environment switches at every call):
-alternates legs of BatchSolver.run_many (20 steps of static4096 from pinned host memory) over the cases below
-and prints the solves/s of every leg plus the medians.  Round 2, one B200: 5 calls in flight 552 k (mean of 7),
-6 calls 537 k, 7 calls 530 k, 8 calls 527 k, every call streamed 527 k; letting the parameter blocks of
-concurrent calls take turns on the PCIe link (tried, removed) changed nothing (536 k against 541 k).
+"""A/B of the number of host calls in flight inside one process: alternates legs of BatchSolver.run_many
+(20 steps of static4096 from pinned host memory) over the depths below and prints the solves/s of every leg
+plus the medians.  Round 2, one B200: 5 calls in flight 552 k (mean of 7), 6 calls 537 k, 7 calls 530 k,
+8 calls 527 k; letting the parameter blocks of concurrent calls take turns on the PCIe link (tried, removed)
+changed nothing (536 k against 541 k).
 usage: python tools/e2e_ab.py [repeats]"""
 import os, sys, time, statistics
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
@@ -18,16 +18,13 @@ for j in range(4):
     pp = t.pinned_empty(p.shape); pp[...] = p; ps.append(pp)
 s = t.BatchSolver(cfg)
 s.run_many(ps + ps, depth=6)
-def leg(depth, steps=20, **env):
-    for a, b in env.items(): os.environ[a] = b
+def leg(depth, steps=20):
     t0 = time.perf_counter(); s.run_many([ps[i % 4] for i in range(steps)], depth=depth); dt = time.perf_counter() - t0
-    for a in env: os.environ.pop(a)
     return 4096 * steps / dt / 1e3
-cases = {"depth 5": (5, {}), "depth 6": (6, {}), "depth 7": (7, {}), "depth 8": (8, {}),
-         "depth 6, every call streamed": (6, {"TTMPC_NO_STREAM": "0"})}
+cases = {"depth 5": 5, "depth 6": 6, "depth 7": 7, "depth 8": 8}
 res = {k: [] for k in cases}
 for r in range(reps):
-    for k, (d, env) in cases.items():
-        res[k].append(leg(d, **env))
+    for k, d in cases.items():
+        res[k].append(leg(d))
 for k, v in res.items():
     print(f"{k:32s} median {statistics.median(v):6.0f} k solves/s   runs {[round(x) for x in v]}", flush=True)

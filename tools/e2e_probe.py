@@ -1,5 +1,5 @@
-"""Diagnostic: host-path throughput (BatchSolver.run_many, pinned inputs) of this process for several
-settings; run several copies at once (one per GPU) to see how ranks disturb each other.
+"""Diagnostic: host-path throughput (BatchSolver.run_many, pinned inputs) of this process at several
+depths; run several copies at once (one per GPU) to see how ranks disturb each other.
 usage: CUDA_VISIBLE_DEVICES=k python tools/e2e_probe.py [start_epoch_seconds]"""
 import os, sys, time
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
@@ -24,21 +24,17 @@ s.run_many(ps + ps, depth=6)
 tag = os.environ.get("LOCAL_RANK", os.environ.get("CUDA_VISIBLE_DEVICES", "?")) + ("/nccl" if os.environ.get("PROBE_NCCL") == "1" else "") + "/omp" + os.environ.get("OMP_NUM_THREADS", "-")
 print(tag, "cpus", len(os.sched_getaffinity(0)), flush=True)
 k = 0
-def leg(name, depth, steps=18, **env):
+def leg(name, depth, steps=18):
     global k
-    for a, b in env.items(): os.environ[a] = b
     # all copies start each leg at the same wall-clock time
     k += 1
     if start:
         while time.time() < start + 6.0 * k: time.sleep(0.001)
     t0 = time.perf_counter(); s.run_many([ps[i % 4] for i in range(steps)], depth=depth); dt = time.perf_counter() - t0
-    for a in env: os.environ.pop(a)
     print(f"{tag} {name}: {1e3 * dt / steps:.2f} ms per step = {4096 * steps / dt / 1e3:.0f} k solves/s", flush=True)
 leg("depth 6", 6)
 if short: sys.exit(0)
 leg("depth 3", 3)
 leg("depth 2", 2)
 leg("depth 1", 1, steps=8)
-leg("depth 6, no chunk streaming", 6, TTMPC_NO_STREAM="1")
-leg("depth 6, staged like pageable", 6, TTMPC_NO_PINNED_INPUT="1")
 leg("depth 6 again", 6)

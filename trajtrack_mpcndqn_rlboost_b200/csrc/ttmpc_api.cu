@@ -115,10 +115,6 @@ static int make_devcfg(const ttmpc_config *c, DevCfg *g) {
       const int ctas = (int)std::min<size_t>(233472 / per_cta, (size_t)(8 / cand));
       if (ctas * cand > best) { best = ctas * cand; wpb = cand; }
     }
-    if (const char *e = std::getenv("TTMPC_WARPS_PER_BLOCK")) {  // tuning: scenes per CTA (1..4)
-      const int v = std::atoi(e);
-      if (v >= 1 && v <= 4 && (size_t)g->smem_per_warp * v <= cap) wpb = v;
-    }
     g->warps_per_block = wpb;
   }
   g->ts = c->ts; g->inv_ts = 1.0 / c->ts; g->h6 = c->ts / 6.0; g->veh_d2 = c->vehicle_width * c->vehicle_width; g->margin = c->social_margin;
@@ -326,10 +322,6 @@ static int grid_for(Workspace *w, const DevCfg &g, int n_scenes, int *grid) {
   CUDA_TRY(solve_occupancy(g, &bps));
   if (bps < 1) return fail(TTMPC_ERR_UNSUPPORTED, "configuration does not fit in shared memory");
   long long want = ((long long)n_scenes + g.warps_per_block - 1) / g.warps_per_block;
-  if (const char *e = std::getenv("TTMPC_MAX_BLOCKS_PER_SM")) {  // diagnostic: occupancy sweeps
-    const int v = std::atoi(e);
-    if (v >= 1 && v < bps) bps = v;
-  }
   long long cap = (long long)w->sm_count * bps;
   *grid = (int)(want < cap ? (want < 1 ? 1 : want) : cap);
   return TTMPC_OK;
@@ -375,9 +367,8 @@ static int solve_device_impl(const ttmpc_config *cfg, int n_scenes, const double
     rc = ensure_dyn(sl, (table ? table : 8) * (size_t)grid * g.warps_per_block);
     if (rc) return rc;
     // more scenes than resident warps: dispatch the likely-long ones first.  Not on the streamed
-    // host path (scenes become available in index order there).  TTMPC_NO_ORDER=1 disables it.
-    const char *no = std::getenv("TTMPC_NO_ORDER");
-    want_order = !d_ready && n_scenes > (long long)grid * g.warps_per_block && !(no && no[0] == '1');
+    // host path (scenes become available in index order there).
+    want_order = !d_ready && n_scenes > (long long)grid * g.warps_per_block;
     if (want_order) {
       rc = ensure_order(sl, 2 * (size_t)n_scenes + 64);
       if (rc) return rc;
@@ -395,9 +386,8 @@ static int solve_device_impl(const ttmpc_config *cfg, int n_scenes, const double
   A.inner_iters = res->inner_iters; A.pred_states = res->pred_states; A.evals = res->evals;
   A.dyn_scratch = sl->dyn_scratch; A.work_counter = sl->work_counter; A.stats = w->stats;
   A.run_stats = sl->run_stats;  // [0] evaluations, [1] count of finished scenes of this launch
-  { const char *ne = std::getenv("TTMPC_NO_EARLY_HELP"); if (ne && ne[0] == '1') A.run_stats = nullptr; }
   // the running average behind the early-helper threshold is per launch (workloads differ by 30x)
-  if (A.run_stats) CUDA_TRY(cudaMemsetAsync(A.run_stats, 0, 2 * sizeof(unsigned long long), st));
+  CUDA_TRY(cudaMemsetAsync(A.run_stats, 0, 2 * sizeof(unsigned long long), st));
   A.n_scenes = n_scenes; A.use_u0 = use_u0; A.use_y0 = use_y0;
   A.order = nullptr;
   if (want_order) {
@@ -469,37 +459,21 @@ extern "C" int ttmpc_fleet_step_device(const ttmpc_config *cfg, const ttmpc_flee
 
 // Cumulative device-side counters since the last reset:
 // [0] cost-only evaluations [1] cost+gradient evaluations [2] dynamic-obstacle
-// bodies executed [3] PANOC iterations.  Synchronises the device.
-extern "C" int ttmpc_read_stats24(unsigned long long out[24], int reset) {
+// bodies executed [3] PANOC iterations; the TTMPC_PROFILE builds fill the rest of the
+// 24 counters.  Reads the first `count`, resets all 24.  Synchronises the device.
+static int read_stats(unsigned long long *out, int count, int reset) {
   std::lock_guard<std::mutex> lk(g_mu);
   Workspace *w;
   int rc = get_ws(&w);
   if (rc) return rc;
   CUDA_TRY(cudaDeviceSynchronize());
-  CUDA_TRY(cudaMemcpy(out, w->stats, 24 * sizeof(unsigned long long), cudaMemcpyDeviceToHost));
+  CUDA_TRY(cudaMemcpy(out, w->stats, count * sizeof(unsigned long long), cudaMemcpyDeviceToHost));
   if (reset) CUDA_TRY(cudaMemset(w->stats, 0, 192));
   return TTMPC_OK;
 }
-extern "C" int ttmpc_read_stats8(unsigned long long out[8], int reset) {
-  std::lock_guard<std::mutex> lk(g_mu);
-  Workspace *w;
-  int rc = get_ws(&w);
-  if (rc) return rc;
-  CUDA_TRY(cudaDeviceSynchronize());
-  CUDA_TRY(cudaMemcpy(out, w->stats, 8 * sizeof(unsigned long long), cudaMemcpyDeviceToHost));
-  if (reset) CUDA_TRY(cudaMemset(w->stats, 0, 192));
-  return TTMPC_OK;
-}
-extern "C" int ttmpc_read_stats(unsigned long long out[4], int reset) {
-  std::lock_guard<std::mutex> lk(g_mu);
-  Workspace *w;
-  int rc = get_ws(&w);
-  if (rc) return rc;
-  CUDA_TRY(cudaDeviceSynchronize());
-  CUDA_TRY(cudaMemcpy(out, w->stats, 4 * sizeof(unsigned long long), cudaMemcpyDeviceToHost));
-  if (reset) CUDA_TRY(cudaMemset(w->stats, 0, 192));
-  return TTMPC_OK;
-}
+extern "C" int ttmpc_read_stats(unsigned long long out[4], int reset) { return read_stats(out, 4, reset); }
+extern "C" int ttmpc_read_stats8(unsigned long long out[8], int reset) { return read_stats(out, 8, reset); }
+extern "C" int ttmpc_read_stats24(unsigned long long out[24], int reset) { return read_stats(out, 24, reset); }
 
 // Launch geometry the solve kernel would use (for DESIGN/bench reporting).
 extern "C" int ttmpc_launch_info(const ttmpc_config *cfg, int n_scenes, int *grid, int *block,
@@ -602,37 +576,36 @@ extern "C" int ttmpc_solve_batch_host(const ttmpc_config *cfg, int n, const doub
   dres.outer_iters = dout; dres.inner_iters = din; dres.last_fpr = dfpr; dres.f1_infeas = df1;
   dres.f2_norm = df2; dres.penalty = dpen; dres.pred_states = res->pred_states ? dps : nullptr;
   dres.evals = dev;
-  // TTMPC_NO_STREAM=1 (or a profiler / CUDA_LAUNCH_BLOCKING that serialises launches) disables the
-  // overlap: everything is copied first, then the kernel is launched.
-  const char *ns = std::getenv("TTMPC_NO_STREAM");
-  const char *lb = std::getenv("CUDA_LAUNCH_BLOCKING");
   // Streaming the parameters in behind the running kernel gives ONE call its lowest latency (the
   // kernel starts on the first chunk) but costs the dispatch order (scenes become available in
   // index order, the likely-long ones cannot go first).  When other host calls are already in
   // flight the GPU is busy anyway: copy everything, then launch with the dispatch order
   // (measured with six calls in flight: 511 k -> 528 k solves/s end to end; one call alone 21.2 ms
-  // streamed, 22.3 ms unstreamed).  TTMPC_NO_STREAM=0 / 1 forces either.
-  bool stream_in = busy_calls <= 1;
-  if (ns) stream_in = !(ns[0] == '1');
-  if (lb && lb[0] == '1') stream_in = false;
+  // streamed, 22.3 ms unstreamed).  CUDA_LAUNCH_BLOCKING=1 turns streaming off, and is the only
+  // switch that does.  It is not a tuning option: with launches serialised (launch-blocking
+  // debugging, or a profiler that serialises kernels -- set it there too) no chunk is copied while
+  // the gated kernel runs, and the kernel would wait out its 2 s time-out before the unstreamed re-run.
+  const char *lb = std::getenv("CUDA_LAUNCH_BLOCKING");
+  const bool stream_in = busy_calls <= 1 && !(lb && lb[0] == '1');
   if (stream_in) {
     rc = solve_device_impl(cfg, n, dp, use_u0, use_y0 && res->y, h_c0 ? dc0 : nullptr, &dres, st, w, true);
     if (rc) return rc;
   }
   // Pinned (page-locked) caller memory is copied from directly; pageable memory goes through the
   // slot's pinned staging buffer first (a host memcpy, ~10 GB/s per thread).
-  bool pinned_in = false;
-  {
-    cudaPointerAttributes at;
-    if (cudaPointerGetAttributes(&at, h_p) == cudaSuccess) pinned_in = at.type == cudaMemoryTypeHost;
-    else cudaGetLastError();
-    const char *np_ = std::getenv("TTMPC_NO_PINNED_INPUT");
-    if (np_ && np_[0] == '1') pinned_in = false;
-  }
+  cudaPointerAttributes at;
+  const bool pinned_in = cudaPointerGetAttributes(&at, h_p) == cudaSuccess ? at.type == cudaMemoryTypeHost
+                                                                           : (cudaGetLastError(), false);
   {
     int chunk = 256;
     while ((n + chunk - 1) / chunk > 4096) chunk *= 2;
     const int n_chunks = (n + chunk - 1) / chunk;
+    // chunk ci: scenes up to s1, `cnt` parameters from element `off` of the block
+    struct Chunk { int s1; size_t off, cnt; };
+    auto chunk_at = [&](int ci) {
+      const int s0 = ci * chunk, s1 = std::min(s0 + chunk, n);
+      return Chunk{s1, (size_t)s0 * g.np, (size_t)(s1 - s0) * g.np};
+    };
     // The copy into pinned staging is host-memory bound and the kernel cannot run ahead of it: a
     // few worker threads stage the chunks (chunk i by thread i mod T), this thread issues the H2D
     // copies in order as the chunks become ready.  The team shrinks when several calls are in
@@ -644,36 +617,26 @@ extern "C" int ttmpc_solve_batch_host(const ttmpc_config *cfg, int n, const doub
     const double *src = pinned_in ? h_p : hp;
     std::vector<std::atomic<int>> staged(n_chunks);
     for (auto &f : staged) f.store(pinned_in ? 1 : 0, std::memory_order_relaxed);
-    auto stage = [&](int t) {
-      for (int ci = t; ci < n_chunks; ci += T) {
-        const int s0 = ci * chunk, s1 = s0 + chunk < n ? s0 + chunk : n;
-        const size_t off = (size_t)s0 * g.np, cnt = (size_t)(s1 - s0) * g.np;
-        std::memcpy(hp + off, h_p + off, sizeof(double) * cnt);
-        staged[ci].store(1, std::memory_order_release);
-      }
+    auto stage = [&](int ci) {
+      const Chunk c = chunk_at(ci);
+      std::memcpy(hp + c.off, h_p + c.off, sizeof(double) * c.cnt);
+      staged[ci].store(1, std::memory_order_release);
     };
     std::vector<std::thread> workers;
-    for (int t = 1; t < T; t++) workers.emplace_back(stage, t);
+    for (int t = 1; t < T; t++)
+      workers.emplace_back([&, t] { for (int ci = t; ci < n_chunks; ci += T) stage(ci); });
     int rc_copy = TTMPC_OK;
     int mine = 0;  // next chunk this thread stages itself (thread 0's share)
     for (int ci = 0; ci < n_chunks; ci++) {
       while (!staged[ci].load(std::memory_order_acquire)) {
-        if (mine < n_chunks) {  // do own share while waiting
-          const int s0 = mine * chunk, s1 = s0 + chunk < n ? s0 + chunk : n;
-          const size_t off = (size_t)s0 * g.np, cnt = (size_t)(s1 - s0) * g.np;
-          std::memcpy(hp + off, h_p + off, sizeof(double) * cnt);
-          staged[mine].store(1, std::memory_order_release);
-          mine += T;
-        } else {
-          std::this_thread::yield();
-        }
+        if (mine < n_chunks) { stage(mine); mine += T; }  // do own share while waiting
+        else std::this_thread::yield();
       }
-      const int s0 = ci * chunk, s1 = s0 + chunk < n ? s0 + chunk : n;
-      const size_t off = (size_t)s0 * g.np, cnt = (size_t)(s1 - s0) * g.np;
-      if (rc_copy == TTMPC_OK &&
-          (cudaMemcpyAsync(dp + off, src + off, sizeof(double) * cnt, cudaMemcpyHostToDevice, cs) != cudaSuccess ||
-           (w->h_ready[ci] = s1,
-            cudaMemcpyAsync(w->ready, w->h_ready + ci, sizeof(int), cudaMemcpyHostToDevice, cs) != cudaSuccess)))
+      if (rc_copy != TTMPC_OK) continue;
+      const Chunk c = chunk_at(ci);
+      w->h_ready[ci] = c.s1;
+      if (cudaMemcpyAsync(dp + c.off, src + c.off, sizeof(double) * c.cnt, cudaMemcpyHostToDevice, cs) != cudaSuccess ||
+          cudaMemcpyAsync(w->ready, w->h_ready + ci, sizeof(int), cudaMemcpyHostToDevice, cs) != cudaSuccess)
         rc_copy = TTMPC_ERR_CUDA;
     }
     for (auto &th : workers) th.join();
