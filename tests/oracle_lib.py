@@ -111,6 +111,15 @@ def eval_warp(cfg, u, p, c=0.0, y=None):
     return float(f[0]), F2[:cfg.Ndynobs], float(ps[0]), g
 
 
+def rollout(cfg, u, p):
+    """States after each of the N steps of one scene (unicycle RK4 from p's start, libm order): [N, 3]."""
+    lib = load()
+    u = np.ascontiguousarray(u, np.float64); p = np.ascontiguousarray(p, np.float64)
+    st = np.zeros((cfg.N_hor, 3))
+    lib.ttmpc_oracle_rollout(C.byref(cfg), _p(u), _p(p), _p(st))
+    return st
+
+
 def sincos(x):
     lib = load()
     s = C.c_double(); c = C.c_double()

@@ -32,7 +32,11 @@ def _rect_halfspaces(cx, cy, hx, hy, ang):
 
 def make_scenes(n: int, cfg: TtmpcConfig, seed: int = 0, n_static: int = 4, n_dynamic: int = 0,
                 mode_speed: float = 1.2, blocking_fraction: float = 0.1, mpc: Configurator = None):
-    """Returns p [n, np] float64 (and a dict with the pieces, for tests)."""
+    """Returns p [n, np] float64.
+
+    Static obstacles are only placed when the configuration has 4-edge slots (nstcobs = 12);
+    with any other edge count the static block stays zero.  Other robots are never placed: the
+    c block is all zeros.  Live obstacles always fill the first slots."""
     rng = np.random.default_rng(seed)
     mpc = mpc or Configurator()
     N, ts = cfg.N_hor, cfg.ts
@@ -60,8 +64,10 @@ def make_scenes(n: int, cfg: TtmpcConfig, seed: int = 0, n_static: int = 4, n_dy
                   + (k - leg1[:, None]) * np.sin(h2)[:, None])
     rth = np.where(on1, heading[:, None], h2[:, None])
     # some scenes end their path early (goal inside the horizon): tail padded with the last state
+    # (at least 3 samples kept; horizons of 3 or less keep 1..N-1, and a horizon of 1 cannot end early)
     short = rng.random(n) < 0.15
-    n_keep = np.where(short, rng.integers(3, N, n), N)
+    lo = min(3, N - 1)
+    n_keep = np.where(short, rng.integers(lo, N, n), N) if lo >= 1 else np.full(n, N)
     idx = np.minimum(np.arange(N)[None, :], n_keep[:, None] - 1)
     rx = np.take_along_axis(rx, idx, 1); ry = np.take_along_axis(ry, idx, 1)
     rth = np.take_along_axis(rth, idx, 1)
