@@ -12,7 +12,11 @@ HDRS      := include/ttmpc.h $(CSRC)/ttmpc_device.cuh $(CSRC)/ttmpc_launch.cuh
 
 all: $(LIB) $(ORACLE)
 
+# the rolled build serves batches larger than the resident warps: registers for 3 CTAs of 128 threads per SM
+# (168 registers: 12 resident scenes per SM, six 64-thread CTAs for the default shapes; CTAs of up to 4
+# scenes, as the API picks for large tables, still launch); its run-time-dimension kernel keeps 255 registers
 $(CSRC)/ttmpc_solve_small.o: $(CSRC)/ttmpc_solve.cu
+$(CSRC)/ttmpc_solve_small.o: NVFLAGS += -DTTMPC_MIN_BLOCKS=3 -DTTMPC_MIN_BLOCKS_RUNTIME=2
 
 $(CSRC)/%.o: $(CSRC)/%.cu $(HDRS)
 	$(NVCC) $(NVFLAGS) -c $< -o $@

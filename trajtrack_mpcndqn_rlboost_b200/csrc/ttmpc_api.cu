@@ -99,10 +99,11 @@ static int make_devcfg(const ttmpc_config *c, DevCfg *g) {
   g->np = g->off_qdyn + N;
   g->smem_per_warp = smem_bytes_per_warp(N, g->Nother, g->Nstc, g->nstcobs, g->Ndyn, g->mem);
   {
-    // 2 scenes per CTA (4 CTAs per SM for the default shapes: 8 resident scenes per SM at 255
-    // registers per thread, each owner has one potential helper).  Small CTAs release their SM share as soon as both scenes are done,
-    // which is what lets the next batch in (batches in flight: +4 % over 4 scenes per CTA, same
-    // time for a batch alone).  Large configurations: one scene per CTA if two do not fit.
+    // 2 scenes per CTA (default shapes: 4 CTAs per SM of the unrolled build at 255 registers per thread,
+    // 6 of the rolled build at 168; each owner has one potential helper).  Small CTAs release their SM
+    // share as soon as both scenes are done, which is what lets the next batch in (batches in flight:
+    // +4 % over 4 scenes per CTA, same time for a batch alone).  Large configurations: one scene per CTA
+    // if two do not fit.
     const size_t cap = 232448 - 256;
     if ((size_t)g->smem_per_warp > cap)
       return fail(TTMPC_ERR_UNSUPPORTED, "configuration does not fit in shared memory: " +
@@ -112,6 +113,10 @@ static int make_devcfg(const ttmpc_config *c, DevCfg *g) {
     for (int cand : {2, 3, 4, 1}) {
       const size_t per_cta = (size_t)g->smem_per_warp * cand + 96 + 1024;  // + CtaHelp + the 1 KB the driver reserves per CTA
       if ((size_t)g->smem_per_warp * cand > cap) continue;
+      // 8 warps per SM: the register limit of the unrolled build (255 registers).  Both builds launch
+      // this CTA size, and the unrolled one, which serves batches that fit its resident warps, must
+      // not lose warps; the rolled build then holds as many of these CTAs as its 168 registers and
+      // the shared memory allow (6 for the default shapes).
       const int ctas = (int)std::min<size_t>(233472 / per_cta, (size_t)(8 / cand));
       if (ctas * cand > best) { best = ctas * cand; wpb = cand; }
     }
@@ -317,13 +322,39 @@ static int ensure_staging(Slot *w, size_t bytes) {
   return TTMPC_OK;
 }
 
-static int grid_for(Workspace *w, const DevCfg &g, int n_scenes, int *grid) {
-  int bps = 0;
-  CUDA_TRY(solve_occupancy(g, &bps));
+static int grid_for_occupancy(Workspace *w, const DevCfg &g, int n_scenes, int bps, int *grid) {
   if (bps < 1) return fail(TTMPC_ERR_UNSUPPORTED, "configuration does not fit in shared memory");
   long long want = ((long long)n_scenes + g.warps_per_block - 1) / g.warps_per_block;
   long long cap = (long long)w->sm_count * bps;
   *grid = (int)(want < cap ? (want < 1 ? 1 : want) : cap);
+  return TTMPC_OK;
+}
+static int grid_for(Workspace *w, const DevCfg &g, int n_scenes, int *grid) {
+  int bps = 0;
+  CUDA_TRY(solve_occupancy(g, &bps));
+  return grid_for_occupancy(w, g, n_scenes, bps, grid);
+}
+// Two builds of the solve kernel, bit-identical results: unrolled hot loops (255 registers) when every
+// scene has a warp from the start (latency-bound), rolled loops (168 registers, more resident warps:
+// 12 per SM for the default shapes) when the batch queues behind the unrolled build's resident warps.
+// The grid is sized from the occupancy of the build that runs.  TTMPC_CODE=small|unrolled forces one.
+struct SolvePlan { int grid, blocks_per_sm; bool small_code; };
+static int plan_solve(Workspace *w, const DevCfg &g, int n_scenes, SolvePlan *pl) {
+  int bps = 0, grid = 0;
+  CUDA_TRY(solve_occupancy(g, &bps));
+  int rc = grid_for_occupancy(w, g, n_scenes, bps, &grid);
+  if (rc) return rc;
+  bool small_code = n_scenes > (long long)grid * g.warps_per_block;
+  if (const char *e = std::getenv("TTMPC_CODE")) {
+    if (e[0] == 's') small_code = true;
+    else if (e[0] == 'u') small_code = false;
+  }
+  if (small_code) {
+    CUDA_TRY(solve_occupancy_small(g, &bps));
+    rc = grid_for_occupancy(w, g, n_scenes, bps, &grid);
+    if (rc) return rc;
+  }
+  pl->grid = grid; pl->blocks_per_sm = bps; pl->small_code = small_code;
   return TTMPC_OK;
 }
 
@@ -352,7 +383,7 @@ static int solve_device_impl(const ttmpc_config *cfg, int n_scenes, const double
   Workspace *w;
   Slot *sl = host_slot;
   const int *d_ready = (host_slot && gated) ? host_slot->ready : nullptr;
-  int grid;
+  SolvePlan plan;
   bool want_order = false;
   {
     std::lock_guard<std::mutex> lk(g_mu);
@@ -361,14 +392,14 @@ static int solve_device_impl(const ttmpc_config *cfg, int n_scenes, const double
     // host path: the caller's slot (streamed inputs gated by its `ready` counter); device path:
     // the slot of the stream
     if (!sl) { rc = slot_for_stream(w, st, &sl); if (rc) return rc; }
-    rc = grid_for(w, g, n_scenes, &grid);
+    rc = plan_solve(w, g, n_scenes, &plan);
     if (rc) return rc;
     const size_t table = (size_t)DYN_FIELDS * g.Ndyn * g.N * sizeof(double);
-    rc = ensure_dyn(sl, (table ? table : 8) * (size_t)grid * g.warps_per_block);
+    rc = ensure_dyn(sl, (table ? table : 8) * (size_t)plan.grid * g.warps_per_block);
     if (rc) return rc;
     // more scenes than resident warps: dispatch the likely-long ones first.  Not on the streamed
     // host path (scenes become available in index order there).
-    want_order = !d_ready && n_scenes > (long long)grid * g.warps_per_block;
+    want_order = !d_ready && n_scenes > (long long)plan.grid * g.warps_per_block;
     if (want_order) {
       rc = ensure_order(sl, 2 * (size_t)n_scenes + 64);
       if (rc) return rc;
@@ -394,16 +425,8 @@ static int solve_device_impl(const ttmpc_config *cfg, int n_scenes, const double
     CUDA_TRY(launch_rank_scenes(g, d_p, n_scenes, sl->order + n_scenes, sl->order, st));
     A.order = sl->order;
   }
-  // two builds of the same kernel, bit-identical results: unrolled hot loops when every scene has a
-  // warp from the start (latency-bound), rolled loops when the batch queues behind the resident
-  // warps (bound by the instruction cache with 12 warps per SM).  TTMPC_CODE=small|unrolled forces one.
-  bool small_code = n_scenes > (long long)grid * g.warps_per_block;
-  if (const char *e = std::getenv("TTMPC_CODE")) {
-    if (e[0] == 's') small_code = true;
-    else if (e[0] == 'u') small_code = false;
-  }
-  if (small_code) CUDA_TRY(launch_solve_small(g, A, grid, st));
-  else CUDA_TRY(launch_solve(g, A, grid, st));
+  if (plan.small_code) CUDA_TRY(launch_solve_small(g, A, plan.grid, st));
+  else CUDA_TRY(launch_solve(g, A, plan.grid, st));
   return TTMPC_OK;
 }
 
@@ -475,7 +498,8 @@ extern "C" int ttmpc_read_stats(unsigned long long out[4], int reset) { return r
 extern "C" int ttmpc_read_stats8(unsigned long long out[8], int reset) { return read_stats(out, 8, reset); }
 extern "C" int ttmpc_read_stats24(unsigned long long out[24], int reset) { return read_stats(out, 24, reset); }
 
-// Launch geometry the solve kernel would use (for DESIGN/bench reporting).
+// Launch geometry the solve of an n_scenes batch would use, of the build that would run it (for
+// DESIGN/bench reporting).
 extern "C" int ttmpc_launch_info(const ttmpc_config *cfg, int n_scenes, int *grid, int *block,
                                  int *smem_bytes, int *blocks_per_sm, int *sm_count) {
   DevCfg g;
@@ -485,15 +509,13 @@ extern "C" int ttmpc_launch_info(const ttmpc_config *cfg, int n_scenes, int *gri
   Workspace *w;
   rc = get_ws(&w);
   if (rc) return rc;
-  int gr;
-  rc = grid_for(w, g, n_scenes, &gr);
+  SolvePlan plan;
+  rc = plan_solve(w, g, n_scenes, &plan);
   if (rc) return rc;
-  int bps = 0;
-  CUDA_TRY(solve_occupancy(g, &bps));
-  if (grid) *grid = gr;
+  if (grid) *grid = plan.grid;
   if (block) *block = g.warps_per_block * 32;
   if (smem_bytes) *smem_bytes = g.smem_per_warp * g.warps_per_block;
-  if (blocks_per_sm) *blocks_per_sm = bps;
+  if (blocks_per_sm) *blocks_per_sm = plan.blocks_per_sm;
   if (sm_count) *sm_count = w->sm_count;
   return TTMPC_OK;
 }

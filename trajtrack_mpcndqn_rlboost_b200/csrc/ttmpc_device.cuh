@@ -40,7 +40,7 @@ constexpr int MAX_MEM = 16;
 constexpr int MAX_EDGE = 8;
 constexpr int DYN_FIELDS = 10;  // per (obstacle, step): see stage_scene
 #ifndef TT_DYN_SLOTS
-#define TT_DYN_SLOTS 4
+#define TT_DYN_SLOTS 1
 #endif
 constexpr int DYN_SLOTS = TT_DYN_SLOTS;  // live dynamic obstacles whose table rows are kept in shared memory
 
@@ -266,6 +266,24 @@ __device__ __forceinline__ double pdot(double a0, double a1, double b0, double b
 // ---------------------------------------------------------------- per-warp state
 // Everything a warp needs that is uniform across lanes lives in shared memory
 // (broadcast reads), so the eval routine can be a real (non-inlined) function.
+// PANOC scalars of the solve kernel (ttmpc_solve.cu) that are read a few times per iteration, away from the
+// dependent chain of the line search: warp-uniform, kept in the warp's context rather than in registers.
+struct PanocCold {
+  double L, sigma, lb_gamma;
+  double ip;              // <grad, fpr>, reduced together with |fpr|^2
+  double env_dd, env_g2;  // |gstep - u_half|^2 and |grad|^2 of the current gradient step / half step: from the
+                          // accepted line-search evaluation, or formed where the solver takes the step itself
+  double tau;             // line-search step of the current candidate
+  double rhs_ls;          // right-hand side of the line search's envelope test
+  int iteration;          // PANOC steps taken in this inner solve
+  int lb_active, lb_head, lb_first;  // L-BFGS ring: pairs held, newest slot, no pair yet
+};
+// The L-BFGS state panoc_step saves before it updates L-BFGS speculatively (tail helpers) and restores
+// when the speculation is lost.
+struct SpecSave {
+  double lb_gamma;
+  int lb_first, lb_head, lb_active;
+};
 struct WarpCtx {
   const double *p;   // this scene's packed parameter vector (global)
   double *dyn;       // this warp's dynamic-obstacle table (global scratch, L2 resident)
@@ -281,6 +299,14 @@ struct WarpCtx {
   unsigned fleet_live;               // bit j: other robot j can matter inside the box
   double lipc;                       // PANOC: GAMMA_L_COEFF / (2 gamma) of the current gamma
   double icm_c, icm;                 // 1 / max(c, 1) of the last penalty c this warp evaluated with
+  // solve_scene's outer-loop (ALM) state: warp-uniform, changes once per outer iteration and is live
+  // across every evaluation of the inner loop.  Kept here, not in registers, so that the rolled build
+  // fits 168 registers per thread (12 resident scenes per SM) without spilling.
+  PanocCold pc;
+  SpecSave spec;
+  double akkt_tol, f_final, last_fpr, dy_norm, dy_norm_plus, f2_norm, f2_norm_plus;
+  unsigned long long t_start, panoc_iters;
+  int inner_count, exit_status, num_outer, scene, in_time;
 #ifdef TTMPC_PROFILE
   long long prof[8];                 // cycles per phase (diagnostic build only)
   long long eprof[10];               // cycles per section of eval_psi
@@ -297,13 +323,15 @@ struct WarpSmem {
   float2 *fleet;  // [Nother][N] other robots' (x, y), fp32 copy for the contact prefilter
   float *dynb;    // [Ndyn][N][3] conservative fp32 bounding test: cx cy R2
   double *dynt;   // [DYN_SLOTS][DYN_FIELDS][N] table rows of the first live dynamic obstacles
-  double2 *lbs;   // [(mem+1)][NP]  L-BFGS s rows; NP = N|1 (odd stride: rows read by
-  double2 *lby;   // [(mem+1)][NP]  different lanes fall in different banks)
+  double2 *lbs;   // [(mem+1)][N]  L-BFGS s rows (lane k reads element k of a row: no bank conflict)
+  double2 *lby;   // [(mem+1)][N]  L-BFGS y rows
   double *rho;    // [mem+1]
-  double *alpha;  // [2*(mem+1)]  gamma*a_c and (a_c - beta_c) of the last apply
+  double2 *gprev; // [N] previous gradient of the PANOC iteration (AKKT residual); lanes >= N: zero
+  double2 *olds;  // [32] L-BFGS old_state of every lane (lanes >= N included: their entries need not be zero)
+  double2 *oldg;  // [32] L-BFGS old_g
   // mailbox of the tail helpers (see ttmpc_solve.cu): the owner's request / the helper's answer
   double2 *hreq;  // [N] evaluation point (v, w)
-  double2 *hres;  // [N] gradient (gv, gw)
+  double2 *hres;  // [N] gradient (gv, gw): the same row as hreq
   double2 *yrow;  // [N] the owner's current multipliers (ya, yw)
   struct HelpHdr *hhdr;
 };
@@ -350,11 +378,10 @@ __host__ __device__ inline int smem_bytes_per_warp(int N, int Nother, int Nstc, 
   b += (sizeof(float2) * (size_t)Nother * N + 15) / 16 * 16;
   b += (sizeof(float) * 3 * (size_t)Ndyn * N + 15) / 16 * 16;
   b += sizeof(double) * (size_t)(Ndyn ? DYN_SLOTS * DYN_FIELDS * N : 0);
-  const int NP = N | 1;
-  b += sizeof(double2) * (size_t)(mem + 1) * NP * 2;
+  b += sizeof(double2) * (size_t)(mem + 1) * N * 2;
   b += sizeof(double) * ((mem + 2) / 2 * 2);
-  b += sizeof(double) * (2 * (mem + 1));
-  b += sizeof(double2) * 3 * (size_t)N + (sizeof(HelpHdr) + 15) / 16 * 16;  // mailbox rows + header
+  b += sizeof(double2) * ((size_t)N + 64);
+  b += sizeof(double2) * 2 * (size_t)N + (sizeof(HelpHdr) + 15) / 16 * 16;  // mailbox rows + header
   return (int)((b + 15) / 16 * 16);
 }
 
@@ -367,9 +394,8 @@ __device__ __forceinline__ WarpSmem carve(unsigned char *base, const DevCfg &g) 
   const int N = DM::N(g), MEM = DM::mem(g), Nother = DM::Nother(g), Nstc = DM::Nstc(g),
             nstcobs = 3 * DM::ne(g), Ndyn = DM::Ndyn(g);
   w.ctx = reinterpret_cast<WarpCtx *>(q); q += (sizeof(WarpCtx) + 15) / 16 * 16;
-  const int NP = N | 1;
-  w.lbs = reinterpret_cast<double2 *>(q); q += sizeof(double2) * (size_t)(MEM + 1) * NP;
-  w.lby = reinterpret_cast<double2 *>(q); q += sizeof(double2) * (size_t)(MEM + 1) * NP;
+  w.lbs = reinterpret_cast<double2 *>(q); q += sizeof(double2) * (size_t)(MEM + 1) * N;
+  w.lby = reinterpret_cast<double2 *>(q); q += sizeof(double2) * (size_t)(MEM + 1) * N;
   w.fleet = reinterpret_cast<float2 *>(q); q += (sizeof(float2) * (size_t)Nother * N + 15) / 16 * 16;
   w.dynb = reinterpret_cast<float *>(q); q += (sizeof(float) * 3 * (size_t)Ndyn * N + 15) / 16 * 16;
   w.dynt = reinterpret_cast<double *>(q); q += sizeof(double) * (size_t)(Ndyn ? DYN_SLOTS * DYN_FIELDS * N : 0);
@@ -378,9 +404,13 @@ __device__ __forceinline__ WarpSmem carve(unsigned char *base, const DevCfg &g) 
   w.D = reinterpret_cast<double *>(q); q += sizeof(double) * ((Ndyn + 1) / 2 * 2);
   w.vref = reinterpret_cast<double *>(q); q += sizeof(double) * ((N + 1) / 2 * 2);
   w.rho = reinterpret_cast<double *>(q); q += sizeof(double) * ((MEM + 2) / 2 * 2);
-  w.alpha = reinterpret_cast<double *>(q); q += sizeof(double) * (2 * (MEM + 1));
+  w.gprev = reinterpret_cast<double2 *>(q); q += sizeof(double2) * (size_t)N;
+  w.olds = reinterpret_cast<double2 *>(q); q += sizeof(double2) * 32;
+  w.oldg = reinterpret_cast<double2 *>(q); q += sizeof(double2) * 32;
+  // the answer overwrites the request: the helper reads the point before it evaluates, and the owner
+  // posts the next request only after it has collected the answer
   w.hreq = reinterpret_cast<double2 *>(q); q += sizeof(double2) * (size_t)N;
-  w.hres = reinterpret_cast<double2 *>(q); q += sizeof(double2) * (size_t)N;
+  w.hres = w.hreq;
   w.yrow = reinterpret_cast<double2 *>(q); q += sizeof(double2) * (size_t)N;
   w.hhdr = reinterpret_cast<HelpHdr *>(q);
   return w;

@@ -42,6 +42,7 @@ cudaError_t launch_rank_scenes(const DevCfg &g, const double *p, int n, int *scr
                                cudaStream_t st);
 cudaError_t launch_eval(const DevCfg &g, const EvalArgs &A, int grid, cudaStream_t st);
 cudaError_t solve_occupancy(const DevCfg &g, int *blocks_per_sm);
+cudaError_t solve_occupancy_small(const DevCfg &g, int *blocks_per_sm);  // the rolled build
 cudaError_t launch_probe(const DevCfg &g, const double *p, double *dyn, long long *out, int reps,
                          cudaStream_t st);
 // fleet step (ttmpc_fleet.cu)

@@ -24,11 +24,17 @@
 // places of the loop; the API launches it for batches larger than the resident warps.  Only the
 // solve kernel and its launcher exist in that build, under these names:
 #ifndef TTMPC_MIN_BLOCKS
-// 128-thread CTAs per SM the register budget is sized for: 2 -> 255 registers, no spills, 8 resident
-// scenes per SM; 3 -> 168 registers, 300 bytes of spills, 12 scenes per SM.  The SM is bound by
-// instruction fetch from 8 warps on (same bulk rate either way), and without the spill traffic one
-// scene alone is 15 % faster (1.50 -> 1.30 ms p50) and a 4096-scene batch alone 9 % (24.0 -> 21.8 ms).
+// CTAs of TTMPC_MAX_THREADS threads per SM the register budget is sized for.  Unrolled build: 2 of 128
+// -> up to 255 registers, 8 resident scenes per SM.  Rolled build (Makefile): 3 of 128 -> 168 registers,
+// 12 resident scenes per SM (six 64-thread CTAs for the default shapes), without spills: the PANOC / ALM state that is read a few times per
+// iteration lives in the warp's shared memory (WarpCtx, the L-BFGS old_state / old_g rows), not in
+// registers (DESIGN.md section 3.1).
 #define TTMPC_MIN_BLOCKS 2
+#endif
+#ifndef TTMPC_MIN_BLOCKS_RUNTIME
+// the same for the run-time-dimension kernel (DimsRuntime), which needs more registers than the
+// specialised shapes: it keeps its 255 registers in both builds
+#define TTMPC_MIN_BLOCKS_RUNTIME TTMPC_MIN_BLOCKS
 #endif
 #ifndef TTMPC_MAX_THREADS
 #define TTMPC_MAX_THREADS 128  // CTA size the register budget is computed for (the API launches 64)
@@ -36,7 +42,7 @@
 #ifdef TTMPC_SMALL_CODE
 #define solve_kernel solve_kernel_small
 #define launch_solve launch_solve_small
-#define solve_occupancy_impl solve_occupancy_small_impl
+#define solve_occupancy solve_occupancy_small
 #endif
 
 namespace ttmpc {
@@ -49,6 +55,9 @@ constexpr double LIPSCHITZ_UPDATE_EPSILON = 1e-6;
 constexpr int MAX_LIPSCHITZ_UPDATE_ITERATIONS = 10;
 constexpr double MAX_LIPSCHITZ_CONSTANT = 1e9;
 constexpr int MAX_LINESEARCH_ITERATIONS = 10;
+// The line search's tau starts at 1 and only halves, so tau = 2^-k exactly after k halvings:
+// k < MAX_LINESEARCH_ITERATIONS  <=>  tau > 2^-MAX_LINESEARCH_ITERATIONS
+constexpr double MIN_LINESEARCH_TAU = 1.0 / (1 << MAX_LINESEARCH_ITERATIONS);
 constexpr double MIN_L_ESTIMATE = 1e-10;
 // lbfgs settings chosen by PANOCCache::new
 constexpr double CBFGS_EPSILON = 1e-8;
@@ -58,19 +67,14 @@ constexpr double SY_EPSILON = 1e-10;
 struct Lane {
   double u0, u1;          // current iterate
   double g0, g1;          // gradient at u (or u_plus during the line search)
-  double gp0, gp1;        // previous gradient (AKKT residual)
   double h0, h1;          // u_half_step
   double d0, d1;          // L-BFGS direction
   double f0, f1;          // gamma * fixed point residual
-  double os0, os1, og0, og1;  // lbfgs old_state / old_g
 };
 
 struct Uni {  // warp-uniform scalars
-  double gamma, L, sigma, cost, norm_fpr, tau, akkt_tol, lb_gamma;
-  double ip;              // <grad, fpr>, reduced together with |fpr|^2
-  double env_dd, env_g2;  // |gstep - u_half|^2 and |grad|^2 of the current gradient step / half step: from the
-                          // accepted line-search evaluation, or formed where the solver takes the step itself
-  int iteration, lb_active, lb_head, lb_first;
+  double gamma, cost, norm_fpr;
+  PanocCold *pc;  // the rest, in the warp's context
 };
 
 __device__ __forceinline__ void project(const DevCfg &g, double a0, double a1, double &o0, double &o1) {
@@ -91,7 +95,7 @@ __device__ __forceinline__ void set_lip_coeff(const Uni &U, const WarpSmem &sm) 
   __syncwarp();
 }
 __device__ __forceinline__ void set_gamma_terms(Uni &U, const WarpSmem &sm) {
-  U.sigma = tt_div(1.0 - GAMMA_L_COEFF, 4.0 * U.gamma);
+  U.pc->sigma = tt_div(1.0 - GAMMA_L_COEFF, 4.0 * U.gamma);
   set_lip_coeff(U, sm);
 }
 // x / gamma for the forward-backward envelope.  x = |gradient step - half step|^2 / 2 is exactly zero
@@ -116,15 +120,24 @@ __device__ __forceinline__ double div_env(double x, double y) {
 // instruction-cache hit rate from 69 % to 94 % and the issue rate up by 43 %.  The literal recursion
 // is ~1.5 KB, executes fewer instructions (no Gram upkeep), and its reduction latency is hidden
 // by the other warps.  The CPU oracle's WARP order mirrors it (lb_apply with butterfly dots).
+// lbfgs old_state / old_g := the current iterate and residual (per-lane rows of the warp's shared memory)
+__device__ __forceinline__ void set_old(const WarpSmem &sm, const Lane &z, int lane) {
+  sm.olds[lane] = make_double2(z.u0, z.u1);
+  sm.oldg[lane] = make_double2(z.f0, z.f1);
+}
+// Returns whether the pair was accepted.  keep_old = false leaves old_state / old_g unchanged: the
+// speculative update of panoc_step stores them (z.os = z.u, z.og = z.f) only once the speculation holds,
+// so that a lost speculation has nothing per lane to restore.
 template <class DM>
-__device__ __forceinline__ void lbfgs_update(const DevCfg &g, const WarpSmem &sm, Lane &z, Uni &U,
-                                             int lane) {
-  const int N = DM::N(g), NP = N | 1, MEM = DM::mem(g), M1 = MEM + 1;
-  const double sv0 = z.u0 - z.os0, sv1 = z.u1 - z.os1;
-  const double yv0 = z.f0 - z.og0, yv1 = z.f1 - z.og1;
+__device__ __forceinline__ bool lbfgs_update(const DevCfg &g, const WarpSmem &sm, Lane &z, Uni &U,
+                                             int lane, bool keep_old = true) {
+  const int N = DM::N(g), MEM = DM::mem(g), M1 = MEM + 1;
+  const double2 os = sm.olds[lane], og = sm.oldg[lane];
+  const double sv0 = z.u0 - os.x, sv1 = z.u1 - os.y;
+  const double yv0 = z.f0 - og.x, yv1 = z.f1 - og.y;
   bool accept = true;
   double ys = 0.0, yy = 0.0;
-  if (!U.lb_first) {
+  if (!U.pc->lb_first) {
     double ss = pdot(sv0, sv1, sv0, sv1);
     ys = pdot(sv0, sv1, yv0, yv1); yy = pdot(yv0, yv1, yv0, yv1);
     wsum3(ys, ss, yy);
@@ -133,21 +146,26 @@ __device__ __forceinline__ void lbfgs_update(const DevCfg &g, const WarpSmem &sm
     accept = !(ss <= 2.2250738585072014e-308 || ys <= SY_EPSILON) &&
              (lhs > rhs && isfinite(lhs) && isfinite(rhs));
   }
-  if (!accept) return;
-  z.os0 = z.u0; z.os1 = z.u1; z.og0 = z.f0; z.og1 = z.f1;
-  if (U.lb_first) { U.lb_first = 0; return; }
+  if (!accept) return false;
+  if (keep_old) set_old(sm, z, lane);
+  if (U.pc->lb_first) {
+    __syncwarp();
+    U.pc->lb_first = 0;
+    return true;
+  }
   // rotate_right(1): scratch slot becomes slot 0
-  U.lb_head = U.lb_head + MEM; if (U.lb_head >= M1) U.lb_head -= M1;
-  const int k0 = U.lb_head;
+  int k0 = U.pc->lb_head + MEM; if (k0 >= M1) k0 -= M1;
+  const int active = min(MEM, U.pc->lb_active + 1);
   const double rho = tt_div(1.0, ys);
   if (lane < N) {
-    sm.lbs[k0 * NP + lane] = make_double2(sv0, sv1);
-    sm.lby[k0 * NP + lane] = make_double2(yv0, yv1);
+    sm.lbs[k0 * N + lane] = make_double2(sv0, sv1);
+    sm.lby[k0 * N + lane] = make_double2(yv0, yv1);
   }
   if (lane == 0) sm.rho[k0] = rho;
-  U.lb_gamma = tt_div(tt_div(1.0, rho), yy);
-  U.lb_active = min(MEM, U.lb_active + 1);
+  U.pc->lb_gamma = tt_div(tt_div(1.0, rho), yy);
   __syncwarp();
+  U.pc->lb_head = k0; U.pc->lb_active = active;
+  return true;
 }
 
 // lbfgs::apply_hessian on the direction.  The 2 m inner products of the recursion are one dependent chain
@@ -157,26 +175,26 @@ __device__ __forceinline__ void lbfgs_update(const DevCfg &g, const WarpSmem &sm
 template <class DM>
 __device__ __forceinline__ void lbfgs_apply(const DevCfg &g, const WarpSmem &sm, Lane &z,
                                             const Uni &U, int lane) {
-  const int m = U.lb_active;
+  const int m = U.pc->lb_active;
   if (m == 0) return;
-  const int N = DM::N(g), NP = N | 1, M1 = DM::mem(g) + 1;
+  const int N = DM::N(g), M1 = DM::mem(g) + 1;
   const bool act = lane < N;
   const int lk = act ? lane : N - 1;
   double q0 = z.d0, q1 = z.d1, a_me = 0.0;  // lane i keeps alpha_i
-  int k = U.lb_head;
+  int k = U.pc->lb_head;
 #pragma unroll 1
   for (int i = 0; i < m; i++) {  // newest to oldest
-    const double2 s = sm.lbs[k * NP + lk], y = sm.lby[k * NP + lk];
+    const double2 s = sm.lbs[k * N + lk], y = sm.lby[k * N + lk];
     const double a = sm.rho[k] * wsum_inl(act ? pdot(s.x, s.y, q0, q1) : 0.0);
     if (lane == i) a_me = a;
     q0 = fma(-a, y.x, q0); q1 = fma(-a, y.y, q1);
     k = (k + 1 == M1) ? 0 : k + 1;
   }
-  q0 = U.lb_gamma * q0; q1 = U.lb_gamma * q1;
+  q0 = U.pc->lb_gamma * q0; q1 = U.pc->lb_gamma * q1;
 #pragma unroll 1
   for (int i = m - 1; i >= 0; i--) {  // oldest to newest
     k = (k == 0) ? M1 - 1 : k - 1;
-    const double2 s = sm.lbs[k * NP + lk], y = sm.lby[k * NP + lk];
+    const double2 s = sm.lbs[k * N + lk], y = sm.lby[k * N + lk];
     const double beta = sm.rho[k] * wsum_inl(act ? pdot(y.x, y.y, q0, q1) : 0.0);
     const double cf = __shfl_sync(FULL, a_me, i) - beta;
     q0 = fma(cf, s.x, q0); q1 = fma(cf, s.y, q1);
@@ -210,19 +228,30 @@ struct CtaHelp {
   int helper[8];  // helper[m] = warp helping owner m, or -1
   int epoch[8];   // serial number of warp w's current scene (a helper serves one scene)
 };
+// Dynamic shared memory of a solve CTA: the CtaHelp table first, at a fixed address (a warp finds its
+// helper slot from its own index instead of holding a pointer in registers), then one region per warp.
+extern __shared__ __align__(16) unsigned char smem_raw[];
+__device__ __forceinline__ CtaHelp *cta_help() { return reinterpret_cast<CtaHelp *>(smem_raw); }
+__device__ __forceinline__ unsigned char *warp_region(const DevCfg &g, int w) {
+  return smem_raw + sizeof(CtaHelp) + (size_t)w * g.smem_per_warp;
+}
 struct HelpCtl {
   bool enabled;              // helpers exist in this launch and none has timed out on this warp
   bool timed_out;            // a request was abandoned after the time-out: helpers stay off for this
                              // warp until the launch ends, and the abandoned request is waited for
                              // before the scene tables are re-staged (see solve_kernel)
-  volatile int *slot;        // &cta->helper[me]
   bool pending;              // a posted request has not been collected yet
 };
+__device__ __forceinline__ int ld_volatile_shared(unsigned addr) {
+  int v;
+  asm volatile("ld.volatile.shared.s32 %0, [%1];" : "=r"(v) : "r"(addr));
+  return v;
+}
 // HELP = false: the instantiation of panoc_step without any request path (see solve_scene)
 template <bool HELP>
 __device__ __forceinline__ bool help_available(const HelpCtl &hc) {
   if constexpr (!HELP) return false;
-  else return hc.enabled && *hc.slot >= 0;
+  else return hc.enabled && ld_volatile_shared((unsigned)__cvta_generic_to_shared(&cta_help()->helper[threadIdx.x >> 5])) >= 0;
 }
 // Collect the posted evaluation.  false = the helper did not answer in time (treated as gone).
 __device__ __forceinline__ bool help_wait(HelpCtl &hc, const WarpSmem &sm, int lane, int N, EvalOut &e) {
@@ -307,7 +336,7 @@ __device__ __forceinline__ void compute_fpr(Lane &z, Uni &U) {
   double nf = pdot(z.f0, z.f1, z.f0, z.f1), ip = pdot(z.g0, z.g1, z.f0, z.f1);
   wsum2(nf, ip);
   U.norm_fpr = tt_sqrt(nf);
-  U.ip = ip;
+  U.pc->ip = ip;
 }
 // The gradient step s = a - gamma g lives only here and in eval_psi: nothing reads it later except the two
 // envelope scalars, which are formed right away where the solver needs them (ENV).
@@ -320,16 +349,16 @@ __device__ __forceinline__ void gradient_and_half_step(const DevCfg &g, Lane &z,
     const double e0 = s0 - z.h0, e1 = s1 - z.h1;
     double dist2 = pdot(e0, e1, e0, e1), gg = pdot(z.g0, z.g1, z.g0, z.g1);
     wsum2(dist2, gg);
-    U.env_dd = dist2; U.env_g2 = gg;
+    U.pc->env_dd = dist2; U.pc->env_g2 = gg;
   }
 }
 
 // Serve owner m (helper slot already taken) until its current scene ends.
 // false = nothing happened for 3 s (the caller gives up helping).
 template <class DM>
-__device__ bool serve_owner(const DevCfg &g, CtaHelp *cta, unsigned char *smem_raw, int m, int epoch_m,
+__device__ bool serve_owner(const DevCfg &g, CtaHelp *cta, int m, int epoch_m,
                             const WarpSmem &mine, int lane) {
-  unsigned char *base_m = smem_raw + (size_t)m * g.smem_per_warp;
+  unsigned char *base_m = warp_region(g, m);
   const WarpSmem own = carve<DM>(base_m, g);
   const int N = g.N;
   unsigned long long t_idle = globaltimer_ns();
@@ -384,10 +413,9 @@ __device__ bool serve_owner(const DevCfg &g, CtaHelp *cta, unsigned char *smem_r
 
 // A warp that ran out of scenes serves its CTA-mates until none of them owns a scene.
 template <class DM>
-__device__ void helper_loop(const DevCfg &g, const SolveArgs &A, CtaHelp *cta, unsigned char *smem_raw,
-                            int warp, int lane) {
+__device__ void helper_loop(const DevCfg &g, const SolveArgs &A, CtaHelp *cta, int warp, int lane) {
   const int W = g.warps_per_block;
-  const WarpSmem mine = carve<DM>(smem_raw + (size_t)warp * g.smem_per_warp, g);
+  const WarpSmem mine = carve<DM>(warp_region(g, warp), g);
   const unsigned long long t_start = globaltimer_ns();
   while (true) {
     int m = -1, any_busy = 0, ep = 0;
@@ -409,7 +437,7 @@ __device__ void helper_loop(const DevCfg &g, const SolveArgs &A, CtaHelp *cta, u
       __nanosleep(2000);
       continue;
     }
-    if (!serve_owner<DM>(g, cta, smem_raw, m, ep, mine, lane)) return;
+    if (!serve_owner<DM>(g, cta, m, ep, mine, lane)) return;
   }
 }
 
@@ -420,7 +448,7 @@ __device__ void helper_loop(const DevCfg &g, const SolveArgs &A, CtaHelp *cta, u
 // run_stats = {sum of evaluations, count} over finished scenes.
 template <class DM>
 __device__ bool help_long_running_mate(const DevCfg &g, const SolveArgs &A, CtaHelp *cta,
-                                       unsigned char *smem_raw, int warp, int lane) {
+                                       int warp, int lane) {
   int m = -1, ep = 0;
   if (lane == 0) {
     const unsigned long long nd = *reinterpret_cast<volatile unsigned long long *>(A.run_stats + 1);
@@ -433,7 +461,7 @@ __device__ bool help_long_running_mate(const DevCfg &g, const SolveArgs &A, CtaH
         if (!*reinterpret_cast<volatile int *>(&cta->busy[cand]) ||
             *reinterpret_cast<volatile int *>(&cta->helper[cand]) != -1)
           continue;
-        const volatile WarpCtx *cx = reinterpret_cast<const volatile WarpCtx *>(smem_raw + (size_t)cand * g.smem_per_warp);
+        const volatile WarpCtx *cx = reinterpret_cast<const volatile WarpCtx *>(warp_region(g, cand));
         ep = *reinterpret_cast<volatile int *>(&cta->epoch[cand]);
         if (cx->n_cost + cx->n_grad > thr && atomicCAS(&cta->helper[cand], -1, warp) == -1) { m = cand; break; }
       }
@@ -442,9 +470,15 @@ __device__ bool help_long_running_mate(const DevCfg &g, const SolveArgs &A, CtaH
   m = __shfl_sync(FULL, m, 0);
   ep = __shfl_sync(FULL, ep, 0);
   if (m < 0) return false;
-  const WarpSmem mine = carve<DM>(smem_raw + (size_t)warp * g.smem_per_warp, g);
-  serve_owner<DM>(g, cta, smem_raw, m, ep, mine, lane);
+  const WarpSmem mine = carve<DM>(warp_region(g, warp), g);
+  serve_owner<DM>(g, cta, m, ep, mine, lane);
   return true;
+}
+
+__device__ __forceinline__ void halve_tau(Uni &U) {
+  const double t = U.pc->tau / 2.0;
+  __syncwarp();  // every lane has read tau
+  U.pc->tau = t;
 }
 
 // PANOCEngine::step.  Returns true to continue.
@@ -452,11 +486,13 @@ template <class DM, bool HELP>
 __device__ __forceinline__ bool panoc_step(const DevCfg &g, const WarpSmem &sm, int lane, const Problem &pb,
                            Lane &z, Uni &U, double tolerance, HelpCtl &hc) {
   PROF_BEGIN(t_step)
-  if (U.iteration >= 1) { z.gp0 = z.g0; z.gp1 = z.g1; }
+  const bool act = lane < DM::N(g);
+  if (U.pc->iteration >= 1 && act) sm.gprev[lane] = make_double2(z.g0, z.g1);
   compute_fpr(z, U);
   if (__builtin_expect(U.norm_fpr < tolerance, 0)) {
-    const double r0 = fma(U.gamma, z.g0 - z.gp0, z.f0), r1 = fma(U.gamma, z.g1 - z.gp1, z.f1);
-    if (sqrt(wsum(pdot(r0, r1, r0, r1))) < U.akkt_tol) return false;
+    const double2 gp = act ? sm.gprev[lane] : make_double2(0.0, 0.0);
+    const double r0 = fma(U.gamma, z.g0 - gp.x, z.f0), r1 = fma(U.gamma, z.g1 - gp.y, z.f1);
+    if (sqrt(wsum(pdot(r0, r1, r0, r1))) < sm.ctx->akkt_tol) return false;
   }
   // update_lipschitz_constant (+ lbfgs_direction).  With a helper the Lipschitz check
   // psi(u_half) runs on the helper while this warp already updates / applies L-BFGS on the
@@ -470,14 +506,14 @@ __device__ __forceinline__ bool panoc_step(const DevCfg &g, const WarpSmem &sm, 
   {
     double cost_half = 0.0;
     const bool spec = __builtin_expect(help_available<HELP>(hc), 0);
-    int s_first = 0, s_head = 0, s_active = 0;
-    double s_gamma = 0.0, s_os0 = 0.0, s_os1 = 0.0, s_og0 = 0.0, s_og1 = 0.0;
+    bool s_accept = false;
+    SpecSave &sv = sm.ctx->spec;
     if (spec) {
       PROF_BEGIN(tp)
       help_post(hc, sm, lane, DM::N(g), z.h0, z.h1, pb.c, 0, 0.0);
       PROF_END(tp, 4)  // helper timeline: post
-      s_first = U.lb_first; s_head = U.lb_head; s_active = U.lb_active;
-      s_gamma = U.lb_gamma; s_os0 = z.os0; s_os1 = z.os1; s_og0 = z.og0; s_og1 = z.og1;
+      sv.lb_first = U.pc->lb_first; sv.lb_head = U.pc->lb_head; sv.lb_active = U.pc->lb_active;
+      sv.lb_gamma = U.pc->lb_gamma;
     }
 #pragma unroll 1
     for (int pass = 0; pass < 2; pass++) {
@@ -485,10 +521,11 @@ __device__ __forceinline__ bool panoc_step(const DevCfg &g, const WarpSmem &sm, 
         PROF_BEGIN(tl)
         {
           PROF_BEGIN(t0)
-          lbfgs_update<DM>(g, sm, z, U, lane);
+          const bool acc = lbfgs_update<DM>(g, sm, z, U, lane, pass != 0);
+          if (pass == 0) s_accept = acc;
           PROF_END(t0, 2)
         }
-        if (U.iteration > 0) {
+        if (U.pc->iteration > 0) {
           PROF_BEGIN(t0)
           z.d0 = z.f0; z.d1 = z.f1;
           lbfgs_apply<DM>(g, sm, z, U, lane);
@@ -510,24 +547,27 @@ __device__ __forceinline__ bool panoc_step(const DevCfg &g, const WarpSmem &sm, 
       }
       if (!got) cost_half = eval_cost<DM>(g, sm, lane, pb, z.h0, z.h1, hc);
       if (spec) {
-        const double rhs0 = U.cost + LIPSCHITZ_UPDATE_EPSILON * fabs(U.cost) - U.ip +
+        const double rhs0 = U.cost + LIPSCHITZ_UPDATE_EPSILON * fabs(U.cost) - U.pc->ip +
                             sm.ctx->lipc * (U.norm_fpr * U.norm_fpr);
-        if (cost_half > rhs0 && U.L < MAX_LIPSCHITZ_CONSTANT) {  // speculation lost
-          U.lb_first = s_first; U.lb_head = s_head; U.lb_active = s_active; U.lb_gamma = s_gamma;
-          z.os0 = s_os0; z.os1 = s_os1; z.og0 = s_og0; z.og1 = s_og1;
+        if (cost_half > rhs0 && U.pc->L < MAX_LIPSCHITZ_CONSTANT) {  // speculation lost
+          U.pc->lb_first = sv.lb_first; U.pc->lb_head = sv.lb_head; U.pc->lb_active = sv.lb_active;
+          U.pc->lb_gamma = sv.lb_gamma;
         } else {
           lbfgs_done = true;
+          if (s_accept) set_old(sm, z, lane);
         }
       }
       int it = 0;
       while (true) {
-        const double rhs = U.cost + LIPSCHITZ_UPDATE_EPSILON * fabs(U.cost) - U.ip +
+        const double rhs = U.cost + LIPSCHITZ_UPDATE_EPSILON * fabs(U.cost) - U.pc->ip +
                            sm.ctx->lipc * (U.norm_fpr * U.norm_fpr);
         if (!(cost_half > rhs && it < MAX_LIPSCHITZ_UPDATE_ITERATIONS &&
-              U.L < MAX_LIPSCHITZ_CONSTANT))
+              U.pc->L < MAX_LIPSCHITZ_CONSTANT))
           break;
-        U.lb_active = 0; U.lb_first = 1;  // lbfgs.reset()
-        U.L *= 2.0;
+        U.pc->lb_active = 0; U.pc->lb_first = 1;  // lbfgs.reset()
+        const double L2 = U.pc->L * 2.0;
+        __syncwarp();
+        U.pc->L = L2;
         U.gamma /= 2.0;
         set_lip_coeff(U, sm);
         gradient_and_half_step<false>(g, z, U, z.u0, z.u1);
@@ -536,32 +576,31 @@ __device__ __forceinline__ bool panoc_step(const DevCfg &g, const WarpSmem &sm, 
         it++;
       }
       // gamma moved: the envelope scalars of the new gradient step / half step (iteration 0 takes its own step below)
-      if (it > 0 && U.iteration > 0) gradient_and_half_step<true>(g, z, U, z.u0, z.u1);
-      if (it > 0) U.sigma = tt_div(1.0 - GAMMA_L_COEFF, 4.0 * U.gamma);  // gamma moved
+      if (it > 0 && U.pc->iteration > 0) gradient_and_half_step<true>(g, z, U, z.u0, z.u1);
+      if (it > 0) U.pc->sigma = tt_div(1.0 - GAMMA_L_COEFF, 4.0 * U.gamma);  // gamma moved
     }
   }
-  if (U.iteration == 0) {
+  if (U.pc->iteration == 0) {
     // update_no_linesearch
     z.u0 = z.h0; z.u1 = z.h1;
     U.cost = eval_grad<DM>(g, sm, lane, pb, z.u0, z.u1, z.g0, z.g1, hc);
     gradient_and_half_step<true>(g, z, U, z.u0, z.u1);
   } else {
     // linesearch on the forward-backward envelope
-    const double dist2 = U.env_dd, gg = U.env_g2;  // same vectors as in the evaluation / step that produced this iterate
+    const double dist2 = U.pc->env_dd, gg = U.pc->env_g2;  // same vectors as in the evaluation / step that produced this iterate
     const double fbe = U.cost - 0.5 * U.gamma * gg + div_env(0.5 * dist2, U.gamma);
-    const double rhs_ls = fbe - U.sigma * (U.norm_fpr * U.norm_fpr);
-    U.tau = 1.0;
-    int nls = 0;
+    U.pc->rhs_ls = fbe - U.pc->sigma * (U.norm_fpr * U.norm_fpr);
+    U.pc->tau = 1.0;
     double p0, p1;
     while (true) {
-      const double one_m = 1.0 - U.tau;
-      p0 = fma(-U.tau, z.d0, fma(-one_m, z.f0, z.u0));
-      p1 = fma(-U.tau, z.d1, fma(-one_m, z.f1, z.u1));
+      const double one_m = 1.0 - U.pc->tau;
+      p0 = fma(-U.pc->tau, z.d0, fma(-one_m, z.f0, z.u0));
+      p1 = fma(-U.pc->tau, z.d1, fma(-one_m, z.f1, z.u1));
       // with a helper: the next candidate (tau/2) is evaluated speculatively at the same time
       bool posted = false;
       double n0 = 0.0, n1 = 0.0;
-      if (__builtin_expect(nls < MAX_LINESEARCH_ITERATIONS && help_available<HELP>(hc), 0)) {
-        const double tau2 = U.tau / 2.0, one_m2 = 1.0 - tau2;
+      if (__builtin_expect(U.pc->tau > MIN_LINESEARCH_TAU && help_available<HELP>(hc), 0)) {
+        const double tau2 = U.pc->tau / 2.0, one_m2 = 1.0 - tau2;
         n0 = fma(-tau2, z.d0, fma(-one_m2, z.f0, z.u0));
         n1 = fma(-tau2, z.d1, fma(-one_m2, z.f1, z.u1));
         help_post(hc, sm, lane, DM::N(g), n0, n1, pb.c, 1, U.gamma);
@@ -576,10 +615,9 @@ __device__ __forceinline__ bool panoc_step(const DevCfg &g, const WarpSmem &sm, 
       U.cost = e.psi;
       z.g0 = e.gv; z.g1 = e.gw; z.h0 = e.h0; z.h1 = e.h1;
       double lhs_ls = U.cost - 0.5 * U.gamma * e.g2 + div_env(0.5 * e.dd, U.gamma);
-      U.env_dd = e.dd; U.env_g2 = e.g2;
-      if (!(lhs_ls > rhs_ls && nls < MAX_LINESEARCH_ITERATIONS)) break;
-      U.tau /= 2.0;
-      nls++;
+      U.pc->env_dd = e.dd; U.pc->env_g2 = e.g2;
+      if (!(lhs_ls > U.pc->rhs_ls && U.pc->tau > MIN_LINESEARCH_TAU)) break;
+      halve_tau(U);
       if (posted && help_wait(hc, sm, lane, DM::N(g), e)) {  // the helper's evaluation is the one at this tau
         if (lane == 0) sm.ctx->n_grad++;
         p0 = n0; p1 = n1;
@@ -587,36 +625,44 @@ __device__ __forceinline__ bool panoc_step(const DevCfg &g, const WarpSmem &sm, 
         z.g0 = e.gv; z.g1 = e.gw;
         gradient_and_half_step<false>(g, z, U, p0, p1);  // same s = p - gamma g, h = proj(s) the evaluation formed
         lhs_ls = U.cost - 0.5 * U.gamma * e.g2 + div_env(0.5 * e.dd, U.gamma);
-        U.env_dd = e.dd; U.env_g2 = e.g2;
-        if (!(lhs_ls > rhs_ls && nls < MAX_LINESEARCH_ITERATIONS)) break;
-        U.tau /= 2.0;
-        nls++;
+        U.pc->env_dd = e.dd; U.pc->env_g2 = e.g2;
+        if (!(lhs_ls > U.pc->rhs_ls && U.pc->tau > MIN_LINESEARCH_TAU)) break;
+        halve_tau(U);
       }
     }
     z.u0 = p0; z.u1 = p1;
   }
-  U.iteration++;
+  {
+    const int it1 = U.pc->iteration + 1;
+    __syncwarp();
+    U.pc->iteration = it1;
+  }
   PROF_END(t_step, 7)  // whole step
   return true;
 }
 
 __device__ __forceinline__ void panoc_reset(Uni &U) {
-  U.lb_active = 0; U.lb_first = 1; U.env_dd = 0.0; U.env_g2 = 0.0;
-  U.tau = 1.0; U.L = 0.0; U.sigma = 0.0; U.cost = 0.0; U.iteration = 0; U.gamma = 0.0;
+  U.pc->lb_active = 0; U.pc->lb_first = 1; U.pc->env_dd = 0.0; U.pc->env_g2 = 0.0;
+  U.pc->tau = 1.0; U.pc->L = 0.0; U.pc->sigma = 0.0; U.cost = 0.0; U.pc->iteration = 0; U.gamma = 0.0;
 }
 
 // One scene, start to finish.
+// The outer-loop (ALM) scalars live in the warp's context (WarpCtx).  They are warp-uniform: every lane
+// stores the same value, and where a value is read and replaced in the same outer iteration, every lane
+// reads it before the __syncwarp() that precedes the stores.
 template <class DM>
 __device__ void solve_scene(const DevCfg &g, const WarpSmem &sm, const SolveArgs &A, int scene,
-                            int lane, unsigned long long *wstats, HelpCtl &hc) {
+                            int lane, HelpCtl &hc) {
   const int N = g.N;
   const bool act = lane < N;
-  const unsigned long long t_start = globaltimer_ns();
+  WarpCtx *const cx = sm.ctx;
+  cx->t_start = __shfl_sync(FULL, globaltimer_ns(), 0);
 #ifdef TTMPC_PROFILE
   const long long t_clk0 = clock64();
 #endif
   Lane z;
   Uni U;
+  U.pc = &cx->pc;
   Problem pb;
   z.u0 = z.u1 = 0.0;
   pb.ya = pb.yw = 0.0;
@@ -631,27 +677,31 @@ __device__ void solve_scene(const DevCfg &g, const WarpSmem &sm, const SolveArgs
     }
   }
   pb.c = A.c0 ? A.c0[scene] : g.c0;
-  z.g0 = z.g1 = z.gp0 = z.gp1 = z.h0 = z.h1 = 0.0;
-  z.d0 = z.d1 = z.f0 = z.f1 = z.os0 = z.os1 = z.og0 = z.og1 = 0.0;
-  U.lb_head = 0; U.lb_gamma = 1.0; U.norm_fpr = 0.0;
+  z.g0 = z.g1 = z.h0 = z.h1 = 0.0;
+  if (act) sm.gprev[lane] = make_double2(0.0, 0.0);
+  z.d0 = z.d1 = z.f0 = z.f1 = 0.0;
+  sm.olds[lane] = make_double2(0.0, 0.0);
+  sm.oldg[lane] = make_double2(0.0, 0.0);
+  U.pc->lb_head = 0; U.pc->lb_gamma = 1.0; U.norm_fpr = 0.0;
   panoc_reset(U);
-  U.akkt_tol = g.init_tol;
+  cx->akkt_tol = g.init_tol;
 
   double yp_a = 0.0, yp_w = 0.0;  // y_plus
-  double delta_y_norm = 0.0, delta_y_norm_plus = 0.0, f2_norm = 0.0, f2_norm_plus = 0.0;
-  double last_fpr = 0.0, f_final = 0.0;
-  int alm_iter = 0, inner_count = 0, num_outer = 0, exit_status = TTMPC_CONVERGED;
-  unsigned long long panoc_iters = 0;
+  cx->dy_norm = 0.0; cx->dy_norm_plus = 0.0; cx->f2_norm = 0.0; cx->f2_norm_plus = 0.0;
+  cx->last_fpr = 0.0; cx->f_final = 0.0;
+  cx->inner_count = 0; cx->exit_status = TTMPC_CONVERGED; cx->panoc_iters = 0;
+  cx->num_outer = 0;
+  cx->scene = scene;
   const double SMALL_EPSILON = 2.220446049250313e-16;
 
-  bool in_time = true;  // OpEn: max_duration (AlmOptimizer::solve / PANOCOptimizer::solve)
-  for (int outer = 1; outer <= g.max_outer; outer++) {
+  cx->in_time = 1;  // OpEn: max_duration (AlmOptimizer::solve / PANOCOptimizer::solve)
+  for (int outer = 1; outer <= g.max_outer; outer = cx->num_outer + 1) {  // the counter lives in the context
     if (g.max_ns) {  // no time left before this outer iteration: NotConvergedOutOfTime
-      unsigned long long el = globaltimer_ns() - t_start;
+      unsigned long long el = globaltimer_ns() - cx->t_start;
       el = __shfl_sync(FULL, el, 0);
-      if (el > g.max_ns) { exit_status = TTMPC_NOT_CONVERGED_OUT_OF_TIME; in_time = false; break; }
+      if (el > g.max_ns) { cx->exit_status = TTMPC_NOT_CONVERGED_OUT_OF_TIME; cx->in_time = 0; break; }
     }
-    num_outer++;
+    cx->num_outer = outer;
     pb.ya = clipd(pb.ya, -1e12, 1e12);
     pb.yw = clipd(pb.yw, -1e12, 1e12);
     help_drain(hc, sm, lane, N);
@@ -676,43 +726,48 @@ __device__ void solve_scene(const DevCfg &g, const WarpSmem &sm, const SolveArgs
         double nh = pdot(h0, h1, h0, h1);
         double nd = pdot(e0, e1, e0, e1);
         wsum2(nh, nd);
-        U.L = sqrt(nd) / sqrt(nh);
+        U.pc->L = sqrt(nd) / sqrt(nh);
       }
-      U.gamma = GAMMA_L_COEFF / fmax(U.L, MIN_L_ESTIMATE);
+      U.gamma = GAMMA_L_COEFF / fmax(U.pc->L, MIN_L_ESTIMATE);
       set_gamma_terms(U, sm);
       gradient_and_half_step<false>(g, z, U, z.u0, z.u1);
 
-      // PANOCOptimizer::solve main loop (one call site: step, then count)
-      int num_iter = 0;
-      bool cont = true;
+      // PANOCOptimizer::solve main loop (one call site: step, then count).  OpEn's iteration count
+      // num_iter is the step counter after every step that continues, and one less after a step that
+      // continues but ends the loop by the iteration or time limit; OpEn's `cont` is num_iter < max_inner
+      // of the steps before the current one.
+      bool flag;
       while (true) {
         // Two instantiations of the step: the plain one (no request path at all) runs while no
         // helper is attached to this warp -- every iteration of a bulk batch -- and keeps the hot
         // loop ~2 KB shorter (it is bound by the instruction cache, DESIGN.md section 6); the
         // helper-aware one takes over the moment a helper attaches (tail of a batch, one scene
         // alone).  Same arithmetic: results do not depend on which one ran.
-        bool flag;
-        if (__builtin_expect(hc.enabled && *hc.slot >= 0, 0))
+        if (__builtin_expect(help_available<true>(hc), 0))
           flag = panoc_step<DM, true>(g, sm, lane, pb, z, U, g.tol, hc);
         else
           flag = panoc_step<DM, false>(g, sm, lane, pb, z, U, g.tol, hc);
-        if (!(flag && cont && in_time)) break;
-        num_iter++;
-        cont = num_iter < g.max_inner;
+        if (!(flag && U.pc->iteration - 1 < g.max_inner && cx->in_time)) break;
         if (g.max_ns) {
-          unsigned long long el = globaltimer_ns() - t_start;
+          unsigned long long el = globaltimer_ns() - cx->t_start;
           el = __shfl_sync(FULL, el, 0);
-          in_time = el <= g.max_ns;
+          cx->in_time = el <= g.max_ns;
         }
       }
+      const int num_iter = flag ? U.pc->iteration - 1 : U.pc->iteration;
+      const bool cont = num_iter < g.max_inner;
       const bool finite = isfinite(z.u0) && isfinite(z.u1);
-      if (!__all_sync(FULL, finite)) { exit_status = TTMPC_NOT_FINITE; inner_count += num_iter; break; }
+      const int ic = cx->inner_count + num_iter;
+      const unsigned long long pi = cx->panoc_iters + num_iter;
+      const bool all_finite = __all_sync(FULL, finite);
+      __syncwarp();
+      cx->inner_count = ic;
+      if (!all_finite) { cx->exit_status = TTMPC_NOT_FINITE; break; }
       z.u0 = z.h0; z.u1 = z.h1;
       inner_status = !cont ? TTMPC_NOT_CONVERGED_ITERATIONS
-                           : (!in_time ? TTMPC_NOT_CONVERGED_OUT_OF_TIME : TTMPC_CONVERGED);
-      inner_count += num_iter;
-      panoc_iters += num_iter;
-      last_fpr = U.norm_fpr;
+                           : (!cx->in_time ? TTMPC_NOT_CONVERGED_OUT_OF_TIME : TTMPC_CONVERGED);
+      cx->panoc_iters = pi;
+      cx->last_fpr = U.norm_fpr;
     }
     // ---------------- multipliers, infeasibility (alm_optimizer.rs step())
     double F1a = 0.0, F1w = 0.0;
@@ -729,39 +784,49 @@ __device__ void solve_scene(const DevCfg &g, const WarpSmem &sm, const SolveArgs
       yp_w = pb.yw + pb.c * (F1w - t);
       if (!act) { yp_a = 0.0; yp_w = 0.0; }
     }
+    double f2_norm_plus;
     {
       // c = 0: the multipliers do not enter f, F2
       const EvalOut e = eval_psi<DM>(&g, reinterpret_cast<unsigned char *>(sm.ctx), z.u0, z.u1, 0.0, 0.0,
                                      0.0, nullptr, false, 0.0);
       if (lane == 0) sm.ctx->n_cost++;
       f2_norm_plus = sqrt(e.f2sq);
-      f_final = e.f;
+      cx->f2_norm_plus = f2_norm_plus;
+      cx->f_final = e.f;
     }
+    double delta_y_norm_plus;
     {
       const double da = yp_a - pb.ya, dw = yp_w - pb.yw;
       delta_y_norm_plus = sqrt(wsum(pdot(da, dw, da, dw)));
+      cx->dy_norm_plus = delta_y_norm_plus;
     }
+    const double akkt_tol = cx->akkt_tol;
+    const int alm_iter = cx->num_outer - 1;  // AlmOptimizer's iteration counter
     const bool crit1 = alm_iter > 0 && delta_y_norm_plus <= pb.c * g.delta_tol + SMALL_EPSILON;
     const bool crit2 = f2_norm_plus <= g.delta_tol + SMALL_EPSILON;
-    const bool crit3 = U.akkt_tol <= g.tol + SMALL_EPSILON;
-    if (crit1 && crit2 && crit3) { exit_status = inner_status; break; }
+    const bool crit3 = akkt_tol <= g.tol + SMALL_EPSILON;
+    if (crit1 && crit2 && crit3) { cx->exit_status = inner_status; break; }
     // is_penalty_stall_criterion: iteration 0, or both infeasibilities decreased enough
-    const bool crit_alm = delta_y_norm_plus <= g.suff_dec * delta_y_norm + SMALL_EPSILON;
-    const bool crit_pm = g.Ndyn == 0 || f2_norm_plus <= g.suff_dec * f2_norm + SMALL_EPSILON;
+    const bool crit_alm = delta_y_norm_plus <= g.suff_dec * cx->dy_norm + SMALL_EPSILON;
+    const bool crit_pm = g.Ndyn == 0 || f2_norm_plus <= g.suff_dec * cx->f2_norm + SMALL_EPSILON;
     const bool stall = alm_iter == 0 || (crit_alm && crit_pm);
     if (!stall) pb.c *= g.pen_factor;
-    U.akkt_tol = fmax(U.akkt_tol * g.tol_factor, g.tol);
-    z.gp0 = 0.0; z.gp1 = 0.0;  // set_akkt_tolerance allocates a fresh zero vector
-    alm_iter++;
-    delta_y_norm = delta_y_norm_plus;
-    f2_norm = f2_norm_plus;
+    __syncwarp();
+    cx->akkt_tol = fmax(akkt_tol * g.tol_factor, g.tol);
+    if (act) sm.gprev[lane] = make_double2(0.0, 0.0);  // set_akkt_tolerance allocates a fresh zero vector
+    cx->dy_norm = delta_y_norm_plus;
+    cx->f2_norm = f2_norm_plus;
     pb.ya = yp_a; pb.yw = yp_w;
   }
-  if (exit_status != TTMPC_NOT_FINITE && in_time && num_outer == g.max_outer)
+  help_drain(hc, sm, lane, N);  // no evaluation on this scene's tables may still be in flight
+  __syncwarp();
+  int exit_status = cx->exit_status;
+  const int num_outer = cx->num_outer;
+  if (exit_status != TTMPC_NOT_FINITE && cx->in_time && num_outer == g.max_outer)
     exit_status = TTMPC_NOT_CONVERGED_ITERATIONS;
 
-  help_drain(hc, sm, lane, N);  // no evaluation on this scene's tables may still be in flight
   // ---------------- results
+  scene = cx->scene;
   if (act) {
     A.u[(size_t)scene * 2 * N + 2 * lane] = z.u0;
     A.u[(size_t)scene * 2 * N + 2 * lane + 1] = z.u1;
@@ -774,28 +839,35 @@ __device__ void solve_scene(const DevCfg &g, const WarpSmem &sm, const SolveArgs
     eval_psi<DM>(&g, reinterpret_cast<unsigned char *>(sm.ctx), z.u0, z.u1, 0.0, 0.0, 0.0,
                  A.pred_states + (size_t)scene * N * 3, false, 0.0);
   if (lane == 0) {
-    if (A.cost) A.cost[scene] = f_final;
+    if (A.cost) A.cost[scene] = cx->f_final;
     if (A.exit_status) A.exit_status[scene] = exit_status;
     if (A.outer_iters) A.outer_iters[scene] = num_outer;
-    if (A.inner_iters) A.inner_iters[scene] = inner_count;
-    if (A.last_fpr) A.last_fpr[scene] = last_fpr;
-    if (A.f1_infeas) A.f1_infeas[scene] = delta_y_norm_plus / pb.c;
-    if (A.f2_norm) A.f2_norm[scene] = f2_norm_plus;
+    if (A.inner_iters) A.inner_iters[scene] = cx->inner_count;
+    if (A.last_fpr) A.last_fpr[scene] = cx->last_fpr;
+    if (A.f1_infeas) A.f1_infeas[scene] = cx->dy_norm_plus / pb.c;
+    if (A.f2_norm) A.f2_norm[scene] = cx->f2_norm_plus;
     if (A.penalty) A.penalty[scene] = pb.c;
     if (A.evals) {
       A.evals[4 * scene] = sm.ctx->n_cost; A.evals[4 * scene + 1] = sm.ctx->n_grad;
-      A.evals[4 * scene + 2] = (long long)(globaltimer_ns() - t_start);
-      A.evals[4 * scene + 3] = (long long)t_start;
+      A.evals[4 * scene + 2] = (long long)(globaltimer_ns() - cx->t_start);
+      A.evals[4 * scene + 3] = (long long)cx->t_start;
     }
-    wstats[0] += sm.ctx->n_cost;
-    wstats[1] += sm.ctx->n_grad;
-    wstats[2] += sm.ctx->n_body;
-    wstats[3] += panoc_iters;
+    // device-wide counters, added once per scene (a per-warp running sum would hold 8 registers
+    // for the whole kernel)
+    if (A.stats) {
+      atomicAdd(A.stats + 0, (unsigned long long)sm.ctx->n_cost);
+      atomicAdd(A.stats + 1, (unsigned long long)sm.ctx->n_grad);
+      atomicAdd(A.stats + 2, (unsigned long long)sm.ctx->n_body);
+      atomicAdd(A.stats + 3, cx->panoc_iters);
 #ifdef TTMPC_PROFILE
-    // 4: cost evals, 5: grad evals, 6: lbfgs update + apply, 7: whole solve (cycles)
-    wstats[4] += sm.ctx->prof[0]; wstats[5] += sm.ctx->prof[1];
-    wstats[6] += sm.ctx->prof[2] + sm.ctx->prof[3];
-    wstats[7] += clock64() - t_clk0;
+      // 4: cost evals, 5: grad evals, 6: lbfgs update + apply, 7: whole solve (cycles)
+      atomicAdd(A.stats + 4, (unsigned long long)sm.ctx->prof[0]);
+      atomicAdd(A.stats + 5, (unsigned long long)sm.ctx->prof[1]);
+      atomicAdd(A.stats + 6, (unsigned long long)(sm.ctx->prof[2] + sm.ctx->prof[3]));
+      atomicAdd(A.stats + 7, (unsigned long long)(clock64() - t_clk0));
+#endif
+    }
+#ifdef TTMPC_PROFILE
 #ifndef TTMPC_PROFILE_STAGE
     sm.ctx->eprof[9] = sm.ctx->prof[3];  // L-BFGS apply alone (slot 6 holds update + apply)
 #else
@@ -811,26 +883,21 @@ __device__ void solve_scene(const DevCfg &g, const WarpSmem &sm, const SolveArgs
 }
 
 template <class DM>
-__global__ void __launch_bounds__(TTMPC_MAX_THREADS, TTMPC_MIN_BLOCKS) solve_kernel(const __grid_constant__ DevCfg g,
+__global__ void __launch_bounds__(TTMPC_MAX_THREADS, DM::kN ? TTMPC_MIN_BLOCKS : TTMPC_MIN_BLOCKS_RUNTIME) solve_kernel(const __grid_constant__ DevCfg g,
                                                     const __grid_constant__ SolveArgs A) {
-  extern __shared__ __align__(16) unsigned char smem_raw[];
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-  const WarpSmem sm = carve<DM>(smem_raw + (size_t)warp * g.smem_per_warp, g);
-  const int gwarp = blockIdx.x * g.warps_per_block + warp;
-  double *dyn = A.dyn_scratch + (size_t)gwarp * DYN_FIELDS * g.Ndyn * g.N;
-  CtaHelp *cta = reinterpret_cast<CtaHelp *>(smem_raw + (size_t)g.warps_per_block * g.smem_per_warp);
+  const WarpSmem sm = carve<DM>(warp_region(g, warp), g);
+  CtaHelp *cta = cta_help();
   if (threadIdx.x < 8) { cta->busy[threadIdx.x] = 0; cta->helper[threadIdx.x] = -1; cta->epoch[threadIdx.x] = 0; }
   __syncthreads();
   HelpCtl hc;
   hc.enabled = A.helpers != 0;
   hc.timed_out = false;
-  hc.slot = &cta->helper[warp];
   hc.pending = false;
   if (lane == 0) sm.hhdr->state = 0;
-  unsigned long long wstats[8] = {0, 0, 0, 0, 0, 0, 0, 0};
   bool had_scene = false;
   while (true) {
-    if (had_scene && A.helpers && A.run_stats && help_long_running_mate<DM>(g, A, cta, smem_raw, warp, lane))
+    if (had_scene && A.helpers && A.run_stats && help_long_running_mate<DM>(g, A, cta, warp, lane))
       continue;
     int scene = 0;
     if (lane == 0) scene = atomicAdd(A.work_counter, 1);
@@ -883,12 +950,15 @@ __global__ void __launch_bounds__(TTMPC_MAX_THREADS, TTMPC_MIN_BLOCKS) solve_ker
 #ifdef TTMPC_PROFILE_STAGE
     const long long t_stage0 = clock64();
 #endif
-    stage_scene(g, sm, A.p + (size_t)scene * g.np, dyn, lane);
+    {
+      const int gwarp = blockIdx.x * g.warps_per_block + warp;
+      stage_scene(g, sm, A.p + (size_t)scene * g.np, A.dyn_scratch + (size_t)gwarp * DYN_FIELDS * g.Ndyn * g.N, lane);
+    }
 #ifdef TTMPC_PROFILE_STAGE
     if (lane == 0 && A.eprof) atomicAdd(A.eprof + 9, (unsigned long long)(clock64() - t_stage0));  // staging cycles (slot of the apply timer)
 #endif
     hc.enabled = A.helpers != 0 && !hc.timed_out;
-    solve_scene<DM>(g, sm, A, scene, lane, wstats, hc);
+    solve_scene<DM>(g, sm, A, scene, lane, hc);
     if (lane == 0) {
       *reinterpret_cast<volatile int *>(&cta->busy[warp]) = 0;
       if (A.run_stats) {
@@ -899,11 +969,7 @@ __global__ void __launch_bounds__(TTMPC_MAX_THREADS, TTMPC_MIN_BLOCKS) solve_ker
     __syncwarp();
   }
   // out of scenes: help the CTA-mates that still own one
-  if (A.helpers) helper_loop<DM>(g, A, cta, smem_raw, warp, lane);
-  if (lane == 0 && A.stats) {
-    for (int i = 0; i < 8; i++)
-      if (wstats[i]) atomicAdd(A.stats + i, wstats[i]);
-  }
+  if (A.helpers) helper_loop<DM>(g, A, cta, warp, lane);
 }
 
 
@@ -965,9 +1031,8 @@ __global__ void __launch_bounds__(256) order_scenes_kernel(int n, const int *__r
 template <class DM>
 __global__ void __launch_bounds__(128) eval_kernel(const __grid_constant__ DevCfg g,
                                                    const __grid_constant__ EvalArgs A) {
-  extern __shared__ __align__(16) unsigned char smem_raw[];
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-  const WarpSmem sm = carve<DM>(smem_raw + (size_t)warp * g.smem_per_warp, g);
+  const WarpSmem sm = carve<DM>(smem_raw + (size_t)warp * g.smem_per_warp, g);  // no CtaHelp table here
   const int gwarp = blockIdx.x * g.warps_per_block + warp;
   const int nwarps = gridDim.x * g.warps_per_block;
   double *dyn = A.dyn_scratch + (size_t)gwarp * DYN_FIELDS * g.Ndyn * g.N;
@@ -1041,11 +1106,12 @@ __global__ void __launch_bounds__(128, 3) probe_kernel(const __grid_constant__ D
   for (int i = 0; i < reps; i++) acc = wsum(acc * 1e-3 + v);
   long long t3 = clock64();
   Lane z; Uni U;
-  z.d0 = v; z.d1 = w; U.lb_active = g.mem; U.lb_head = 0; U.lb_gamma = 0.7;
+  U.pc = &sm.ctx->pc;
+  z.d0 = v; z.d1 = w; U.pc->lb_active = g.mem; U.pc->lb_head = 0; U.pc->lb_gamma = 0.7;
   if (lane < g.N)
     for (int k = 0; k <= g.mem; k++) {
-      sm.lbs[k * (g.N | 1) + lane] = make_double2(0.01 * (k + 1), 0.02);
-      sm.lby[k * (g.N | 1) + lane] = make_double2(0.03, 0.01 * (k + 2));
+      sm.lbs[k * g.N + lane] = make_double2(0.01 * (k + 1), 0.02);
+      sm.lby[k * g.N + lane] = make_double2(0.03, 0.01 * (k + 2));
     }
   if (lane <= g.mem) sm.rho[lane] = 0.5;
   __syncwarp();
@@ -1161,7 +1227,7 @@ cudaError_t launch_solve(const DevCfg &g, const SolveArgs &A, int grid, cudaStre
   });
 }
 // resident blocks per SM of the kernel launch_solve would pick
-cudaError_t solve_occupancy_impl(const DevCfg &g, int *blocks_per_sm) {
+cudaError_t solve_occupancy(const DevCfg &g, int *blocks_per_sm) {
   const size_t smem = (size_t)g.smem_per_warp * g.warps_per_block + sizeof(CtaHelp);
   return with_solve_dims(g, [&](auto dm) -> cudaError_t {
     using DM = decltype(dm);
@@ -1191,7 +1257,6 @@ cudaError_t launch_eval(const DevCfg &g, const EvalArgs &A, int grid, cudaStream
   }
   return cudaGetLastError();
 }
-cudaError_t solve_occupancy(const DevCfg &g, int *blocks_per_sm) { return solve_occupancy_impl(g, blocks_per_sm); }
 cudaError_t launch_probe(const DevCfg &g, const double *p, double *dyn, long long *out, int reps,
                          cudaStream_t st) {
   const size_t smem = (size_t)g.smem_per_warp * g.warps_per_block;
