@@ -43,7 +43,7 @@
 extern "C" {
 #endif
 
-#define TTMPC_VERSION 100
+#define TTMPC_VERSION 101
 
 /* exit_status codes; names are the strings the OpEn python binding returns
  * (format!("{:?}", ExitStatus)), which the reference matches against
@@ -276,6 +276,20 @@ enum {
   TTMPC_FLEET_REACHED = 1,  /* check_termination_condition: get_action -> None    */
   TTMPC_FLEET_FAILED = 2    /* solver error (the reference raises RuntimeError)   */
 };
+/* ttmpc_fleet.options: bit mask of opt-in behaviours of ttmpc_fleet_step_device (0 = none; the
+ * pack and advance entry points ignore it).  Other bits -> TTMPC_ERR_BAD_ARG.                  */
+enum {
+  /* Start the solve of every robot that is RUNNING after this step's goal test from its previous
+   * solution shifted by one step, u'[k] = u[k+1] for k < N-1 and u'[N-1] = u[N-1], if that
+   * solve's exit status was TTMPC_CONVERGED, and from zeros otherwise (run_step's initial_guess).
+   * The previous step's outputs are read from res->u and res->exit_status, which must therefore
+   * hold zeros before the first step.  Multipliers still follow use_y0.                         */
+  TTMPC_FLEET_WARM_START = 1,
+  /* Solve only the robots that are RUNNING (get_action returns None before the solver is called
+   * once the goal test holds).  The result rows of the other robots -- every member of res --
+   * keep the values of the last step in which they were solved.                               */
+  TTMPC_FLEET_SKIP_STOPPED = 2
+};
 typedef struct ttmpc_fleet {
   int n;            /* robots                                                         */
   int ref_stride;   /* rows per robot in ref_traj                                     */
@@ -291,7 +305,7 @@ typedef struct ttmpc_fleet {
   int stc_shared;
   int n_dyn_live;   /* moving obstacles described by dyn_cur / dyn_last (<= Ndynobs)  */
   int action_steps; /* config.action_steps; only 1 is supported                       */
-  int _pad;
+  int options;      /* TTMPC_FLEET_* bit mask of the step; C callers must zero it         */
   const double *other;    /* [n][ns*N*Nother] other-robot predictions or NULL (zeros) */
   const double *dyn;      /* [n][Ndynobs*ndynobs*N] ready-made rows or NULL           */
   double *dyn_cur;  /* [n][n_dyn_live][2] current obstacle positions (in/out) or NULL */
@@ -325,8 +339,10 @@ int ttmpc_fleet_pack_device(const ttmpc_config *cfg, const ttmpc_fleet *fleet, d
 /* d_u [n][nu*N] solutions, d_exit_status [n] of the solve that used d_p. */
 int ttmpc_fleet_advance_device(const ttmpc_config *cfg, const ttmpc_fleet *fleet,
                                const double *d_u, const int *d_exit_status, void *stream);
-/* pack + solve (cold start, like run_step with initial_guess=None; multipliers carried in
- * res->y when use_y0 != 0, like the reference's Solver object) + advance, on `stream`. */
+/* pack + solve + advance, on `stream`.  The solve starts from zeros (run_step with
+ * initial_guess=None) unless fleet->options has TTMPC_FLEET_WARM_START, and runs every robot
+ * unless it has TTMPC_FLEET_SKIP_STOPPED.  Multipliers are carried in res->y when use_y0 != 0,
+ * like the reference's Solver object. */
 int ttmpc_fleet_step_device(const ttmpc_config *cfg, const ttmpc_fleet *fleet, double *d_p,
                             int use_y0, const ttmpc_result *res, void *stream);
 

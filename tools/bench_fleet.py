@@ -1,15 +1,21 @@
 #!/usr/bin/env python
-"""Closed-loop fleet step on one GPU: n robots, K control steps without touching the host.
+"""Closed-loop fleet drive on one GPU, with and without the fleet-step options.
 
-  python tools/bench_fleet.py [n=4096] [steps=30]
+  python tools/bench_fleet.py [n=4096] [max_steps=200]
 
-Per step = pack + solve + advance (ttmpc_fleet_step_device).  Prints one JSON line with the
-p50 / p90 step time, robot-steps/s, the share of pack and advance, the HBM rate of the pack
-kernel against MEASURED_PEAKS.json, and the CPU oracle (reference order, all host cores) doing the
-same step on a bounded sample.  Appended to gpurun_out/bench_fleet.json.
+Each leg builds the same seeded fleet and calls FleetPlanner.step() -- pack + solve + advance,
+multipliers carried from step to step -- until every robot has stopped or max_steps steps have
+run.  Legs: options off (0), warm start (W), skip stopped robots (S) and both (WS), run
+interleaved as 0 W S WS WS S W 0 so that drift of the card affects every option alike.  Per leg:
+drive time (sum of the per-step event times), step p50 / p90, PANOC iterations (device counters,
+ttmpc_read_stats) and reached / failed / running robots at the end.  The card's name and power
+limit are read in the same run.  Also the CPU oracle (reference order, all host cores) doing one
+plain step on a bounded sample.  Prints one JSON line.
 """
+import ctypes as C
 import json
 import os
+import subprocess
 import sys
 import time
 
@@ -18,62 +24,81 @@ import numpy as np
 import torch
 
 import trajtrack_mpcndqn_rlboost_b200 as t
+from trajtrack_mpcndqn_rlboost_b200 import _lib
 from trajtrack_mpcndqn_rlboost_b200.fleet import work_mode
 from tests import oracle_lib as O
 
-ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+LEGS = ["0", "W", "S", "WS", "WS", "S", "W", "0"]
+
+
+def card():
+    try:
+        pl = subprocess.run(["nvidia-smi", "--query-gpu=power.limit", "--format=csv,noheader", "-i",
+                             str(torch.cuda.current_device())], capture_output=True, text=True, timeout=30).stdout.strip()
+    except (OSError, subprocess.SubprocessError):
+        pl = None
+    return dict(gpu=torch.cuda.get_device_name(), power_limit=pl or None)
+
+
+def make(n, mc, fl):
+    fp = t.FleetPlanner(mc, fl["init"], fl["goal"], fl["paths"], mode="work")
+    fp.update_static_constraints(fl["static_polys"], per_robot=True)
+    fp.set_moving_obstacles(fl["moving_pos"], fl["moving_disp"])
+    return fp
+
+
+def drive(fp, leg, max_steps):
+    stats = (C.c_ulonglong * 4)()
+    _lib.check(fp.lib.ttmpc_read_stats(stats, 1), "ttmpc_read_stats")
+    ev = []
+    for k in range(max_steps):
+        e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+        e0.record()
+        fp.step(warm_start="W" in leg, skip_stopped="S" in leg)
+        e1.record()
+        ev.append((e0, e1))
+        if k % 5 == 4 and int((fp.status == 0).sum()) == 0:
+            break
+    torch.cuda.synchronize()
+    _lib.check(fp.lib.ttmpc_read_stats(stats, 0), "ttmpc_read_stats")
+    ms = [a.elapsed_time(b) for a, b in ev]
+    status = fp.status.cpu().numpy()
+    q = lambda p: float(np.quantile(ms, p))
+    return dict(leg=leg, steps=len(ms), drive_ms=float(np.sum(ms)), step_ms_p50=q(0.5), step_ms_p90=q(0.9),
+                panoc_iters=int(stats[3]), reached=int((status == 1).sum()), failed=int((status == 2).sum()),
+                running=int((status == 0).sum()))
 
 
 def main():
     n = int(sys.argv[1]) if len(sys.argv) > 1 else 4096
-    steps = int(sys.argv[2]) if len(sys.argv) > 2 else 30
+    max_steps = int(sys.argv[2]) if len(sys.argv) > 2 else 200
     mc = t.Configurator()
     fl = t.scenes.make_fleet(n, seed=1000)
-    fp = t.FleetPlanner(mc, fl["init"], fl["goal"], fl["paths"], mode="work")
-    fp.update_static_constraints(fl["static_polys"], per_robot=True)
-    fp.set_moving_obstacles(fl["moving_pos"], fl["moving_disp"])
-    ev = lambda: torch.cuda.Event(enable_timing=True)
-    for _ in range(3):          # warm-up steps (they do advance the fleet)
-        fp.step()
+    warm = make(n, mc, fl)      # module loads and first-launch costs stay out of the legs
+    for _ in range(3):
+        warm.step(warm_start=True, skip_stopped=True)
     torch.cuda.synchronize()
-    t_step, t_pack, t_adv, iters, running = [], [], [], [], []
-    for k in range(steps):
-        e0, e1, e2, e3 = ev(), ev(), ev(), ev()
-        e0.record(); fp.pack(); e1.record()
-        r = fp._result_struct()
-        import ctypes as C
-        from trajtrack_mpcndqn_rlboost_b200 import _lib
-        st = torch.cuda.current_stream().cuda_stream
-        _lib.check(fp.lib.ttmpc_solve_batch_device(C.byref(fp.cfg), n, fp.p.data_ptr(), 0, 0, None, C.byref(r), st), "solve")
-        e2.record(); fp.advance(); e3.record()
-        torch.cuda.synchronize()
-        t_step.append(e0.elapsed_time(e3)); t_pack.append(e0.elapsed_time(e1)); t_adv.append(e2.elapsed_time(e3))
-        iters.append(float(fp.inner.float().mean())); running.append(int((fp.status == 0).sum()))
-    q = lambda a, p: float(np.quantile(a, p))
-    peaks = json.load(open(os.path.join(ROOT, "MEASURED_PEAKS.json"))) if os.path.exists(os.path.join(ROOT, "MEASURED_PEAKS.json")) else {}
-    pack_bytes = fp.p.numel() * 8 + n * (fp.N * 3 * 8 + 12 * 8 + fp.stc.shape[1] * 8)   # row written + ref window, state, own static rows read
-    out = dict(workload=f"fleet{n}", robots=n, steps=steps, step_ms_p50=q(t_step, 0.5), step_ms_p90=q(t_step, 0.9),
-               robot_steps_per_s=n / (q(t_step, 0.5) * 1e-3), pack_ms_p50=q(t_pack, 0.5), advance_ms_p50=q(t_adv, 0.5),
-               pack_GBps=pack_bytes / (q(t_pack, 0.5) * 1e-3) / 1e9, hbm_peak_GBps=peaks.get("hbm_gbs"),
-               mean_inner_iters=float(np.mean(iters)), running_last=running[-1],
-               step_ms=[round(x, 1) for x in t_step], inner_iters=[round(x, 1) for x in iters])
-    # CPU: the same step with the oracle (reference operation order), bounded sample
+    legs = [drive(make(n, mc, fl), leg, max_steps) for leg in LEGS]
+    mean = {}
+    for leg in dict.fromkeys(LEGS):
+        rs = [r for r in legs if r["leg"] == leg]
+        mean[leg] = {k: float(np.mean([r[k] for r in rs])) for k in ("drive_ms", "step_ms_p50", "step_ms_p90", "panoc_iters")}
+        mean[leg].update({k: rs[-1][k] for k in ("steps", "reached", "failed", "running")})
+    out = dict(workload=f"fleet{n}", robots=n, max_steps=max_steps, **card(), legs=legs, mean=mean)
+    # CPU: one plain step with the oracle (reference operation order), bounded sample
     ns = min(n, 256)
     tuning, base = work_mode(mc, "work")
-    fh = O.FleetHost(fp.cfg, fl["init"][:ns], fl["goal"][:ns], fp.ref_traj.cpu().numpy()[:ns], fp.ref_len.cpu().numpy()[:ns],
-                     fp.stc.cpu().numpy()[:ns], tuning, base, mc.low_speed, dyn_cur=fl["moving_pos"][:ns], dyn_disp=fl["moving_disp"][:ns])
+    fh = O.FleetHost(warm.cfg, fl["init"][:ns], fl["goal"][:ns], warm.ref_traj.cpu().numpy()[:ns], warm.ref_len.cpu().numpy()[:ns],
+                     warm.stc.cpu().numpy()[:ns], tuning, base, mc.low_speed, dyn_cur=fl["moving_pos"][:ns], dyn_disp=fl["moving_disp"][:ns])
     cores = os.cpu_count() or 1
     t0 = time.perf_counter()
     for _ in range(2):
         p = O.fleet_pack(fh, use_libm=True)
-        ref = O.solve_batch(fp.cfg, p, threads=cores, warp=False)
+        ref = O.solve_batch(warm.cfg, p, threads=cores, warp=False)
         O.fleet_advance(fh, ref["u"], ref["exit_status"], use_libm=True)
     dt = (time.perf_counter() - t0) / 2
     out["cpu_baseline"] = dict(robot_steps_per_s=ns / dt, cores=cores, kind="port", sample=f"{ns} robots x 2 steps")
     print(json.dumps(out))
-    os.makedirs(os.path.join(ROOT, "gpurun_out"), exist_ok=True)
-    with open(os.path.join(ROOT, "gpurun_out", "bench_fleet.json"), "a") as f:
-        f.write(json.dumps(out) + "\n")
 
 
 if __name__ == "__main__":

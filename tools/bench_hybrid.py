@@ -6,8 +6,10 @@
 
 all device-resident (ttdqn_internal_obs_device, ttdqn_observe_act_device, ttdqn_rl_ref_device,
 ttmpc_fleet_step_device); whether the hint is used is decided per step and environment by the
-HintSwitcher logic inside the pack kernel.  python tools/bench_hybrid.py [n=16384] [steps=10]
+HintSwitcher logic inside the pack kernel.
+  python tools/bench_hybrid.py [n=16384] [steps=10] [--warm-start] [--skip-stopped]
 """
+import argparse
 import json
 import os
 import sys
@@ -22,8 +24,13 @@ ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
 
 def main():
-    n = int(sys.argv[1]) if len(sys.argv) > 1 else 16384
-    steps = int(sys.argv[2]) if len(sys.argv) > 2 else 10
+    ap = argparse.ArgumentParser()
+    ap.add_argument("n", type=int, nargs="?", default=16384)
+    ap.add_argument("steps", type=int, nargs="?", default=10)
+    ap.add_argument("--warm-start", action="store_true", help="FleetPlanner.step(warm_start=True)")
+    ap.add_argument("--skip-stopped", action="store_true", help="FleetPlanner.step(skip_stopped=True)")
+    a = ap.parse_args()
+    n, steps = a.n, a.steps
     mc = t.Configurator()
     fl = t.scenes.make_fleet(n, seed=1000)
     fp = t.FleetPlanner(mc, fl["init"], fl["goal"], fl["paths"], mode="work")
@@ -64,7 +71,8 @@ def main():
         comp.observe_act_device(fp.state, xy, off, sol, cnt, internal, old, out, qs)
         t.dqn.rl_ref_device(agent5, out["action"], steps=fp.N, ts=mc.ts, ref_speed=1.0, out=rl)
         e[1].record()
-        fp.step(keep_multipliers=os.environ.get('KEEP_Y', '1') == '1')
+        fp.step(keep_multipliers=os.environ.get('KEEP_Y', '1') == '1', warm_start=a.warm_start,
+                skip_stopped=a.skip_stopped)
         e[2].record()
         if times is not None:
             torch.cuda.synchronize()
@@ -76,7 +84,7 @@ def main():
     for _ in range(steps):
         one_step(times)
     tt = np.array(times)
-    res = dict(workload=f"hybrid{n}", envs=n, steps=steps, step_ms_p50=float(np.median(tt[:, 0])),
+    res = dict(workload=f"hybrid{n}", envs=n, warm_start=a.warm_start, skip_stopped=a.skip_stopped, steps=steps, step_ms_p50=float(np.median(tt[:, 0])),
                step_ms_p90=float(np.quantile(tt[:, 0], 0.9)), dqn_part_ms_p50=float(np.median(tt[:, 1])),
                env_steps_per_s=n / (float(np.median(tt[:, 0])) * 1e-3),
                actions_hist=np.bincount(out["action"].cpu().numpy(), minlength=9).tolist(),

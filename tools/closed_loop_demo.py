@@ -1,7 +1,9 @@
 #!/usr/bin/env python
 """Functional check of the whole stack: n robots drive their reference paths to the goal with the
 device-resident fleet loop; reports how many arrive, the closest approach to the static obstacles
-and the tracking error.  python tools/closed_loop_demo.py [n=1024] [max_steps=200]"""
+and the tracking error.
+  python tools/closed_loop_demo.py [n=1024] [max_steps=200] [--warm-start] [--skip-stopped]"""
+import argparse
 import json
 import os
 import sys
@@ -25,8 +27,13 @@ def point_poly_clearance(px, py, polys):
 
 
 def main():
-    n = int(sys.argv[1]) if len(sys.argv) > 1 else 1024
-    max_steps = int(sys.argv[2]) if len(sys.argv) > 2 else 200
+    ap = argparse.ArgumentParser()
+    ap.add_argument("n", type=int, nargs="?", default=1024)
+    ap.add_argument("max_steps", type=int, nargs="?", default=200)
+    ap.add_argument("--warm-start", action="store_true", help="FleetPlanner.step(warm_start=True)")
+    ap.add_argument("--skip-stopped", action="store_true", help="FleetPlanner.step(skip_stopped=True)")
+    a = ap.parse_args()
+    n, max_steps = a.n, a.max_steps
     mc = t.Configurator()
     fl = t.scenes.make_fleet(n, seed=7)
     fp = t.FleetPlanner(mc, fl["init"], fl["goal"], fl["paths"], mode="work")
@@ -38,7 +45,7 @@ def main():
     e0.record()
     steps = 0
     for k in range(max_steps):
-        fp.step()
+        fp.step(warm_start=a.warm_start, skip_stopped=a.skip_stopped)
         steps += 1
         if k % 5 == 4:
             st = fp.state.cpu().numpy()
@@ -48,7 +55,7 @@ def main():
     e1.record(); torch.cuda.synchronize()
     status = fp.status.cpu().numpy(); st = fp.state.cpu().numpy()
     dist_goal = np.hypot(st[:, 0] - fl["goal"][:, 0], st[:, 1] - fl["goal"][:, 1])
-    out = dict(robots=n, steps=steps, wall_ms=e0.elapsed_time(e1), reached=int((status == 1).sum()),
+    out = dict(robots=n, warm_start=a.warm_start, skip_stopped=a.skip_stopped, steps=steps, wall_ms=e0.elapsed_time(e1), reached=int((status == 1).sum()),
                failed=int((status == 2).sum()), still_running=int((status == 0).sum()),
                dist_to_goal_p50=float(np.median(dist_goal)), dist_to_goal_max=float(dist_goal.max()),
                min_clearance_to_static_obstacles=float(clearance.min()),

@@ -57,6 +57,9 @@ class TtdqnQnet(C.Structure):
     ]
 
 
+FLEET_WARM_START, FLEET_SKIP_STOPPED = 1, 2  # ttmpc_fleet.options bits
+
+
 class TtmpcFleet(C.Structure):
     """struct ttmpc_fleet: raw addresses (device for the product calls, host for the oracle)."""
     _fields_ = [
@@ -64,7 +67,7 @@ class TtmpcFleet(C.Structure):
         ("state", C.c_void_p), ("goal", C.c_void_p), ("last_u", C.c_void_p),
         ("idx_ref", C.c_void_p), ("status", C.c_void_p), ("ref_traj", C.c_void_p),
         ("ref_len", C.c_void_p), ("stc", C.c_void_p),
-        ("stc_shared", C.c_int), ("n_dyn_live", C.c_int), ("action_steps", C.c_int), ("_pad", C.c_int),
+        ("stc_shared", C.c_int), ("n_dyn_live", C.c_int), ("action_steps", C.c_int), ("options", C.c_int),
         ("other", C.c_void_p), ("dyn", C.c_void_p), ("dyn_cur", C.c_void_p),
         ("dyn_last", C.c_void_p), ("dyn_disp", C.c_void_p),
         ("dyn_size", C.c_double), ("tuning", C.c_double * 10),

@@ -358,9 +358,11 @@ static int plan_solve(Workspace *w, const DevCfg &g, int n_scenes, SolvePlan *pl
   return TTMPC_OK;
 }
 
+// skip_status [n] or null: scenes whose entry is non-zero are not solved (fleet step, skip stopped)
 static int solve_device_impl(const ttmpc_config *cfg, int n_scenes, const double *d_p, int use_u0,
                              int use_y0, const double *d_c0, const ttmpc_result *res,
-                             cudaStream_t st, Slot *host_slot, bool gated);
+                             cudaStream_t st, Slot *host_slot, bool gated,
+                             const int *skip_status = nullptr);
 
 extern "C" int ttmpc_solve_batch_device(const ttmpc_config *cfg, int n_scenes, const double *d_p,
                                         int use_u0, int use_y0, const double *d_c0,
@@ -370,7 +372,7 @@ extern "C" int ttmpc_solve_batch_device(const ttmpc_config *cfg, int n_scenes, c
 
 static int solve_device_impl(const ttmpc_config *cfg, int n_scenes, const double *d_p, int use_u0,
                              int use_y0, const double *d_c0, const ttmpc_result *res,
-                             cudaStream_t st, Slot *host_slot, bool gated) {
+                             cudaStream_t st, Slot *host_slot, bool gated, const int *skip_status) {
   DevCfg g;
   int rc = make_devcfg(cfg, &g);
   if (rc) return rc;
@@ -420,6 +422,7 @@ static int solve_device_impl(const ttmpc_config *cfg, int n_scenes, const double
   // the running average behind the early-helper threshold is per launch (workloads differ by 30x)
   CUDA_TRY(cudaMemsetAsync(A.run_stats, 0, 2 * sizeof(unsigned long long), st));
   A.n_scenes = n_scenes; A.use_u0 = use_u0; A.use_y0 = use_y0;
+  A.skip_status = skip_status;
   A.order = nullptr;
   if (want_order) {
     CUDA_TRY(launch_rank_scenes(g, d_p, n_scenes, sl->order + n_scenes, sl->order, st));
@@ -456,7 +459,7 @@ extern "C" int ttmpc_fleet_pack_device(const ttmpc_config *cfg, const ttmpc_flee
   if (rc) return rc;
   if (fleet->n == 0) return TTMPC_OK;
   if (!d_p) return fail(TTMPC_ERR_BAD_ARG, "fleet: d_p is required");
-  CUDA_TRY(launch_fleet_pack(*fleet, d, d_p, (cudaStream_t)stream));
+  CUDA_TRY(launch_fleet_pack(*fleet, d, d_p, nullptr, nullptr, (cudaStream_t)stream));
   return TTMPC_OK;
 }
 extern "C" int ttmpc_fleet_advance_device(const ttmpc_config *cfg, const ttmpc_fleet *fleet,
@@ -473,11 +476,24 @@ extern "C" int ttmpc_fleet_step_device(const ttmpc_config *cfg, const ttmpc_flee
                                        int use_y0, const ttmpc_result *res, void *stream) {
   if (!res || !res->u || !res->exit_status)
     return fail(TTMPC_ERR_BAD_ARG, "fleet: res->u and res->exit_status are required");
-  int rc = ttmpc_fleet_pack_device(cfg, fleet, d_p, stream);
+  FleetDims d;
+  int rc = fleet_dims(cfg, fleet, &d);
   if (rc) return rc;
-  rc = ttmpc_solve_batch_device(cfg, fleet->n, d_p, 0, use_y0, nullptr, res, stream);
+  if (fleet->options & ~(TTMPC_FLEET_WARM_START | TTMPC_FLEET_SKIP_STOPPED))
+    return fail(TTMPC_ERR_BAD_ARG, "fleet: unknown bits in options");
+  if (fleet->n == 0) return TTMPC_OK;
+  if (!d_p) return fail(TTMPC_ERR_BAD_ARG, "fleet: d_p is required");
+  const bool warm = fleet->options & TTMPC_FLEET_WARM_START;
+  const bool skip = fleet->options & TTMPC_FLEET_SKIP_STOPPED;
+  cudaStream_t st = (cudaStream_t)stream;
+  // warm start: the pack kernel shifts res->u of the robots it leaves RUNNING; a zero row there
+  // solves exactly like use_u0 = 0
+  CUDA_TRY(launch_fleet_pack(*fleet, d, d_p, warm ? res->u : nullptr, warm ? res->exit_status : nullptr, st));
+  rc = solve_device_impl(cfg, fleet->n, d_p, warm ? 1 : 0, use_y0, nullptr, res, st, nullptr, false,
+                         skip ? fleet->status : nullptr);
   if (rc) return rc;
-  return ttmpc_fleet_advance_device(cfg, fleet, res->u, res->exit_status, stream);
+  CUDA_TRY(launch_fleet_advance(*fleet, d, res->u, res->exit_status, st));
+  return TTMPC_OK;
 }
 
 // Cumulative device-side counters since the last reset:

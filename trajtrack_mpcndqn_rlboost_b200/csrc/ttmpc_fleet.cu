@@ -106,12 +106,16 @@ __device__ int hint_switch(const ttmpc_fleet &f, int e, int N, const double *ref
 
 // One CTA per robot.  Thread 0 does the scalar decisions (closest reference point, goal test,
 // speed reference); all threads then write the packed vector, element o of the row by thread
-// o mod blockDim (coalesced 8-byte stores).
+// o mod blockDim (coalesced 8-byte stores).  With warm_u (warm start of the fleet step) the CTA of
+// a robot that is RUNNING after the goal test also rewrites its row of warm_u, the initial guess of
+// this step's solve: the previous solution shifted by one step (last control repeated) if that
+// solve converged, zeros otherwise.
 __global__ void __launch_bounds__(128) fleet_pack_kernel(const ttmpc_fleet f, const FleetDims d,
-                                                         double *__restrict__ p_all) {
+                                                         double *__restrict__ p_all, double *warm_u,
+                                                         const int *__restrict__ warm_exit) {
   const int e = blockIdx.x;
   if (e >= f.n) return;
-  __shared__ int s_idx, s_hint, s_sw;
+  __shared__ int s_idx, s_hint, s_sw, s_run;
   __shared__ double s_speed;
   __shared__ double s_dist[SW_MAX_OBS];
   __shared__ unsigned char s_in[32 * SW_MAX_OBS];
@@ -137,6 +141,7 @@ __global__ void __launch_bounds__(128) fleet_pack_kernel(const ttmpc_fleet f, co
       const bool close = fabs(x - goal[0]) <= 0.05 && fabs(y - goal[1]) <= 0.05;
       if (close && fabs(lu[0]) < 0.05) f.status[e] = TTMPC_FLEET_REACHED;
     }
+    s_run = f.status[e] == TTMPC_FLEET_RUNNING;
     s_idx = idx;
     s_sw = (f.sw_state && f.hint && f.use_hint && was_running) ? 1 : 0;
     // speed reference (:248-255)
@@ -175,6 +180,14 @@ __global__ void __launch_bounds__(128) fleet_pack_kernel(const ttmpc_fleet f, co
   }
   if (threadIdx.x == 0) s_hint = (f.hint && f.use_hint && f.use_hint[e]) ? 1 : 0;
   __syncthreads();
+  if (warm_u && s_run) {  // in place: every element is read before any is written
+    double *u = warm_u + (size_t)e * 2 * N;
+    const int o = threadIdx.x, nz = 2 * N;  // nz <= 64 < blockDim
+    double v = 0.0;
+    if (o < nz && warm_exit[e] == TTMPC_CONVERGED) v = u[o + 2 < nz ? o + 2 : o];
+    __syncthreads();
+    if (o < nz) u[o] = v;
+  }
   double *p = p_all + (size_t)e * d.np;
   const int o_refs = 18, o_speed = o_refs + 3 * N, o_other = o_speed + N, o_stc = o_other + d.n_other,
             o_dyn = o_stc + d.n_stc, o_ws = o_dyn + d.n_dyn, o_wd = o_ws + N;
@@ -257,8 +270,9 @@ __global__ void __launch_bounds__(128) fleet_advance_kernel(const ttmpc_fleet f,
   f.last_u[2 * e] = v; f.last_u[2 * e + 1] = w;
 }
 
-cudaError_t launch_fleet_pack(const ttmpc_fleet &f, const FleetDims &d, double *p, cudaStream_t st) {
-  fleet_pack_kernel<<<f.n, 128, 0, st>>>(f, d, p);
+cudaError_t launch_fleet_pack(const ttmpc_fleet &f, const FleetDims &d, double *p, double *warm_u,
+                              const int *warm_exit, cudaStream_t st) {
+  fleet_pack_kernel<<<f.n, 128, 0, st>>>(f, d, p, warm_u, warm_exit);
   return cudaGetLastError();
 }
 cudaError_t launch_fleet_advance(const ttmpc_fleet &f, const FleetDims &d, const double *u,

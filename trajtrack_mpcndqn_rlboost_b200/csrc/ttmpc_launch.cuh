@@ -24,6 +24,8 @@ struct SolveArgs {
                         // (host path streams p in chunks while the kernel already runs)
   unsigned long long *stats;  // [4]: cost evals, grad evals, dyn bodies, panoc iterations
   unsigned long long *run_stats;  // [2]: evaluations and count of finished scenes (early helpers) or null
+  const int *skip_status;  // [n] or null: scenes whose entry is non-zero are not solved (fleet
+                           // status of stopped robots); their result rows are left untouched
   int n_scenes;
   int use_u0, use_y0;
 };
@@ -47,7 +49,10 @@ cudaError_t launch_probe(const DevCfg &g, const double *p, double *dyn, long lon
                          cudaStream_t st);
 // fleet step (ttmpc_fleet.cu)
 struct FleetDims { int N, np, n_other, n_stc, n_dyn; double ts; };
-cudaError_t launch_fleet_pack(const ttmpc_fleet &f, const FleetDims &d, double *p, cudaStream_t st);
+// warm_u / warm_exit (both or neither): the previous step's solutions, shifted in place into the
+// initial guess of every robot that is RUNNING after this step's goal test
+cudaError_t launch_fleet_pack(const ttmpc_fleet &f, const FleetDims &d, double *p, double *warm_u,
+                              const int *warm_exit, cudaStream_t st);
 cudaError_t launch_fleet_advance(const ttmpc_fleet &f, const FleetDims &d, const double *u,
                                  const int *exit_status, cudaStream_t st);
 cudaError_t launch_fp64_peak(double *out, int blocks, int threads, int iters, cudaStream_t st);

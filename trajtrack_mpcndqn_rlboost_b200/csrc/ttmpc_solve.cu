@@ -903,8 +903,10 @@ __global__ void __launch_bounds__(TTMPC_MAX_THREADS, DM::kN ? TTMPC_MIN_BLOCKS :
     if (lane == 0) scene = atomicAdd(A.work_counter, 1);
     scene = __shfl_sync(FULL, scene, 0);
     if (scene >= A.n_scenes) break;
-    had_scene = true;
     if (A.order) scene = A.order[scene];  // likely-long scenes first (rank_scenes_kernel)
+    // skipped scenes: no writes, not counted, the warp stays idle and fetches again
+    if (A.skip_status && A.skip_status[scene] != 0) continue;
+    had_scene = true;
     // owner from here on: warps that find the queue empty may attach as helpers already while
     // the tables are being staged (requests are only posted from solve_scene)
     if (lane == 0) {

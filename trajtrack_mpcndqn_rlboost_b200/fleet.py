@@ -182,7 +182,8 @@ class FleetPlanner:
         r.inner_iters, r.y, r.pred_states = self.inner.data_ptr(), self.y.data_ptr(), self.pred_states.data_ptr()
         return r
 
-    def step(self, keep_multipliers: bool = True, stream=None):
+    def step(self, keep_multipliers: bool = True, warm_start: bool = False, skip_stopped: bool = False,
+             stream=None):
         """One control step of every robot, asynchronous on the current torch stream.
 
         keep_multipliers=True (default) is what the reference's control loop does: the PyO3 ``Solver``
@@ -190,12 +191,20 @@ class FleetPlanner:
         the ones the next ``run()`` starts from (``self.y`` lives on the device between steps and is
         passed in / out of the solve).  False starts every step from y = 0 (a fresh solver object).
 
+        warm_start=True starts the solve of every running robot from its previous solution shifted
+        by one step (the last control repeated) when that solve converged, and from zeros otherwise
+        (``TTMPC_FLEET_WARM_START``; ``run_step(..., initial_guess)`` in the reference).  ``self.u``
+        and ``self.exit_status`` start as zeros, so a warm first step equals a cold one.
+        skip_stopped=True solves only the robots that are still RUNNING; the result rows of the
+        others keep what their last solve wrote (``TTMPC_FLEET_SKIP_STOPPED``).  Both default to off.
+
         ``pred_states`` is the rollout of u* from the state the step STARTED in (p.s), i.e. one step
         earlier than ``TrajectoryGenerator.run_step``'s list, which re-applies u from the post-step
         state (trajectory_generator.py:296-301; ``planner.TrajectoryGenerator`` reproduces that list
         on the host)."""
         st = stream if stream is not None else self.torch.cuda.current_stream().cuda_stream
         f, r = self._fleet_struct(), self._result_struct()
+        f.options = (_lib.FLEET_WARM_START if warm_start else 0) | (_lib.FLEET_SKIP_STOPPED if skip_stopped else 0)
         _lib.check(self.lib.ttmpc_fleet_step_device(C.byref(self.cfg), C.byref(f), self.p.data_ptr(),
                                                     1 if keep_multipliers else 0, C.byref(r), st),
                    "ttmpc_fleet_step_device")
