@@ -43,7 +43,7 @@
 extern "C" {
 #endif
 
-#define TTMPC_VERSION 101
+#define TTMPC_VERSION 102
 
 /* exit_status codes; names are the strings the OpEn python binding returns
  * (format!("{:?}", ExitStatus)), which the reference matches against
@@ -374,10 +374,6 @@ int ttmpc_read_stats(unsigned long long out[4], int reset);
 /* Launch geometry the solve kernel uses for n_scenes (reporting only). */
 int ttmpc_launch_info(const ttmpc_config *cfg, int n_scenes, int *grid, int *block,
                       int *smem_bytes, int *blocks_per_sm, int *sm_count);
-
-/* Single-warp latency probe (diagnostics): cycles per call of {cost eval, gradient
- * eval, butterfly sum, L-BFGS apply, fp64 divide, sqrt, dependent DFMA, checksum}. */
-int ttmpc_probe_latency(const ttmpc_config *cfg, const double *h_p, long long out[8], int reps);
 
 /* FP64 FMA-pipe peak probe: runs a dependent-chain-free DFMA kernel on every
  * SM and returns achieved TFLOP/s (used by bench.py as the roofline

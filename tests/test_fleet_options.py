@@ -35,7 +35,7 @@ def test_warm_start_rule_on_hand_made_rows():
     assert np.array_equal(warm_start(np.zeros(1, np.int32), u1, np.zeros(1, np.int32)), u1)
 
 
-def test_fleet_struct_layout_matches_header(tmp_path):
+def test_fleet_struct_layout_and_version_match_header(tmp_path):
     src = tmp_path / "layout.c"
     src.write_text('#include <stddef.h>\n#include <stdio.h>\n#include "ttmpc.h"\n'
                    'int main(void) { printf("%zu %zu %zu %d %d %d\\n", sizeof(ttmpc_fleet), '
@@ -50,5 +50,5 @@ def test_fleet_struct_layout_matches_header(tmp_path):
     assert C.sizeof(_lib.TtmpcFleet) == size
     assert _lib.TtmpcFleet.options.offset == off_options == off_action + 4
     assert (_lib.FLEET_WARM_START, _lib.FLEET_SKIP_STOPPED) == (warm, skip)
-    assert version == 101
+    assert version == 102 == _lib.load().ttmpc_version()
     assert _lib.TtmpcFleet().options == 0

@@ -106,7 +106,6 @@ SYMBOLS = {
     "ttmpc_read_stats": (_I, [C.POINTER(C.c_ulonglong), _I]),
     "ttmpc_launch_info": (_I, [_CFG, _I] + [C.POINTER(C.c_int)] * 5),
     "ttmpc_measure_fp64_peak": (_I, [C.POINTER(_D), _VP]),
-    "ttmpc_probe_latency": (_I, [_CFG, _VP, C.POINTER(C.c_longlong), _I]),
     "ttdqn_last_error": (C.c_char_p, []),
     "ttdqn_default_layout": (None, [_LAY]),
     "ttdqn_observe_act_device": (_I, [_LAY, _QN, _I] + [_VP] * 12 + [_VP]),

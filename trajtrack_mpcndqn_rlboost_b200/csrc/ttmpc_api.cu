@@ -157,10 +157,11 @@ struct Slot {
   void *hbuf = nullptr; size_t hbytes = 0;
 };
 constexpr int MAX_STREAM_SLOTS = 16, MAX_HOST_SLOTS = 8;
+constexpr int N_STATS = 4;  // the solve kernel's device counters (ttmpc_read_stats)
 struct Workspace {
   int device = -1;
   int sm_count = 0;
-  unsigned long long *stats = nullptr;  // 24 x u64, shared by every slot (atomics)
+  unsigned long long *stats = nullptr;  // [N_STATS] device counters, shared by every slot (atomics)
   std::vector<Slot *> slots;
 };
 static std::mutex g_mu;
@@ -175,8 +176,8 @@ static int get_ws(Workspace **out) {
   Workspace w;
   w.device = dev;
   CUDA_TRY(cudaDeviceGetAttribute(&w.sm_count, cudaDevAttrMultiProcessorCount, dev));
-  CUDA_TRY(cudaMalloc(&w.stats, 192));
-  CUDA_TRY(cudaMemset(w.stats, 0, 192));
+  CUDA_TRY(cudaMalloc(&w.stats, N_STATS * sizeof(unsigned long long)));
+  CUDA_TRY(cudaMemset(w.stats, 0, N_STATS * sizeof(unsigned long long)));
   g_ws.reserve(16);
   g_ws.push_back(w);
   *out = &g_ws.back();
@@ -410,7 +411,6 @@ static int solve_device_impl(const ttmpc_config *cfg, int n_scenes, const double
   CUDA_TRY(cudaMemsetAsync(sl->work_counter, 0, sizeof(int), st));
   const char *nh = std::getenv("TTMPC_NO_HELPERS");
   SolveArgs A;
-  A.eprof = w->stats + 8;  // stats block is 24 x u64: [0..7] counters, [8..17] eval sections
   A.helpers = (nh && nh[0] == '1') ? 0 : 1;  // TTMPC_NO_HELPERS=1 disables the tail helpers
   A.ready = d_ready; A.timeout_flag = d_ready ? sl->ready + 1 : nullptr;
   A.p = d_p; A.c0 = d_c0; A.u = res->u; A.y = res->y; A.cost = res->cost;
@@ -498,21 +498,17 @@ extern "C" int ttmpc_fleet_step_device(const ttmpc_config *cfg, const ttmpc_flee
 
 // Cumulative device-side counters since the last reset:
 // [0] cost-only evaluations [1] cost+gradient evaluations [2] dynamic-obstacle
-// bodies executed [3] PANOC iterations; the TTMPC_PROFILE builds fill the rest of the
-// 24 counters.  Reads the first `count`, resets all 24.  Synchronises the device.
-static int read_stats(unsigned long long *out, int count, int reset) {
+// bodies executed [3] PANOC iterations.  Synchronises the device.
+extern "C" int ttmpc_read_stats(unsigned long long out[N_STATS], int reset) {
   std::lock_guard<std::mutex> lk(g_mu);
   Workspace *w;
   int rc = get_ws(&w);
   if (rc) return rc;
   CUDA_TRY(cudaDeviceSynchronize());
-  CUDA_TRY(cudaMemcpy(out, w->stats, count * sizeof(unsigned long long), cudaMemcpyDeviceToHost));
-  if (reset) CUDA_TRY(cudaMemset(w->stats, 0, 192));
+  CUDA_TRY(cudaMemcpy(out, w->stats, N_STATS * sizeof(unsigned long long), cudaMemcpyDeviceToHost));
+  if (reset) CUDA_TRY(cudaMemset(w->stats, 0, N_STATS * sizeof(unsigned long long)));
   return TTMPC_OK;
 }
-extern "C" int ttmpc_read_stats(unsigned long long out[4], int reset) { return read_stats(out, 4, reset); }
-extern "C" int ttmpc_read_stats8(unsigned long long out[8], int reset) { return read_stats(out, 8, reset); }
-extern "C" int ttmpc_read_stats24(unsigned long long out[24], int reset) { return read_stats(out, 24, reset); }
 
 // Launch geometry the solve of an n_scenes batch would use, of the build that would run it (for
 // DESIGN/bench reporting).
@@ -785,24 +781,6 @@ extern "C" int ttmpc_eval_batch_host(const ttmpc_config *cfg, int n, const doubl
   if (h_psi) TRY_OR_CLEAN(cudaMemcpy(h_psi, dpsi, sizeof(double) * nn, cudaMemcpyDeviceToHost));
   if (h_grad) TRY_OR_CLEAN(cudaMemcpy(h_grad, dgrad, sizeof(double) * nn * nu, cudaMemcpyDeviceToHost));
   cleanup();
-  return TTMPC_OK;
-}
-
-// Latency probe (diagnostics): h_p = one scene's parameters (host); out[8] cycles of
-// {cost eval, grad eval, wsum, lbfgs apply (mem pairs), div, sqrt, dfma, checksum}.
-extern "C" int ttmpc_probe_latency(const ttmpc_config *cfg, const double *h_p, long long out[8], int reps) {
-  DevCfg g;
-  int rc = make_devcfg(cfg, &g);
-  if (rc) return rc;
-  double *dp = nullptr, *dyn = nullptr; long long *dout = nullptr;
-  CUDA_TRY(cudaMalloc(&dp, sizeof(double) * g.np));
-  CUDA_TRY(cudaMalloc(&dyn, sizeof(double) * DYN_FIELDS * (g.Ndyn > 0 ? g.Ndyn : 1) * g.N));
-  CUDA_TRY(cudaMalloc(&dout, 64));
-  CUDA_TRY(cudaMemcpy(dp, h_p, sizeof(double) * g.np, cudaMemcpyHostToDevice));
-  CUDA_TRY(launch_probe(g, dp, dyn, dout, reps, 0));
-  CUDA_TRY(cudaDeviceSynchronize());
-  CUDA_TRY(cudaMemcpy(out, dout, 64, cudaMemcpyDeviceToHost));
-  cudaFree(dp); cudaFree(dyn); cudaFree(dout);
   return TTMPC_OK;
 }
 

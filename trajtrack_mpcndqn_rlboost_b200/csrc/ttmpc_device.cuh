@@ -39,10 +39,10 @@ constexpr unsigned FULL = 0xffffffffu;
 constexpr int MAX_MEM = 16;
 constexpr int MAX_EDGE = 8;
 constexpr int DYN_FIELDS = 10;  // per (obstacle, step): see stage_scene
-#ifndef TT_DYN_SLOTS
-#define TT_DYN_SLOTS 1
-#endif
-constexpr int DYN_SLOTS = TT_DYN_SLOTS;  // live dynamic obstacles whose table rows are kept in shared memory
+// live dynamic obstacles whose table rows are kept in shared memory; the rest stay in the warp's global
+// table.  One, not more: each further slot costs 1.6 KB per warp (default shapes), and 12 warps of the
+// rolled build must fit the shared memory of an SM.
+constexpr int DYN_SLOTS = 1;
 
 struct DevCfg {
   int N, Nother, Nstc, ne, nstcobs, Ndyn, mem, max_inner, max_outer;
@@ -307,10 +307,6 @@ struct WarpCtx {
   double akkt_tol, f_final, last_fpr, dy_norm, dy_norm_plus, f2_norm, f2_norm_plus;
   unsigned long long t_start, panoc_iters;
   int inner_count, exit_status, num_outer, scene, in_time;
-#ifdef TTMPC_PROFILE
-  long long prof[8];                 // cycles per phase (diagnostic build only)
-  long long eprof[10];               // cycles per section of eval_psi
-#endif
 };
 
 struct HelpHdr;
@@ -454,10 +450,6 @@ __device__ inline void stage_part1(const DevCfg &g, const WarpSmem &sm, const do
     c->qrpd = q[7]; c->acc_pen = q[8]; c->wacc_pen = q[9];
     c->n_cost = 0; c->n_grad = 0; c->n_body = 0;
     c->lipc = 0.0; c->icm_c = NAN; c->icm = 0.0;  // NaN never compares equal: the first evaluation fills the pair
-#ifdef TTMPC_PROFILE
-    for (int i = 0; i < 8; i++) c->prof[i] = 0;
-    for (int i = 0; i < 10; i++) c->eprof[i] = 0;
-#endif
   }
   // reference-path segments: path_ref has N+1 points, last duplicated (l.190-191)
   const double *r = p + g.off_r;
@@ -600,29 +592,15 @@ __device__ inline void stage_part2(const DevCfg &g, const WarpSmem &sm, const do
 }
 
 // Staging = part 1 + part 2, straight from the scene's row of the parameter block (read once;
-// ~35 us per scene, 1 % of an average solve: measured with -DTTMPC_PROFILE_STAGE, tools/stage_profile.py).
+// ~35 us per scene, 1 % of an average solve: measured in round 1 with a cycle-counting build of the
+// kernel, since removed; DESIGN.md section 6).
 // A cp.async.bulk landing zone in the (then empty) L-BFGS ring was tried and dropped: part 2 is
 // bound by its 300 sincos + 1200 divisions, not by the loads, and its 14.4 KB block does not fit the ring.
 __device__ inline void stage_scene(const DevCfg &g, const WarpSmem &sm, const double *p,
                                    double *dyn_scratch, int lane) {
-#ifdef TTMPC_PROFILE_STAGE
-  const long long td0 = clock64();
-#endif
   stage_part1(g, sm, p, p, dyn_scratch, lane);
-#ifdef TTMPC_PROFILE_STAGE
-  const long long td1 = clock64();
-#endif
   stage_part2(g, sm, p + g.off_od, p + g.off_qdyn, dyn_scratch, lane);
-#ifdef TTMPC_PROFILE_STAGE
-  if (lane == 0) { sm.ctx->prof[4] += td1 - td0; sm.ctx->prof[5] += clock64() - td1; }
-#endif
 }
-
-#ifdef TTMPC_PROFILE
-#define EPROF(slot) { const long long tt_ = clock64(); if (lane == 0 && !Dalt) sm.ctx->eprof[slot] += tt_ - ep_t; ep_t = tt_; }
-#else
-#define EPROF(slot)
-#endif
 
 // ---------------------------------------------------------------- evaluation
 struct EvalOut {
@@ -680,9 +658,6 @@ __device__ __noinline__ EvalOut eval_psi(const DevCfg *gp, unsigned char *smem_b
   const int lk = act ? lane : N - 1;  // table column this lane reads
   const double ts = g.ts;
 
-#ifdef TTMPC_PROFILE
-  long long ep_t = clock64();
-#endif
   // ---- terms of (v, w) alone: speed reference + control action (l.203-204), accelerations and the ALM
   //      distance (l.250-264).  Formed HERE, ahead of the rollout: the kernel runs two warps per scheduler
   //      and its top stall is the fixed-latency dependency wait, and the rollout that follows is one long
@@ -748,7 +723,6 @@ __device__ __noinline__ EvalOut eval_psi(const DevCfg *gp, unsigned char *smem_b
   // every rolled-out position inside the scene's box?  then only the "live" robots / obstacles
   // can contribute (the others are farther than their radius from every point of the box)
   const bool in_box = __all_sync(FULL, fabs(X - cx->x0) < cx->box_half && fabs(Y - cx->y0) < cx->box_half);
-  EPROF(0)
   double cost;               // this lane's share of f
   double gx = 0.0, gy = 0.0; // d psi / d position_{k+1}
   double S_loc = 0.0, gSx = 0.0, gSy = 0.0;
@@ -840,7 +814,6 @@ __device__ __noinline__ EvalOut eval_psi(const DevCfg *gp, unsigned char *smem_b
       gy = cx->qrpd * (2.0 * fma(cs, sd.y, -qy));
     }
   }
-  EPROF(1)
   // ---- speed reference + control action (l.203-204)
   cost += t_vel;
   cost += t_ctl;
@@ -885,7 +858,6 @@ __device__ __noinline__ EvalOut eval_psi(const DevCfg *gp, unsigned char *smem_b
       if (GRAD) { gx = fma(1000.0, fx, gx); gy = fma(1000.0, fy, gy); }
     }
   }
-  EPROF(2)
   // ---- dynamic obstacles (l.225-237): hard penalty D_j and soft cost.
   //      fp32 bounding test from shared memory first; the exact fp64 body (global
   //      table) only runs for pairs that can be non-zero.
@@ -970,7 +942,6 @@ __device__ __noinline__ EvalOut eval_psi(const DevCfg *gp, unsigned char *smem_b
     __syncwarp();
   }
   }  // fleet_todo | dyn_todo
-  EPROF(3)
   // ---- terminal cost (l.242)
   double gt = 0.0;
   // both terminal weights zero (config/mpc_default.yaml): every term below is a signed zero; the block is
@@ -989,7 +960,6 @@ __device__ __noinline__ EvalOut eval_psi(const DevCfg *gp, unsigned char *smem_b
 TT_UNROLL_4
     for (int i = 0; i < Nstc; i++) static_obstacle(i);
   }
-  EPROF(4)
   // ---- accelerations: cost (l.250-264) and the ALM set C = acc bounds
   cost += t_acc;
   // ---- lanes beyond the horizon contribute nothing
@@ -997,7 +967,6 @@ TT_UNROLL_4
     cost = 0.0; gx = 0.0; gy = 0.0; S_loc = 0.0; gSx = 0.0; gSy = 0.0;
     aa = 0.0; aw = 0.0; ea = 0.0; ew = 0.0; alm = 0.0;
   }
-  EPROF(5)
   // ---- static sum: needed before the gradient (weight c * sum F2); zero in most evaluations
   double S = 0.0;
   if (__builtin_expect(__any_sync(FULL, S_loc != 0.0), 0)) S = wsum(S_loc);
@@ -1024,7 +993,6 @@ TT_UNROLL_4
   out.h0 = out.h1 = out.dd = out.g2 = 0.0;
   double ddp = 0.0, g2p = 0.0;
 
-  EPROF(6)
   if (GRAD) {
     double gv = 0.0, gw = 0.0;
     // hard-penalty gradient: c * sum_j F2_j * (grad S + grad D_j)
@@ -1081,12 +1049,10 @@ TT_UNROLL_4
       g2p = pdot(gv, gw, gv, gw);
     }
   }
-  EPROF(7)
   // ---- one batched reduction: f, ALM distance (and the line-search scalars)
   wsum4(cost, alm, ddp, g2p, lane);
   out.f = cost; out.dd = ddp; out.g2 = g2p;
   out.psi = cost + c * alm / 2 + c * f2sq / 2;
-  EPROF(8)
   return out;
 }
 

@@ -17,7 +17,6 @@ struct SolveArgs {
   double *dyn_scratch;  // [total_warps][DYN_FIELDS*Ndyn*N]
   int *work_counter;    // dynamic scene queue
   const int *order;     // optional dispatch order (likely-long scenes first) or null
-  unsigned long long *eprof;  // [10] eval section cycles (diagnostic build) or null
   int helpers;          // 1: warps that run out of scenes help their CTA-mates (tail of a batch)
   int *timeout_flag;    // set to 1 if a wait on `ready` timed out (host then re-runs unstreamed)
   const int *ready;     // optional: number of scenes whose parameters have landed in d_p
@@ -45,8 +44,6 @@ cudaError_t launch_rank_scenes(const DevCfg &g, const double *p, int n, int *scr
 cudaError_t launch_eval(const DevCfg &g, const EvalArgs &A, int grid, cudaStream_t st);
 cudaError_t solve_occupancy(const DevCfg &g, int *blocks_per_sm);
 cudaError_t solve_occupancy_small(const DevCfg &g, int *blocks_per_sm);  // the rolled build
-cudaError_t launch_probe(const DevCfg &g, const double *p, double *dyn, long long *out, int reps,
-                         cudaStream_t st);
 // fleet step (ttmpc_fleet.cu)
 struct FleetDims { int N, np, n_other, n_stc, n_dyn; double ts; };
 // warm_u / warm_exit (both or neither): the previous step's solutions, shifted in place into the

@@ -11,8 +11,6 @@
 // butterfly all-reduces.
 #include "ttmpc_device.cuh"
 #include "ttmpc_launch.cuh"
-#include <algorithm>
-#include <cstdlib>
 #include <map>
 #include <mutex>
 #include <tuple>
@@ -24,7 +22,8 @@
 // places of the loop; the API launches it for batches larger than the resident warps.  Only the
 // solve kernel and its launcher exist in that build, under these names:
 #ifndef TTMPC_MIN_BLOCKS
-// CTAs of TTMPC_MAX_THREADS threads per SM the register budget is sized for.  Unrolled build: 2 of 128
+// CTAs of 128 threads per SM the register budget is sized for (__launch_bounds__ of solve_kernel; the
+// API launches CTAs of 64 threads for the default shapes).  Unrolled build: 2 of 128
 // -> up to 255 registers, 8 resident scenes per SM.  Rolled build (Makefile): 3 of 128 -> 168 registers,
 // 12 resident scenes per SM (six 64-thread CTAs for the default shapes), without spills: the PANOC / ALM state that is read a few times per
 // iteration lives in the warp's shared memory (WarpCtx, the L-BFGS old_state / old_g rows), not in
@@ -35,9 +34,6 @@
 // the same for the run-time-dimension kernel (DimsRuntime), which needs more registers than the
 // specialised shapes: it keeps its 255 registers in both builds
 #define TTMPC_MIN_BLOCKS_RUNTIME TTMPC_MIN_BLOCKS
-#endif
-#ifndef TTMPC_MAX_THREADS
-#define TTMPC_MAX_THREADS 128  // CTA size the register budget is computed for (the API launches 64)
 #endif
 #ifdef TTMPC_SMALL_CODE
 #define solve_kernel solve_kernel_small
@@ -208,14 +204,6 @@ __device__ __forceinline__ unsigned long long globaltimer_ns() {
   return t;
 }
 
-#ifdef TTMPC_PROFILE
-#define PROF_BEGIN(v) const long long v = clock64();
-#define PROF_END(v, slot) if (lane == 0) sm.ctx->prof[slot] += clock64() - v;
-#else
-#define PROF_BEGIN(v)
-#define PROF_END(v, slot)
-#endif
-
 // ---------------------------------------------------------------- tail helpers
 // When the scene queue is empty, warps without work help the CTA-mates that still own a
 // long-running scene: the owner posts evaluation points into a mailbox, the helper evaluates
@@ -310,10 +298,8 @@ struct Problem {  // what eval needs besides the point
 template <class DM>
 __device__ __forceinline__ double eval_cost(const DevCfg &g, const WarpSmem &sm, int lane,
                                             const Problem &pb, double a0, double a1, HelpCtl &hc) {
-  PROF_BEGIN(t0)
   EvalOut e = eval_psi<DM>(&g, reinterpret_cast<unsigned char *>(sm.ctx), a0, a1, pb.c, pb.ya,
                            pb.yw, nullptr, false, 0.0);
-  PROF_END(t0, 0)
   if (lane == 0) sm.ctx->n_cost++;
   return e.psi;
 }
@@ -321,10 +307,8 @@ template <class DM>
 __device__ __forceinline__ double eval_grad(const DevCfg &g, const WarpSmem &sm, int lane,
                                             const Problem &pb, double a0, double a1, double &o0,
                                             double &o1, HelpCtl &hc) {
-  PROF_BEGIN(t0)
   EvalOut e = eval_psi<DM>(&g, reinterpret_cast<unsigned char *>(sm.ctx), a0, a1, pb.c, pb.ya, pb.yw,
                            nullptr, true, 0.0);
-  PROF_END(t0, 1)
   if (lane == 0) sm.ctx->n_grad++;
   o0 = e.gv; o1 = e.gw;
   return e.psi;
@@ -485,7 +469,6 @@ __device__ __forceinline__ void halve_tau(Uni &U) {
 template <class DM, bool HELP>
 __device__ __forceinline__ bool panoc_step(const DevCfg &g, const WarpSmem &sm, int lane, const Problem &pb,
                            Lane &z, Uni &U, double tolerance, HelpCtl &hc) {
-  PROF_BEGIN(t_step)
   const bool act = lane < DM::N(g);
   if (U.pc->iteration >= 1 && act) sm.gprev[lane] = make_double2(z.g0, z.g1);
   compute_fpr(z, U);
@@ -509,37 +492,25 @@ __device__ __forceinline__ bool panoc_step(const DevCfg &g, const WarpSmem &sm, 
     bool s_accept = false;
     SpecSave &sv = sm.ctx->spec;
     if (spec) {
-      PROF_BEGIN(tp)
       help_post(hc, sm, lane, DM::N(g), z.h0, z.h1, pb.c, 0, 0.0);
-      PROF_END(tp, 4)  // helper timeline: post
       sv.lb_first = U.pc->lb_first; sv.lb_head = U.pc->lb_head; sv.lb_active = U.pc->lb_active;
       sv.lb_gamma = U.pc->lb_gamma;
     }
 #pragma unroll 1
     for (int pass = 0; pass < 2; pass++) {
       if (pass == 0 ? spec : !lbfgs_done) {
-        PROF_BEGIN(tl)
-        {
-          PROF_BEGIN(t0)
-          const bool acc = lbfgs_update<DM>(g, sm, z, U, lane, pass != 0);
-          if (pass == 0) s_accept = acc;
-          PROF_END(t0, 2)
-        }
+        const bool acc = lbfgs_update<DM>(g, sm, z, U, lane, pass != 0);
+        if (pass == 0) s_accept = acc;
         if (U.pc->iteration > 0) {
-          PROF_BEGIN(t0)
           z.d0 = z.f0; z.d1 = z.f1;
           lbfgs_apply<DM>(g, sm, z, U, lane);
-          PROF_END(t0, 3)
         }
-        if (pass == 0) { PROF_END(tl, 5) }  // speculative L-BFGS
       }
       if (pass == 1) break;
       bool got = false;
       if (spec) {
         EvalOut r;
-        PROF_BEGIN(tw)
         got = hc.pending && help_wait(hc, sm, lane, DM::N(g), r);
-        PROF_END(tw, 6)  // waiting for the helper's psi(u_half)
         if (got) {
           cost_half = r.psi;
           if (lane == 0) sm.ctx->n_cost++;
@@ -607,10 +578,8 @@ __device__ __forceinline__ bool panoc_step(const DevCfg &g, const WarpSmem &sm, 
         posted = hc.pending;
       }
       // cost, gradient, gradient step, half step and both envelope scalars in one evaluation
-      PROF_BEGIN(t0)
       EvalOut e = eval_psi<DM>(&g, reinterpret_cast<unsigned char *>(sm.ctx), p0, p1, pb.c,
                                pb.ya, pb.yw, nullptr, true, U.gamma);
-      PROF_END(t0, 1)
       if (lane == 0) sm.ctx->n_grad++;
       U.cost = e.psi;
       z.g0 = e.gv; z.g1 = e.gw; z.h0 = e.h0; z.h1 = e.h1;
@@ -637,7 +606,6 @@ __device__ __forceinline__ bool panoc_step(const DevCfg &g, const WarpSmem &sm, 
     __syncwarp();
     U.pc->iteration = it1;
   }
-  PROF_END(t_step, 7)  // whole step
   return true;
 }
 
@@ -657,9 +625,6 @@ __device__ void solve_scene(const DevCfg &g, const WarpSmem &sm, const SolveArgs
   const bool act = lane < N;
   WarpCtx *const cx = sm.ctx;
   cx->t_start = __shfl_sync(FULL, globaltimer_ns(), 0);
-#ifdef TTMPC_PROFILE
-  const long long t_clk0 = clock64();
-#endif
   Lane z;
   Uni U;
   U.pc = &cx->pc;
@@ -859,31 +824,12 @@ __device__ void solve_scene(const DevCfg &g, const WarpSmem &sm, const SolveArgs
       atomicAdd(A.stats + 1, (unsigned long long)sm.ctx->n_grad);
       atomicAdd(A.stats + 2, (unsigned long long)sm.ctx->n_body);
       atomicAdd(A.stats + 3, cx->panoc_iters);
-#ifdef TTMPC_PROFILE
-      // 4: cost evals, 5: grad evals, 6: lbfgs update + apply, 7: whole solve (cycles)
-      atomicAdd(A.stats + 4, (unsigned long long)sm.ctx->prof[0]);
-      atomicAdd(A.stats + 5, (unsigned long long)sm.ctx->prof[1]);
-      atomicAdd(A.stats + 6, (unsigned long long)(sm.ctx->prof[2] + sm.ctx->prof[3]));
-      atomicAdd(A.stats + 7, (unsigned long long)(clock64() - t_clk0));
-#endif
     }
-#ifdef TTMPC_PROFILE
-#ifndef TTMPC_PROFILE_STAGE
-    sm.ctx->eprof[9] = sm.ctx->prof[3];  // L-BFGS apply alone (slot 6 holds update + apply)
-#else
-    sm.ctx->eprof[9] = 0;
-    sm.ctx->eprof[8] = sm.ctx->prof[4]; sm.ctx->eprof[7] = sm.ctx->prof[5];  // staging part 1 / part 2
-#endif
-#ifdef TTMPC_PROFILE_HELP
-    for (int i = 0; i < 4; i++) sm.ctx->eprof[i] = sm.ctx->prof[4 + i];  // helper timeline instead of eval sections
-#endif
-    if (A.eprof) for (int i = 0; i < 10; i++) atomicAdd(A.eprof + i, (unsigned long long)sm.ctx->eprof[i]);
-#endif
   }
 }
 
 template <class DM>
-__global__ void __launch_bounds__(TTMPC_MAX_THREADS, DM::kN ? TTMPC_MIN_BLOCKS : TTMPC_MIN_BLOCKS_RUNTIME) solve_kernel(const __grid_constant__ DevCfg g,
+__global__ void __launch_bounds__(128, DM::kN ? TTMPC_MIN_BLOCKS : TTMPC_MIN_BLOCKS_RUNTIME) solve_kernel(const __grid_constant__ DevCfg g,
                                                     const __grid_constant__ SolveArgs A) {
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
   const WarpSmem sm = carve<DM>(warp_region(g, warp), g);
@@ -949,16 +895,10 @@ __global__ void __launch_bounds__(TTMPC_MAX_THREADS, DM::kN ? TTMPC_MIN_BLOCKS :
       }
       __threadfence();
     }
-#ifdef TTMPC_PROFILE_STAGE
-    const long long t_stage0 = clock64();
-#endif
     {
       const int gwarp = blockIdx.x * g.warps_per_block + warp;
       stage_scene(g, sm, A.p + (size_t)scene * g.np, A.dyn_scratch + (size_t)gwarp * DYN_FIELDS * g.Ndyn * g.N, lane);
     }
-#ifdef TTMPC_PROFILE_STAGE
-    if (lane == 0 && A.eprof) atomicAdd(A.eprof + 9, (unsigned long long)(clock64() - t_stage0));  // staging cycles (slot of the apply timer)
-#endif
     hc.enabled = A.helpers != 0 && !hc.timed_out;
     solve_scene<DM>(g, sm, A, scene, lane, hc);
     if (lane == 0) {
@@ -1068,69 +1008,6 @@ __global__ void __launch_bounds__(128) eval_kernel(const __grid_constant__ DevCf
       if (A.psi) A.psi[scene] = e.psi;
     }
     __syncwarp();
-  }
-}
-
-// ------------------------------------------------------------------ latency probe (diagnostics)
-// One warp, one scene: cycles of a cost-only eval, a gradient eval, a butterfly sum, a
-// 10-pair L-BFGS apply and a double division, each averaged over `reps` back-to-back calls.
-template <class DM>
-__global__ void __launch_bounds__(128, 3) probe_kernel(const __grid_constant__ DevCfg g, const double *p,
-                                                       double *dyn, long long *out, int reps,
-                                                       int warps) {
-  // `warps` warps of every CTA run the same measurement on their own copy of the scene
-  // (grid x warps > 1 shows how the latencies change when the SM is shared); block 0 /
-  // warp 0 reports
-  extern __shared__ __align__(16) unsigned char smem_all[];
-  const int lane = threadIdx.x & 31, warp_id = threadIdx.x >> 5;
-  if (warp_id >= warps) return;
-  unsigned char *smem_raw = smem_all + (size_t)warp_id * g.smem_per_warp;
-  const WarpSmem sm = carve<DM>(smem_raw, g);
-  stage_scene(g, sm, p, dyn, lane);
-  {  // desynchronise the warps
-    const long long until = clock64() + ((blockIdx.x * 4 + warp_id) * 7919) % 9000;
-    while (clock64() < until) {}
-  }
-  double v = lane < g.N ? 0.8 : 0.0, w = lane < g.N ? 0.05 : 0.0, acc = 0.0;
-  long long t0 = clock64();
-  for (int i = 0; i < reps; i++) {
-    EvalOut e = eval_psi<DM>(&g, smem_raw, v, w, 10.0, 0.0, 0.0, nullptr, false, 0.0);
-    v += 1e-9 * e.psi * 0.0 + 1e-12;
-    acc += e.psi;
-  }
-  long long t1 = clock64();
-  for (int i = 0; i < reps; i++) {
-    EvalOut e = eval_psi<DM>(&g, smem_raw, v, w, 10.0, 0.0, 0.0, nullptr, true, 1e-3);
-    v += e.gv * 1e-300; w += e.gw * 1e-300;
-    acc += e.psi;
-  }
-  long long t2 = clock64();
-  for (int i = 0; i < reps; i++) acc = wsum(acc * 1e-3 + v);
-  long long t3 = clock64();
-  Lane z; Uni U;
-  U.pc = &sm.ctx->pc;
-  z.d0 = v; z.d1 = w; U.pc->lb_active = g.mem; U.pc->lb_head = 0; U.pc->lb_gamma = 0.7;
-  if (lane < g.N)
-    for (int k = 0; k <= g.mem; k++) {
-      sm.lbs[k * g.N + lane] = make_double2(0.01 * (k + 1), 0.02);
-      sm.lby[k * g.N + lane] = make_double2(0.03, 0.01 * (k + 2));
-    }
-  if (lane <= g.mem) sm.rho[lane] = 0.5;
-  __syncwarp();
-  for (int i = 0; i < reps; i++) { lbfgs_apply<DM>(g, sm, z, U, lane); z.d0 *= 1e-3; z.d1 *= 1e-3; }
-  long long t4 = clock64();
-  double d = 1.0 + acc * 1e-30;
-  for (int i = 0; i < reps; i++) d = 1.0 / (d + 0.5);
-  long long t5 = clock64();
-  for (int i = 0; i < reps; i++) d = sqrt(d + 0.5);
-  long long t6 = clock64();
-  double f = d;
-  for (int i = 0; i < reps; i++) f = fma(f, 0.999, 1e-3);
-  long long t7 = clock64();
-  if (lane == 0 && blockIdx.x == 0 && warp_id == 0) {
-    out[0] = (t1 - t0) / reps; out[1] = (t2 - t1) / reps; out[2] = (t3 - t2) / reps;
-    out[3] = (t4 - t3) / reps; out[4] = (t5 - t4) / reps; out[5] = (t6 - t5) / reps;
-    out[6] = (t7 - t6) / reps; out[7] = (long long)(acc + z.d0 + d + f);
   }
 }
 
@@ -1256,22 +1133,6 @@ cudaError_t launch_eval(const DevCfg &g, const EvalArgs &A, int grid, cudaStream
   } else {
     if ((e = set_smem(eval_kernel<DimsRuntime>, smem)) != cudaSuccess) return e;
     eval_kernel<DimsRuntime><<<grid, g.warps_per_block * 32, smem, st>>>(g, A);
-  }
-  return cudaGetLastError();
-}
-cudaError_t launch_probe(const DevCfg &g, const double *p, double *dyn, long long *out, int reps,
-                         cudaStream_t st) {
-  const size_t smem = (size_t)g.smem_per_warp * g.warps_per_block;
-  cudaError_t e;
-  int grid = 1, warps = 1;  // diagnostics: TTMPC_PROBE_GRID x TTMPC_PROBE_WARPS warps run the probe together
-  if (const char *s = std::getenv("TTMPC_PROBE_GRID")) grid = std::max(1, std::atoi(s));
-  if (const char *s = std::getenv("TTMPC_PROBE_WARPS")) warps = std::min(std::max(1, std::atoi(s)), g.warps_per_block);
-  if (is_default_dims(g)) {
-    if ((e = set_smem(probe_kernel<DimsDefault>, smem)) != cudaSuccess) return e;
-    probe_kernel<DimsDefault><<<grid, 128, smem, st>>>(g, p, dyn, out, reps, warps);
-  } else {
-    if ((e = set_smem(probe_kernel<DimsRuntime>, smem)) != cudaSuccess) return e;
-    probe_kernel<DimsRuntime><<<grid, 128, smem, st>>>(g, p, dyn, out, reps, warps);
   }
   return cudaGetLastError();
 }
