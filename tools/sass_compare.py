@@ -1,8 +1,9 @@
 #!/usr/bin/env python
-"""Kernel-by-kernel SASS comparison of two builds of the same object:
-    tools/sass_compare.py [--mask-params] <a.o> <b.o>
+"""Kernel-by-kernel SASS comparison of two builds of the same object or library:
+    tools/sass_compare.py [--mask-params] <a.o|a.so> <b.o|b.so>
 cuobjdump prints each __global__ function (with its inlined copies of the __noinline__ helpers) as a
 section of its own; addresses and encodings are dropped, the rest is compared section by section.
+Kernels are matched by name, so two libraries linked from different sets of objects compare too.
 Under the arithmetic contract (ttmpc_device.cuh) a refactor that leaves a kernel byte-identical here
 cannot have changed its results.  --mask-params masks constant-bank-0 operands (c[0x0][...]: the kernel
 parameters), for a change that only moves a field of an argument struct.  Exit status 1 when any kernel
@@ -22,6 +23,8 @@ def kernels(obj):
         m = re.match(r"\s+Function : (\S+)", line)
         if m:
             cur = d.setdefault(m.group(1), [])
+        elif line.startswith("Fatbin"):  # header of the next cubin (source file name): no function's code
+            cur = None
         elif cur is not None:
             s = re.sub(r"/\*[0-9a-f]{4,}\*/|/\* 0x[0-9a-f]+ \*/", "", line).strip()
             if MASK_PARAMS:

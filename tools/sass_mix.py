@@ -25,7 +25,8 @@ subprocess.run(["cuobjdump", "-xelf", "all", os.path.abspath(obj)], cwd=d, captu
 cub = [f for f in os.listdir(d) if f.endswith(".cubin")][0]
 dis = subprocess.run(["nvdisasm", "-g", "-c", os.path.join(d, cub)], capture_output=True, text=True).stdout.split("\n")
 key = re.sub(r"[^0-9]", " ", kernel.split("Dims<")[1].split(">")[0]).split()          # template arguments of the captured kernel
-sec = "Dims" + "".join("ILi%sE" % key[0] if i == 0 else "Li%sE" % k for i, k in enumerate(key))
+name = re.findall(r"\w+", kernel.split("<")[0])[-1]                                       # solve_kernel or solve_kernel_small
+sec = "%d%sINS_4Dims" % (len(name), name) + "".join("ILi%sE" % key[0] if i == 0 else "Li%sE" % k for i, k in enumerate(key))
 start = [i for i, l in enumerate(dis) if l.startswith(".text.") and sec in l][0]
 func = "kernel body"; fn_of = {}
 for l in dis[start + 1:]:

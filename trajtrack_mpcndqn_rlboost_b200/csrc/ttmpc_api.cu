@@ -332,17 +332,17 @@ static int grid_for_occupancy(Workspace *w, const DevCfg &g, int n_scenes, int b
 }
 static int grid_for(Workspace *w, const DevCfg &g, int n_scenes, int *grid) {
   int bps = 0;
-  CUDA_TRY(solve_occupancy(g, &bps));
+  CUDA_TRY(solve_occupancy(g, false, &bps));
   return grid_for_occupancy(w, g, n_scenes, bps, grid);
 }
-// Two builds of the solve kernel, bit-identical results: unrolled hot loops (255 registers) when every
-// scene has a warp from the start (latency-bound), rolled loops (168 registers, more resident warps:
-// 12 per SM for the default shapes) when the batch queues behind the unrolled build's resident warps.
-// The grid is sized from the occupancy of the build that runs.  TTMPC_CODE=small|unrolled forces one.
+// Two variants of the solve kernel, bit-identical results: solve_kernel (255 registers) when every
+// scene has a warp from the start (latency-bound), solve_kernel_small (168 registers, more resident
+// warps: 12 per SM for the default shapes) when the batch queues behind solve_kernel's resident warps.
+// The grid is sized from the occupancy of the variant that runs.  TTMPC_CODE=small|unrolled forces one.
 struct SolvePlan { int grid, blocks_per_sm; bool small_code; };
 static int plan_solve(Workspace *w, const DevCfg &g, int n_scenes, SolvePlan *pl) {
   int bps = 0, grid = 0;
-  CUDA_TRY(solve_occupancy(g, &bps));
+  CUDA_TRY(solve_occupancy(g, false, &bps));
   int rc = grid_for_occupancy(w, g, n_scenes, bps, &grid);
   if (rc) return rc;
   bool small_code = n_scenes > (long long)grid * g.warps_per_block;
@@ -351,7 +351,7 @@ static int plan_solve(Workspace *w, const DevCfg &g, int n_scenes, SolvePlan *pl
     else if (e[0] == 'u') small_code = false;
   }
   if (small_code) {
-    CUDA_TRY(solve_occupancy_small(g, &bps));
+    CUDA_TRY(solve_occupancy(g, true, &bps));
     rc = grid_for_occupancy(w, g, n_scenes, bps, &grid);
     if (rc) return rc;
   }
@@ -428,8 +428,7 @@ static int solve_device_impl(const ttmpc_config *cfg, int n_scenes, const double
     CUDA_TRY(launch_rank_scenes(g, d_p, n_scenes, sl->order + n_scenes, sl->order, st));
     A.order = sl->order;
   }
-  if (plan.small_code) CUDA_TRY(launch_solve_small(g, A, plan.grid, st));
-  else CUDA_TRY(launch_solve(g, A, plan.grid, st));
+  CUDA_TRY(launch_solve(g, A, plan.grid, plan.small_code, st));
   return TTMPC_OK;
 }
 

@@ -25,14 +25,6 @@
 
 #include "../../include/ttmpc.h"
 
-// Unroll policy of the hot loops.  The kernel is bound by instruction-cache refills (DESIGN.md
-// section 6), so every unroll factor is a trade between dependent-issue latency and code bytes;
-// -DTTMPC_SMALL_CODE builds the variant with the static-obstacle loop rolled.
-#ifdef TTMPC_SMALL_CODE
-#define TT_UNROLL_4 _Pragma("unroll 1")
-#else
-#define TT_UNROLL_4 _Pragma("unroll 4")
-#endif
 namespace ttmpc {
 
 constexpr unsigned FULL = 0xffffffffu;
@@ -353,6 +345,8 @@ struct Dims {
   // find-first-set / shifts are ~10 instructions each on sm_100)
   using dmask = typename DynMask<(N_ == 0 || ND_ > 32)>::type;
   static constexpr int kN = N_, kNstc = NS_;
+  // unroll factor of the static-obstacle loop in eval_psi (see Rolled)
+  static constexpr int kStaticUnroll = 4;
   __device__ __forceinline__ static int mem(const DevCfg &g) { return N_ ? MEM_ : g.mem; }
   __device__ __forceinline__ static int N(const DevCfg &g) { return N_ ? N_ : g.N; }
   __device__ __forceinline__ static int Nother(const DevCfg &g) { return N_ ? NO_ : g.Nother; }
@@ -362,6 +356,14 @@ struct Dims {
 };
 using DimsRuntime = Dims<0, 0, 0, 0, 0>;
 using DimsDefault = Dims<20, 10, 10, 4, 15, 10>;
+// The same dimensions with the static-obstacle loop rolled: the code of solve_kernel_small.  The
+// kernel is bound by instruction-cache refills (DESIGN.md section 6), so an unroll factor trades
+// dependent-issue latency against code bytes; with 12 warps per SM at different places of the loop,
+// the smaller loop body wins.  Same arithmetic in the same order: bit-identical results.
+template <class DM>
+struct Rolled : DM {
+  static constexpr int kStaticUnroll = 1;
+};
 
 __host__ __device__ inline int smem_bytes_per_warp(int N, int Nother, int Nstc, int nstcobs, int Ndyn,
                                                    int mem) {
@@ -957,7 +959,7 @@ __device__ __noinline__ EvalOut eval_psi(const DevCfg *gp, unsigned char *smem_b
   }
   // ---- static obstacles (l.214-220), in obstacle order like the reference fold
   {
-TT_UNROLL_4
+#pragma unroll(DM::kStaticUnroll)
     for (int i = 0; i < Nstc; i++) static_obstacle(i);
   }
   // ---- accelerations: cost (l.250-264) and the ALM set C = acc bounds

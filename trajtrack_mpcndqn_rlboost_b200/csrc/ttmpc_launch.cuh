@@ -36,14 +36,12 @@ struct EvalArgs {
   int n_scenes;
 };
 
-cudaError_t launch_solve(const DevCfg &g, const SolveArgs &A, int grid, cudaStream_t st);
-// the rolled-loop build of the same kernel (ttmpc_solve_small.cu): bulk batches
-cudaError_t launch_solve_small(const DevCfg &g, const SolveArgs &A, int grid, cudaStream_t st);
+// rolled: solve_kernel_small (bulk batches) instead of solve_kernel, see ttmpc_solve.cu
+cudaError_t launch_solve(const DevCfg &g, const SolveArgs &A, int grid, bool rolled, cudaStream_t st);
 cudaError_t launch_rank_scenes(const DevCfg &g, const double *p, int n, int *scratch, int *order,
                                cudaStream_t st);
 cudaError_t launch_eval(const DevCfg &g, const EvalArgs &A, int grid, cudaStream_t st);
-cudaError_t solve_occupancy(const DevCfg &g, int *blocks_per_sm);
-cudaError_t solve_occupancy_small(const DevCfg &g, int *blocks_per_sm);  // the rolled build
+cudaError_t solve_occupancy(const DevCfg &g, bool rolled, int *blocks_per_sm);
 // fleet step (ttmpc_fleet.cu)
 struct FleetDims { int N, np, n_other, n_stc, n_dyn; double ts; };
 // warm_u / warm_exit (both or neither): the previous step's solutions, shifted in place into the

@@ -15,31 +15,11 @@
 #include <mutex>
 #include <tuple>
 
-// This file is compiled twice (Makefile).  ttmpc_solve.o: hot loops unrolled -- lowest latency of a
-// single scene, ~47 KB of SASS per PANOC iteration.  ttmpc_solve_small.o (ttmpc_solve_small.cu,
-// -DTTMPC_SMALL_CODE): every hot loop rolled -- same arithmetic in the same order, bit-identical
-// results, smaller loop body, better instruction-cache behaviour with 12 warps per SM at different
-// places of the loop; the API launches it for batches larger than the resident warps.  Only the
-// solve kernel and its launcher exist in that build, under these names:
-#ifndef TTMPC_MIN_BLOCKS
-// CTAs of 128 threads per SM the register budget is sized for (__launch_bounds__ of solve_kernel; the
-// API launches CTAs of 64 threads for the default shapes).  Unrolled build: 2 of 128
-// -> up to 255 registers, 8 resident scenes per SM.  Rolled build (Makefile): 3 of 128 -> 168 registers,
-// 12 resident scenes per SM (six 64-thread CTAs for the default shapes), without spills: the PANOC / ALM state that is read a few times per
-// iteration lives in the warp's shared memory (WarpCtx, the L-BFGS old_state / old_g rows), not in
-// registers (DESIGN.md section 3.1).
-#define TTMPC_MIN_BLOCKS 2
-#endif
-#ifndef TTMPC_MIN_BLOCKS_RUNTIME
-// the same for the run-time-dimension kernel (DimsRuntime), which needs more registers than the
-// specialised shapes: it keeps its 255 registers in both builds
-#define TTMPC_MIN_BLOCKS_RUNTIME TTMPC_MIN_BLOCKS
-#endif
-#ifdef TTMPC_SMALL_CODE
-#define solve_kernel solve_kernel_small
-#define launch_solve launch_solve_small
-#define solve_occupancy solve_occupancy_small
-#endif
+// The solve kernel comes in two variants with bit-identical results (solve_main below):
+// solve_kernel, for batches in which every scene has a warp from the start (lowest latency of a single
+// scene), and solve_kernel_small, for batches that queue behind the resident warps (12 scenes per SM).
+// They differ in the register budget of their launch bounds and in the unroll factor of the
+// static-obstacle loop (Rolled in ttmpc_device.cuh).
 
 namespace ttmpc {
 
@@ -829,8 +809,7 @@ __device__ void solve_scene(const DevCfg &g, const WarpSmem &sm, const SolveArgs
 }
 
 template <class DM>
-__global__ void __launch_bounds__(128, DM::kN ? TTMPC_MIN_BLOCKS : TTMPC_MIN_BLOCKS_RUNTIME) solve_kernel(const __grid_constant__ DevCfg g,
-                                                    const __grid_constant__ SolveArgs A) {
+__device__ __forceinline__ void solve_main(const DevCfg &g, const SolveArgs &A) {
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
   const WarpSmem sm = carve<DM>(warp_region(g, warp), g);
   CtaHelp *cta = cta_help();
@@ -914,9 +893,25 @@ __global__ void __launch_bounds__(128, DM::kN ? TTMPC_MIN_BLOCKS : TTMPC_MIN_BLO
   if (A.helpers) helper_loop<DM>(g, A, cta, warp, lane);
 }
 
+// The register budget is set by the CTAs of 128 threads per SM named in __launch_bounds__ (the API
+// launches CTAs of 64 threads for the default shapes).  solve_kernel: 2 -> up to 255 registers,
+// 8 resident scenes per SM, for the latency of a single scene.  solve_kernel_small: 3 -> 168
+// registers, 12 resident scenes per SM (six 64-thread CTAs for the default shapes), without spills:
+// the PANOC / ALM state that is read a few times per iteration lives in the warp's shared memory
+// (WarpCtx, the L-BFGS old_state / old_g rows), not in registers (DESIGN.md section 3.1).  The
+// run-time-dimension kernel (DimsRuntime) needs more registers than the specialised shapes and keeps
+// its 255 in both variants.
+template <class DM>
+__global__ void __launch_bounds__(128, 2) solve_kernel(const __grid_constant__ DevCfg g,
+                                                       const __grid_constant__ SolveArgs A) {
+  solve_main<DM>(g, A);
+}
+template <class DM>
+__global__ void __launch_bounds__(128, DM::kN ? 3 : 2) solve_kernel_small(const __grid_constant__ DevCfg g,
+                                                                          const __grid_constant__ SolveArgs A) {
+  solve_main<Rolled<DM>>(g, A);
+}
 
-
-#ifndef TTMPC_SMALL_CODE  // everything below exists once, in the unrolled build
 // ------------------------------------------------------------------ dispatch order
 // Solve lengths span 50x and a batch ends when its slowest scene does, so scenes that are likely
 // to run long should start first.  A cheap, result-neutral predictor: how many points of the
@@ -1023,7 +1018,6 @@ __global__ void fp64_peak_kernel(double *out, int iters) {
   out[blockIdx.x * blockDim.x + threadIdx.x] = a0 + a1 + a2 + a3 + a4 + a5 + a6 + a7;
 }
 
-#endif  // !TTMPC_SMALL_CODE
 }  // namespace ttmpc
 
 // ------------------------------------------------------------------ launch helpers (host)
@@ -1086,34 +1080,32 @@ static cudaError_t cached_occupancy(K kernel, int block, size_t smem, int *block
   X(32, 10, 10, 4, 15, 10)    \
   X(20, 10, 4, 4, 4, 10)      \
   X(20, 10, 20, 4, 30, 10)
-template <class F>
-static cudaError_t with_solve_dims(const DevCfg &g, F &&f) {
-#define X(n, no, ns, e, nd, m) \
-  if (g.N == n && g.Nother == no && g.Nstc == ns && g.ne == e && g.Ndyn == nd && g.mem == m) return f(Dims<n, no, ns, e, nd, m>{});
+using SolveKernel = void (*)(DevCfg, SolveArgs);
+// the solve kernel for the dimensions of g: solve_kernel_small when `rolled`, else solve_kernel
+static SolveKernel solve_kernel_for(const DevCfg &g, bool rolled) {
+#define X(n, no, ns, e, nd, m)                                                                  \
+  if (g.N == n && g.Nother == no && g.Nstc == ns && g.ne == e && g.Ndyn == nd && g.mem == m) \
+    return rolled ? solve_kernel_small<Dims<n, no, ns, e, nd, m>> : solve_kernel<Dims<n, no, ns, e, nd, m>>;
   TTMPC_SOLVE_SHAPES(X)
 #undef X
-  return f(DimsRuntime{});
+  return rolled ? solve_kernel_small<DimsRuntime> : solve_kernel<DimsRuntime>;
+}
+static size_t solve_smem(const DevCfg &g) {
+  return (size_t)g.smem_per_warp * g.warps_per_block + sizeof(CtaHelp);
 }
 
-cudaError_t launch_solve(const DevCfg &g, const SolveArgs &A, int grid, cudaStream_t st) {
-  const size_t smem = (size_t)g.smem_per_warp * g.warps_per_block + sizeof(CtaHelp);
-  return with_solve_dims(g, [&](auto dm) -> cudaError_t {
-    using DM = decltype(dm);
-    cudaError_t e;
-    if ((e = set_smem(solve_kernel<DM>, smem)) != cudaSuccess) return e;
-    solve_kernel<DM><<<grid, g.warps_per_block * 32, smem, st>>>(g, A);
-    return cudaGetLastError();
-  });
+cudaError_t launch_solve(const DevCfg &g, const SolveArgs &A, int grid, bool rolled, cudaStream_t st) {
+  const SolveKernel kernel = solve_kernel_for(g, rolled);
+  const size_t smem = solve_smem(g);
+  cudaError_t e;
+  if ((e = set_smem(kernel, smem)) != cudaSuccess) return e;
+  kernel<<<grid, g.warps_per_block * 32, smem, st>>>(g, A);
+  return cudaGetLastError();
 }
 // resident blocks per SM of the kernel launch_solve would pick
-cudaError_t solve_occupancy(const DevCfg &g, int *blocks_per_sm) {
-  const size_t smem = (size_t)g.smem_per_warp * g.warps_per_block + sizeof(CtaHelp);
-  return with_solve_dims(g, [&](auto dm) -> cudaError_t {
-    using DM = decltype(dm);
-    return cached_occupancy(solve_kernel<DM>, g.warps_per_block * 32, smem, blocks_per_sm);
-  });
+cudaError_t solve_occupancy(const DevCfg &g, bool rolled, int *blocks_per_sm) {
+  return cached_occupancy(solve_kernel_for(g, rolled), g.warps_per_block * 32, solve_smem(g), blocks_per_sm);
 }
-#ifndef TTMPC_SMALL_CODE
 // scratch: cls[n] | hist[16] | cursor[16]   (ints; hist and cursor zeroed here)
 cudaError_t launch_rank_scenes(const DevCfg &g, const double *p, int n, int *scratch, int *order,
                                cudaStream_t st) {
@@ -1141,5 +1133,4 @@ cudaError_t launch_fp64_peak(double *out, int blocks, int threads, int iters, cu
   return cudaGetLastError();
 }
 
-#endif  // !TTMPC_SMALL_CODE
 }  // namespace ttmpc
