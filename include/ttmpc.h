@@ -256,14 +256,14 @@ int ttdqn_observe_act_host(const ttdqn_scene_layout *lay, const ttdqn_qnet *qnet
  * (src/interface_mpc.py:80-92, src/mpc_traj_tracker/trajectory_generator.py:203-274):
  *
  *   pack    : termination test (check_termination_condition, :158-164), closest point of
- *             the global reference trajectory in the window [idx-1, idx+5) and the N
- *             reference states from there (get_local_ref_traj, :203-230), speed
+ *             the global reference trajectory in the window [idx-k, idx+5k) (k = action_steps)
+ *             and the N reference states from there (get_local_ref_traj, :203-230), speed
  *             reference from the distance to the goal (:248-255), dynamic-obstacle rows
  *             extrapolated from two consecutive positions (main.py:80-89,
  *             est_dyn_obs_positions), and the packed parameter vector in the block
  *             order of :257-260.
  *   solve   : ttmpc_solve_batch_device.
- *   advance : state <- unicycle RK4 step with the first control (run_solver, :291-294;
+ *   advance : state <- unicycle RK4 step with u[k-1] (run_solver, :291-294;
  *             motion_model.py:153-176), last action, solver failure flag
  *             (NotFiniteComputation -> the reference raises), obstacle positions moved by
  *             their per-step displacement.
@@ -280,8 +280,9 @@ enum {
  * pack and advance entry points ignore it).  Other bits -> TTMPC_ERR_BAD_ARG.                  */
 enum {
   /* Start the solve of every robot that is RUNNING after this step's goal test from its previous
-   * solution shifted by one step, u'[k] = u[k+1] for k < N-1 and u'[N-1] = u[N-1], if that
-   * solve's exit status was TTMPC_CONVERGED, and from zeros otherwise (run_step's initial_guess).
+   * solution shifted by the k = action_steps controls it applied, u'[j] = u[j+k] for j < N-k and
+   * u'[j] = u[N-1] otherwise, if that solve's exit status was TTMPC_CONVERGED, and from zeros
+   * otherwise (run_step's initial_guess).
    * The previous step's outputs are read from res->u and res->exit_status, which must therefore
    * hold zeros before the first step.  Multipliers still follow use_y0.                         */
   TTMPC_FLEET_WARM_START = 1,
@@ -304,7 +305,20 @@ typedef struct ttmpc_fleet {
                              shared row block when stc_shared != 0                   */
   int stc_shared;
   int n_dyn_live;   /* moving obstacles described by dyn_cur / dyn_last (<= Ndynobs)  */
-  int action_steps; /* config.action_steps; only 1 is supported                       */
+  /* config.action_steps = k: controls of one solution a robot applies before the next solve.
+   * 1 everywhere; 1..N_hor in ttmpc_fleet_step_device (out of range -> TTMPC_ERR_BAD_ARG; the
+   * pack and advance entry points return TTMPC_ERR_UNSUPPORTED for k != 1).  With k > 1:
+   *  - run_solver computes each of its k taken states from the state the step started in, with
+   *    u[0] .. u[k-1], and continues from the last one; advance therefore takes one RK4 step with
+   *    u[k-1], and last_u becomes u[k-1] (past_actions[-1]), which pack puts into p.  The other
+   *    taken states are not an output: rebuild them from p[0:3] (that state) and res->u.
+   *  - the goal test reads the FIRST control u[0] of the previous solution
+   *    (InterfaceMpc._last_action = actions[0]) from res->u, which must therefore hold zeros
+   *    before the first step, as for TTMPC_FLEET_WARM_START.
+   *  - moving obstacles still move by dyn_disp once per control step, and the dynamic-obstacle
+   *    rows still extrapolate from the positions of two consecutive control steps (main.py:80-89).
+   *  - res->pred_states stays the rollout of u* from p.s.                                       */
+  int action_steps;
   int options;      /* TTMPC_FLEET_* bit mask of the step; C callers must zero it         */
   const double *other;    /* [n][ns*N*Nother] other-robot predictions or NULL (zeros) */
   const double *dyn;      /* [n][Ndynobs*ndynobs*N] ready-made rows or NULL           */
@@ -342,7 +356,7 @@ int ttmpc_fleet_advance_device(const ttmpc_config *cfg, const ttmpc_fleet *fleet
 /* pack + solve + advance, on `stream`.  The solve starts from zeros (run_step with
  * initial_guess=None) unless fleet->options has TTMPC_FLEET_WARM_START, and runs every robot
  * unless it has TTMPC_FLEET_SKIP_STOPPED.  Multipliers are carried in res->y when use_y0 != 0,
- * like the reference's Solver object. */
+ * like the reference's Solver object.  The only entry point that takes action_steps > 1. */
 int ttmpc_fleet_step_device(const ttmpc_config *cfg, const ttmpc_fleet *fleet, double *d_p,
                             int use_y0, const ttmpc_result *res, void *stream);
 

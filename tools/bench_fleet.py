@@ -1,17 +1,22 @@
 #!/usr/bin/env python
 """Closed-loop fleet drive on one GPU, with and without the fleet-step options.
 
-  python tools/bench_fleet.py [n=4096] [max_steps=200]
+  python tools/bench_fleet.py [n=4096] [max_steps=200] [--action-steps k]
 
 Each leg builds the same seeded fleet and calls FleetPlanner.step() -- pack + solve + advance,
 multipliers carried from step to step -- until every robot has stopped or max_steps steps have
 run.  Legs: options off (0), warm start (W), skip stopped robots (S) and both (WS), run
-interleaved as 0 W S WS WS S W 0 so that drift of the card affects every option alike.  Per leg:
-drive time (sum of the per-step event times), step p50 / p90, PANOC iterations (device counters,
-ttmpc_read_stats) and reached / failed / running robots at the end.  The card's name and power
-limit are read in the same run.  Also the CPU oracle (reference order, all host cores) doing one
-plain step on a bounded sample.  Prints one JSON line.
+interleaved as 0 W S WS WS S W 0 so that drift of the card affects every option alike.  Every leg
+runs with the same action_steps k.  Per leg: drive time (sum of the per-step event times), step
+p50 / p90, PANOC iterations (device counters, ttmpc_read_stats), reached / failed / running
+robots at the end, and two rates over the drive time: robot-seconds per wall-second (k * ts of
+robot time for every robot that moved in a step, the time the reference's loop accounts for) and
+metres driven per wall-second (the robots' summed displacement; with k > 1 a step moves a robot by
+one RK4 step with its k-th control, see include/ttmpc.h).  The card's name and power limit are read
+in the same run.  Also the CPU oracle (reference order, all host cores) doing one plain step on a
+bounded sample.  Prints one JSON line.
 """
+import argparse
 import ctypes as C
 import json
 import os
@@ -40,8 +45,8 @@ def card():
     return dict(gpu=torch.cuda.get_device_name(), power_limit=pl or None)
 
 
-def make(n, mc, fl):
-    fp = t.FleetPlanner(mc, fl["init"], fl["goal"], fl["paths"], mode="work")
+def make(n, mc, fl, k):
+    fp = t.FleetPlanner(mc, fl["init"], fl["goal"], fl["paths"], mode="work", action_steps=k)
     fp.update_static_constraints(fl["static_polys"], per_robot=True)
     fp.set_moving_obstacles(fl["moving_pos"], fl["moving_disp"])
     return fp
@@ -51,12 +56,17 @@ def drive(fp, leg, max_steps):
     stats = (C.c_ulonglong * 4)()
     _lib.check(fp.lib.ttmpc_read_stats(stats, 1), "ttmpc_read_stats")
     ev = []
+    moved = torch.zeros((), dtype=torch.int64, device=fp.state.device)     # robots that moved, summed over steps
+    metres = torch.zeros((), dtype=torch.float64, device=fp.state.device)
     for k in range(max_steps):
+        xy = fp.state[:, :2].clone()                                        # outside the timed window
         e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
         e0.record()
         fp.step(warm_start="W" in leg, skip_stopped="S" in leg)
         e1.record()
         ev.append((e0, e1))
+        moved += (fp.status == 0).sum()    # RUNNING after a step = took this step's controls
+        metres += (fp.state[:, :2] - xy).norm(dim=1).sum()
         if k % 5 == 4 and int((fp.status == 0).sum()) == 0:
             break
     torch.cuda.synchronize()
@@ -64,27 +74,35 @@ def drive(fp, leg, max_steps):
     ms = [a.elapsed_time(b) for a, b in ev]
     status = fp.status.cpu().numpy()
     q = lambda p: float(np.quantile(ms, p))
+    drive_s = float(np.sum(ms)) * 1e-3
     return dict(leg=leg, steps=len(ms), drive_ms=float(np.sum(ms)), step_ms_p50=q(0.5), step_ms_p90=q(0.9),
+                robot_s_per_s=int(moved) * fp.action_steps * fp.config.ts / drive_s,
+                metres_per_s=float(metres) / drive_s,
                 panoc_iters=int(stats[3]), reached=int((status == 1).sum()), failed=int((status == 2).sum()),
                 running=int((status == 0).sum()))
 
 
 def main():
-    n = int(sys.argv[1]) if len(sys.argv) > 1 else 4096
-    max_steps = int(sys.argv[2]) if len(sys.argv) > 2 else 200
+    ap = argparse.ArgumentParser()
+    ap.add_argument("n", type=int, nargs="?", default=4096)
+    ap.add_argument("max_steps", type=int, nargs="?", default=200)
+    ap.add_argument("--action-steps", type=int, default=1, help="FleetPlanner(action_steps=k)")
+    a = ap.parse_args()
+    n, max_steps, ks = a.n, a.max_steps, a.action_steps
     mc = t.Configurator()
     fl = t.scenes.make_fleet(n, seed=1000)
-    warm = make(n, mc, fl)      # module loads and first-launch costs stay out of the legs
+    warm = make(n, mc, fl, ks)  # module loads and first-launch costs stay out of the legs
     for _ in range(3):
         warm.step(warm_start=True, skip_stopped=True)
     torch.cuda.synchronize()
-    legs = [drive(make(n, mc, fl), leg, max_steps) for leg in LEGS]
+    legs = [drive(make(n, mc, fl, ks), leg, max_steps) for leg in LEGS]
     mean = {}
     for leg in dict.fromkeys(LEGS):
         rs = [r for r in legs if r["leg"] == leg]
-        mean[leg] = {k: float(np.mean([r[k] for r in rs])) for k in ("drive_ms", "step_ms_p50", "step_ms_p90", "panoc_iters")}
+        mean[leg] = {k: float(np.mean([r[k] for r in rs]))
+                     for k in ("drive_ms", "step_ms_p50", "step_ms_p90", "robot_s_per_s", "metres_per_s", "panoc_iters")}
         mean[leg].update({k: rs[-1][k] for k in ("steps", "reached", "failed", "running")})
-    out = dict(workload=f"fleet{n}", robots=n, max_steps=max_steps, **card(), legs=legs, mean=mean)
+    out = dict(workload=f"fleet{n}", robots=n, max_steps=max_steps, action_steps=ks, **card(), legs=legs, mean=mean)
     # CPU: one plain step with the oracle (reference operation order), bounded sample
     ns = min(n, 256)
     tuning, base = work_mode(mc, "work")

@@ -7,7 +7,7 @@
 all device-resident (ttdqn_internal_obs_device, ttdqn_observe_act_device, ttdqn_rl_ref_device,
 ttmpc_fleet_step_device); whether the hint is used is decided per step and environment by the
 HintSwitcher logic inside the pack kernel.
-  python tools/bench_hybrid.py [n=16384] [steps=10] [--warm-start] [--skip-stopped]
+  python tools/bench_hybrid.py [n=16384] [steps=10] [--warm-start] [--skip-stopped] [--action-steps k]
 """
 import argparse
 import json
@@ -29,11 +29,12 @@ def main():
     ap.add_argument("steps", type=int, nargs="?", default=10)
     ap.add_argument("--warm-start", action="store_true", help="FleetPlanner.step(warm_start=True)")
     ap.add_argument("--skip-stopped", action="store_true", help="FleetPlanner.step(skip_stopped=True)")
+    ap.add_argument("--action-steps", type=int, default=1, help="FleetPlanner(action_steps=k)")
     a = ap.parse_args()
     n, steps = a.n, a.steps
     mc = t.Configurator()
     fl = t.scenes.make_fleet(n, seed=1000)
-    fp = t.FleetPlanner(mc, fl["init"], fl["goal"], fl["paths"], mode="work")
+    fp = t.FleetPlanner(mc, fl["init"], fl["goal"], fl["paths"], mode="work", action_steps=a.action_steps)
     fp.update_static_constraints(fl["static_polys"], per_robot=True)
     fp.set_moving_obstacles(fl["moving_pos"], fl["moving_disp"])
     # lidar geometry: each env's rectangles (padded by the robot radius) + a boundary ring
@@ -84,7 +85,8 @@ def main():
     for _ in range(steps):
         one_step(times)
     tt = np.array(times)
-    res = dict(workload=f"hybrid{n}", envs=n, warm_start=a.warm_start, skip_stopped=a.skip_stopped, steps=steps, step_ms_p50=float(np.median(tt[:, 0])),
+    res = dict(workload=f"hybrid{n}", envs=n, warm_start=a.warm_start, skip_stopped=a.skip_stopped,
+               action_steps=a.action_steps, steps=steps, step_ms_p50=float(np.median(tt[:, 0])),
                step_ms_p90=float(np.quantile(tt[:, 0], 0.9)), dqn_part_ms_p50=float(np.median(tt[:, 1])),
                env_steps_per_s=n / (float(np.median(tt[:, 0])) * 1e-3),
                actions_hist=np.bincount(out["action"].cpu().numpy(), minlength=9).tolist(),

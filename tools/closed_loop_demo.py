@@ -2,7 +2,7 @@
 """Functional check of the whole stack: n robots drive their reference paths to the goal with the
 device-resident fleet loop; reports how many arrive, the closest approach to the static obstacles
 and the tracking error.
-  python tools/closed_loop_demo.py [n=1024] [max_steps=200] [--warm-start] [--skip-stopped]"""
+  python tools/closed_loop_demo.py [n=1024] [max_steps=200] [--warm-start] [--skip-stopped] [--action-steps k]"""
 import argparse
 import json
 import os
@@ -32,11 +32,12 @@ def main():
     ap.add_argument("max_steps", type=int, nargs="?", default=200)
     ap.add_argument("--warm-start", action="store_true", help="FleetPlanner.step(warm_start=True)")
     ap.add_argument("--skip-stopped", action="store_true", help="FleetPlanner.step(skip_stopped=True)")
+    ap.add_argument("--action-steps", type=int, default=1, help="FleetPlanner(action_steps=k)")
     a = ap.parse_args()
     n, max_steps = a.n, a.max_steps
     mc = t.Configurator()
     fl = t.scenes.make_fleet(n, seed=7)
-    fp = t.FleetPlanner(mc, fl["init"], fl["goal"], fl["paths"], mode="work")
+    fp = t.FleetPlanner(mc, fl["init"], fl["goal"], fl["paths"], mode="work", action_steps=a.action_steps)
     fp.update_static_constraints(fl["static_polys"], per_robot=True)
     fp.set_moving_obstacles(fl["moving_pos"], fl["moving_disp"])
     polys = np.array(fl["static_polys"], dtype=np.float64)               # [n][k][4][2]
@@ -55,7 +56,7 @@ def main():
     e1.record(); torch.cuda.synchronize()
     status = fp.status.cpu().numpy(); st = fp.state.cpu().numpy()
     dist_goal = np.hypot(st[:, 0] - fl["goal"][:, 0], st[:, 1] - fl["goal"][:, 1])
-    out = dict(robots=n, warm_start=a.warm_start, skip_stopped=a.skip_stopped, steps=steps, wall_ms=e0.elapsed_time(e1), reached=int((status == 1).sum()),
+    out = dict(robots=n, warm_start=a.warm_start, skip_stopped=a.skip_stopped, action_steps=a.action_steps, steps=steps, wall_ms=e0.elapsed_time(e1), reached=int((status == 1).sum()),
                failed=int((status == 2).sum()), still_running=int((status == 0).sum()),
                dist_to_goal_p50=float(np.median(dist_goal)), dist_to_goal_max=float(dist_goal.max()),
                min_clearance_to_static_obstacles=float(clearance.min()),

@@ -441,7 +441,6 @@ static int fleet_dims(const ttmpc_config *cfg, const ttmpc_fleet *f, FleetDims *
   if (f->n > 0 && (!f->state || !f->goal || !f->last_u || !f->idx_ref || !f->status || !f->ref_traj ||
                    !f->ref_len || !f->stc))
     return fail(TTMPC_ERR_BAD_ARG, "fleet: state, goal, last_u, idx_ref, status, ref_traj, ref_len, stc are required");
-  if (f->action_steps != 1) return fail(TTMPC_ERR_UNSUPPORTED, "fleet: only action_steps = 1 is supported");
   if (f->ref_stride < 1) return fail(TTMPC_ERR_BAD_ARG, "fleet: ref_stride must be >= 1");
   if (f->dyn_cur && (!f->dyn_last || !f->dyn_disp || f->n_dyn_live < 0 || f->n_dyn_live > cfg->Ndynobs))
     return fail(TTMPC_ERR_BAD_ARG, "fleet: dyn_cur needs dyn_last, dyn_disp and 0 <= n_dyn_live <= Ndynobs");
@@ -456,6 +455,8 @@ extern "C" int ttmpc_fleet_pack_device(const ttmpc_config *cfg, const ttmpc_flee
   FleetDims d;
   int rc = fleet_dims(cfg, fleet, &d);
   if (rc) return rc;
+  if (fleet->action_steps != 1)
+    return fail(TTMPC_ERR_UNSUPPORTED, "fleet: action_steps != 1 is only supported by the whole step (ttmpc_fleet_step_device)");
   if (fleet->n == 0) return TTMPC_OK;
   if (!d_p) return fail(TTMPC_ERR_BAD_ARG, "fleet: d_p is required");
   CUDA_TRY(launch_fleet_pack(*fleet, d, d_p, nullptr, nullptr, (cudaStream_t)stream));
@@ -466,6 +467,8 @@ extern "C" int ttmpc_fleet_advance_device(const ttmpc_config *cfg, const ttmpc_f
   FleetDims d;
   int rc = fleet_dims(cfg, fleet, &d);
   if (rc) return rc;
+  if (fleet->action_steps != 1)
+    return fail(TTMPC_ERR_UNSUPPORTED, "fleet: action_steps != 1 is only supported by the whole step (ttmpc_fleet_step_device)");
   if (fleet->n == 0) return TTMPC_OK;
   if (!d_u) return fail(TTMPC_ERR_BAD_ARG, "fleet: d_u is required");
   CUDA_TRY(launch_fleet_advance(*fleet, d, d_u, d_exit_status, (cudaStream_t)stream));
@@ -480,14 +483,18 @@ extern "C" int ttmpc_fleet_step_device(const ttmpc_config *cfg, const ttmpc_flee
   if (rc) return rc;
   if (fleet->options & ~(TTMPC_FLEET_WARM_START | TTMPC_FLEET_SKIP_STOPPED))
     return fail(TTMPC_ERR_BAD_ARG, "fleet: unknown bits in options");
+  if (fleet->action_steps < 1 || fleet->action_steps > cfg->N_hor)
+    return fail(TTMPC_ERR_BAD_ARG, "fleet: action_steps must be in 1..N_hor");
   if (fleet->n == 0) return TTMPC_OK;
   if (!d_p) return fail(TTMPC_ERR_BAD_ARG, "fleet: d_p is required");
   const bool warm = fleet->options & TTMPC_FLEET_WARM_START;
   const bool skip = fleet->options & TTMPC_FLEET_SKIP_STOPPED;
   cudaStream_t st = (cudaStream_t)stream;
   // warm start: the pack kernel shifts res->u of the robots it leaves RUNNING; a zero row there
-  // solves exactly like use_u0 = 0
-  CUDA_TRY(launch_fleet_pack(*fleet, d, d_p, warm ? res->u : nullptr, warm ? res->exit_status : nullptr, st));
+  // solves exactly like use_u0 = 0.  action_steps > 1: its goal test reads the first control of
+  // the previous solution, which res->u still holds.
+  double *prev_u = (warm || fleet->action_steps > 1) ? res->u : nullptr;
+  CUDA_TRY(launch_fleet_pack(*fleet, d, d_p, prev_u, warm ? res->exit_status : nullptr, st));
   rc = solve_device_impl(cfg, fleet->n, d_p, warm ? 1 : 0, use_y0, nullptr, res, st, nullptr, false,
                          skip ? fleet->status : nullptr);
   if (rc) return rc;

@@ -106,12 +106,14 @@ __device__ int hint_switch(const ttmpc_fleet &f, int e, int N, const double *ref
 
 // One CTA per robot.  Thread 0 does the scalar decisions (closest reference point, goal test,
 // speed reference); all threads then write the packed vector, element o of the row by thread
-// o mod blockDim (coalesced 8-byte stores).  With warm_u (warm start of the fleet step) the CTA of
-// a robot that is RUNNING after the goal test also rewrites its row of warm_u, the initial guess of
-// this step's solve: the previous solution shifted by one step (last control repeated) if that
-// solve converged, zeros otherwise.
+// o mod blockDim (coalesced 8-byte stores).  prev_u holds the previous step's solutions.  With
+// action_steps = k > 1 the goal test reads their first control (InterfaceMpc._last_action =
+// actions[0]) while p packs last_u = u[k-1] (past_actions[-1]); with k = 1 both are last_u.  With
+// warm_exit (warm start of the fleet step) the CTA of a robot that is RUNNING after the goal test
+// also rewrites its row of prev_u, the initial guess of this step's solve: the previous solution
+// shifted by k steps (last control repeated) if that solve converged, zeros otherwise.
 __global__ void __launch_bounds__(128) fleet_pack_kernel(const ttmpc_fleet f, const FleetDims d,
-                                                         double *__restrict__ p_all, double *warm_u,
+                                                         double *__restrict__ p_all, double *prev_u,
                                                          const int *__restrict__ warm_exit) {
   const int e = blockIdx.x;
   if (e >= f.n) return;
@@ -137,9 +139,11 @@ __global__ void __launch_bounds__(128) fleet_pack_kernel(const ttmpc_fleet f, co
       }
       idx = arg;
       f.idx_ref[e] = idx;
-      // check_termination_condition (:158-164): np.allclose(atol=0.05, rtol=0) and |v| < 0.05
+      // check_termination_condition (:158-164): np.allclose(atol=0.05, rtol=0) and |v| < 0.05.
+      // Runs before the warm-start rewrite of the same prev_u row (behind a __syncthreads).
       const bool close = fabs(x - goal[0]) <= 0.05 && fabs(y - goal[1]) <= 0.05;
-      if (close && fabs(lu[0]) < 0.05) f.status[e] = TTMPC_FLEET_REACHED;
+      const double v0 = f.action_steps > 1 ? prev_u[(size_t)e * 2 * N] : lu[0];
+      if (close && fabs(v0) < 0.05) f.status[e] = TTMPC_FLEET_REACHED;
     }
     s_run = f.status[e] == TTMPC_FLEET_RUNNING;
     s_idx = idx;
@@ -180,11 +184,14 @@ __global__ void __launch_bounds__(128) fleet_pack_kernel(const ttmpc_fleet f, co
   }
   if (threadIdx.x == 0) s_hint = (f.hint && f.use_hint && f.use_hint[e]) ? 1 : 0;
   __syncthreads();
-  if (warm_u && s_run) {  // in place: every element is read before any is written
-    double *u = warm_u + (size_t)e * 2 * N;
+  if (warm_exit && s_run) {  // in place: every element is read before any is written
+    double *u = prev_u + (size_t)e * 2 * N;
     const int o = threadIdx.x, nz = 2 * N;  // nz <= 64 < blockDim
     double v = 0.0;
-    if (o < nz && warm_exit[e] == TTMPC_CONVERGED) v = u[o + 2 < nz ? o + 2 : o];
+    if (o < nz && warm_exit[e] == TTMPC_CONVERGED) {  // u'[j] = u[min(j + k, N - 1)]
+      const int src = o + 2 * f.action_steps, last = nz - 2 + (o & 1);
+      v = u[src < last ? src : last];
+    }
     __syncthreads();
     if (o < nz) u[o] = v;
   }
@@ -233,7 +240,10 @@ __global__ void __launch_bounds__(128) fleet_pack_kernel(const ttmpc_fleet f, co
   }
 }
 
-// One thread per robot: obstacles move, RUNNING robots take the first control.
+// One thread per robot: obstacles move (once per control step), RUNNING robots take their step.
+// With action_steps = k, run_solver (trajectory_generator.py:291-294) computes each of its k taken
+// states from the state the step started in, with u[i], and continues from the last one: the new
+// state is one RK4 step with u[k-1], which is also the new last action (past_actions[-1]).
 __global__ void __launch_bounds__(128) fleet_advance_kernel(const ttmpc_fleet f, const FleetDims d,
                                                             const double *__restrict__ u_all,
                                                             const int *__restrict__ exit_status) {
@@ -252,7 +262,8 @@ __global__ void __launch_bounds__(128) fleet_advance_kernel(const ttmpc_fleet f,
   if (exit_status && exit_status[e] == TTMPC_NOT_FINITE) { f.status[e] = TTMPC_FLEET_FAILED; return; }
   const double *u = u_all + (size_t)e * 2 * d.N;
   double *st = f.state + 3 * e;
-  const double v = u[0], w = u[1], ts = d.ts;
+  const int j = 2 * (f.action_steps - 1);
+  const double v = u[j], w = u[j + 1], ts = d.ts;
   // unicycle_model, RK4 branch, in numpy's operation order (motion_model.py:166-174)
   double s, c;
   tt_sincos(st[2], &s, &c);
@@ -270,9 +281,9 @@ __global__ void __launch_bounds__(128) fleet_advance_kernel(const ttmpc_fleet f,
   f.last_u[2 * e] = v; f.last_u[2 * e + 1] = w;
 }
 
-cudaError_t launch_fleet_pack(const ttmpc_fleet &f, const FleetDims &d, double *p, double *warm_u,
+cudaError_t launch_fleet_pack(const ttmpc_fleet &f, const FleetDims &d, double *p, double *prev_u,
                               const int *warm_exit, cudaStream_t st) {
-  fleet_pack_kernel<<<f.n, 128, 0, st>>>(f, d, p, warm_u, warm_exit);
+  fleet_pack_kernel<<<f.n, 128, 0, st>>>(f, d, p, prev_u, warm_exit);
   return cudaGetLastError();
 }
 cudaError_t launch_fleet_advance(const ttmpc_fleet &f, const FleetDims &d, const double *u,

@@ -44,9 +44,10 @@ cudaError_t launch_eval(const DevCfg &g, const EvalArgs &A, int grid, cudaStream
 cudaError_t solve_occupancy(const DevCfg &g, bool rolled, int *blocks_per_sm);
 // fleet step (ttmpc_fleet.cu)
 struct FleetDims { int N, np, n_other, n_stc, n_dyn; double ts; };
-// warm_u / warm_exit (both or neither): the previous step's solutions, shifted in place into the
-// initial guess of every robot that is RUNNING after this step's goal test
-cudaError_t launch_fleet_pack(const ttmpc_fleet &f, const FleetDims &d, double *p, double *warm_u,
+// prev_u: the previous step's solutions, required when warm_exit != null or action_steps > 1
+// (the goal test then reads their first control).  warm_exit != null: warm start -- prev_u is
+// shifted in place into the initial guess of every robot that is RUNNING after the goal test.
+cudaError_t launch_fleet_pack(const ttmpc_fleet &f, const FleetDims &d, double *p, double *prev_u,
                               const int *warm_exit, cudaStream_t st);
 cudaError_t launch_fleet_advance(const ttmpc_fleet &f, const FleetDims &d, const double *u,
                                  const int *exit_status, cudaStream_t st);

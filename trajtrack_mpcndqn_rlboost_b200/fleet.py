@@ -47,7 +47,11 @@ class FleetPlanner:
 
     def __init__(self, config: Configurator, init_states: np.ndarray, goal_states: np.ndarray,
                  ref_paths: Sequence[Sequence], mode: str = "work", device: str = "cuda",
-                 stc_weights: float = 1e3, dyn_weights: float = 1e3, **solver_overrides):
+                 stc_weights: float = 1e3, dyn_weights: float = 1e3, action_steps: int = 1,
+                 **solver_overrides):
+        """action_steps: controls of each solution a robot applies before its next solve
+        (``config.action_steps``; pass it to mirror a configuration).  1..N_hor, checked by the
+        first ``step()``; values other than 1 work only through ``step()``."""
         import torch
         self.torch = torch
         self.config = config
@@ -56,6 +60,7 @@ class FleetPlanner:
         self.n = n = len(ref_paths)
         self.N = config.N_hor
         self.np = self.lib.ttmpc_num_params(C.byref(self.cfg))
+        self.action_steps = int(action_steps)
         self.tuning, self.base_speed = work_mode(config, mode)
         init_states = np.asarray(init_states, dtype=np.float64).reshape(n, 3)
         goal_states = np.asarray(goal_states, dtype=np.float64).reshape(n, 3)
@@ -156,7 +161,7 @@ class FleetPlanner:
         f.idx_ref, f.status = self.idx_ref.data_ptr(), self.status.data_ptr()
         f.ref_traj, f.ref_len = self.ref_traj.data_ptr(), self.ref_len.data_ptr()
         f.stc, f.stc_shared = self.stc.data_ptr(), self.stc_shared
-        f.n_dyn_live, f.action_steps = self.n_dyn_live, 1
+        f.n_dyn_live, f.action_steps = self.n_dyn_live, self.action_steps
         f.other = self.other.data_ptr() if self.other is not None else None
         f.dyn = None
         if self.dyn_cur is not None:
@@ -198,6 +203,12 @@ class FleetPlanner:
         skip_stopped=True solves only the robots that are still RUNNING; the result rows of the
         others keep what their last solve wrote (``TTMPC_FLEET_SKIP_STOPPED``).  Both default to off.
 
+        With ``action_steps = k > 1`` the step does what ``InterfaceMpc`` does with
+        ``config.action_steps = k`` (include/ttmpc.h, ``action_steps``): the state takes one RK4
+        step with u[k-1] from the state the step started in (``run_solver`` computes each taken
+        state from there) and ``last_u`` becomes u[k-1]; the goal test of the next step reads u[0]
+        of this solution.  A warm start shifts by k.  Moving obstacles still move once per step.
+
         ``pred_states`` is the rollout of u* from the state the step STARTED in (p.s), i.e. one step
         earlier than ``TrajectoryGenerator.run_step``'s list, which re-applies u from the post-step
         state (trajectory_generator.py:296-301; ``planner.TrajectoryGenerator`` reproduces that list
@@ -211,11 +222,13 @@ class FleetPlanner:
         self.steps += 1
 
     def pack(self, stream=None):
+        """The pack kernel alone (action_steps = 1 only: raises TtmpcError otherwise)."""
         st = stream if stream is not None else self.torch.cuda.current_stream().cuda_stream
         f = self._fleet_struct()
         _lib.check(self.lib.ttmpc_fleet_pack_device(C.byref(self.cfg), C.byref(f), self.p.data_ptr(), st), "fleet pack")
 
     def advance(self, stream=None):
+        """The advance kernel alone (action_steps = 1 only: raises TtmpcError otherwise)."""
         st = stream if stream is not None else self.torch.cuda.current_stream().cuda_stream
         f = self._fleet_struct()
         _lib.check(self.lib.ttmpc_fleet_advance_device(C.byref(self.cfg), C.byref(f), self.u.data_ptr(),
