@@ -7,10 +7,11 @@ NVFLAGS   := -gencode arch=compute_100a,code=sm_100a -lineinfo -O3 -std=c++17 -f
              -Xcompiler -fPIC -Xcompiler -O2
 LIB       := $(PKG)/libttmpc.so
 ORACLE    := oracle/libttmpc_oracle.so
+TASKS_ORACLE := oracle/libttfleet_tasks_oracle.so
 CU        := $(CSRC)/ttmpc_solve.cu $(CSRC)/ttmpc_api.cu $(CSRC)/ttmpc_fleet.cu $(CSRC)/ttdqn.cu
 HDRS      := include/ttmpc.h $(CSRC)/ttmpc_device.cuh $(CSRC)/ttmpc_launch.cuh
 
-all: $(LIB) $(ORACLE)
+all: $(LIB) $(ORACLE) $(TASKS_ORACLE)
 
 $(CSRC)/%.o: $(CSRC)/%.cu $(HDRS)
 	$(NVCC) $(NVFLAGS) -c $< -o $@
@@ -22,7 +23,10 @@ $(LIB): $(CU:.cu=.o)
 $(ORACLE): oracle/ttmpc_oracle.c oracle/ttdqn_oracle.c oracle/ttfleet_oracle.c oracle/ttmpc_oracle.h include/ttmpc.h
 	$(CC) -O2 -fPIC -shared -ffp-contract=off -Wall -o $@ oracle/ttmpc_oracle.c oracle/ttdqn_oracle.c oracle/ttfleet_oracle.c -lm -lpthread
 
+$(TASKS_ORACLE): oracle/ttfleet_tasks_oracle.c
+	$(CC) -O2 -fPIC -shared -ffp-contract=off -Wall -o $@ $< -lm
+
 clean:
-	rm -f $(CSRC)/*.o $(LIB) $(ORACLE)
+	rm -f $(CSRC)/*.o $(LIB) $(ORACLE) $(TASKS_ORACLE)
 
 .PHONY: all clean

@@ -274,7 +274,9 @@ int ttdqn_observe_act_host(const ttdqn_scene_layout *lay, const ttdqn_qnet *qnet
 enum {
   TTMPC_FLEET_RUNNING = 0,  /* get_action returned an action                      */
   TTMPC_FLEET_REACHED = 1,  /* check_termination_condition: get_action -> None    */
-  TTMPC_FLEET_FAILED = 2    /* solver error (the reference raises RuntimeError)   */
+  TTMPC_FLEET_FAILED = 2,   /* solver error (the reference raises RuntimeError)   */
+  TTMPC_FLEET_BAD_TASK = 3  /* ttmpc_fleet_step_tasks_device: the task taken next cannot be
+                               driven (see ttmpc_fleet_tasks); the robot stops       */
 };
 /* ttmpc_fleet.options: bit mask of opt-in behaviours of ttmpc_fleet_step_device (0 = none; the
  * pack and advance entry points ignore it).  Other bits -> TTMPC_ERR_BAD_ARG.                  */
@@ -295,12 +297,13 @@ typedef struct ttmpc_fleet {
   int n;            /* robots                                                         */
   int ref_stride;   /* rows per robot in ref_traj                                     */
   double *state;    /* [n][3] x y theta, in/out                                       */
-  const double *goal;     /* [n][3]                                                   */
+  const double *goal;     /* [n][3]  (written by ttmpc_fleet_step_tasks_device)        */
   double *last_u;   /* [n][2] last applied action, in/out (zeros before the first)    */
   int *idx_ref;     /* [n] index into the global reference trajectory, in/out         */
   int *status;      /* [n] TTMPC_FLEET_*, in/out (robots not RUNNING are left alone)  */
-  const double *ref_traj; /* [n][ref_stride][3] get_global_ref_traj output            */
-  const int *ref_len;     /* [n] valid rows                                           */
+  const double *ref_traj; /* [n][ref_stride][3] get_global_ref_traj output; written by
+                             ttmpc_fleet_step_tasks_device when a robot takes a task  */
+  const int *ref_len;     /* [n] valid rows (written by ttmpc_fleet_step_tasks_device) */
   const double *stc;      /* static half-space rows: [n][Nstcobs*nstcobs], or one
                              shared row block when stc_shared != 0                   */
   int stc_shared;
@@ -359,6 +362,54 @@ int ttmpc_fleet_advance_device(const ttmpc_config *cfg, const ttmpc_fleet *fleet
  * like the reference's Solver object.  The only entry point that takes action_steps > 1. */
 int ttmpc_fleet_step_device(const ttmpc_config *cfg, const ttmpc_fleet *fleet, double *d_p,
                             int use_y0, const ttmpc_result *res, void *stream);
+
+/* Task queues of ttmpc_fleet_step_tasks_device: robot e has count[e] tasks, a goal [3] and a
+ * polyline path of path_n (1..max_nodes) nodes each; next[e] of them have been taken.  All device
+ * pointers.
+ *
+ * In the pack kernel, after the goal test, a robot that is TTMPC_FLEET_REACHED and has a task left
+ * takes the next one -- a robot that arrived in this step as well as one that was parked before
+ * its tasks were queued -- and does what InterfaceMpc.initialization(state, goal, path, mode)
+ * does with it:
+ *   - goal <- the task's goal; ref_traj / ref_len <- get_global_ref_traj(ts, path, state,
+ *     base_speed) (trajectory_generator.py:160-201), sampled from the robot's current state with
+ *     the device's arithmetic (sqrt(fma(dx,dx,dy*dy)), IEEE division, a 1-ulp atan2): within ulps of
+ *     the Python sampler, not bit for bit;
+ *   - idx_ref <- 0 and last_u <- 0 (past_actions is reset); status <- RUNNING; next[e] += 1;
+ *   - the closest-point search and the goal test run again on the new task, so a robot whose
+ *     consecutive goals lie within the 5 cm goal box takes several tasks in one step.  With
+ *     action_steps = k > 1 the goal test still reads u[0] of the previous solution from res->u
+ *     (InterfaceMpc._last_action, which initialization keeps).
+ * The rest of the step is unchanged: the robot is packed and solved in this step, its multipliers
+ * carry over in res->y (the reference keeps its Solver object), and with TTMPC_FLEET_WARM_START a
+ * robot that took a task in this step starts from zeros (its previous solution tracked another
+ * trajectory).  With the HintSwitcher on, a robot that took a task is switched once, if it is
+ * RUNNING afterwards, on the new task's original local reference.  TTMPC_FLEET_REACHED thus means
+ * that the last queued task is done.
+ *
+ * A task that cannot be driven -- no node, a walk the reference would index past the last node in
+ * (a node it lands on within 1e-9 of the last one), no row or more than ref_stride rows -- sets
+ * status TTMPC_FLEET_BAD_TASK and advances next[e] past it; goal, ref_traj, ref_len, idx_ref and
+ * last_u keep the previous task's values.                                                       */
+typedef struct ttmpc_fleet_tasks {
+  int max_tasks, max_nodes;
+  const int *count;      /* [n] queued tasks, 0..max_tasks                          */
+  int *next;             /* [n] in/out: queued tasks taken so far (zeros at first)  */
+  const double *goal;    /* [n][max_tasks][3]                                       */
+  const double *path_xy; /* [n][max_tasks][max_nodes][2]                            */
+  const int *path_n;     /* [n][max_tasks]                                          */
+  double *path_out;      /* [n][max_nodes][2] or NULL: current path, in the layout  */
+  int *path_out_n;       /* [n]                   ttdqn_internal_obs_device reads   */
+} ttmpc_fleet_tasks;
+/* ttmpc_fleet_step_device with task queues: writes fleet->goal, fleet->ref_traj and fleet->ref_len
+ * of the robots that take a task (and their path_out rows when path_out != NULL).  With every count
+ * zero it computes exactly what ttmpc_fleet_step_device computes.  tasks == NULL, max_tasks < 0,
+ * max_nodes < 1, a NULL array other than path_out / path_out_n with max_tasks > 0, or path_out
+ * without path_out_n -> TTMPC_ERR_BAD_ARG before any device work.  The pack and advance entry
+ * points take no tasks. */
+int ttmpc_fleet_step_tasks_device(const ttmpc_config *cfg, const ttmpc_fleet *fleet,
+                                  const ttmpc_fleet_tasks *tasks, double *d_p, int use_y0,
+                                  const ttmpc_result *res, void *stream);
 
 /* ------------------------------------------------------------------------
  * DQN side of the hybrid loop (src/main.py:174-193), device-resident.

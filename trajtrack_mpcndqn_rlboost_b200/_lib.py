@@ -80,11 +80,21 @@ class TtmpcFleet(C.Structure):
     ]
 
 
+class TtmpcFleetTasks(C.Structure):
+    """struct ttmpc_fleet_tasks: per-robot task queues of ttmpc_fleet_step_tasks_device (device addresses)."""
+    _fields_ = [
+        ("max_tasks", C.c_int), ("max_nodes", C.c_int),
+        ("count", C.c_void_p), ("next", C.c_void_p), ("goal", C.c_void_p), ("path_xy", C.c_void_p),
+        ("path_n", C.c_void_p), ("path_out", C.c_void_p), ("path_out_n", C.c_void_p),
+    ]
+
+
 # every symbol include/ttmpc.h declares, with its signature
 _VP, _I, _D = C.c_void_p, C.c_int, C.c_double
 _CFG, _RES = C.POINTER(TtmpcConfig), C.POINTER(TtmpcResult)
 _LAY, _QN = C.POINTER(TtdqnLayout), C.POINTER(TtdqnQnet)
 _FLT = C.POINTER(TtmpcFleet)
+_TSK = C.POINTER(TtmpcFleetTasks)
 SYMBOLS = {
     "ttmpc_default_config": (None, [_CFG]),
     "ttmpc_num_params": (_I, [_CFG]),
@@ -103,6 +113,7 @@ SYMBOLS = {
     "ttmpc_fleet_pack_device": (_I, [_CFG, _FLT, _VP, _VP]),
     "ttmpc_fleet_advance_device": (_I, [_CFG, _FLT, _VP, _VP, _VP]),
     "ttmpc_fleet_step_device": (_I, [_CFG, _FLT, _VP, _I, _RES, _VP]),
+    "ttmpc_fleet_step_tasks_device": (_I, [_CFG, _FLT, _TSK, _VP, _I, _RES, _VP]),
     "ttmpc_read_stats": (_I, [C.POINTER(C.c_ulonglong), _I]),
     "ttmpc_launch_info": (_I, [_CFG, _I] + [C.POINTER(C.c_int)] * 5),
     "ttmpc_measure_fp64_peak": (_I, [C.POINTER(_D), _VP]),

@@ -459,7 +459,7 @@ extern "C" int ttmpc_fleet_pack_device(const ttmpc_config *cfg, const ttmpc_flee
     return fail(TTMPC_ERR_UNSUPPORTED, "fleet: action_steps != 1 is only supported by the whole step (ttmpc_fleet_step_device)");
   if (fleet->n == 0) return TTMPC_OK;
   if (!d_p) return fail(TTMPC_ERR_BAD_ARG, "fleet: d_p is required");
-  CUDA_TRY(launch_fleet_pack(*fleet, d, d_p, nullptr, nullptr, (cudaStream_t)stream));
+  CUDA_TRY(launch_fleet_pack(*fleet, d, d_p, nullptr, nullptr, nullptr, (cudaStream_t)stream));
   return TTMPC_OK;
 }
 extern "C" int ttmpc_fleet_advance_device(const ttmpc_config *cfg, const ttmpc_fleet *fleet,
@@ -474,8 +474,9 @@ extern "C" int ttmpc_fleet_advance_device(const ttmpc_config *cfg, const ttmpc_f
   CUDA_TRY(launch_fleet_advance(*fleet, d, d_u, d_exit_status, (cudaStream_t)stream));
   return TTMPC_OK;
 }
-extern "C" int ttmpc_fleet_step_device(const ttmpc_config *cfg, const ttmpc_fleet *fleet, double *d_p,
-                                       int use_y0, const ttmpc_result *res, void *stream) {
+// ttmpc_fleet_step_device and ttmpc_fleet_step_tasks_device; tasks == nullptr: no queues
+static int fleet_step(const ttmpc_config *cfg, const ttmpc_fleet *fleet, const ttmpc_fleet_tasks *tasks,
+                      double *d_p, int use_y0, const ttmpc_result *res, void *stream) {
   if (!res || !res->u || !res->exit_status)
     return fail(TTMPC_ERR_BAD_ARG, "fleet: res->u and res->exit_status are required");
   FleetDims d;
@@ -494,12 +495,27 @@ extern "C" int ttmpc_fleet_step_device(const ttmpc_config *cfg, const ttmpc_flee
   // solves exactly like use_u0 = 0.  action_steps > 1: its goal test reads the first control of
   // the previous solution, which res->u still holds.
   double *prev_u = (warm || fleet->action_steps > 1) ? res->u : nullptr;
-  CUDA_TRY(launch_fleet_pack(*fleet, d, d_p, prev_u, warm ? res->exit_status : nullptr, st));
+  CUDA_TRY(launch_fleet_pack(*fleet, d, d_p, prev_u, warm ? res->exit_status : nullptr, tasks, st));
   rc = solve_device_impl(cfg, fleet->n, d_p, warm ? 1 : 0, use_y0, nullptr, res, st, nullptr, false,
                          skip ? fleet->status : nullptr);
   if (rc) return rc;
   CUDA_TRY(launch_fleet_advance(*fleet, d, res->u, res->exit_status, st));
   return TTMPC_OK;
+}
+extern "C" int ttmpc_fleet_step_device(const ttmpc_config *cfg, const ttmpc_fleet *fleet, double *d_p,
+                                       int use_y0, const ttmpc_result *res, void *stream) {
+  return fleet_step(cfg, fleet, nullptr, d_p, use_y0, res, stream);
+}
+extern "C" int ttmpc_fleet_step_tasks_device(const ttmpc_config *cfg, const ttmpc_fleet *fleet,
+                                             const ttmpc_fleet_tasks *tasks, double *d_p, int use_y0,
+                                             const ttmpc_result *res, void *stream) {
+  if (!tasks || tasks->max_tasks < 0 || tasks->max_nodes < 1)
+    return fail(TTMPC_ERR_BAD_ARG, "fleet tasks: null, max_tasks < 0 or max_nodes < 1");
+  if (tasks->max_tasks > 0 && (!tasks->count || !tasks->next || !tasks->goal || !tasks->path_xy || !tasks->path_n))
+    return fail(TTMPC_ERR_BAD_ARG, "fleet tasks: count, next, goal, path_xy and path_n are required");
+  if (tasks->path_out && !tasks->path_out_n)
+    return fail(TTMPC_ERR_BAD_ARG, "fleet tasks: path_out needs path_out_n");
+  return fleet_step(cfg, fleet, tasks, d_p, use_y0, res, stream);
 }
 
 // Cumulative device-side counters since the last reset:

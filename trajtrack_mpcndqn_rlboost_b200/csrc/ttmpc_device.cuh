@@ -77,6 +77,57 @@ __host__ __device__ __forceinline__ void tt_sincos(double x, double *s, double *
   *s = so; *c = co;
 }
 
+// ---------------------------------------------------------------- atan2
+// fdlibm's __ieee754_atan2 / atan (argument reduction by atan(1/2), atan(1), atan(3/2), atan(inf),
+// 11-term odd minimax polynomial, hi/lo table of atan at the reduction points) with Horner in fma
+// and one correction fdlibm lacks: the rounding error of y/x, fma(-t, x, y) / x, enters through
+// d atan / dt = 1 / (1 + t^2).  <= 1 ulp.  CUDA's atan2 and glibc's differ from each other in the
+// last bit; this one is the same function on the device and in the CPU oracle (ttmpc_oracle_atan2).
+__host__ __device__ __forceinline__ double tt_atan_ratio(double ay, double ax) {  // atan(ay / ax), ay, ax > 0
+  const double t = ay / ax;
+  if (!(t <= 0x1p60)) return 1.57079632679489655800e+00;  // |y/x| > 2^60 (or overflow): pi/2
+  if (t < 0x1p-27) return t;                               // atan(t) = t to the last bit
+  const double e = fma(-t, ax, ay) / ax / fma(t, t, 1.0);  // (y/x - t) / (1 + t^2)
+  double r, hi, lo;
+  int id;
+  if (t < 0.4375) { id = -1; r = t; hi = lo = 0.0; }
+  else if (t < 0.6875) { id = 0; r = (2.0 * t - 1.0) / (2.0 + t); hi = 4.63647609000806093515e-01; lo = 2.26987774529616870924e-17; }
+  else if (t < 1.1875) { id = 1; r = (t - 1.0) / (t + 1.0); hi = 7.85398163397448278999e-01; lo = 3.06161699786838301793e-17; }
+  else if (t < 2.4375) { id = 2; r = (t - 1.5) / fma(1.5, t, 1.0); hi = 9.82793723247329054082e-01; lo = 1.39033110312309984516e-17; }
+  else { id = 3; r = -1.0 / t; hi = 1.57079632679489655800e+00; lo = 6.12323399573676603587e-17; }
+  const double z = r * r, w = z * z;
+  double s1 = fma(w, 1.62858201153657823623e-02, 4.97687799461593236017e-02);
+  s1 = fma(w, s1, 6.66107313738753120669e-02);
+  s1 = fma(w, s1, 9.09088713343650656196e-02);
+  s1 = fma(w, s1, 1.42857142725034663711e-01);
+  s1 = fma(w, s1, 3.33333333333329318027e-01);
+  double s2 = fma(w, -3.65315727442169155270e-02, -5.83357013379057348645e-02);
+  s2 = fma(w, s2, -7.69187620504482999495e-02);
+  s2 = fma(w, s2, -1.11111104054623557880e-01);
+  s2 = fma(w, s2, -1.99999999998764832476e-01);
+  const double s = fma(z, s1, w * s2);
+  if (id < 0) return r - fma(r, s, -e);
+  return hi - ((fma(r, s, -lo) - r) - e);
+}
+__host__ __device__ __forceinline__ double tt_atan2(double y, double x) {
+  const double pi = 3.1415926535897931160e+00, pi_lo = 1.2246467991473531772e-16;
+  if (x != x || y != y) return x + y;
+  const double ax = fabs(x), ay = fabs(y);
+  const bool xneg = signbit(x);
+  double z;
+  if (ay == 0.0) z = xneg ? pi : 0.0;                             // atan2(+-0, x)
+  else if (ax == INFINITY) {
+    if (ay == INFINITY) z = xneg ? 2.35619449019234483700e+00 : 7.85398163397448278999e-01;
+    else z = xneg ? pi : 0.0;
+  }
+  else if (ax == 0.0 || ay == INFINITY) z = 1.57079632679489655800e+00;
+  else {
+    z = tt_atan_ratio(ay, ax);
+    if (xneg) z = pi - (z - pi_lo);
+  }
+  return copysign(z, y);
+}
+
 // Same function for the hot path (eval_psi): the coefficients come from the constant bank, so
 // every DFMA takes its constant as an operand.  With literals ptxas materialises each 64-bit
 // constant with two UMOVs -- 28 of the 85 instructions of one inlined tt_sincos, three of them per

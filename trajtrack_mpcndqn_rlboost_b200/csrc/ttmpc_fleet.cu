@@ -104,6 +104,54 @@ __device__ int hint_switch(const ttmpc_fleet &f, int e, int N, const double *ref
   return st[0];
 }
 
+// get_global_ref_traj (trajectory_generator.py:160-201) of a queued task from (px, py): rows
+// (x, y, heading) into out (nullptr: count only).  Returns the row count, or -1 for a task that
+// cannot be driven: no node, a walk that would index past the last node (the reference raises),
+// no row, or more than cap rows.  Python's operation order; oracle: ttfleet_oracle_global_ref_traj.
+__device__ int global_ref_walk(const double *path, int n_nodes, double px, double py, double ts, double speed,
+                               int cap, double *out) {
+  if (n_nodes < 1) return -1;
+  double tx = path[0], ty = path[1], ux = 0.0, uy = 0.0, gap = 0.0;
+  int k = 0, rows = 0;
+  bool alive = true;
+  while (alive) {
+    for (;;) {
+      gap = hyp2(tx - px, ty - py);
+      if (gap < 1e-9) {
+        k += 1;
+        if (k > n_nodes - 1) return -1;
+        tx = path[2 * k]; ty = path[2 * k + 1];
+        break;
+      }
+      ux = (tx - px) / gap; uy = (ty - py) / gap;
+      const double eta = gap / speed;
+      if (eta > ts) { px = px + ux * speed * ts; py = py + uy * speed * ts; break; }
+      px = px + ux * speed * eta; py = py + uy * speed * eta;
+      k += 1;
+      if (k > n_nodes - 1) { alive = false; break; }
+      tx = path[2 * k]; ty = path[2 * k + 1];
+    }
+    if (!(gap < 1e-9)) {
+      if (rows >= cap) return -1;  // also bounds the walk
+      if (out) { out[3 * rows] = px; out[3 * rows + 1] = py; out[3 * rows + 2] = tt_atan2(uy, ux); }
+      rows++;
+    }
+  }
+  return rows > 0 ? rows : -1;
+}
+
+// get_local_ref_traj (trajectory_generator.py:214-219): first minimum in the window [idx-k, idx+5k)
+__device__ __forceinline__ int local_ref_idx(const double *ref, int L, int idx, int k, double x, double y) {
+  int lo = idx - 1 * k; if (lo < 0) lo = 0;
+  int hi = idx + 5 * k; if (hi > L) hi = L;
+  double best = INFINITY; int arg = lo;
+  for (int i = lo; i < hi; i++) {
+    const double dist = hyp2(x - ref[3 * i], y - ref[3 * i + 1]);
+    if (dist < best) { best = dist; arg = i; }
+  }
+  return arg;
+}
+
 // One CTA per robot.  Thread 0 does the scalar decisions (closest reference point, goal test,
 // speed reference); all threads then write the packed vector, element o of the row by thread
 // o mod blockDim (coalesced 8-byte stores).  prev_u holds the previous step's solutions.  With
@@ -112,42 +160,75 @@ __device__ int hint_switch(const ttmpc_fleet &f, int e, int N, const double *ref
 // warm_exit (warm start of the fleet step) the CTA of a robot that is RUNNING after the goal test
 // also rewrites its row of prev_u, the initial guess of this step's solve: the previous solution
 // shifted by k steps (last control repeated) if that solve converged, zeros otherwise.
+// tk.count != nullptr (ttmpc_fleet_step_tasks_device): after the goal test thread 0 lets a REACHED
+// robot take its next queued task (include/ttmpc.h, ttmpc_fleet_tasks): it samples the task's
+// reference trajectory into the robot's ref_traj rows, sets goal, ref_len, idx_ref, last_u and
+// status, and repeats the search and the goal test on the new task.  The other threads read the
+// new rows and last_u from global memory and the new ref_len from s_len, all behind the barrier.
 __global__ void __launch_bounds__(128) fleet_pack_kernel(const ttmpc_fleet f, const FleetDims d,
                                                          double *__restrict__ p_all, double *prev_u,
-                                                         const int *__restrict__ warm_exit) {
+                                                         const int *__restrict__ warm_exit,
+                                                         const ttmpc_fleet_tasks tk) {
   const int e = blockIdx.x;
   if (e >= f.n) return;
-  __shared__ int s_idx, s_hint, s_sw, s_run;
+  __shared__ int s_idx, s_hint, s_sw, s_run, s_len, s_new;
   __shared__ double s_speed;
   __shared__ double s_dist[SW_MAX_OBS];
   __shared__ unsigned char s_in[32 * SW_MAX_OBS];
   const double *st = f.state + 3 * e, *goal = f.goal + 3 * e, *lu = f.last_u + 2 * e;
   const double *ref = f.ref_traj + (size_t)e * f.ref_stride * 3;
-  const int L = f.ref_len[e], N = d.N;
+  const int N = d.N;
   if (threadIdx.x == 0) {
-    int idx = f.idx_ref[e];
+    int idx = f.idx_ref[e], L = f.ref_len[e];
     const double x = st[0], y = st[1];
     const bool was_running = f.status[e] == TTMPC_FLEET_RUNNING;
+    // check_termination_condition (:158-164): np.allclose(atol=0.05, rtol=0) and |v| < 0.05.
+    // Runs before the warm-start rewrite of the same prev_u row (behind a __syncthreads).
     if (f.status[e] == TTMPC_FLEET_RUNNING) {
-      // get_local_ref_traj (trajectory_generator.py:214-219): first minimum in the window
-      int lo = idx - 1 * f.action_steps; if (lo < 0) lo = 0;
-      int hi = idx + 5 * f.action_steps; if (hi > L) hi = L;
-      double best = INFINITY; int arg = lo;
-      for (int i = lo; i < hi; i++) {
-        const double dist = hyp2(x - ref[3 * i], y - ref[3 * i + 1]);
-        if (dist < best) { best = dist; arg = i; }
-      }
-      idx = arg;
+      idx = local_ref_idx(ref, L, idx, f.action_steps, x, y);
       f.idx_ref[e] = idx;
-      // check_termination_condition (:158-164): np.allclose(atol=0.05, rtol=0) and |v| < 0.05.
-      // Runs before the warm-start rewrite of the same prev_u row (behind a __syncthreads).
       const bool close = fabs(x - goal[0]) <= 0.05 && fabs(y - goal[1]) <= 0.05;
       const double v0 = f.action_steps > 1 ? prev_u[(size_t)e * 2 * N] : lu[0];
       if (close && fabs(v0) < 0.05) f.status[e] = TTMPC_FLEET_REACHED;
     }
+    bool took = false;
+    if (tk.count) {
+      int next = tk.next[e];
+      const int count = min(tk.count[e], tk.max_tasks);
+      while (f.status[e] == TTMPC_FLEET_REACHED && next < count) {  // InterfaceMpc.initialization
+        const size_t t = (size_t)e * tk.max_tasks + next;
+        const double *path = tk.path_xy + t * tk.max_nodes * 2;
+        const int pn = tk.path_n[t];
+        next += 1;
+        const int rows = pn <= tk.max_nodes ? global_ref_walk(path, pn, x, y, d.ts, f.base_speed, f.ref_stride, nullptr) : -1;
+        if (rows < 0) { f.status[e] = TTMPC_FLEET_BAD_TASK; break; }
+        global_ref_walk(path, pn, x, y, d.ts, f.base_speed, f.ref_stride, const_cast<double *>(ref));
+        L = rows;
+        const_cast<int *>(f.ref_len)[e] = rows;
+        double *g = const_cast<double *>(goal);
+        g[0] = tk.goal[3 * t]; g[1] = tk.goal[3 * t + 1]; g[2] = tk.goal[3 * t + 2];
+        f.last_u[2 * e] = 0.0; f.last_u[2 * e + 1] = 0.0;
+        if (tk.path_out) {
+          for (int i = 0; i < 2 * pn; i++) tk.path_out[(size_t)e * tk.max_nodes * 2 + i] = path[i];
+          tk.path_out_n[e] = pn;
+        }
+        f.status[e] = TTMPC_FLEET_RUNNING;
+        took = true;
+        idx = local_ref_idx(ref, L, 0, f.action_steps, x, y);
+        f.idx_ref[e] = idx;
+        // _last_action is kept: with k > 1 the first control of the previous solution, with k = 1
+        // the last applied control, which passed |v| < 0.05 when the robot stopped
+        const bool close = fabs(x - g[0]) <= 0.05 && fabs(y - g[1]) <= 0.05;
+        const double v0 = f.action_steps > 1 ? prev_u[(size_t)e * 2 * N] : 0.0;
+        if (close && fabs(v0) < 0.05) f.status[e] = TTMPC_FLEET_REACHED;
+      }
+      tk.next[e] = next;
+    }
     s_run = f.status[e] == TTMPC_FLEET_RUNNING;
     s_idx = idx;
-    s_sw = (f.sw_state && f.hint && f.use_hint && was_running) ? 1 : 0;
+    s_len = L;
+    s_new = took;
+    s_sw = (f.sw_state && f.hint && f.use_hint && (took ? s_run : was_running)) ? 1 : 0;
     // speed reference (:248-255)
     const double dist = hyp2(x - goal[0], y - goal[1]);
     double v = f.base_speed;
@@ -158,7 +239,7 @@ __global__ void __launch_bounds__(128) fleet_pack_kernel(const ttmpc_fleet f, co
     s_speed = v;
   }
   __syncthreads();
-  const int idx = s_idx;
+  const int idx = s_idx, L = s_len;
   // hybrid mode: main.py:200 evaluates HintSwitcher.switch before get_action's goal test.  The
   // geometric predicates are independent: one obstacle distance / one (point, obstacle)
   // containment per thread, then thread 0 walks the state machine over them.
@@ -188,7 +269,7 @@ __global__ void __launch_bounds__(128) fleet_pack_kernel(const ttmpc_fleet f, co
     double *u = prev_u + (size_t)e * 2 * N;
     const int o = threadIdx.x, nz = 2 * N;  // nz <= 64 < blockDim
     double v = 0.0;
-    if (o < nz && warm_exit[e] == TTMPC_CONVERGED) {  // u'[j] = u[min(j + k, N - 1)]
+    if (o < nz && warm_exit[e] == TTMPC_CONVERGED && !s_new) {  // u'[j] = u[min(j + k, N - 1)]
       const int src = o + 2 * f.action_steps, last = nz - 2 + (o & 1);
       v = u[src < last ? src : last];
     }
@@ -282,8 +363,10 @@ __global__ void __launch_bounds__(128) fleet_advance_kernel(const ttmpc_fleet f,
 }
 
 cudaError_t launch_fleet_pack(const ttmpc_fleet &f, const FleetDims &d, double *p, double *prev_u,
-                              const int *warm_exit, cudaStream_t st) {
-  fleet_pack_kernel<<<f.n, 128, 0, st>>>(f, d, p, prev_u, warm_exit);
+                              const int *warm_exit, const ttmpc_fleet_tasks *tasks, cudaStream_t st) {
+  ttmpc_fleet_tasks tk = {};
+  if (tasks && tasks->max_tasks > 0) tk = *tasks;
+  fleet_pack_kernel<<<f.n, 128, 0, st>>>(f, d, p, prev_u, warm_exit, tk);
   return cudaGetLastError();
 }
 cudaError_t launch_fleet_advance(const ttmpc_fleet &f, const FleetDims &d, const double *u,

@@ -47,8 +47,9 @@ struct FleetDims { int N, np, n_other, n_stc, n_dyn; double ts; };
 // prev_u: the previous step's solutions, required when warm_exit != null or action_steps > 1
 // (the goal test then reads their first control).  warm_exit != null: warm start -- prev_u is
 // shifted in place into the initial guess of every robot that is RUNNING after the goal test.
+// tasks != null with max_tasks > 0: REACHED robots take their next queued task (checked by the API).
 cudaError_t launch_fleet_pack(const ttmpc_fleet &f, const FleetDims &d, double *p, double *prev_u,
-                              const int *warm_exit, cudaStream_t st);
+                              const int *warm_exit, const ttmpc_fleet_tasks *tasks, cudaStream_t st);
 cudaError_t launch_fleet_advance(const ttmpc_fleet &f, const FleetDims &d, const double *u,
                                  const int *exit_status, cudaStream_t st);
 cudaError_t launch_fp64_peak(double *out, int blocks, int threads, int iters, cudaStream_t st);

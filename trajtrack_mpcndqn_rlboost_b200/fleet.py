@@ -7,9 +7,13 @@ reference's control loop does per robot per step (src/main.py:155-172, decision_
     traj_gen.update_dynamic_constraints(pred)                 # main.py:80-89 est_dyn_obs_positions
     action, pred_states, cost = traj_gen.get_action(ref)      # interface_mpc.py:80-92
 
-through ``ttmpc_fleet_step_device`` (pack -> solve -> advance, include/ttmpc.h).  The global
-reference trajectories are sampled once on the host with the same
-``TrajectoryGenerator.get_global_ref_traj`` the single-robot mirror uses.
+through ``ttmpc_fleet_step_device`` (pack -> solve -> advance, include/ttmpc.h).  The first global
+reference trajectories are sampled on the host with the same
+``TrajectoryGenerator.get_global_ref_traj`` the single-robot mirror uses.  Tasks queued with
+``FleetPlanner.set_tasks`` are taken on the device (``ttmpc_fleet_step_tasks_device``) and their
+trajectories are sampled there, from the state in which a robot takes the task; they agree with
+the host sampler to within a few ulps, not bit for bit (the device uses ``sqrt(fma(dx, dx, dy*dy))``
+and its own 1-ulp atan2 where Python uses ``math.hypot`` and ``math.atan2``).
 """
 from __future__ import annotations
 
@@ -23,7 +27,8 @@ from .geometry import polygon_halfspace_representation
 from .mpc_config import Configurator
 from .planner import TrajectoryGenerator
 
-RUNNING, REACHED, FAILED = 0, 1, 2
+RUNNING, REACHED, FAILED, BAD_TASK = 0, 1, 2, 3
+GOAL_REACH = 0.08  # a robot that stops at a goal is within its 5 cm box: at most 0.0708 m away
 DYN_OBS_SIZE = 0.8 + 0.8  # main.py:32
 
 
@@ -94,6 +99,8 @@ class FleetPlanner:
         self.pred_states = torch.zeros(n, self.N, 3, **f64)
         self.hint = None       # [n][N][2] DQN hint positions (rl_ref) and the per-robot switch
         self.use_hint = None
+        self.tasks = None      # _lib.TtmpcFleetTasks of the queued tasks (set_tasks), None: no queue
+        self.task_next = None  # [n] int32: queued tasks taken so far
         self.steps = 0
 
     # ------------------------------------------------------------------ obstacles
@@ -153,6 +160,76 @@ class FleetPlanner:
         if self.use_hint is None:
             self.use_hint = t.zeros(self.n, dtype=t.int32, device=dev)
 
+    # ------------------------------------------------------------------ tasks
+    def ref_rows_bound(self, start_xy, path) -> int:
+        """An upper bound of the rows ``get_global_ref_traj`` gives for ``path`` from any start within
+        GOAL_REACH of ``start_xy``: every row but the last advances the walker by base_speed*ts of
+        arc length, so rows <= length / (base_speed*ts) + 1 (+1 for rounding)."""
+        nodes = np.asarray(path, dtype=np.float64).reshape(-1, 2)
+        if len(nodes) == 0:
+            return 1
+        length = float(np.hypot(*(nodes[0] - np.asarray(start_xy, dtype=np.float64)[:2]))) + GOAL_REACH
+        length += float(np.hypot(*np.diff(nodes, axis=0).T).sum()) if len(nodes) > 1 else 0.0
+        return int(length / (self.base_speed * self.config.ts)) + 2
+
+    def set_tasks(self, goals: Sequence[Sequence], paths: Sequence[Sequence], dqn_paths=None):
+        """Replace every robot's task queue.  goals[e]: the goals [3] of robot e's tasks, paths[e]: one
+        polyline (list of (x, y) nodes) per task.  A robot that has reached its goal takes its next
+        task inside the step, on the device: ``InterfaceMpc.initialization(state, goal, path, mode)``
+        (include/ttmpc.h, ``ttmpc_fleet_tasks``); ``task_next`` counts the tasks taken, and
+        ``REACHED`` then means that the last task is done.  A task that cannot be driven stops its
+        robot with status ``BAD_TASK``.
+
+        ``ref_stride`` grows, keeping the rows, to cover every queued task from a start within
+        GOAL_REACH of the goal before it.  dqn_paths=(path_xy [n][m][2] float64, path_n [n] int32),
+        the CUDA tensors the hybrid loop passes to ``dqn.internal_obs_device``: the step writes each
+        robot's current path there when it takes a task (m must hold the longest task path)."""
+        t = self.torch
+        n = self.n
+        if len(goals) != n or len(paths) != n or any(len(g) != len(p) for g, p in zip(goals, paths)):
+            raise ValueError("set_tasks: one list of goals and one of paths per robot, of equal lengths")
+        T = max(len(g) for g in goals)
+        M = max([1] + [len(q) for pl in paths for q in pl])
+        if dqn_paths is not None:
+            if dqn_paths[0].shape[1] < M:
+                raise ValueError(f"set_tasks: dqn path buffer holds {dqn_paths[0].shape[1]} nodes, tasks need {M}")
+            M = int(dqn_paths[0].shape[1])
+        dev = self.state.device
+        if T == 0:
+            self.tasks, self.task_next = None, t.zeros(n, dtype=t.int32, device=dev)
+            return
+        goal = np.zeros((n, T, 3))
+        xy = np.zeros((n, T, M, 2))
+        pn = np.zeros((n, T), np.int32)
+        stride = self.ref_stride
+        prev = self.goal.cpu().numpy()
+        for e in range(n):
+            start = prev[e, :2]
+            for k, (g, q) in enumerate(zip(goals[e], paths[e])):
+                goal[e, k] = np.asarray(g, dtype=np.float64).reshape(3)
+                a = np.asarray(q, dtype=np.float64).reshape(-1, 2)
+                xy[e, k, :len(a)] = a
+                pn[e, k] = len(a)
+                stride = max(stride, self.ref_rows_bound(start, a))
+                start = goal[e, k, :2]
+        if stride > self.ref_stride:
+            ref = t.zeros(n, stride, 3, dtype=t.float64, device=dev)
+            ref[:, :self.ref_stride] = self.ref_traj
+            self.ref_traj, self.ref_stride = ref, stride
+        self.task_count = t.tensor([len(g) for g in goals], dtype=t.int32, device=dev)
+        self.task_next = t.zeros(n, dtype=t.int32, device=dev)
+        self.task_goal = t.tensor(goal, dtype=t.float64, device=dev)
+        self.task_path = t.tensor(xy, dtype=t.float64, device=dev)
+        self.task_path_n = t.tensor(pn, dtype=t.int32, device=dev)
+        tk = _lib.TtmpcFleetTasks()
+        tk.max_tasks, tk.max_nodes = T, M
+        tk.count, tk.next = self.task_count.data_ptr(), self.task_next.data_ptr()
+        tk.goal, tk.path_xy, tk.path_n = self.task_goal.data_ptr(), self.task_path.data_ptr(), self.task_path_n.data_ptr()
+        if dqn_paths is not None:
+            tk.path_out, tk.path_out_n = dqn_paths[0].data_ptr(), dqn_paths[1].data_ptr()
+        self.dqn_paths = dqn_paths
+        self.tasks = tk if int(self.task_count.sum()) > 0 else None
+
     # ------------------------------------------------------------------ the step
     def _fleet_struct(self) -> _lib.TtmpcFleet:
         f = _lib.TtmpcFleet()
@@ -209,6 +286,9 @@ class FleetPlanner:
         state from there) and ``last_u`` becomes u[k-1]; the goal test of the next step reads u[0]
         of this solution.  A warm start shifts by k.  Moving obstacles still move once per step.
 
+        With tasks queued (``set_tasks``) a robot that reaches its goal takes its next task in the
+        same step and is packed and solved on it; with warm_start it then starts from zeros.
+
         ``pred_states`` is the rollout of u* from the state the step STARTED in (p.s), i.e. one step
         earlier than ``TrajectoryGenerator.run_step``'s list, which re-applies u from the post-step
         state (trajectory_generator.py:296-301; ``planner.TrajectoryGenerator`` reproduces that list
@@ -216,9 +296,14 @@ class FleetPlanner:
         st = stream if stream is not None else self.torch.cuda.current_stream().cuda_stream
         f, r = self._fleet_struct(), self._result_struct()
         f.options = (_lib.FLEET_WARM_START if warm_start else 0) | (_lib.FLEET_SKIP_STOPPED if skip_stopped else 0)
-        _lib.check(self.lib.ttmpc_fleet_step_device(C.byref(self.cfg), C.byref(f), self.p.data_ptr(),
-                                                    1 if keep_multipliers else 0, C.byref(r), st),
-                   "ttmpc_fleet_step_device")
+        if self.tasks is not None:
+            _lib.check(self.lib.ttmpc_fleet_step_tasks_device(C.byref(self.cfg), C.byref(f), C.byref(self.tasks),
+                                                              self.p.data_ptr(), 1 if keep_multipliers else 0,
+                                                              C.byref(r), st), "ttmpc_fleet_step_tasks_device")
+        else:
+            _lib.check(self.lib.ttmpc_fleet_step_device(C.byref(self.cfg), C.byref(f), self.p.data_ptr(),
+                                                        1 if keep_multipliers else 0, C.byref(r), st),
+                       "ttmpc_fleet_step_device")
         self.steps += 1
 
     def pack(self, stream=None):

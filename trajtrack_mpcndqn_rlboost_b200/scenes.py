@@ -167,3 +167,51 @@ def make_fleet(n: int, seed: int = 0, n_static: int = 4, n_moving: int = 2):
     return dict(init=init, goal=goal, paths=paths, static_polys=polys,
                 moving_pos=np.stack([ox, oy], axis=-1),
                 moving_disp=np.stack([vmag * np.cos(vdir), vmag * np.sin(vdir)], axis=-1))
+
+
+def make_missions(n: int, tasks: int, seed: int = 0, n_moving: int = 2, max_static: int = 10):
+    """Synthetic missions for FleetPlanner.set_tasks: every robot gets a chain of ``tasks`` tasks,
+    each a two-leg path (4-8 m per leg) that starts at the goal of the task before it (the first at
+    the robot's start), one rectangle beside every leg while the ``max_static`` static slots last, and
+    obstacles crossing its first leg at constant velocity as in ``make_fleet``.
+
+    Returns make_fleet's keys for the first task (init, goal, paths, static_polys, moving_pos,
+    moving_disp) and task_goals / task_paths: per robot, the goals [3] and paths of the other
+    ``tasks - 1`` tasks, in the form ``FleetPlanner.set_tasks`` takes."""
+    rng = np.random.default_rng(seed)
+    x0 = rng.uniform(8.0, 32.0, n); y0 = rng.uniform(8.0, 32.0, n)
+    heading = rng.uniform(-np.pi, np.pi, n)
+    lateral = rng.normal(0.0, 0.1, n)
+    init = np.stack([x0 - lateral * np.sin(heading), y0 + lateral * np.cos(heading),
+                     heading + rng.normal(0.0, 0.2, n)], axis=1)
+    goals, paths, polys = [[] for _ in range(n)], [[] for _ in range(n)], [[] for _ in range(n)]
+    ax, ay, h = x0.copy(), y0.copy(), heading.copy()
+    for k in range(tasks):
+        if k:
+            h = h + rng.uniform(-2.5, 2.5, n)                  # the next task leaves in a new direction
+        leg1 = rng.uniform(4.0, 8.0, n); leg2 = rng.uniform(4.0, 8.0, n)
+        h2 = h + rng.uniform(-0.9, 0.9, n)
+        mx, my = ax + leg1 * np.cos(h), ay + leg1 * np.sin(h)
+        gx, gy = mx + leg2 * np.cos(h2), my + leg2 * np.sin(h2)
+        for (sx, sy, lh, ll) in ((ax, ay, h, leg1), (mx, my, h2, leg2)):
+            along = rng.uniform(0.25, 0.75, n) * ll
+            side = rng.choice([-1.0, 1.0], n) * rng.uniform(1.3, 3.0, n)
+            cx = sx + along * np.cos(lh) - side * np.sin(lh)
+            cy = sy + along * np.sin(lh) + side * np.cos(lh)
+            hx = rng.uniform(0.3, 0.9, n); hy = rng.uniform(0.3, 0.9, n)
+            for i in range(n):
+                if len(polys[i]) < max_static:
+                    polys[i].append([(cx[i] - hx[i], cy[i] - hy[i]), (cx[i] + hx[i], cy[i] - hy[i]),
+                                     (cx[i] + hx[i], cy[i] + hy[i]), (cx[i] - hx[i], cy[i] + hy[i])])
+        for i in range(n):
+            goals[i].append((gx[i], gy[i], 0.0))
+            paths[i].append([(ax[i], ay[i]), (mx[i], my[i]), (gx[i], gy[i])])
+        ax, ay, h = gx, gy, h2
+    a = rng.uniform(3.0, 9.0, (n, n_moving)); s = rng.choice([-1.0, 1.0], (n, n_moving)) * rng.uniform(3.0, 5.0, (n, n_moving))
+    ox = x0[:, None] + a * np.cos(heading)[:, None] - s * np.sin(heading)[:, None]
+    oy = y0[:, None] + a * np.sin(heading)[:, None] + s * np.cos(heading)[:, None]
+    vdir = rng.uniform(-np.pi, np.pi, (n, n_moving)); vmag = rng.uniform(0.0, 0.05, (n, n_moving))
+    return dict(init=init, goal=np.array([g[0] for g in goals]), paths=[p[0] for p in paths],
+                static_polys=polys, task_goals=[g[1:] for g in goals], task_paths=[p[1:] for p in paths],
+                moving_pos=np.stack([ox, oy], axis=-1),
+                moving_disp=np.stack([vmag * np.cos(vdir), vmag * np.sin(vdir)], axis=-1))
