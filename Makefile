@@ -8,10 +8,11 @@ NVFLAGS   := -gencode arch=compute_100a,code=sm_100a -lineinfo -O3 -std=c++17 -f
 LIB       := $(PKG)/libttmpc.so
 ORACLE    := oracle/libttmpc_oracle.so
 TASKS_ORACLE := oracle/libttfleet_tasks_oracle.so
+MONITOR_ORACLE := oracle/libttfleet_monitor_oracle.so
 CU        := $(CSRC)/ttmpc_solve.cu $(CSRC)/ttmpc_api.cu $(CSRC)/ttmpc_fleet.cu $(CSRC)/ttdqn.cu
 HDRS      := include/ttmpc.h $(CSRC)/ttmpc_device.cuh $(CSRC)/ttmpc_launch.cuh
 
-all: $(LIB) $(ORACLE) $(TASKS_ORACLE)
+all: $(LIB) $(ORACLE) $(TASKS_ORACLE) $(MONITOR_ORACLE)
 
 $(CSRC)/%.o: $(CSRC)/%.cu $(HDRS)
 	$(NVCC) $(NVFLAGS) -c $< -o $@
@@ -26,7 +27,10 @@ $(ORACLE): oracle/ttmpc_oracle.c oracle/ttdqn_oracle.c oracle/ttfleet_oracle.c o
 $(TASKS_ORACLE): oracle/ttfleet_tasks_oracle.c
 	$(CC) -O2 -fPIC -shared -ffp-contract=off -Wall -o $@ $< -lm
 
+$(MONITOR_ORACLE): oracle/ttfleet_monitor_oracle.c include/ttmpc.h
+	$(CC) -O2 -fPIC -shared -ffp-contract=off -Wall -o $@ $< -lm
+
 clean:
-	rm -f $(CSRC)/*.o $(LIB) $(ORACLE) $(TASKS_ORACLE)
+	rm -f $(CSRC)/*.o $(LIB) $(ORACLE) $(TASKS_ORACLE) $(MONITOR_ORACLE)
 
 .PHONY: all clean

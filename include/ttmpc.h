@@ -275,8 +275,10 @@ enum {
   TTMPC_FLEET_RUNNING = 0,  /* get_action returned an action                      */
   TTMPC_FLEET_REACHED = 1,  /* check_termination_condition: get_action -> None    */
   TTMPC_FLEET_FAILED = 2,   /* solver error (the reference raises RuntimeError)   */
-  TTMPC_FLEET_BAD_TASK = 3  /* ttmpc_fleet_step_tasks_device: the task taken next cannot be
+  TTMPC_FLEET_BAD_TASK = 3, /* ttmpc_fleet_step_tasks_device: the task taken next cannot be
                                driven (see ttmpc_fleet_tasks); the robot stops       */
+  TTMPC_FLEET_COLLIDED = 4  /* ttmpc_fleet_monitor_device with stop_on_contact: the robot
+                               touched an obstacle while RUNNING; the robot stops    */
 };
 /* ttmpc_fleet.options: bit mask of opt-in behaviours of ttmpc_fleet_step_device (0 = none; the
  * pack and advance entry points ignore it).  Other bits -> TTMPC_ERR_BAD_ARG.                  */
@@ -410,6 +412,66 @@ typedef struct ttmpc_fleet_tasks {
 int ttmpc_fleet_step_tasks_device(const ttmpc_config *cfg, const ttmpc_fleet *fleet,
                                   const ttmpc_fleet_tasks *tasks, double *d_p, int use_y0,
                                   const ttmpc_result *res, void *stream);
+
+/* Obstacle-contact and tracking monitor of ttmpc_fleet_monitor_device: what the closed loop did in
+ * the step that just ran, per robot, on the device.  All arrays are device pointers.
+ *
+ * Swept clearance.  The monitor runs after the step's advance, so robot e moved on the chord from
+ * prev_xy[e] to state[e][0:2] and each moving obstacle j moved from dyn_last[e][j] to
+ * dyn_cur[e][j].  clearance[e] is the minimum over the step of
+ *   - per static polygon (a slot with nv < 3 is unused): the distance of the chord to the polygon
+ *     minus robot_radius.  The polygon is a vertex ring, possibly non-convex (even-odd rule, strict
+ *     interior as shapely's Polygon.contains); the distance is 0 if an endpoint is inside or the
+ *     chord properly crosses an edge, else the least of the endpoint-to-edge and vertex-to-chord
+ *     distances.  A zero-length chord gives shapely's Polygon.distance(Point);
+ *   - per moving obstacle (when fleet->dyn_cur != NULL): the disc of radius moving_radius centred
+ *     on the obstacle; both move linearly in time, so the distance is that of the origin to the
+ *     segment from prev_xy - dyn_last to state - dyn_cur, minus (moving_radius + robot_radius);
+ * and +inf for a robot without obstacles.  The chord stands in for the RK4 arc: with |w| <= 0.5
+ * rad/s, v <= 1.5 m/s and ts = 0.2 s the arc leaves its chord by at most v ts (|w| ts) / 8, about
+ * 4 mm.  Every robot is monitored, a parked one too (a moving obstacle may run into it).
+ * Contact: clearance <= 0.  Then contact_steps[e] += 1, and first_contact[e] <- step if it is < 0.
+ * min_clearance[e] <- min(min_clearance[e], clearance[e]).
+ *
+ * Tracking.  For a robot that is TTMPC_FLEET_RUNNING when the monitor runs (exactly the robots
+ * that moved in this step): the distance of state[e][0:2] to the polyline through ref_traj rows
+ * max(idx_ref - k, 0) .. min(idx_ref + 5k, ref_len) - 1 (k = action_steps), the window the next
+ * pack's closest-point search scans; with one row the point distance.  deviation_max[e] <- max,
+ * deviation_sum[e] += it, moved_steps[e] += 1.
+ *
+ * stop_on_contact != 0: a robot that is RUNNING and in contact gets status TTMPC_FLEET_COLLIDED
+ * (after its deviation is taken).  It then stays where it is: pack and advance leave robots that
+ * are not RUNNING alone, TTMPC_FLEET_SKIP_STOPPED skips its solve, and only REACHED robots take
+ * queued tasks.  With stop_on_contact == 0 the monitor writes only the arrays of this struct.
+ *
+ * Arithmetic: plain IEEE mul / add in a fixed order (no contraction), so a C restatement compiled
+ * with -ffp-contract=off matches it bit for bit.  Start values: prev_xy = the states before the
+ * first step, min_clearance = +inf, first_contact = -1, the other in/out arrays 0.             */
+typedef struct ttmpc_fleet_monitor {
+  const double *poly_xy;  /* [n or 1][max_poly][max_pv][2] static polygons or NULL (none)     */
+  const int *poly_nv;     /* [n or 1][max_poly] vertex counts (< 3: unused slot)              */
+  int max_poly, max_pv;   /* max_poly >= 0; max_pv >= 3 when poly_xy != NULL                  */
+  int poly_shared;        /* != 0: one polygon block for every robot                          */
+  int stop_on_contact;
+  double robot_radius;    /* >= 0: the robot is a disc of this radius                         */
+  double moving_radius;   /* >= 0: radius of the moving obstacles' discs                      */
+  int step;               /* written to first_contact                                        */
+  int _pad;
+  double *prev_xy;        /* [n][2] in/out: position at the previous call (set to state[0:2]) */
+  double *clearance;      /* [n] out: this step's swept clearance                            */
+  double *min_clearance;  /* [n] in/out: running minimum                                     */
+  int *contact_steps;     /* [n] in/out: steps with clearance <= 0                           */
+  int *first_contact;     /* [n] in/out: step of the first contact, -1 before it             */
+  double *deviation_max;  /* [n] in/out: largest tracking deviation over the moved steps     */
+  double *deviation_sum;  /* [n] in/out: summed tracking deviation over the moved steps      */
+  int *moved_steps;       /* [n] in/out: steps in which the robot was RUNNING                 */
+} ttmpc_fleet_monitor;
+/* Run the monitor on `stream` after ttmpc_fleet_step_device or ttmpc_fleet_step_tasks_device (one
+ * thread per robot).  mon == NULL, a NULL in/out array, poly_xy without poly_nv, max_poly < 0,
+ * max_pv < 3 with polygons, a negative or non-finite radius, action_steps outside 1..N_hor or a
+ * fleet the step would reject -> TTMPC_ERR_BAD_ARG before any device work. */
+int ttmpc_fleet_monitor_device(const ttmpc_config *cfg, const ttmpc_fleet *fleet,
+                               const ttmpc_fleet_monitor *mon, void *stream);
 
 /* ------------------------------------------------------------------------
  * DQN side of the hybrid loop (src/main.py:174-193), device-resident.

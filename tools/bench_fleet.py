@@ -9,8 +9,10 @@ run.  Legs: options off (0), warm start (W), skip stopped robots (S) and both (W
 interleaved as 0 W S WS WS S W 0 so that drift of the card affects every option alike.  Every leg
 runs with the same action_steps k.  Per leg: drive time (sum of the per-step event times), step
 p50 / p90, PANOC iterations (device counters, ttmpc_read_stats), reached / failed / running
-robots at the end, and two rates over the drive time: robot-seconds per wall-second (k * ts of
-robot time for every robot that moved in a step, the time the reference's loop accounts for) and
+robots at the end, robots that touched an obstacle (the default monitor of
+FleetPlanner.enable_monitor, run after each step's end event, outside the timed window), and two
+rates over the drive time: robot-seconds per wall-second (k * ts of robot time for every robot
+that moved in a step, the time the reference's loop accounts for) and
 metres driven per wall-second (the robots' summed displacement; with k > 1 a step moves a robot by
 one RK4 step with its k-th control, see include/ttmpc.h).  The card's name and power limit are read
 in the same run.  Also the CPU oracle (reference order, all host cores) doing one plain step on a
@@ -49,6 +51,7 @@ def make(n, mc, fl, k):
     fp = t.FleetPlanner(mc, fl["init"], fl["goal"], fl["paths"], mode="work", action_steps=k)
     fp.update_static_constraints(fl["static_polys"], per_robot=True)
     fp.set_moving_obstacles(fl["moving_pos"], fl["moving_disp"])
+    fp.enable_monitor()
     return fp
 
 
@@ -62,8 +65,9 @@ def drive(fp, leg, max_steps):
         xy = fp.state[:, :2].clone()                                        # outside the timed window
         e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
         e0.record()
-        fp.step(warm_start="W" in leg, skip_stopped="S" in leg)
+        fp.step(warm_start="W" in leg, skip_stopped="S" in leg, monitor=False)
         e1.record()
+        fp.run_monitor()
         ev.append((e0, e1))
         moved += (fp.status == 0).sum()    # RUNNING after a step = took this step's controls
         metres += (fp.state[:, :2] - xy).norm(dim=1).sum()
@@ -79,7 +83,7 @@ def drive(fp, leg, max_steps):
                 robot_s_per_s=int(moved) * fp.action_steps * fp.config.ts / drive_s,
                 metres_per_s=float(metres) / drive_s,
                 panoc_iters=int(stats[3]), reached=int((status == 1).sum()), failed=int((status == 2).sum()),
-                running=int((status == 0).sum()))
+                running=int((status == 0).sum()), contact=int((fp.contact_steps > 0).sum()))
 
 
 def main():
@@ -101,7 +105,7 @@ def main():
         rs = [r for r in legs if r["leg"] == leg]
         mean[leg] = {k: float(np.mean([r[k] for r in rs]))
                      for k in ("drive_ms", "step_ms_p50", "step_ms_p90", "robot_s_per_s", "metres_per_s", "panoc_iters")}
-        mean[leg].update({k: rs[-1][k] for k in ("steps", "reached", "failed", "running")})
+        mean[leg].update({k: rs[-1][k] for k in ("steps", "reached", "failed", "running", "contact")})
     out = dict(workload=f"fleet{n}", robots=n, max_steps=max_steps, action_steps=ks, **card(), legs=legs, mean=mean)
     # CPU: one plain step with the oracle (reference operation order), bounded sample
     ns = min(n, 256)

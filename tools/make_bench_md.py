@@ -3,7 +3,7 @@
 r2_bench_static4096.json (headline), r2_bench_reference.json, r2_multi_<tag>_n<N>.json (tools/r2_multi.sh,
 tools/r2_single_sweep.sh), profiles/r2_parity_distribution_{gpu,cpu}.json, r2_qnet.json, r2_fleet.json,
 r2_hybrid.json, r2_single_latency.txt, profiles/r2_roofline_inputs.json, r2_missions.json (tools/bench_missions.py,
-one line per fleet size), r2_missions_profile.json (its --profile-pack line)."""
+one line per fleet size), r2_missions_profile.json (its --profile-pack line), r2_monitor.json (tools/bench_monitor.py)."""
 import glob
 import json
 import os
@@ -81,6 +81,37 @@ def missions_section(ms, prof):
         out.append(f"`fleet_pack_kernel` with {p['robots']} robots (`--profile-pack`, torch.profiler): {p['all_switch']['pack_us']:.0f} µs "
                    f"in a step in which every robot takes a task ({p['switched_in_first_step']} switched), "
                    f"{p['no_switch']['pack_us']:.0f} µs in the next step, in which none does.\n")
+    return out
+
+
+def monitor_section(mo):
+    """Lines of the "Fleet monitor" section: the line of tools/bench_monitor.py."""
+    if not mo:
+        return []
+    out = ["## Fleet monitor (`tools/bench_monitor.py`; swept clearance, contacts and tracking deviation after every step)\n",
+           f"Kernel time of `fleet_monitor_kernel` on `make_fleet(n, seed=1000)` geometry (4 rectangles and 2 moving obstacles "
+           f"per robot, the chords of the third step), one pair of CUDA events per launch, {mo['gpu']}, power limit {mo['power_limit']}.\n",
+           "| robots | launches | µs p50 | µs mean |", "|---:|---:|---:|---:|"]
+    for k in mo["kernel"]:
+        out.append(f"| {k['robots']} | {k['launches']} | {k['kernel_us_p50']:.1f} | {k['kernel_us_mean']:.1f} |")
+    out.append("")
+    out.append("One thread per robot: both sizes are a single wave of CTAs (32 and 128 on 148 SMs), so the time is the "
+               "latency of one robot's chain of fp64 divisions and square roots, not a throughput.\n")
+    d = mo.get("drive")
+    if d:
+        q = d["min_clearance_quantiles"]
+        out.append(f"Drive: `make_fleet({d['robots']}, seed=1000)`, {d['steps']} steps, options {d['options']}, default monitor (robot "
+                   f"centre against the polygons the MPC sees, moving obstacles as discs of {d['moving_radius']} m). Reached / failed / "
+                   f"running {d['reached']} / {d['failed']} / {d['running']}; robots with contact {d['robots_with_contact']} "
+                   f"({d['contact_steps_total']} robot-steps in contact); min_clearance quantiles 0 / 1 / 5 / 10 / 50 %: "
+                   + " / ".join(f"{q[k]:.3f}" for k in ("0.0", "0.01", "0.05", "0.1", "0.5"))
+                   + f" m; tracking deviation mean {d['deviation_mean']:.3f} m, max {d['deviation_max']:.3f} m.\n")
+    s = mo.get("drive_static_only")
+    if s:
+        q = s["min_clearance_quantiles"]
+        out.append(f"The same drive with moving_radius = 0, i.e. the rectangles alone: robots with contact {s['robots_with_contact']} "
+                   f"({s['contact_steps_total']} robot-steps); min_clearance quantiles "
+                   + " / ".join(f"{q[k]:.3f}" for k in ("0.0", "0.01", "0.05", "0.1", "0.5")) + " m.\n")
     return out
 
 
@@ -221,13 +252,16 @@ def main():
         out.append(f"Each leg drives the same seeded fleet until every robot has stopped or {fl[0]['max_steps']} steps have run. "
                    "Options: 0 = none, W = warm start, S = skip stopped robots. The legs ran interleaved (0 W S WS WS S W 0); "
                    f"each row is the mean of an option's two legs. {fl[0]['gpu']}, power limit {fl[0]['power_limit']}.\n")
-        out.append("| robots | options | steps | drive time (s) | ms / step p50 | p90 | PANOC iterations | reached / failed / running |")
-        out.append("|---:|:--|---:|---:|---:|---:|---:|:--|")
+        out.append("Robots with contact: robots whose swept clearance was <= 0 in some step (the default monitor of "
+                   "`FleetPlanner.enable_monitor`, run outside the timed window; – where the line has no count).\n")
+        out.append("| robots | options | steps | drive time (s) | ms / step p50 | p90 | PANOC iterations | reached / failed / running | robots with contact |")
+        out.append("|---:|:--|---:|---:|---:|---:|---:|:--|---:|")
         for r in fl:
             for leg, m in r["mean"].items():
                 out.append(f"| {r['robots']} | {leg} | {m['steps']} | {m['drive_ms'] / 1e3:.2f} | {m['step_ms_p50']:.1f} | {m['step_ms_p90']:.1f} | "
-                           f"{m['panoc_iters']:,.0f} | {m['reached']} / {m['failed']} / {m['running']} |")
+                           f"{m['panoc_iters']:,.0f} | {m['reached']} / {m['failed']} / {m['running']} | {m.get('contact', '–')} |")
         out.append("")
+    out += monitor_section(last(os.path.join(G, "r2_monitor.json")))
     out += missions_section(list({r["robots"]: r for r in jl(os.path.join(G, "r2_missions.json"))}.values()),
                             last(os.path.join(G, "r2_missions_profile.json")))
     hy = last(os.path.join(G, "r2_hybrid.json"))

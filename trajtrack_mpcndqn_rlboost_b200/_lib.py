@@ -89,12 +89,27 @@ class TtmpcFleetTasks(C.Structure):
     ]
 
 
+class TtmpcFleetMonitor(C.Structure):
+    """struct ttmpc_fleet_monitor: obstacle-contact and tracking monitor of ttmpc_fleet_monitor_device
+    (device addresses)."""
+    _fields_ = [
+        ("poly_xy", C.c_void_p), ("poly_nv", C.c_void_p),
+        ("max_poly", C.c_int), ("max_pv", C.c_int), ("poly_shared", C.c_int), ("stop_on_contact", C.c_int),
+        ("robot_radius", C.c_double), ("moving_radius", C.c_double),
+        ("step", C.c_int), ("_pad", C.c_int),
+        ("prev_xy", C.c_void_p), ("clearance", C.c_void_p), ("min_clearance", C.c_void_p),
+        ("contact_steps", C.c_void_p), ("first_contact", C.c_void_p), ("deviation_max", C.c_void_p),
+        ("deviation_sum", C.c_void_p), ("moved_steps", C.c_void_p),
+    ]
+
+
 # every symbol include/ttmpc.h declares, with its signature
 _VP, _I, _D = C.c_void_p, C.c_int, C.c_double
 _CFG, _RES = C.POINTER(TtmpcConfig), C.POINTER(TtmpcResult)
 _LAY, _QN = C.POINTER(TtdqnLayout), C.POINTER(TtdqnQnet)
 _FLT = C.POINTER(TtmpcFleet)
 _TSK = C.POINTER(TtmpcFleetTasks)
+_MON = C.POINTER(TtmpcFleetMonitor)
 SYMBOLS = {
     "ttmpc_default_config": (None, [_CFG]),
     "ttmpc_num_params": (_I, [_CFG]),
@@ -114,6 +129,7 @@ SYMBOLS = {
     "ttmpc_fleet_advance_device": (_I, [_CFG, _FLT, _VP, _VP, _VP]),
     "ttmpc_fleet_step_device": (_I, [_CFG, _FLT, _VP, _I, _RES, _VP]),
     "ttmpc_fleet_step_tasks_device": (_I, [_CFG, _FLT, _TSK, _VP, _I, _RES, _VP]),
+    "ttmpc_fleet_monitor_device": (_I, [_CFG, _FLT, _MON, _VP]),
     "ttmpc_read_stats": (_I, [C.POINTER(C.c_ulonglong), _I]),
     "ttmpc_launch_info": (_I, [_CFG, _I] + [C.POINTER(C.c_int)] * 5),
     "ttmpc_measure_fp64_peak": (_I, [C.POINTER(_D), _VP]),

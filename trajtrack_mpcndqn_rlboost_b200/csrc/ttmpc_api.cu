@@ -2,6 +2,7 @@
 // Host-side only: argument checking, workspace management, staging copies.
 #include <cuda_runtime.h>
 
+#include <cmath>
 #include <cstdio>
 #include <cstdlib>
 #include <cstring>
@@ -516,6 +517,26 @@ extern "C" int ttmpc_fleet_step_tasks_device(const ttmpc_config *cfg, const ttmp
   if (tasks->path_out && !tasks->path_out_n)
     return fail(TTMPC_ERR_BAD_ARG, "fleet tasks: path_out needs path_out_n");
   return fleet_step(cfg, fleet, tasks, d_p, use_y0, res, stream);
+}
+extern "C" int ttmpc_fleet_monitor_device(const ttmpc_config *cfg, const ttmpc_fleet *fleet,
+                                          const ttmpc_fleet_monitor *mon, void *stream) {
+  FleetDims d;
+  int rc = fleet_dims(cfg, fleet, &d);
+  if (rc) return rc;
+  if (fleet->action_steps < 1 || fleet->action_steps > cfg->N_hor)
+    return fail(TTMPC_ERR_BAD_ARG, "fleet: action_steps must be in 1..N_hor");
+  if (!mon) return fail(TTMPC_ERR_BAD_ARG, "fleet monitor: null");
+  if (!mon->prev_xy || !mon->clearance || !mon->min_clearance || !mon->contact_steps || !mon->first_contact ||
+      !mon->deviation_max || !mon->deviation_sum || !mon->moved_steps)
+    return fail(TTMPC_ERR_BAD_ARG, "fleet monitor: every in/out array is required");
+  if (mon->max_poly < 0 || (mon->poly_xy && (!mon->poly_nv || mon->max_pv < 3)))
+    return fail(TTMPC_ERR_BAD_ARG, "fleet monitor: polygons need poly_nv, max_poly >= 0 and max_pv >= 3");
+  if (!(mon->robot_radius >= 0.0 && mon->robot_radius < INFINITY) ||
+      !(mon->moving_radius >= 0.0 && mon->moving_radius < INFINITY))
+    return fail(TTMPC_ERR_BAD_ARG, "fleet monitor: radii must be finite and >= 0");
+  if (fleet->n == 0) return TTMPC_OK;
+  CUDA_TRY(launch_fleet_monitor(*fleet, *mon, (cudaStream_t)stream));
+  return TTMPC_OK;
 }
 
 // Cumulative device-side counters since the last reset:

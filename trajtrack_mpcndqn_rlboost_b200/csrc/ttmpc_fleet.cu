@@ -4,8 +4,9 @@
 // See include/ttmpc.h ("Fleet step") for the contract; oracle/ttfleet_oracle.c is the CPU
 // restatement these kernels match bit for bit (use_libm = 0).
 //
-// Both kernels are copy / scalar work: pack writes the n x np parameter block once, coalesced
-// (HBM-bound, 21 KB per robot), advance touches 5 doubles per robot.
+// The kernels are copy / scalar work: pack writes the n x np parameter block once, coalesced
+// (HBM-bound, 21 KB per robot), advance touches 5 doubles per robot, the monitor (run after the
+// step, include/ttmpc.h: ttmpc_fleet_monitor) reads a robot's polygons, obstacles and reference rows.
 #include <cuda_runtime.h>
 
 #include "ttmpc_device.cuh"
@@ -24,16 +25,20 @@ __device__ __forceinline__ bool poly_contains(const double *xy, int nv, double p
   }
   return in;
 }
+// distance of (px, py) to the segment from (ax, ay) to (bx, by)
+__device__ __forceinline__ double seg_distance(double ax, double ay, double bx, double by, double px, double py) {
+  const double dx = bx - ax, dy = by - ay;
+  const double len2 = dx * dx + dy * dy;
+  double t = 0.0;
+  if (len2 > 0.0) { t = ((px - ax) * dx + (py - ay) * dy) / len2; t = t < 0.0 ? 0.0 : (t > 1.0 ? 1.0 : t); }
+  const double qx = ax + t * dx - px, qy = ay + t * dy - py;
+  return sqrt(qx * qx + qy * qy);
+}
 __device__ __forceinline__ double poly_distance(const double *xy, int nv, double px, double py) {
   if (poly_contains(xy, nv, px, py)) return 0.0;
   double best = INFINITY;
   for (int i = 0, j = nv - 1; i < nv; j = i++) {
-    const double ax = xy[2 * j], ay = xy[2 * j + 1], dx = xy[2 * i] - ax, dy = xy[2 * i + 1] - ay;
-    const double len2 = dx * dx + dy * dy;
-    double t = 0.0;
-    if (len2 > 0.0) { t = ((px - ax) * dx + (py - ay) * dy) / len2; t = t < 0.0 ? 0.0 : (t > 1.0 ? 1.0 : t); }
-    const double qx = ax + t * dx - px, qy = ay + t * dy - py;
-    const double d = sqrt(qx * qx + qy * qy);
+    const double d = seg_distance(xy[2 * j], xy[2 * j + 1], xy[2 * i], xy[2 * i + 1], px, py);
     if (d < best) best = d;
   }
   return best;
@@ -360,6 +365,93 @@ __global__ void __launch_bounds__(128) fleet_advance_kernel(const ttmpc_fleet f,
   st[1] = st[1] + sixth * (((k1y + 2.0 * k2y) + 2.0 * k3y) + k4y);
   st[2] = st[2] + sixth * (((k1t + 2.0 * k2t) + 2.0 * k3t) + k4t);
   f.last_u[2 * e] = v; f.last_u[2 * e + 1] = w;
+}
+
+// Distance of the chord (x0, y0) -> (x1, y1) to a polygon ring: 0 if an endpoint is inside or the
+// chord properly crosses an edge, else the least endpoint-to-edge and vertex-to-chord distance (the
+// distance of two segments that do not cross).  A chord that touches an edge without crossing it
+// gets its distance from the touching endpoint or vertex.  Zero length: poly_distance.
+__device__ double swept_poly_distance(const double *xy, int nv, double x0, double y0, double x1, double y1) {
+  if (poly_contains(xy, nv, x0, y0) || poly_contains(xy, nv, x1, y1)) return 0.0;
+  const bool moved = x0 != x1 || y0 != y1;
+  const double cx = x1 - x0, cy = y1 - y0;
+  double best = INFINITY;
+  for (int i = 0, j = nv - 1; i < nv; j = i++) {
+    const double ax = xy[2 * j], ay = xy[2 * j + 1], bx = xy[2 * i], by = xy[2 * i + 1];
+    double d = seg_distance(ax, ay, bx, by, x0, y0);
+    if (moved) {
+      const double ex = bx - ax, ey = by - ay;  // orientations of the chord ends to the edge, and back
+      const double o0 = ex * (y0 - ay) - ey * (x0 - ax), o1 = ex * (y1 - ay) - ey * (x1 - ax);
+      const double oa = cx * (ay - y0) - cy * (ax - x0), ob = cx * (by - y0) - cy * (bx - x0);
+      if (((o0 > 0.0 && o1 < 0.0) || (o0 < 0.0 && o1 > 0.0)) && ((oa > 0.0 && ob < 0.0) || (oa < 0.0 && ob > 0.0)))
+        return 0.0;
+      const double d1 = seg_distance(ax, ay, bx, by, x1, y1), dv = seg_distance(x0, y0, x1, y1, ax, ay);
+      if (d1 < d) d = d1;
+      if (dv < d) d = dv;
+    }
+    if (d < best) best = d;
+  }
+  return best;
+}
+
+// One thread per robot: the obstacle-contact and tracking monitor of the step that just ran
+// (include/ttmpc.h, ttmpc_fleet_monitor).  oracle/ttfleet_monitor_oracle.c restates it.
+__global__ void __launch_bounds__(128) fleet_monitor_kernel(const ttmpc_fleet f, const ttmpc_fleet_monitor m) {
+  const int e = blockIdx.x * blockDim.x + threadIdx.x;
+  if (e >= f.n) return;
+  double *pv = m.prev_xy + 2 * e;
+  const double x0 = pv[0], y0 = pv[1], x1 = f.state[3 * e], y1 = f.state[3 * e + 1];
+  double c = INFINITY;
+  if (m.poly_xy) {
+    const double *pxy = m.poly_xy + (m.poly_shared ? 0 : (size_t)e * m.max_poly * m.max_pv * 2);
+    const int *pnv = m.poly_nv + (m.poly_shared ? 0 : (size_t)e * m.max_poly);
+    for (int o = 0; o < m.max_poly; o++) {
+      const int nv = min(pnv[o], m.max_pv);
+      if (nv < 3) continue;
+      const double d = swept_poly_distance(pxy + (size_t)o * m.max_pv * 2, nv, x0, y0, x1, y1) - m.robot_radius;
+      if (d < c) c = d;
+    }
+  }
+  if (f.dyn_cur) {  // robot relative to the obstacle: prev - last -> state - cur, linear in time
+    const double r = m.moving_radius + m.robot_radius;
+    for (int j = 0; j < f.n_dyn_live; j++) {
+      const double *cur = f.dyn_cur + ((size_t)e * f.n_dyn_live + j) * 2;
+      const double *last = f.dyn_last + ((size_t)e * f.n_dyn_live + j) * 2;
+      const double d = seg_distance(x0 - last[0], y0 - last[1], x1 - cur[0], y1 - cur[1], 0.0, 0.0) - r;
+      if (d < c) c = d;
+    }
+  }
+  m.clearance[e] = c;
+  if (c < m.min_clearance[e]) m.min_clearance[e] = c;
+  const bool contact = c <= 0.0;
+  if (contact) {
+    m.contact_steps[e] += 1;
+    if (m.first_contact[e] < 0) m.first_contact[e] = m.step;
+  }
+  if (f.status[e] == TTMPC_FLEET_RUNNING) {
+    const int k = f.action_steps, L = f.ref_len[e], idx = f.idx_ref[e];
+    const double *ref = f.ref_traj + (size_t)e * f.ref_stride * 3;
+    int lo = idx - k; if (lo < 0) lo = 0;
+    int hi = idx + 5 * k; if (hi > L) hi = L;
+    double dev = seg_distance(ref[3 * lo], ref[3 * lo + 1], ref[3 * lo], ref[3 * lo + 1], x1, y1);
+    if (hi - lo >= 2) {
+      dev = INFINITY;
+      for (int i = lo + 1; i < hi; i++) {
+        const double d = seg_distance(ref[3 * i - 3], ref[3 * i - 2], ref[3 * i], ref[3 * i + 1], x1, y1);
+        if (d < dev) dev = d;
+      }
+    }
+    if (dev > m.deviation_max[e]) m.deviation_max[e] = dev;
+    m.deviation_sum[e] = m.deviation_sum[e] + dev;
+    m.moved_steps[e] += 1;
+    if (m.stop_on_contact && contact) f.status[e] = TTMPC_FLEET_COLLIDED;
+  }
+  pv[0] = x1; pv[1] = y1;
+}
+
+cudaError_t launch_fleet_monitor(const ttmpc_fleet &f, const ttmpc_fleet_monitor &m, cudaStream_t st) {
+  fleet_monitor_kernel<<<(f.n + 127) / 128, 128, 0, st>>>(f, m);
+  return cudaGetLastError();
 }
 
 cudaError_t launch_fleet_pack(const ttmpc_fleet &f, const FleetDims &d, double *p, double *prev_u,

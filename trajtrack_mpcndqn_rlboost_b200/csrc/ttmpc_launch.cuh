@@ -52,6 +52,7 @@ cudaError_t launch_fleet_pack(const ttmpc_fleet &f, const FleetDims &d, double *
                               const int *warm_exit, const ttmpc_fleet_tasks *tasks, cudaStream_t st);
 cudaError_t launch_fleet_advance(const ttmpc_fleet &f, const FleetDims &d, const double *u,
                                  const int *exit_status, cudaStream_t st);
+cudaError_t launch_fleet_monitor(const ttmpc_fleet &f, const ttmpc_fleet_monitor &m, cudaStream_t st);
 cudaError_t launch_fp64_peak(double *out, int blocks, int threads, int iters, cudaStream_t st);
 
 }  // namespace ttmpc

@@ -7,7 +7,10 @@ reference's control loop does per robot per step (src/main.py:155-172, decision_
     traj_gen.update_dynamic_constraints(pred)                 # main.py:80-89 est_dyn_obs_positions
     action, pred_states, cost = traj_gen.get_action(ref)      # interface_mpc.py:80-92
 
-through ``ttmpc_fleet_step_device`` (pack -> solve -> advance, include/ttmpc.h).  The first global
+through ``ttmpc_fleet_step_device`` (pack -> solve -> advance, include/ttmpc.h).  With
+``FleetPlanner.enable_monitor`` every step is followed by ``ttmpc_fleet_monitor_device``, which
+records per robot on the device how close it came to its obstacles over the step (swept clearance,
+contacts) and how far it was from its reference path.  The first global
 reference trajectories are sampled on the host with the same
 ``TrajectoryGenerator.get_global_ref_traj`` the single-robot mirror uses.  Tasks queued with
 ``FleetPlanner.set_tasks`` are taken on the device (``ttmpc_fleet_step_tasks_device``) and their
@@ -27,7 +30,7 @@ from .geometry import polygon_halfspace_representation
 from .mpc_config import Configurator
 from .planner import TrajectoryGenerator
 
-RUNNING, REACHED, FAILED, BAD_TASK = 0, 1, 2, 3
+RUNNING, REACHED, FAILED, BAD_TASK, COLLIDED = 0, 1, 2, 3, 4
 GOAL_REACH = 0.08  # a robot that stops at a goal is within its 5 cm box: at most 0.0708 m away
 DYN_OBS_SIZE = 0.8 + 0.8  # main.py:32
 
@@ -101,6 +104,8 @@ class FleetPlanner:
         self.use_hint = None
         self.tasks = None      # _lib.TtmpcFleetTasks of the queued tasks (set_tasks), None: no queue
         self.task_next = None  # [n] int32: queued tasks taken so far
+        self.static_polys = None  # (polygons, per_robot) of the last update_static_constraints
+        self.monitor = None    # _lib.TtmpcFleetMonitor (enable_monitor), None: no monitor
         self.steps = 0
 
     # ------------------------------------------------------------------ obstacles
@@ -118,6 +123,7 @@ class FleetPlanner:
         data = [rows(pl) for pl in obstacle_list] if per_robot else [rows(obstacle_list)]
         self.stc = self.torch.tensor(np.array(data, dtype=np.float64), device=self.state.device)
         self.stc_shared = 0 if per_robot else 1
+        self.static_polys = (obstacle_list, per_robot)
 
     def set_moving_obstacles(self, positions: np.ndarray, displacement_per_step: np.ndarray):
         """positions, displacement_per_step: [n][k][2].  Every step the planner sees
@@ -142,6 +148,19 @@ class FleetPlanner:
         polygons: the processed (inflated) static obstacle polygons, shared or one list per robot;
         moving obstacles enter as circle_to_rect squares of radius DYN_OBS_SIZE."""
         t = self.torch
+        xy, nv = self._polygon_rings(polygons, per_robot)
+        dev = self.state.device
+        self.sw_poly_xy, self.sw_poly_nv = t.tensor(xy, device=dev), t.tensor(nv, device=dev)
+        self.sw_shape = (xy.shape[1], xy.shape[2], 0 if per_robot else 1)
+        self.sw_params = (float(max_switch_distance), float(min_detach_distance), int(min_detach_steps))
+        self.sw_state = t.zeros(self.n, 2, dtype=t.int32, device=dev)
+        if self.use_hint is None:
+            self.use_hint = t.zeros(self.n, dtype=t.int32, device=dev)
+
+    @staticmethod
+    def _polygon_rings(polygons, per_robot: bool):
+        """Vertex rings of polygons (shared, or one list per robot) in the layout the kernels read:
+        xy [n or 1][max_poly][max_pv][2] float64, nv [n or 1][max_poly] int32 (0: unused slot)."""
         lists = polygons if per_robot else [polygons]
         max_poly = max(1, max(len(pl) for pl in lists))
         max_pv = max(3, max((len(poly) for pl in lists for poly in pl), default=3))
@@ -152,13 +171,69 @@ class FleetPlanner:
                 a = np.asarray(poly, np.float64).reshape(-1, 2)
                 xy[i, j, :len(a)] = a
                 nv[i, j] = len(a)
+        return xy, nv
+
+    # ------------------------------------------------------------------ monitor
+    def enable_monitor(self, polygons=None, per_robot: Optional[bool] = None, robot_radius: float = 0.0,
+                       moving_radius: float = DYN_OBS_SIZE, stop_on_contact: bool = False):
+        """Run the obstacle-contact and tracking monitor (``ttmpc_fleet_monitor_device``, include/ttmpc.h)
+        after every ``step()``, on the step's stream.
+
+        polygons: static obstacles as vertex rings, shared or (per_robot=True) one list per robot;
+        default: the polygons last given to ``update_static_constraints``, with their per_robot flag.
+        The robot is a disc of robot_radius, a moving obstacle a disc of moving_radius.  The defaults
+        monitor the region the MPC's constraints exclude: the robot centre against the polygons the
+        MPC sees, and the DYN_OBS_SIZE discs the pack writes for moving obstacles.
+
+        Per robot, on the device (reset here; ``prev_xy`` starts at the current state):
+        ``clearance`` (the last step's swept clearance, +inf before the first), ``min_clearance``,
+        ``contact_steps`` (steps with clearance <= 0), ``first_contact`` (index of the first such
+        ``step()`` call, counted from the planner's construction; -1: none), and over the steps in
+        which the robot moved ``deviation_max``, ``deviation_sum`` and ``moved_steps``.
+        stop_on_contact=True: a RUNNING robot in contact stops with status ``COLLIDED``."""
+        t = self.torch
+        if polygons is None and self.static_polys is not None:
+            polygons, stored = self.static_polys
+            per_robot = stored if per_robot is None else per_robot
+        per_robot = bool(per_robot)
+        if not (np.isfinite(robot_radius) and robot_radius >= 0.0 and np.isfinite(moving_radius) and moving_radius >= 0.0):
+            raise ValueError("enable_monitor: radii must be finite and >= 0")
+        if per_robot and polygons is not None and len(polygons) != self.n:
+            raise ValueError(f"enable_monitor: {len(polygons)} polygon lists for {self.n} robots")
         dev = self.state.device
-        self.sw_poly_xy, self.sw_poly_nv = t.tensor(xy, device=dev), t.tensor(nv, device=dev)
-        self.sw_shape = (max_poly, max_pv, 0 if per_robot else 1)
-        self.sw_params = (float(max_switch_distance), float(min_detach_distance), int(min_detach_steps))
-        self.sw_state = t.zeros(self.n, 2, dtype=t.int32, device=dev)
-        if self.use_hint is None:
-            self.use_hint = t.zeros(self.n, dtype=t.int32, device=dev)
+        m = _lib.TtmpcFleetMonitor()
+        self.mon_poly_xy = self.mon_poly_nv = None
+        if polygons is not None:
+            xy, nv = self._polygon_rings(polygons, per_robot)
+            self.mon_poly_xy, self.mon_poly_nv = t.tensor(xy, device=dev), t.tensor(nv, device=dev)
+            m.poly_xy, m.poly_nv = self.mon_poly_xy.data_ptr(), self.mon_poly_nv.data_ptr()
+            m.max_poly, m.max_pv, m.poly_shared = xy.shape[1], xy.shape[2], 0 if per_robot else 1
+        m.robot_radius, m.moving_radius = float(robot_radius), float(moving_radius)
+        m.stop_on_contact = 1 if stop_on_contact else 0
+        f64 = dict(dtype=t.float64, device=dev)
+        i32 = dict(dtype=t.int32, device=dev)
+        self.prev_xy = self.state[:, :2].clone()
+        self.clearance = t.full((self.n,), float("inf"), **f64)
+        self.min_clearance = t.full((self.n,), float("inf"), **f64)
+        self.contact_steps = t.zeros(self.n, **i32)
+        self.first_contact = t.full((self.n,), -1, **i32)
+        self.deviation_max = t.zeros(self.n, **f64)
+        self.deviation_sum = t.zeros(self.n, **f64)
+        self.moved_steps = t.zeros(self.n, **i32)
+        for name in ("prev_xy", "clearance", "min_clearance", "contact_steps", "first_contact", "deviation_max",
+                     "deviation_sum", "moved_steps"):
+            setattr(m, name, getattr(self, name).data_ptr())
+        self.monitor = m
+
+    def run_monitor(self, stream=None):
+        """Run the monitor on the last ``step()``.  ``step()`` calls this itself unless it is called
+        with monitor=False.  Needs ``enable_monitor``."""
+        if self.monitor is None:
+            raise RuntimeError("run_monitor: call enable_monitor first")
+        st = stream if stream is not None else self.torch.cuda.current_stream().cuda_stream
+        self.monitor.step = self.steps - 1
+        _lib.check(self.lib.ttmpc_fleet_monitor_device(C.byref(self.cfg), C.byref(self._fleet_struct()),
+                                                       C.byref(self.monitor), st), "ttmpc_fleet_monitor_device")
 
     # ------------------------------------------------------------------ tasks
     def ref_rows_bound(self, start_xy, path) -> int:
@@ -265,7 +340,7 @@ class FleetPlanner:
         return r
 
     def step(self, keep_multipliers: bool = True, warm_start: bool = False, skip_stopped: bool = False,
-             stream=None):
+             stream=None, monitor: bool = True):
         """One control step of every robot, asynchronous on the current torch stream.
 
         keep_multipliers=True (default) is what the reference's control loop does: the PyO3 ``Solver``
@@ -292,7 +367,11 @@ class FleetPlanner:
         ``pred_states`` is the rollout of u* from the state the step STARTED in (p.s), i.e. one step
         earlier than ``TrajectoryGenerator.run_step``'s list, which re-applies u from the post-step
         state (trajectory_generator.py:296-301; ``planner.TrajectoryGenerator`` reproduces that list
-        on the host)."""
+        on the host).
+
+        With the monitor enabled (``enable_monitor``) the step ends with it, on the same stream;
+        monitor=False leaves it to a ``run_monitor()`` call before the next step (a benchmark that
+        times the step alone does that)."""
         st = stream if stream is not None else self.torch.cuda.current_stream().cuda_stream
         f, r = self._fleet_struct(), self._result_struct()
         f.options = (_lib.FLEET_WARM_START if warm_start else 0) | (_lib.FLEET_SKIP_STOPPED if skip_stopped else 0)
@@ -305,6 +384,8 @@ class FleetPlanner:
                                                         1 if keep_multipliers else 0, C.byref(r), st),
                        "ttmpc_fleet_step_device")
         self.steps += 1
+        if self.monitor is not None and monitor:
+            self.run_monitor(st)
 
     def pack(self, stream=None):
         """The pack kernel alone (action_steps = 1 only: raises TtmpcError otherwise)."""
