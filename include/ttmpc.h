@@ -248,6 +248,35 @@ int ttdqn_observe_act_host(const ttdqn_scene_layout *lay, const ttdqn_qnet *qnet
                            float *h_ext, float *h_q, int *h_action,
                            double *h_seg_dist, double *h_ray_dist);
 
+/* Moving obstacles in the observation: n_live solid rings per env, each a vertex template placed
+ * at its obstacle's current centre.  Ring o of env e has vertices
+ *   centre[e][o] + shape_xy[e or 0][o][v],  v < shape_nv[e or 0][o]
+ * (one fp64 add per coordinate).  Like a static solid ring it is even-odd filled: an agent inside
+ * one gives 0 in every sector and on every ray.  A template with shape_nv < 3 is not seen; counts
+ * above max_pv are read as max_pv.  All arrays are device pointers.                               */
+typedef struct ttdqn_moving {
+  int n_live;              /* moving obstacles per env, >= 0                                   */
+  int max_pv;              /* vertex slots per template, 3..32                                 */
+  int shape_shared;        /* != 0: one template block for every env                           */
+  int _pad;
+  const double *centre;    /* [n][n_live][2] current centres, e.g. ttmpc_fleet.dyn_cur         */
+  const double *shape_xy;  /* [n or 1][n_live][max_pv][2] vertex offsets from the centre       */
+  const int *shape_nv;     /* [n or 1][n_live] vertex counts (< 3: not seen)                   */
+} ttdqn_moving;
+/* ttdqn_observe_act_device with the moving rings of mv.  The result equals that of
+ * ttdqn_observe_act_device given the same rings (centre + offset) appended as static solid rings,
+ * bit for bit; mv == NULL or n_live == 0 computes exactly what ttdqn_observe_act_device computes.
+ * n_live < 0, max_pv outside 3..32 or a NULL array with n_live > 0 -> TTMPC_ERR_BAD_ARG before
+ * any device work. */
+int ttdqn_observe_act_moving_device(const ttdqn_scene_layout *lay, const ttdqn_qnet *qnet,
+                                    int n_envs, const double *d_agent,
+                                    const double *d_poly_xy, const int *d_poly_off,
+                                    const int *d_is_solid, const int *d_n_poly,
+                                    const ttdqn_moving *mv,
+                                    const float *d_internal, float *d_old_ext,
+                                    float *d_ext, float *d_q, int *d_action,
+                                    double *d_seg_dist, double *d_ray_dist, void *stream);
+
 /* ------------------------------------------------------------------------
  * Fleet step: the caller side of the solve, batched on the device.
  *

@@ -8,10 +8,22 @@ all device-resident (ttdqn_internal_obs_device, ttdqn_observe_act_device, ttdqn_
 ttmpc_fleet_step_device); whether the hint is used is decided per step and environment by the
 HintSwitcher logic inside the pack kernel.
   python tools/bench_hybrid.py [n=16384] [steps=10] [--warm-start] [--skip-stopped] [--action-steps k]
+                               [--lidar-moving] [--monitor]
+
+--lidar-moving: the lidar also sees the moving obstacles, as the circle_to_rect squares the
+HintSwitcher uses, at the positions the step's pack treats as current (ttdqn_observe_act_moving_device;
+FleetPlanner.enable_dqn(moving_shape="rect") does the same).  Off by default, so that numbers stay
+comparable with earlier runs.
+--monitor: the default monitor of FleetPlanner.enable_monitor, run after each step's end event,
+outside the timed window (as tools/bench_fleet.py does); reports reached robots, robots with a
+contact and the deepest entry into a moving obstacle's disc (-min clearance; a static polygon's
+clearance is never below 0).  The 3 warm-up steps count for the monitor too.
+The card's name and power limit are read in the same run.
 """
 import argparse
 import json
 import os
+import subprocess
 import sys
 
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
@@ -19,8 +31,18 @@ import numpy as np
 import torch
 
 import trajtrack_mpcndqn_rlboost_b200 as t
+from trajtrack_mpcndqn_rlboost_b200.fleet import DYN_OBS_SIZE, REACHED
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+
+
+def card():
+    try:
+        pl = subprocess.run(["nvidia-smi", "--query-gpu=power.limit", "--format=csv,noheader", "-i",
+                             str(torch.cuda.current_device())], capture_output=True, text=True, timeout=30).stdout.strip()
+    except (OSError, subprocess.SubprocessError):
+        pl = None
+    return dict(gpu=torch.cuda.get_device_name(), power_limit=pl or None)
 
 
 def main():
@@ -30,6 +52,8 @@ def main():
     ap.add_argument("--warm-start", action="store_true", help="FleetPlanner.step(warm_start=True)")
     ap.add_argument("--skip-stopped", action="store_true", help="FleetPlanner.step(skip_stopped=True)")
     ap.add_argument("--action-steps", type=int, default=1, help="FleetPlanner(action_steps=k)")
+    ap.add_argument("--lidar-moving", action="store_true", help="the lidar sees the moving obstacles' squares")
+    ap.add_argument("--monitor", action="store_true", help="run the fleet monitor outside the timed window")
     a = ap.parse_args()
     n, steps = a.n, a.steps
     mc = t.Configurator()
@@ -62,6 +86,13 @@ def main():
     agent5 = torch.empty(n, 5, dtype=torch.float64, device="cuda")
     fp.set_hint(rl, use)
     fp.enable_hint_switch(fl["static_polys"], per_robot=True)      # HintSwitcher(10, 2, 10), main.py:129
+    moving = None
+    if a.lidar_moving:                                              # the switcher's squares, one template for all
+        k = fp.n_dyn_live
+        moving = (fp.dyn_cur, torch.from_numpy(np.repeat(t.dqn.rect_shape(DYN_OBS_SIZE)[None, None], k, 1)).cuda(),
+                  torch.full((1, k), 4, dtype=torch.int32, device="cuda"))
+    if a.monitor:
+        fp.enable_monitor()
     ev = lambda: torch.cuda.Event(enable_timing=True)
 
     def one_step(times=None):
@@ -69,12 +100,14 @@ def main():
         e[0].record()
         agent5[:, :3] = fp.state; agent5[:, 3:] = fp.last_u          # env.set_agent_state (main.py:175-176)
         t.dqn.internal_obs_device(agent5, pxy, pcnt, out=internal, progress=progress)
-        comp.observe_act_device(fp.state, xy, off, sol, cnt, internal, old, out, qs)
+        comp.observe_act_device(fp.state, xy, off, sol, cnt, internal, old, out, qs, moving=moving)
         t.dqn.rl_ref_device(agent5, out["action"], steps=fp.N, ts=mc.ts, ref_speed=1.0, out=rl)
         e[1].record()
         fp.step(keep_multipliers=os.environ.get('KEEP_Y', '1') == '1', warm_start=a.warm_start,
-                skip_stopped=a.skip_stopped)
+                skip_stopped=a.skip_stopped, monitor=False)
         e[2].record()
+        if a.monitor:
+            fp.run_monitor()
         if times is not None:
             torch.cuda.synchronize()
             times.append((e[0].elapsed_time(e[2]), e[0].elapsed_time(e[1])))
@@ -85,13 +118,16 @@ def main():
     for _ in range(steps):
         one_step(times)
     tt = np.array(times)
-    res = dict(workload=f"hybrid{n}", envs=n, warm_start=a.warm_start, skip_stopped=a.skip_stopped,
-               action_steps=a.action_steps, steps=steps, step_ms_p50=float(np.median(tt[:, 0])),
+    res = dict(workload=f"hybrid{n}", envs=n, **card(), warm_start=a.warm_start, skip_stopped=a.skip_stopped,
+               action_steps=a.action_steps, lidar_moving=a.lidar_moving, steps=steps, step_ms_p50=float(np.median(tt[:, 0])),
                step_ms_p90=float(np.quantile(tt[:, 0], 0.9)), dqn_part_ms_p50=float(np.median(tt[:, 1])),
                env_steps_per_s=n / (float(np.median(tt[:, 0])) * 1e-3),
                actions_hist=np.bincount(out["action"].cpu().numpy(), minlength=9).tolist(),
                running=int((fp.status == 0).sum()), mean_inner_iters=float(fp.inner.float().mean()),
                hint_on=int(fp.use_hint.sum()))
+    if a.monitor:
+        res.update(reached=int((fp.status == REACHED).sum()), robots_with_contact=int((fp.contact_steps > 0).sum()),
+                   deepest_moving_disc_entry=max(0.0, -float(fp.min_clearance.min())))
     print(json.dumps(res))
     os.makedirs(os.path.join(ROOT, "gpurun_out"), exist_ok=True)
     with open(os.path.join(ROOT, "gpurun_out", "bench_hybrid.json"), "a") as f:

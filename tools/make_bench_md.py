@@ -3,7 +3,9 @@
 r2_bench_static4096.json (headline), r2_bench_reference.json, r2_multi_<tag>_n<N>.json (tools/r2_multi.sh,
 tools/r2_single_sweep.sh), profiles/r2_parity_distribution_{gpu,cpu}.json, r2_qnet.json, r2_fleet.json,
 r2_hybrid.json, r2_single_latency.txt, profiles/r2_roofline_inputs.json, r2_missions.json (tools/bench_missions.py,
-one line per fleet size), r2_missions_profile.json (its --profile-pack line), r2_monitor.json (tools/bench_monitor.py)."""
+one line per fleet size), r2_missions_profile.json (its --profile-pack line), r2_monitor.json (tools/bench_monitor.py),
+r2_lidar_moving.json (tools/bench_lidar_moving.py), r2_hybrid_lidar.json (tools/bench_hybrid.py timing runs with and
+without --lidar-moving), r2_hybrid_drive.json (its --monitor drives)."""
 import glob
 import json
 import os
@@ -112,6 +114,44 @@ def monitor_section(mo):
         out.append(f"The same drive with moving_radius = 0, i.e. the rectangles alone: robots with contact {s['robots_with_contact']} "
                    f"({s['contact_steps_total']} robot-steps); min_clearance quantiles "
                    + " / ".join(f"{q[k]:.3f}" for k in ("0.0", "0.01", "0.05", "0.1", "0.5")) + " m.\n")
+    return out
+
+
+def lidar_moving_section(lm, hy, drive):
+    """Lines of the "Moving obstacles in the lidar" section: the line of tools/bench_lidar_moving.py, the lines of
+    tools/bench_hybrid.py with and without --lidar-moving (hy: timing runs, drive: --monitor runs)."""
+    if not (lm or hy or drive):
+        return []
+    out = ["## Moving obstacles in the DQN's lidar (`ttdqn_observe_act_moving_device`, `--lidar-moving`)\n"]
+    if lm:
+        m = lm["ms_per_call_median"]
+        out.append(f"`tools/bench_lidar_moving.py`, {lm['n_envs']} environments, observation + Q-network per call (median of "
+                   f"{lm['rounds']} rounds of {lm['calls']} calls), {lm['gpu']}, power limit {lm['power_limit']}: static rings alone "
+                   f"{m['static']:.3f} ms; with 2 moving squares through the new path {m['moving2']:.3f} ms; the same 2 squares "
+                   f"appended as static rings {m['appended2']:.3f} ms. Outputs of the last two identical: {lm['moving2_equals_appended2']}.\n")
+    if hy:
+        rows = {}
+        for r in hy:
+            rows.setdefault(bool(r.get("lidar_moving")), []).append(r)
+        out.append(f"`tools/bench_hybrid.py {hy[0]['envs']} {hy[0]['steps']}` (runs alternated, mean over the runs of each run's per-step p50), "
+                   f"{hy[0]['gpu']}, power limit {hy[0]['power_limit']}:\n")
+        out += ["| lidar | runs | ms / step p50 | DQN part ms p50 | env-steps / s | hint on |", "|:--|---:|---:|---:|---:|---:|"]
+        for mv, rs in sorted(rows.items()):
+            med = lambda k: sum(r[k] for r in rs) / len(rs)
+            out.append(f"| {'static + moving squares' if mv else 'static only'} | {len(rs)} | {med('step_ms_p50'):.2f} | "
+                       f"{med('dqn_part_ms_p50'):.3f} | {med('env_steps_per_s'):,.0f} | {rs[-1]['hint_on']} |")
+        out.append("")
+    if drive:
+        d0 = drive[0]
+        out.append(f"Drive: `make_fleet({d0['envs']}, seed=1000)`, {d0['steps'] + 3} steps (3 warm-up + {d0['steps']} timed), warm start + "
+                   f"skip-stopped, the default monitor ({d0['gpu']}, power limit {d0['power_limit']}). This is a finding about the planner, "
+                   "not a target: whether the trained policy steers better with the extra input was not known before this run.\n")
+        out += ["| lidar | reached | running | robots with contact | deepest moving-disc entry (m) | hint on at the end |",
+                "|:--|---:|---:|---:|---:|---:|"]
+        for r in drive:
+            out.append(f"| {'static + moving squares' if r.get('lidar_moving') else 'static only (blind)'} | {r['reached']} | {r['running']} | "
+                       f"{r['robots_with_contact']} | {r['deepest_moving_disc_entry']:.3f} | {r['hint_on']} |")
+        out.append("")
     return out
 
 
@@ -270,6 +310,8 @@ def main():
         out.append(f"{hy['envs']} environments: {hy['step_ms_p50']:.1f} ms per control step (p90 {hy['step_ms_p90']:.1f}) = {hy['env_steps_per_s']:,.0f} env-steps/s "
                    f"(round 1: 1,351,483); DQN part (internal observation + lidar + Q-net + hint rollout) {hy.get('dqn_part_ms_p50', 0):.2f} ms of it; "
                    f"{hy.get('mean_inner_iters', 0):.0f} PANOC iterations per solve.\n")
+    out += lidar_moving_section(last(os.path.join(G, "r2_lidar_moving.json")), jl(os.path.join(G, "r2_hybrid_lidar.json")),
+                                jl(os.path.join(G, "r2_hybrid_drive.json")))
     open(os.path.join(ROOT, "BENCH.md"), "w").write("\n".join(out) + "\n")
     print("\n".join(out))
 

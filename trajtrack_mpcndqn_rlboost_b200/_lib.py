@@ -57,6 +57,14 @@ class TtdqnQnet(C.Structure):
     ]
 
 
+class TtdqnMoving(C.Structure):
+    """struct ttdqn_moving: moving solid rings of ttdqn_observe_act_moving_device (device addresses)."""
+    _fields_ = [
+        ("n_live", C.c_int), ("max_pv", C.c_int), ("shape_shared", C.c_int), ("_pad", C.c_int),
+        ("centre", C.c_void_p), ("shape_xy", C.c_void_p), ("shape_nv", C.c_void_p),
+    ]
+
+
 FLEET_WARM_START, FLEET_SKIP_STOPPED = 1, 2  # ttmpc_fleet.options bits
 
 
@@ -106,7 +114,7 @@ class TtmpcFleetMonitor(C.Structure):
 # every symbol include/ttmpc.h declares, with its signature
 _VP, _I, _D = C.c_void_p, C.c_int, C.c_double
 _CFG, _RES = C.POINTER(TtmpcConfig), C.POINTER(TtmpcResult)
-_LAY, _QN = C.POINTER(TtdqnLayout), C.POINTER(TtdqnQnet)
+_LAY, _QN, _MOV = C.POINTER(TtdqnLayout), C.POINTER(TtdqnQnet), C.POINTER(TtdqnMoving)
 _FLT = C.POINTER(TtmpcFleet)
 _TSK = C.POINTER(TtmpcFleetTasks)
 _MON = C.POINTER(TtmpcFleetMonitor)
@@ -136,6 +144,7 @@ SYMBOLS = {
     "ttdqn_last_error": (C.c_char_p, []),
     "ttdqn_default_layout": (None, [_LAY]),
     "ttdqn_observe_act_device": (_I, [_LAY, _QN, _I] + [_VP] * 12 + [_VP]),
+    "ttdqn_observe_act_moving_device": (_I, [_LAY, _QN, _I] + [_VP] * 5 + [_MOV] + [_VP] * 7 + [_VP]),
     "ttdqn_observe_act_host": (_I, [_LAY, _QN, _I] + [_VP] * 12),
     "ttdqn_internal_obs_device": (_I, [_I, _I, _I, _D, _D, _VP, _VP, _VP, _VP, _VP, _VP]),
     "ttdqn_rl_ref_device": (_I, [_I, _I, _D, _D, _VP, _VP, _VP, _VP]),

@@ -13,7 +13,9 @@
 // the closest point of T^G to A lies on G's boundary whenever A is outside G, so
 // the sector distance is min over edges e of dist(A, e clipped to T); the ray
 // distance is the first hit along the centre ray.  A inside a solid ring gives 0
-// for every sector.  Lanes split the edges; the 16 minima are warp-reduced.
+// for every sector.  Lanes split the edges; the 16 minima are warp-reduced.  Moving
+// solid rings (ttdqn_moving, observe_act_moving_kernel) spread their (ring, edge) pairs over the
+// lanes instead (moving_minima).
 //
 // The Q-network (46-16-16-9 for the reference's ray model) runs on the TENSOR CORES in its own
 // kernel, qnet_mma_kernel: 16 environments per warp tile, mma.sync.m16n8k8 TF32 with fp32
@@ -122,8 +124,70 @@ __device__ __forceinline__ double wmin(double v) {
   return v;
 }
 
-// shared memory per block: Q-net weights (once) + per-warp scratch
-__global__ void __launch_bounds__(128) observe_act_kernel(const __grid_constant__ Args A) {
+// one edge p0 -> p1 into this lane's running sector and ray minima
+__device__ __forceinline__ void edge_minima(const Sector *sec, int ns, double ax, double ay, double L,
+                                            double p0x, double p0y, double p1x, double p1y,
+                                            double (&dseg)[MAX_SEG], double (&dray)[MAX_SEG]) {
+  const double dx = p1x - p0x, dy = p1y - p0y;
+  const double dd = dx * dx + dy * dy;
+#pragma unroll
+  for (int i = 0; i < MAX_SEG; i++) {
+    if (i < ns) {
+      const Sector &S = sec[i];
+      double t0, t1;
+      if (clip_to_triangle(S, p0x, p0y, dx, dy, t0, t1)) {
+        double t = t0;
+        if (dd > 0.0) {
+          t = ((ax - p0x) * dx + (ay - p0y) * dy) / dd;
+          t = fmin(fmax(t, t0), t1);
+        }
+        const double qx = p0x + t * dx - ax, qy = p0y + t * dy - ay;
+        dseg[i] = fmin(dseg[i], sqrt(qx * qx + qy * qy));
+      }
+      dray[i] = fmin(dray[i], ray_seg_hit(ax, ay, S.rx, S.ry, L, p0x, p0y, p1x, p1y));
+    }
+  }
+}
+
+// Moving solid rings (ttdqn_moving): the (ring, edge) pairs are spread over the lanes, 32 / max_pv
+// whole rings per pass, lane = slot * max_pv + edge.  Each lane forms its edge e -> e+1 of ring
+// centre + offset and the even-odd crossing of the pair (e+1, e), which is the pair the static ring
+// loop tests on lane e+1; a ballot masked to the ring's lanes gives the ring's parity.  Every edge
+// is the same arithmetic as for a static ring and min / OR ignore the order, so the result equals
+// that of the rings appended as static solid rings.  Returns whether the agent is inside any ring.
+__device__ __forceinline__ bool moving_minima(const ttdqn_moving &M, int env, int lane, const Sector *sec, int ns,
+                                              double ax, double ay, double L, double (&dseg)[MAX_SEG],
+                                              double (&dray)[MAX_SEG]) {
+  const int pv = M.max_pv, per = 32 / pv, slot = lane / pv, e = lane - slot * pv;
+  const unsigned mask = slot < per ? ((pv == 32 ? FULL : (1u << pv) - 1u) << (slot * pv)) : 0u;
+  const double *cen = M.centre + (size_t)env * M.n_live * 2;
+  const double *sxy = M.shape_xy + (M.shape_shared ? 0 : (size_t)env * M.n_live * pv * 2);
+  const int *snv = M.shape_nv + (M.shape_shared ? 0 : (size_t)env * M.n_live);
+  bool inside = false;
+  for (int o0 = 0; o0 < M.n_live; o0 += per) {
+    const int o = o0 + slot;
+    const int nv = (slot < per && o < M.n_live) ? min(snv[o], pv) : 0;
+    const bool edge = nv >= 3 && e < nv;
+    double p0x = 0.0, p0y = 0.0, p1x = 0.0, p1y = 0.0;
+    int cross = 0;
+    if (edge) {
+      const double cx = cen[2 * o], cy = cen[2 * o + 1], *r = sxy + (size_t)o * pv * 2;
+      const int e2 = (e + 1 == nv) ? 0 : e + 1;
+      p0x = cx + r[2 * e]; p0y = cy + r[2 * e + 1];
+      p1x = cx + r[2 * e2]; p1y = cy + r[2 * e2 + 1];
+      if (((p1y > ay) != (p0y > ay)) && (ax < (p0x - p1x) * (ay - p1y) / (p0y - p1y) + p1x)) cross = 1;
+    }
+    const bool in_ring = (__popc(__ballot_sync(FULL, cross) & mask) & 1) != 0;
+    inside = inside || in_ring;
+    if (edge && !in_ring) edge_minima(sec, ns, ax, ay, L, p0x, p0y, p1x, p1y, dseg, dray);
+  }
+  return __any_sync(FULL, inside);
+}
+
+// shared memory per block: Q-net weights (once) + per-warp scratch.  MOVING: also the moving rings
+// of ttdqn_moving (n_live > 0); the instantiation without them is observe_act_kernel.
+template <bool MOVING>
+__device__ __forceinline__ void observe_act_body(const Args A, const ttdqn_moving M) {
   extern __shared__ __align__(16) unsigned char smem_raw[];
   const int warps = blockDim.x >> 5, warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
   const int ns = A.lay.num_segments;
@@ -188,28 +252,10 @@ __global__ void __launch_bounds__(128) observe_act_kernel(const __grid_constant_
       }
       for (int e = lane; e < nv; e += 32) {
         const int e2 = (e + 1 == nv) ? 0 : e + 1;
-        const double p0x = r[2 * e], p0y = r[2 * e + 1], p1x = r[2 * e2], p1y = r[2 * e2 + 1];
-        const double dx = p1x - p0x, dy = p1y - p0y;
-        const double dd = dx * dx + dy * dy;
-#pragma unroll
-        for (int i = 0; i < MAX_SEG; i++) {
-          if (i < ns) {
-            const Sector &S = sec[i];
-            double t0, t1;
-            if (clip_to_triangle(S, p0x, p0y, dx, dy, t0, t1)) {
-              double t = t0;
-              if (dd > 0.0) {
-                t = ((ax - p0x) * dx + (ay - p0y) * dy) / dd;
-                t = fmin(fmax(t, t0), t1);
-              }
-              const double qx = p0x + t * dx - ax, qy = p0y + t * dy - ay;
-              dseg[i] = fmin(dseg[i], sqrt(qx * qx + qy * qy));
-            }
-            dray[i] = fmin(dray[i], ray_seg_hit(ax, ay, S.rx, S.ry, L, p0x, p0y, p1x, p1y));
-          }
-        }
+        edge_minima(sec, ns, ax, ay, L, r[2 * e], r[2 * e + 1], r[2 * e2], r[2 * e2 + 1], dseg, dray);
       }
     }
+    if (MOVING && moving_minima(M, env, lane, sec, ns, ax, ay, L, dseg, dray)) inside_any = true;
 #pragma unroll
     for (int i = 0; i < MAX_SEG; i++) {
       if (i < ns) {
@@ -270,6 +316,13 @@ __global__ void __launch_bounds__(128) observe_act_kernel(const __grid_constant_
     }
     __syncwarp();
   }
+}
+__global__ void __launch_bounds__(128) observe_act_kernel(const __grid_constant__ Args A) {
+  observe_act_body<false>(A, ttdqn_moving{});
+}
+__global__ void __launch_bounds__(128) observe_act_moving_kernel(const __grid_constant__ Args A,
+                                                                 const __grid_constant__ ttdqn_moving M) {
+  observe_act_body<true>(A, M);
 }
 
 // ------------------------------------------------------------------ Q-network on the tensor cores
@@ -544,17 +597,22 @@ extern "C" void ttdqn_default_layout(ttdqn_scene_layout *l) {
   l->use_memory = 1; l->_pad = 0; l->ray_length = 1000.0; l->max_distance = 10.0;
 }
 
-extern "C" int ttdqn_observe_act_device(const ttdqn_scene_layout *lay, const ttdqn_qnet *qn, int n,
-                                        const double *d_agent, const double *d_poly_xy,
-                                        const int *d_poly_off, const int *d_is_solid,
-                                        const int *d_n_poly, const float *d_internal,
-                                        float *d_old_ext, float *d_ext, float *d_q, int *d_action,
-                                        double *d_seg, double *d_ray, void *stream) {
+static int observe_act(const ttdqn_scene_layout *lay, const ttdqn_qnet *qn, int n, const double *d_agent,
+                       const double *d_poly_xy, const int *d_poly_off, const int *d_is_solid, const int *d_n_poly,
+                       const ttdqn_moving *mv, const float *d_internal, float *d_old_ext, float *d_ext,
+                       float *d_q, int *d_action, double *d_seg, double *d_ray, void *stream) {
   using namespace ttdqn;
   if (!lay || n < 0) return dfail(TTMPC_ERR_BAD_ARG, "layout required, n >= 0");
   if (lay->num_segments < 1 || lay->num_segments > MAX_SEG)
     return dfail(TTMPC_ERR_BAD_CONFIG, "num_segments must be in 1..16");
   if (lay->use_memory && !d_old_ext) return dfail(TTMPC_ERR_BAD_ARG, "use_memory needs d_old_ext");
+  if (mv) {
+    if (mv->n_live < 0) return dfail(TTMPC_ERR_BAD_ARG, "moving: n_live must be >= 0");
+    if (mv->max_pv < 3 || mv->max_pv > 32) return dfail(TTMPC_ERR_BAD_ARG, "moving: max_pv must be in 3..32");
+    if (mv->n_live > 0 && (!mv->centre || !mv->shape_xy || !mv->shape_nv))
+      return dfail(TTMPC_ERR_BAD_ARG, "moving: centre, shape_xy and shape_nv are required with n_live > 0");
+  }
+  const bool moving = mv && mv->n_live > 0;
   if (n == 0) return TTMPC_OK;
   if (!d_agent || !d_poly_xy || !d_poly_off || !d_is_solid || !d_n_poly)
     return dfail(TTMPC_ERR_BAD_ARG, "agent and geometry pointers are required");
@@ -609,13 +667,17 @@ extern "C" int ttdqn_observe_act_device(const ttdqn_scene_layout *lay, const ttd
   size_t per_warp = (sizeof(Sector) * MAX_SEG + sizeof(float) * (size_t)(A.n_in + A.n_h1 + A.n_h2 + A.n_out + 4) + 15) / 16 * 16;
   size_t smem = wbytes + per_warp * warps;
   DQN_TRY(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev));
-  DQN_TRY(cudaFuncSetAttribute(observe_act_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+  const void *kern = moving ? (const void *)observe_act_moving_kernel : (const void *)observe_act_kernel;
+  DQN_TRY(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
   int bps = 0;
-  DQN_TRY(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&bps, observe_act_kernel, warps * 32, smem));
+  DQN_TRY(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&bps, kern, warps * 32, smem));
   if (bps < 1) return dfail(TTMPC_ERR_UNSUPPORTED, "observe_act kernel does not fit");
   long long want = ((long long)n + warps - 1) / warps, cap = (long long)sms * bps;
   const int grid = (int)(want < cap ? want : cap);
-  observe_act_kernel<<<grid, warps * 32, smem, (cudaStream_t)stream>>>(A);
+  if (moving)
+    observe_act_moving_kernel<<<grid, warps * 32, smem, (cudaStream_t)stream>>>(A, *mv);
+  else
+    observe_act_kernel<<<grid, warps * 32, smem, (cudaStream_t)stream>>>(A);
   DQN_TRY(cudaGetLastError());
   if (mma) {
     QArgs Q;
@@ -631,6 +693,27 @@ extern "C" int ttdqn_observe_act_device(const ttdqn_scene_layout *lay, const ttd
     DQN_TRY(cudaFreeAsync(d_obs, (cudaStream_t)stream));
   }
   return TTMPC_OK;
+}
+
+extern "C" int ttdqn_observe_act_device(const ttdqn_scene_layout *lay, const ttdqn_qnet *qn, int n,
+                                        const double *d_agent, const double *d_poly_xy,
+                                        const int *d_poly_off, const int *d_is_solid,
+                                        const int *d_n_poly, const float *d_internal,
+                                        float *d_old_ext, float *d_ext, float *d_q, int *d_action,
+                                        double *d_seg, double *d_ray, void *stream) {
+  return observe_act(lay, qn, n, d_agent, d_poly_xy, d_poly_off, d_is_solid, d_n_poly, nullptr, d_internal,
+                     d_old_ext, d_ext, d_q, d_action, d_seg, d_ray, stream);
+}
+
+extern "C" int ttdqn_observe_act_moving_device(const ttdqn_scene_layout *lay, const ttdqn_qnet *qn, int n,
+                                               const double *d_agent, const double *d_poly_xy,
+                                               const int *d_poly_off, const int *d_is_solid,
+                                               const int *d_n_poly, const ttdqn_moving *mv,
+                                               const float *d_internal, float *d_old_ext, float *d_ext,
+                                               float *d_q, int *d_action, double *d_seg, double *d_ray,
+                                               void *stream) {
+  return observe_act(lay, qn, n, d_agent, d_poly_xy, d_poly_off, d_is_solid, d_n_poly, mv, d_internal,
+                     d_old_ext, d_ext, d_q, d_action, d_seg, d_ray, stream);
 }
 
 extern "C" int ttdqn_observe_act_host(const ttdqn_scene_layout *lay, const ttdqn_qnet *qn, int n,

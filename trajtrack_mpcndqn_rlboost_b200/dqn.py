@@ -17,7 +17,7 @@ from typing import List, Sequence
 import numpy as np
 
 from . import _lib
-from ._lib import TtdqnLayout, TtdqnQnet
+from ._lib import TtdqnLayout, TtdqnMoving, TtdqnQnet
 
 
 def default_layout(max_poly: int = 16, max_vert: int = 512) -> TtdqnLayout:
@@ -122,18 +122,56 @@ class DqnCompanion:
         return dict(ext=ext, q=q, action=act, seg=seg, ray=ray, old_ext=old_ext)
 
     def observe_act_device(self, agent, xy, off, sol, cnt, internal, old_ext, out: dict, qstruct,
-                           stream=None):
-        """All arguments are CUDA torch tensors; out holds ext/q/action/seg/ray tensors."""
+                           stream=None, moving=None):
+        """All arguments are CUDA torch tensors; out holds ext/q/action/seg/ray tensors.
+        moving=(centre [n][k][2] float64, shape_xy [n or 1][k][max_pv][2] float64, shape_nv [n or 1][k]
+        int32): k moving solid rings per env, vertex offsets placed at the centres
+        (ttdqn_observe_act_moving_device); None: the static rings alone."""
         import torch
         st = torch.cuda.current_stream().cuda_stream if stream is None else stream
         dp = lambda t: None if t is None else t.data_ptr()
-        rc = self.lib.ttdqn_observe_act_device(
-            C.byref(self.lay), C.byref(qstruct) if qstruct else None, agent.shape[0], dp(agent), dp(xy),
-            dp(off), dp(sol), dp(cnt), dp(internal), dp(old_ext), dp(out.get("ext")), dp(out.get("q")),
-            dp(out.get("action")), dp(out.get("seg")), dp(out.get("ray")), C.c_void_p(st))
+        outs = (dp(out.get("ext")), dp(out.get("q")), dp(out.get("action")), dp(out.get("seg")), dp(out.get("ray")))
+        qs = C.byref(qstruct) if qstruct else None
+        if moving is None:
+            rc = self.lib.ttdqn_observe_act_device(
+                C.byref(self.lay), qs, agent.shape[0], dp(agent), dp(xy), dp(off), dp(sol), dp(cnt),
+                dp(internal), dp(old_ext), *outs, C.c_void_p(st))
+        else:
+            mv = moving_struct(agent.shape[0], *moving)
+            rc = self.lib.ttdqn_observe_act_moving_device(
+                C.byref(self.lay), qs, agent.shape[0], dp(agent), dp(xy), dp(off), dp(sol), dp(cnt), C.byref(mv),
+                dp(internal), dp(old_ext), *outs, C.c_void_p(st))
         if rc != 0:
-            raise _lib.TtmpcError(f"ttdqn_observe_act_device failed (code {rc})")
+            raise _lib.TtmpcError(f"ttdqn_observe_act_device failed (code {rc}): {self.lib.ttdqn_last_error().decode()}")
         return out
+
+
+def rect_shape(radius: float) -> np.ndarray:
+    """circle_to_rect of a moving obstacle as offsets from its centre, [4][2], in the vertex order the
+    HintSwitcher's squares have (main.py:91-95): centre + rect_shape(r) is that square, bit for bit."""
+    r = float(radius)
+    return np.array([(-r, -r), (r, -r), (r, r), (-r, r)], dtype=np.float64)
+
+
+def moving_struct(n: int, centre, shape_xy, shape_nv) -> TtdqnMoving:
+    """ttdqn_moving of CUDA tensors centre [n][k][2] float64, shape_xy [n or 1][k][max_pv][2] float64
+    and shape_nv [n or 1][k] int32 (shape_xy / shape_nv with one row: one template block for every
+    env).  The tensors must outlive the call that uses the struct."""
+    import torch
+    if centre.dim() != 3 or centre.shape[0] != n or centre.shape[2] != 2 or centre.dtype != torch.float64:
+        raise ValueError(f"moving centre must be float64 [{n}][k][2], got {tuple(centre.shape)} {centre.dtype}")
+    k = centre.shape[1]
+    if (shape_xy.dim() != 4 or shape_xy.shape[0] not in (1, n) or shape_xy.shape[1] != k or shape_xy.shape[3] != 2
+            or shape_xy.dtype != torch.float64 or not 3 <= shape_xy.shape[2] <= 32):
+        raise ValueError(f"moving shape_xy must be float64 [{n} or 1][{k}][3..32][2], got "
+                         f"{tuple(shape_xy.shape)} {shape_xy.dtype}")
+    if tuple(shape_nv.shape) != tuple(shape_xy.shape[:2]) or shape_nv.dtype != torch.int32:
+        raise ValueError(f"moving shape_nv must be int32 {tuple(shape_xy.shape[:2])}, got "
+                         f"{tuple(shape_nv.shape)} {shape_nv.dtype}")
+    if not all(a.is_cuda and a.is_contiguous() for a in (centre, shape_xy, shape_nv)):
+        raise ValueError("moving tensors must be contiguous CUDA tensors")
+    return TtdqnMoving(k, shape_xy.shape[2], 1 if shape_xy.shape[0] == 1 else 0, 0,
+                       centre.data_ptr(), shape_xy.data_ptr(), shape_nv.data_ptr())
 
 
 def pack_paths(paths, max_nodes: int = None):

@@ -106,6 +106,8 @@ class FleetPlanner:
         self.task_next = None  # [n] int32: queued tasks taken so far
         self.static_polys = None  # (polygons, per_robot) of the last update_static_constraints
         self.monitor = None    # _lib.TtmpcFleetMonitor (enable_monitor), None: no monitor
+        self.dqn_paths = None  # (path_xy, path_n) the task step keeps current (set_tasks / enable_dqn)
+        self._dqn = None       # the DQN side of the step (enable_dqn), None: off
         self.steps = 0
 
     # ------------------------------------------------------------------ obstacles
@@ -258,9 +260,12 @@ class FleetPlanner:
         ``ref_stride`` grows, keeping the rows, to cover every queued task from a start within
         GOAL_REACH of the goal before it.  dqn_paths=(path_xy [n][m][2] float64, path_n [n] int32),
         the CUDA tensors the hybrid loop passes to ``dqn.internal_obs_device``: the step writes each
-        robot's current path there when it takes a task (m must hold the longest task path)."""
+        robot's current path there when it takes a task (m must hold the longest task path).  With
+        the DQN enabled (``enable_dqn``) and dqn_paths not given, its path tensors are the ones kept."""
         t = self.torch
         n = self.n
+        if dqn_paths is None and self._dqn is not None:
+            dqn_paths = self._dqn.paths
         if len(goals) != n or len(paths) != n or any(len(g) != len(p) for g, p in zip(goals, paths)):
             raise ValueError("set_tasks: one list of goals and one of paths per robot, of equal lengths")
         T = max(len(g) for g in goals)
@@ -304,6 +309,138 @@ class FleetPlanner:
             tk.path_out, tk.path_out_n = dqn_paths[0].data_ptr(), dqn_paths[1].data_ptr()
         self.dqn_paths = dqn_paths
         self.tasks = tk if int(self.task_count.sum()) > 0 else None
+
+    # ------------------------------------------------------------------ DQN
+    def enable_dqn(self, weights, geometry, paths, layout=None, moving_shape="rect",
+                   moving_radius: float = DYN_OBS_SIZE, ref_speed: float = 1.0, corner_samples: int = 3,
+                   sample_offset: float = 0.0):
+        """Run the DQN side of the hybrid loop (main.py:174-193) at the start of every ``step()``, on
+        the step's stream: ``agent5`` <- (state, last_u); the internal observation
+        (``dqn.internal_obs_device``); lidar observation + Q-network + argmax
+        (``DqnCompanion.observe_act_device``, with ``use_memory`` on the layout's memory rows); the
+        rl_ref rollout of the chosen action into ``self.hint``.  The fleet step follows as before.
+
+        weights: ``dqn.QNetWeights``.  geometry: the CUDA tensors of ``dqn.pack_geometry``
+        (xy [n][max_vert][2] float64, off [n][max_poly+1], solid [n][max_poly], count [n] int32);
+        layout defaults to ``dqn.default_layout`` with those max_poly / max_vert.  paths: the CUDA
+        tensors of ``dqn.pack_paths`` (path_xy [n][m][2] float64, path_n [n] int32); task queues keep
+        them current (``set_tasks``).
+
+        moving_shape: how the lidar sees the moving obstacles of ``set_moving_obstacles``, as solid
+        rings at the positions this step's pack treats as current (``dyn_cur``): ``"rect"`` the
+        ``circle_to_rect`` square of moving_radius the HintSwitcher uses, a ``[k][nv][2]`` array of
+        vertex offsets (one template per moving obstacle, 3 <= nv <= 32), or None (not seen: the
+        static geometry alone).
+
+        Results, overwritten by every step: ``dqn_action`` [n] int32, ``dqn_q`` [n][n_out],
+        ``dqn_ext`` [n][n_ext] float32 and ``hint`` [n][N][2].  Whether a robot follows the hint is
+        decided as without the DQN: ``use_hint`` (zeros unless set), or the switcher of
+        ``enable_hint_switch``."""
+        from types import SimpleNamespace
+
+        from . import dqn
+        t = self.torch
+        n, dev = self.n, self.state.device
+
+        def want(x, name, dtype, shape):
+            if not isinstance(x, t.Tensor) or x.dtype != dtype or tuple(x.shape) != tuple(shape):
+                got = (tuple(x.shape), x.dtype) if isinstance(x, t.Tensor) else type(x).__name__
+                raise ValueError(f"enable_dqn: {name} must be a {dtype} tensor {tuple(shape)}, got {got}")
+
+        if len(geometry) != 4 or len(paths) != 2:
+            raise ValueError("enable_dqn: geometry = (xy, off, solid, count), paths = (path_xy, path_n)")
+        xy, off, sol, cnt = geometry
+        path_xy, path_n = paths
+        if layout is None:
+            if not (isinstance(xy, t.Tensor) and xy.dim() == 3 and isinstance(sol, t.Tensor) and sol.dim() == 2):
+                raise ValueError("enable_dqn: geometry xy must be [n][max_vert][2] and solid [n][max_poly]")
+            layout = dqn.default_layout(max_poly=sol.shape[1], max_vert=xy.shape[1])
+        want(xy, "geometry xy", t.float64, (n, layout.max_vert, 2))
+        want(off, "geometry off", t.int32, (n, layout.max_poly + 1))
+        want(sol, "geometry solid", t.int32, (n, layout.max_poly))
+        want(cnt, "geometry count", t.int32, (n,))
+        if not (isinstance(path_xy, t.Tensor) and path_xy.dim() == 3 and path_xy.shape[1] >= 2):
+            raise ValueError("enable_dqn: path_xy must be [n][m >= 2][2]")
+        want(path_xy, "path_xy", t.float64, (n, path_xy.shape[1], 2))
+        want(path_n, "path_n", t.int32, (n,))
+        if 5 + 3 * int(corner_samples) != layout.n_internal or corner_samples < 0:
+            raise ValueError(f"enable_dqn: 5 + 3 * corner_samples must equal the layout's n_internal {layout.n_internal}")
+        ns = layout.num_segments
+        n_ext = (4 if layout.use_memory else 2) * ns
+        if weights.n_in != n_ext + layout.n_internal:
+            raise ValueError(f"enable_dqn: Q-network input {weights.n_in} != {n_ext} + {layout.n_internal}")
+        shape = None
+        if isinstance(moving_shape, str):
+            if moving_shape != "rect":
+                raise ValueError(f"enable_dqn: moving_shape must be 'rect', a [k][nv][2] array or None, got {moving_shape!r}")
+            if not (np.isfinite(moving_radius) and moving_radius >= 0.0):
+                raise ValueError("enable_dqn: moving_radius must be finite and >= 0")
+            shape = dqn.rect_shape(moving_radius)[None]
+        elif moving_shape is not None:
+            shape = np.asarray(moving_shape, dtype=np.float64)
+            if shape.ndim != 3 or shape.shape[2] != 2 or not 3 <= shape.shape[1] <= 32:
+                raise ValueError(f"enable_dqn: moving_shape must be [k][3..32][2], got {shape.shape}")
+        if not all(x.is_cuda and x.is_contiguous() for x in (xy, off, sol, cnt, path_xy, path_n)):
+            raise ValueError("enable_dqn: geometry and path tensors must be contiguous CUDA tensors")
+        if self.tasks is not None and (self.dqn_paths is None or self.dqn_paths[0] is not path_xy):
+            if self.tasks.max_nodes != path_xy.shape[1]:
+                raise ValueError(f"enable_dqn: path_xy holds {path_xy.shape[1]} nodes, the queued tasks "
+                                 f"{self.tasks.max_nodes}: call set_tasks after enable_dqn")
+            self.tasks.path_out, self.tasks.path_out_n = path_xy.data_ptr(), path_n.data_ptr()
+            self.dqn_paths = (path_xy, path_n)
+        f32 = dict(dtype=t.float32, device=dev)
+        w = [t.from_numpy(a).to(dev) for a in weights.arrays]
+        d = SimpleNamespace(
+            lay=layout, geometry=(xy, off, sol, cnt), paths=(path_xy, path_n), shape=shape, shape_dev=None,
+            ref_speed=float(ref_speed), corner_samples=int(corner_samples), sample_offset=float(sample_offset),
+            comp=dqn.DqnCompanion(layout, weights), w=w,
+            qnet=_lib.TtdqnQnet(weights.n_in, weights.n_h1, weights.n_h2, weights.n_out, *[a.data_ptr() for a in w]),
+            agent5=t.zeros(n, 5, dtype=t.float64, device=dev), internal=t.zeros(n, layout.n_internal, **f32),
+            progress=t.zeros(n, dtype=t.float64, device=dev),
+            old_ext=t.zeros(n, 2 * ns, **f32) if layout.use_memory else None)
+        self.dqn_ext = t.zeros(n, n_ext, **f32)
+        self.dqn_q = t.zeros(n, weights.n_out, **f32)
+        self.dqn_action = t.zeros(n, dtype=t.int32, device=dev)
+        self.hint = t.zeros(n, self.N, 2, dtype=t.float64, device=dev)
+        if self.use_hint is None:
+            self.use_hint = t.zeros(n, dtype=t.int32, device=dev)
+        self._dqn = d
+
+    def _moving_shapes(self):
+        """(shape_xy [1][k][nv][2], shape_nv [1][k]) device tensors of the lidar's moving rings for the
+        current k = n_dyn_live, or None when the lidar does not see moving obstacles."""
+        d = self._dqn
+        if d.shape is None or self.dyn_cur is None or self.n_dyn_live == 0:
+            return None
+        k = self.n_dyn_live
+        if d.shape_dev is None or d.shape_dev[0].shape[1] != k:
+            xy = d.shape
+            if len(xy) == 1:
+                xy = np.repeat(xy, k, axis=0)
+            if len(xy) != k:
+                raise ValueError(f"enable_dqn: {len(xy)} moving shapes for {k} moving obstacles")
+            dev = self.state.device
+            d.shape_dev = (self.torch.tensor(xy[None], device=dev),
+                           self.torch.full((1, k), xy.shape[1], dtype=self.torch.int32, device=dev))
+        return d.shape_dev
+
+    def _dqn_step(self, st, stream):
+        import contextlib
+
+        from . import dqn
+        d, t = self._dqn, self.torch
+        xy, off, sol, cnt = d.geometry
+        with contextlib.nullcontext() if stream is None else t.cuda.stream(t.cuda.ExternalStream(stream)):
+            d.agent5[:, :3] = self.state                                 # env.set_agent_state (main.py:175-176)
+            d.agent5[:, 3:] = self.last_u
+        dqn.internal_obs_device(d.agent5, *d.paths, corner_samples=d.corner_samples, sample_offset=d.sample_offset,
+                                max_distance=d.lay.max_distance, out=d.internal, progress=d.progress, stream=st)
+        shapes = self._moving_shapes()
+        d.comp.observe_act_device(self.state, xy, off, sol, cnt, d.internal, d.old_ext,
+                                  dict(ext=self.dqn_ext, q=self.dqn_q, action=self.dqn_action), d.qnet, stream=st,
+                                  moving=None if shapes is None else (self.dyn_cur, *shapes))
+        dqn.rl_ref_device(d.agent5, self.dqn_action, steps=self.N, ts=self.config.ts, ref_speed=d.ref_speed,
+                          out=self.hint, stream=st)
 
     # ------------------------------------------------------------------ the step
     def _fleet_struct(self) -> _lib.TtmpcFleet:
@@ -371,8 +508,13 @@ class FleetPlanner:
 
         With the monitor enabled (``enable_monitor``) the step ends with it, on the same stream;
         monitor=False leaves it to a ``run_monitor()`` call before the next step (a benchmark that
-        times the step alone does that)."""
+        times the step alone does that).
+
+        With the DQN enabled (``enable_dqn``) the step starts with the DQN side of the hybrid loop,
+        which writes ``hint``, on the same stream."""
         st = stream if stream is not None else self.torch.cuda.current_stream().cuda_stream
+        if self._dqn is not None:
+            self._dqn_step(st, stream)
         f, r = self._fleet_struct(), self._result_struct()
         f.options = (_lib.FLEET_WARM_START if warm_start else 0) | (_lib.FLEET_SKIP_STOPPED if skip_stopped else 0)
         if self.tasks is not None:
