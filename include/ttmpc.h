@@ -199,13 +199,14 @@ int ttmpc_eval_batch_host(const ttmpc_config *cfg, int n_scenes,
  * Batched layout: fixed capacity per env: max_poly rings, max_vert vertices.
  * ------------------------------------------------------------------------ */
 typedef struct ttdqn_scene_layout {
-  int num_segments; /* 8 (rays_reward1.py:20)                              */
+  int num_segments; /* 8 (rays_reward1.py:20); 3..16, else TTMPC_ERR_BAD_CONFIG */
   int max_poly;     /* ring slots per env                                  */
   int max_vert;     /* vertex slots per env (sum over rings)               */
   int n_internal;   /* 14 internal observation entries                     */
   int use_memory;   /* 1: external obs = [seg, ray, old_seg, old_ray]      */
   int _pad;
-  double ray_length;   /* L = 1000 (ext_obsv_sector_and_ray.py:34)         */
+  double ray_length;   /* L = 1000 (ext_obsv_sector_and_ray.py:34): the sector
+                        * triangles reach L, the centre rays are L long     */
   double max_distance; /* normalize_distance max_distance = 10 (utils.py:10) */
 } ttdqn_scene_layout;
 
@@ -214,7 +215,7 @@ typedef struct ttdqn_scene_layout {
  * (SB3 CombinedExtractor concatenates Dict keys in sorted order:
  *  'external' then 'internal').                                           */
 typedef struct ttdqn_qnet {
-  int n_in, n_h1, n_h2, n_out; /* 46, 16, 16, 9 */
+  int n_in, n_h1, n_h2, n_out; /* 46, 16, 16, 9; n_h1, n_h2 1..256, n_out 1..64 */
   const float *w0, *b0, *w1, *b1, *w2, *b2;
 } ttdqn_qnet;
 
@@ -232,7 +233,18 @@ const char *ttdqn_last_error(void);
  *              (NULL when use_memory == 0)
  * outputs (any may be NULL): d_ext [n][n_ext] fp32, d_q [n][n_out] fp32,
  *   d_action [n] int32, d_seg_dist / d_ray_dist [n][num_segments] fp64 raw distances.
- * qnet pointers are device pointers.                                      */
+ * qnet pointers are device pointers.
+ * Sector i is the triangle with apex at the agent and far vertices at ray_length, at angles
+ * theta + i * 2 pi / num_segments -+ pi / num_segments; its ray is the centre line, ray_length long.
+ * A ring's ray hit counts only in the sectors whose triangle the ring meets (the reference
+ * intersects the ray only when the sector intersection is non-empty).
+ * Q-network: 16-wide hidden layers with n_out <= 16 and n_in <= 248 run on the tensor cores (an
+ * exact three-way TF32 split of every operand); every other shape runs on the FMA pipe with fp64
+ * accumulation and one rounding to fp32 per neuron.  The FMA path keeps all weights in shared
+ * memory: 4 * (n_in*n_h1 + n_h1 + n_h1*n_h2 + n_h2 + n_h2*n_out + n_out) bytes rounded up to 16,
+ * plus 4 warps x (1024 + 4 * (n_in + n_h1 + n_h2 + n_out + 4) rounded up to 16) of scratch.  More
+ * than the device's opt-in shared memory per block -> TTMPC_ERR_UNSUPPORTED before any device work
+ * (ttdqn_last_error names both numbers).                                  */
 int ttdqn_observe_act_device(const ttdqn_scene_layout *lay, const ttdqn_qnet *qnet,
                              int n_envs, const double *d_agent,
                              const double *d_poly_xy, const int *d_poly_off,
@@ -511,7 +523,8 @@ int ttmpc_fleet_monitor_device(const ttmpc_config *cfg, const ttmpc_fleet *fleet
  *   corner_samples) -- components/int_obsv_*.py -- with path_progress =
  *   path.project(agent) (environment.py:115).
  *     d_agent5   [n][5]  x y theta v w
- *     d_path_xy  [n][max_nodes][2] reference-path polyline, d_path_n [n] node counts (>= 2)
+ *     d_path_xy  [n][max_nodes][2] reference-path polyline, d_path_n [n] node counts
+ *                (1..max_nodes; one node is a path of length 0 at that point)
  *     d_internal [n][5 + 3*corner_samples] fp32 out, d_progress [n] out (may be NULL)
  * ttdqn_rl_ref_device: the DQN "hint" trajectory: MobileRobot.step(action, ts) followed by
  *   steps-1 x step_with_ref_speed(ts, ref_speed) on a copy of the agent

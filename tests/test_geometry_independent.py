@@ -36,48 +36,58 @@ def boundary_samples(poly, spacing):
     return np.concatenate(out)
 
 
-def brute_sector_ray(agent, rings, solid, ns=8, r_max=40.0, dr=2e-3, dth=2e-4):
+def brute_sector_ray(agent, rings, solid, ns=8, r_max=40.0, dr=2e-3, dth=2e-4, ray_length=None):
     """Reference semantics by sampling: segment i = wedge of half-width pi/ns around angle_i;
-    closest point of wedge ^ geometry, first point of geometry along the centre ray."""
+    closest point of wedge ^ geometry, first point of geometry along the centre ray.
+    ray_length=L: segment i is the triangle with apex at the agent and far vertices at L (the wedge
+    cut at L cos(pi/ns) along its centre line), the ray is L long, and a ring's ray hit counts only
+    when the ring meets the triangle (ext_obsv_sector_and_ray.py looks for the ray hit only when the
+    sector intersection is non-empty)."""
     ax, ay, ath = agent
     seg = np.full(ns, np.inf); ray = np.full(ns, np.inf)
     width = 2 * math.pi / ns
-    rr = np.arange(dr, r_max, dr)
+    rr = np.arange(dr, r_max if ray_length is None else ray_length, dr)
     for i in range(ns):
         ang = ath + i * width
-        # ---- ray: first sample along the centre ray that is inside a solid polygon / crosses a ring
-        pts = np.stack([ax + rr * math.cos(ang), ay + rr * math.sin(ang)], axis=1)
         for poly, sd in zip(rings, solid):
+            # ---- ray: first sample along the centre ray that is inside a solid polygon / crosses a ring
+            pts = np.stack([ax + rr * math.cos(ang), ay + rr * math.sin(ang)], axis=1)
+            ray_g = seg_g = np.inf
             inside = winding_inside(poly, pts)
             if sd:
                 if winding_inside(poly, np.array([[ax, ay]]))[0]:
-                    ray[i] = 0.0
+                    ray_g = 0.0
                 elif inside.any():
-                    ray[i] = min(ray[i], rr[np.argmax(inside)])
+                    ray_g = rr[np.argmax(inside)]
             else:  # LineString: the crossing of the boundary = a change of the inside flag
                 start = winding_inside(poly, np.array([[ax, ay]]))[0]
                 flips = np.nonzero(np.diff(np.concatenate([[start], inside]).astype(int)) != 0)[0]
                 if len(flips):
-                    ray[i] = min(ray[i], rr[flips[0]])
-        # ---- sector: boundary points inside the wedge (the closest point of wedge ^ G lies on G's
-        #      boundary when the agent is outside G) plus, for solid polygons, the wedge's own two
-        #      edge rays entering the polygon
-        for poly, sd in zip(rings, solid):
+                    ray_g = rr[flips[0]]
+            # ---- sector: boundary points inside the wedge (the closest point of wedge ^ G lies on G's
+            #      boundary when the agent is outside G) plus, for solid polygons, the wedge's own two
+            #      edge rays entering the polygon
             if sd and winding_inside(poly, np.array([[ax, ay]]))[0]:
-                seg[i] = 0.0
-                continue
-            b = boundary_samples(poly, dr)
-            rel = np.arctan2(b[:, 1] - ay, b[:, 0] - ax) - ang
-            rel = (rel + math.pi) % (2 * math.pi) - math.pi
-            inw = np.abs(rel) <= width / 2
-            if inw.any():
-                seg[i] = min(seg[i], np.hypot(b[inw, 0] - ax, b[inw, 1] - ay).min())
-            if sd:
-                for edge_ang in (ang - width / 2, ang + width / 2):
-                    e = np.stack([ax + rr * math.cos(edge_ang), ay + rr * math.sin(edge_ang)], axis=1)
-                    ins = winding_inside(poly, e)
-                    if ins.any():
-                        seg[i] = min(seg[i], rr[np.argmax(ins)])
+                seg_g = 0.0
+            else:
+                b = boundary_samples(poly, dr)
+                rel = np.arctan2(b[:, 1] - ay, b[:, 0] - ax) - ang
+                rel = (rel + math.pi) % (2 * math.pi) - math.pi
+                inw = np.abs(rel) <= width / 2
+                if ray_length is not None:      # the triangle: not beyond its far edge
+                    inw &= (b[:, 0] - ax) * math.cos(ang) + (b[:, 1] - ay) * math.sin(ang) <= \
+                        ray_length * math.cos(width / 2)
+                if inw.any():
+                    seg_g = np.hypot(b[inw, 0] - ax, b[inw, 1] - ay).min()
+                if sd:
+                    for edge_ang in (ang - width / 2, ang + width / 2):
+                        e = np.stack([ax + rr * math.cos(edge_ang), ay + rr * math.sin(edge_ang)], axis=1)
+                        ins = winding_inside(poly, e)
+                        if ins.any():
+                            seg_g = min(seg_g, rr[np.argmax(ins)])
+            seg[i] = min(seg[i], seg_g)
+            if ray_length is None or seg_g < np.inf:
+                ray[i] = min(ray[i], ray_g)
     return seg, ray
 
 
@@ -137,3 +147,40 @@ def test_polygon_contains_and_distance_against_winding_number_and_sampling(seed)
         # shapely: a point ON the boundary is not contained, its distance is 0
         v = poly[0]
         assert O.poly_distance(poly, *v) <= 1e-12
+
+
+@pytest.mark.parametrize("ns", [3, 8])
+def test_ray_length_rule_against_dense_sampling(ns):
+    """Short rays (L = 3): obstacles on a centre ray between L cos(pi/ns) and L lie outside every
+    sector triangle; the reference does not see them on the ray either.  Obstacles that reach into
+    the triangle and cross the ray beyond it are seen on the ray."""
+    from tests.dqn_exact_ref import band_square
+    L = 3.0
+    lay = t.dqn.default_layout()
+    lay.num_segments, lay.ray_length = ns, L
+    rng = np.random.default_rng(40 + ns)
+    near = L * math.cos(math.pi / ns)
+    seen_band = seen_reach = 0
+    for k in range(3):
+        ag = np.array([*rng.uniform(5, 15, 2), rng.uniform(-math.pi, math.pi)])
+        rings = [band_square(ag, lay, s, 0.3 + 0.2 * k) for s in range(0, ns, 2)]
+        # a thin bar from inside sector 1's triangle across its ray in the band
+        a = ag[2] + 2 * math.pi / ns
+        u, v = np.array([math.cos(a), math.sin(a)]), np.array([-math.sin(a), math.cos(a)])
+        p1 = ag[:2] + u * (0.5 * (near + L))
+        p2 = ag[:2] + u * (0.8 * near) + v * (0.3 * near * math.tan(math.pi / ns))
+        p1 = p1 + 0.2 * (p1 - p2)
+        nrm = np.array([-(p1 - p2)[1], (p1 - p2)[0]]) / np.hypot(*(p1 - p2)) * 0.01
+        bar = np.array([p2 - nrm, p1 - nrm, p1 + nrm, p2 + nrm])
+        rings.append(bar)
+        solid = [True] * len(rings)
+        seg_o, ray_o = O.observe(lay, ag, rings, solid)
+        seg_b, ray_b = brute_sector_ray(ag, rings, solid, ns=ns, ray_length=L, dr=1e-3)
+        tol = 3e-3 + 2e-4 * L
+        for o, b in ((seg_o, seg_b), (ray_o, ray_b)):
+            assert np.array_equal(np.isfinite(o), np.isfinite(b)), (ns, k, o, b)
+            fin = np.isfinite(o)
+            assert np.abs(o[fin] - b[fin]).max(initial=0.0) <= tol, (ns, k, o, b)
+        seen_band += int(np.isinf(ray_o[0::2]).sum())
+        seen_reach += int(np.isfinite(ray_o[1]) and ray_o[1] > near)
+    assert seen_band >= 3 and seen_reach >= 1, (seen_band, seen_reach)

@@ -12,7 +12,10 @@
 // Geometry: for sector triangle T with apex at the agent A, and a closed ring G,
 // the closest point of T^G to A lies on G's boundary whenever A is outside G, so
 // the sector distance is min over edges e of dist(A, e clipped to T); the ray
-// distance is the first hit along the centre ray.  A inside a solid ring gives 0
+// distance is the first hit along the centre ray of length L, counted only for rings that meet T
+// (the reference intersects the ray with a ring only when the sector intersection is non-empty: a
+// ring crossing the ray between L cos(pi / ns), where the ray leaves T, and L is not seen unless
+// another part of it reaches into T).  A inside a solid ring gives 0
 // for every sector.  Lanes split the edges; the 16 minima are warp-reduced.  Moving
 // solid rings (ttdqn_moving, observe_act_moving_kernel) spread their (ring, edge) pairs over the
 // lanes instead (moving_minima).
@@ -124,8 +127,14 @@ __device__ __forceinline__ double wmin(double v) {
   return v;
 }
 
-// one edge p0 -> p1 into this lane's running sector and ray minima
-__device__ __forceinline__ void edge_minima(const Sector *sec, int ns, double ax, double ay, double L,
+// one edge p0 -> p1 into this lane's running sector and ray minima.  Only ray hits at s <= Lmax are
+// taken: Lmax is L when no vertex of the environment lies beyond Lin, else Lin.  Hits up to Lin lie
+// inside the sector triangle (the ray leaves it at L cos(pi / ns); Lin stays 2^-20 of that short of
+// it), so their ring meets the triangle.  A hit beyond Lin counts only if some edge
+// of its ring meets the triangle (the reference looks for a ring's ray hit only when the sector
+// intersection is non-empty); such a hit needs a vertex farther than Lin from the agent, and only
+// then are a ring's edges passed again, sector by sector, through far_edge_hit / take_ray.
+__device__ __forceinline__ void edge_minima(const Sector *sec, int ns, double ax, double ay, double Lmax,
                                             double p0x, double p0y, double p1x, double p1y,
                                             double (&dseg)[MAX_SEG], double (&dray)[MAX_SEG]) {
   const double dx = p1x - p0x, dy = p1y - p0y;
@@ -144,9 +153,24 @@ __device__ __forceinline__ void edge_minima(const Sector *sec, int ns, double ax
         const double qx = p0x + t * dx - ax, qy = p0y + t * dy - ay;
         dseg[i] = fmin(dseg[i], sqrt(qx * qx + qy * qy));
       }
-      dray[i] = fmin(dray[i], ray_seg_hit(ax, ay, S.rx, S.ry, L, p0x, p0y, p1x, p1y));
+      dray[i] = fmin(dray[i], ray_seg_hit(ax, ay, S.rx, S.ry, Lmax, p0x, p0y, p1x, p1y));
     }
   }
+}
+
+// ray hit of the edge p0 -> p1 in sector i (a run-time index: one copy of the code for the rare
+// rings that reach beyond Lin), and whether the edge meets sector i's triangle
+__device__ __forceinline__ double far_edge_hit(const Sector &S, double ax, double ay, double L, double p0x,
+                                               double p0y, double p1x, double p1y, bool &touch) {
+  double t0, t1;
+  touch = touch || clip_to_triangle(S, p0x, p0y, p1x - p0x, p1y - p0y, t0, t1);
+  return ray_seg_hit(ax, ay, S.rx, S.ry, L, p0x, p0y, p1x, p1y);
+}
+// dray[i] = fmin(dray[i], h) for a run-time i, without indexing the register array
+__device__ __forceinline__ void take_ray(double (&dray)[MAX_SEG], int i, double h) {
+#pragma unroll
+  for (int k = 0; k < MAX_SEG; k++)
+    if (k == i) dray[k] = fmin(dray[k], h);
 }
 
 // Moving solid rings (ttdqn_moving): the (ring, edge) pairs are spread over the lanes, 32 / max_pv
@@ -156,8 +180,8 @@ __device__ __forceinline__ void edge_minima(const Sector *sec, int ns, double ax
 // is the same arithmetic as for a static ring and min / OR ignore the order, so the result equals
 // that of the rings appended as static solid rings.  Returns whether the agent is inside any ring.
 __device__ __forceinline__ bool moving_minima(const ttdqn_moving &M, int env, int lane, const Sector *sec, int ns,
-                                              double ax, double ay, double L, double (&dseg)[MAX_SEG],
-                                              double (&dray)[MAX_SEG]) {
+                                              double ax, double ay, double L, double Lin, double Lfar2,
+                                              double (&dseg)[MAX_SEG], double (&dray)[MAX_SEG]) {
   const int pv = M.max_pv, per = 32 / pv, slot = lane / pv, e = lane - slot * pv;
   const unsigned mask = slot < per ? ((pv == 32 ? FULL : (1u << pv) - 1u) << (slot * pv)) : 0u;
   const double *cen = M.centre + (size_t)env * M.n_live * 2;
@@ -179,7 +203,29 @@ __device__ __forceinline__ bool moving_minima(const ttdqn_moving &M, int env, in
     }
     const bool in_ring = (__popc(__ballot_sync(FULL, cross) & mask) & 1) != 0;
     inside = inside || in_ring;
-    if (edge && !in_ring) edge_minima(sec, ns, ax, ay, L, p0x, p0y, p1x, p1y, dseg, dray);
+    bool far = false;
+    if (edge && !in_ring) {
+      edge_minima(sec, ns, ax, ay, Lin, p0x, p0y, p1x, p1y, dseg, dray);
+      far = (p0x - ax) * (p0x - ax) + (p0y - ay) * (p0y - ay) > Lfar2;
+    }
+    if (__any_sync(FULL, far)) {   // rings reaching beyond Lin: their ray hits count where they meet a triangle
+      const int end = slot * pv + pv;
+#pragma unroll 1
+      for (int i = 0; i < ns; i++) {
+        bool touch = false;
+        double h = INFINITY;
+        if (edge && !in_ring) h = far_edge_hit(sec[i], ax, ay, L, p0x, p0y, p1x, p1y, touch);
+        // OR over the ring's lanes [slot * pv, end): lane l gathers [l, min(l + 2o, end))
+        unsigned tv = touch ? 1u : 0u;
+#pragma unroll
+        for (int o = 1; o < 32; o <<= 1) {
+          const unsigned v = __shfl_down_sync(FULL, tv, o);
+          if (lane + o < end) tv |= v;
+        }
+        tv = __shfl_sync(FULL, tv, (slot * pv) & 31);
+        if (tv) take_ray(dray, i, h);
+      }
+    }
   }
   return __any_sync(FULL, inside);
 }
@@ -215,6 +261,8 @@ __device__ __forceinline__ void observe_act_body(const Args A, const ttdqn_movin
 
   const double L = A.lay.ray_length;
   const double width = 2 * M_PI / ns;
+  const double Lin = L * cos(width / 2) * (1.0 - 0x1p-20);  // ray hits up to here lie inside the triangle
+  const double Lfar2 = Lin * Lin * (1.0 - 0x1p-20);          // a hit beyond Lin needs a vertex this far (squared)
   for (int env = blockIdx.x * warps + warp; env < A.n_envs; env += gridDim.x * warps) {
     const double ax = A.agent[3 * env], ay = A.agent[3 * env + 1], th = A.agent[3 * env + 2];
     const double *xy = A.poly_xy + (size_t)env * A.lay.max_vert * 2;
@@ -231,6 +279,15 @@ __device__ __forceinline__ void observe_act_body(const Args A, const ttdqn_movin
       S.rx = cos(angle); S.ry = sin(angle);
     }
     __syncwarp();
+    // a ray hit beyond Lin needs a vertex farther than Lin: without one (every scene smaller than the
+    // ray) all hits are taken in the edge loop, as they lie inside their triangle
+    bool far_v = false;
+    for (int v = lane; v < poff[npoly > 0 ? npoly : 0] - poff[0]; v += 32) {
+      const double qx = xy[2 * (poff[0] + v)] - ax, qy = xy[2 * (poff[0] + v) + 1] - ay;
+      far_v = far_v || qx * qx + qy * qy > Lfar2;
+    }
+    const bool far_env = __any_sync(FULL, far_v);
+    const double Lx = far_env ? Lin : L;
     double dseg[MAX_SEG], dray[MAX_SEG];
 #pragma unroll
     for (int i = 0; i < MAX_SEG; i++) { dseg[i] = INFINITY; dray[i] = INFINITY; }
@@ -252,10 +309,22 @@ __device__ __forceinline__ void observe_act_body(const Args A, const ttdqn_movin
       }
       for (int e = lane; e < nv; e += 32) {
         const int e2 = (e + 1 == nv) ? 0 : e + 1;
-        edge_minima(sec, ns, ax, ay, L, r[2 * e], r[2 * e + 1], r[2 * e2], r[2 * e2 + 1], dseg, dray);
+        edge_minima(sec, ns, ax, ay, Lx, r[2 * e], r[2 * e + 1], r[2 * e2], r[2 * e2 + 1], dseg, dray);
+      }
+      if (far_env) {   // ray hits beyond Lin count in the sectors whose triangle the ring meets
+#pragma unroll 1
+        for (int i = 0; i < ns; i++) {
+          bool touch = false;
+          double h = INFINITY;
+          for (int e = lane; e < nv; e += 32) {
+            const int e2 = (e + 1 == nv) ? 0 : e + 1;
+            h = fmin(h, far_edge_hit(sec[i], ax, ay, L, r[2 * e], r[2 * e + 1], r[2 * e2], r[2 * e2 + 1], touch));
+          }
+          if (__any_sync(FULL, touch)) take_ray(dray, i, h);
+        }
       }
     }
-    if (MOVING && moving_minima(M, env, lane, sec, ns, ax, ay, L, dseg, dray)) inside_any = true;
+    if (MOVING && moving_minima(M, env, lane, sec, ns, ax, ay, L, Lin, Lfar2, dseg, dray)) inside_any = true;
 #pragma unroll
     for (int i = 0; i < MAX_SEG; i++) {
       if (i < ns) {
@@ -597,14 +666,21 @@ extern "C" void ttdqn_default_layout(ttdqn_scene_layout *l) {
   l->use_memory = 1; l->_pad = 0; l->ray_length = 1000.0; l->max_distance = 10.0;
 }
 
+// num_segments 1 and 2 give sector "triangles" of zero area (the far vertices coincide, or lie on a
+// line with the apex): whether anything is seen then hangs on the last bit of cos / sin
+static int check_layout(const ttdqn_scene_layout *lay, int n) {
+  if (!lay || n < 0) return dfail(TTMPC_ERR_BAD_ARG, "layout required, n >= 0");
+  if (lay->num_segments < 3 || lay->num_segments > ttdqn::MAX_SEG)
+    return dfail(TTMPC_ERR_BAD_CONFIG, "num_segments must be in 3..16");
+  return TTMPC_OK;
+}
+
 static int observe_act(const ttdqn_scene_layout *lay, const ttdqn_qnet *qn, int n, const double *d_agent,
                        const double *d_poly_xy, const int *d_poly_off, const int *d_is_solid, const int *d_n_poly,
                        const ttdqn_moving *mv, const float *d_internal, float *d_old_ext, float *d_ext,
                        float *d_q, int *d_action, double *d_seg, double *d_ray, void *stream) {
   using namespace ttdqn;
-  if (!lay || n < 0) return dfail(TTMPC_ERR_BAD_ARG, "layout required, n >= 0");
-  if (lay->num_segments < 1 || lay->num_segments > MAX_SEG)
-    return dfail(TTMPC_ERR_BAD_CONFIG, "num_segments must be in 1..16");
+  if (int rc = check_layout(lay, n)) return rc;
   if (lay->use_memory && !d_old_ext) return dfail(TTMPC_ERR_BAD_ARG, "use_memory needs d_old_ext");
   if (mv) {
     if (mv->n_live < 0) return dfail(TTMPC_ERR_BAD_ARG, "moving: n_live must be >= 0");
@@ -635,11 +711,21 @@ static int observe_act(const ttdqn_scene_layout *lay, const ttdqn_qnet *qn, int 
   A.action = d_action; A.seg_dist = d_seg; A.ray_dist = d_ray; A.n_envs = n;
   // tensor-core path of the Q-network: 16-wide hidden layers, up to 16 outputs (the reference's
   // SB3 [16, 16] MLP); TTDQN_QNET=fma forces the FMA-pipe path for A/B measurements
-  int dev = 0, sms = 0;
+  int dev = 0, sms = 0, smem_max = 0;
   DQN_TRY(cudaGetDevice(&dev));
   bool mma = qn && qn->n_h1 == 16 && qn->n_h2 == 16 && qn->n_out <= 16 && qn->n_in <= 248;
   if (const char *e = std::getenv("TTDQN_QNET")) mma = mma && !(e[0] == 'f');
   A.obs = nullptr; A.obs_stride = (A.n_in + 7) / 8 * 8; A.defer_net = 0;
+  // shared memory per block: the Q-network's weights and 4 warps' scratch (observe_act_body)
+  const int warps = 4;
+  size_t wbytes = ((size_t)(A.n_in * A.n_h1 + A.n_h1 + A.n_h1 * A.n_h2 + A.n_h2 + A.n_h2 * A.n_out + A.n_out) * sizeof(float) + 15) / 16 * 16;
+  size_t per_warp = (sizeof(Sector) * MAX_SEG + sizeof(float) * (size_t)(A.n_in + A.n_h1 + A.n_h2 + A.n_out + 4) + 15) / 16 * 16;
+  size_t smem = wbytes + per_warp * warps;
+  DQN_TRY(cudaDeviceGetAttribute(&smem_max, cudaDevAttrMaxSharedMemoryPerBlockOptin, dev));
+  if (smem > (size_t)smem_max)
+    return dfail(TTMPC_ERR_UNSUPPORTED, "observe_act needs " + std::to_string(smem) +
+                                            " bytes of shared memory per block (Q-network weights and scratch), "
+                                            "the device allows " + std::to_string(smem_max));
   float *d_obs = nullptr;
   if (mma) {
     // stream-ordered scratch from the device's default memory pool.  The pool's default release
@@ -662,10 +748,6 @@ static int observe_act(const ttdqn_scene_layout *lay, const ttdqn_qnet *qn, int 
     DQN_TRY(cudaMallocAsync((void **)&d_obs, sizeof(float) * (size_t)n * A.obs_stride, (cudaStream_t)stream));
     A.obs = d_obs; A.defer_net = 1;
   }
-  const int warps = 4;
-  size_t wbytes = ((size_t)(A.n_in * A.n_h1 + A.n_h1 + A.n_h1 * A.n_h2 + A.n_h2 + A.n_h2 * A.n_out + A.n_out) * sizeof(float) + 15) / 16 * 16;
-  size_t per_warp = (sizeof(Sector) * MAX_SEG + sizeof(float) * (size_t)(A.n_in + A.n_h1 + A.n_h2 + A.n_out + 4) + 15) / 16 * 16;
-  size_t smem = wbytes + per_warp * warps;
   DQN_TRY(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev));
   const void *kern = moving ? (const void *)observe_act_moving_kernel : (const void *)observe_act_kernel;
   DQN_TRY(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
@@ -722,7 +804,7 @@ extern "C" int ttdqn_observe_act_host(const ttdqn_scene_layout *lay, const ttdqn
                                       const int *h_n_poly, const float *h_internal,
                                       float *h_old_ext, float *h_ext, float *h_q, int *h_action,
                                       double *h_seg, double *h_ray) {
-  if (!lay || n < 0) return dfail(TTMPC_ERR_BAD_ARG, "layout required, n >= 0");
+  if (int rc = check_layout(lay, n)) return rc;
   if (n == 0) return TTMPC_OK;
   const size_t nn = (size_t)n;
   const int ns = lay->num_segments;

@@ -96,6 +96,10 @@ class DqnCompanion:
 
     def __init__(self, lay: TtdqnLayout, weights: QNetWeights = None):
         self.lib = _lib.load()
+        # the library's own layout checks (num_segments 3..16); with no environments nothing else runs
+        rc = self.lib.ttdqn_observe_act_host(C.byref(lay), None, 0, *[None] * 12)
+        if rc != 0:
+            raise _lib.TtmpcError(f"DqnCompanion: bad layout (code {rc}): {self.lib.ttdqn_last_error().decode()}")
         self.lay = lay
         self.weights = weights
         self.ns = lay.num_segments

@@ -355,6 +355,7 @@ class FleetPlanner:
             if not (isinstance(xy, t.Tensor) and xy.dim() == 3 and isinstance(sol, t.Tensor) and sol.dim() == 2):
                 raise ValueError("enable_dqn: geometry xy must be [n][max_vert][2] and solid [n][max_poly]")
             layout = dqn.default_layout(max_poly=sol.shape[1], max_vert=xy.shape[1])
+        comp = dqn.DqnCompanion(layout, weights)       # rejects a bad layout before anything is set
         want(xy, "geometry xy", t.float64, (n, layout.max_vert, 2))
         want(off, "geometry off", t.int32, (n, layout.max_poly + 1))
         want(sol, "geometry solid", t.int32, (n, layout.max_poly))
@@ -393,7 +394,7 @@ class FleetPlanner:
         d = SimpleNamespace(
             lay=layout, geometry=(xy, off, sol, cnt), paths=(path_xy, path_n), shape=shape, shape_dev=None,
             ref_speed=float(ref_speed), corner_samples=int(corner_samples), sample_offset=float(sample_offset),
-            comp=dqn.DqnCompanion(layout, weights), w=w,
+            comp=comp, w=w,
             qnet=_lib.TtdqnQnet(weights.n_in, weights.n_h1, weights.n_h2, weights.n_out, *[a.data_ptr() for a in w]),
             agent5=t.zeros(n, 5, dtype=t.float64, device=dev), internal=t.zeros(n, layout.n_internal, **f32),
             progress=t.zeros(n, dtype=t.float64, device=dev),
