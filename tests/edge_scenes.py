@@ -13,6 +13,8 @@ in place and return it:
 
 ``ref_eval`` computes f, F1 and F2 in ``np.longdouble`` (64-bit mantissa on x86), vectorised over
 scenes: a plain restatement of oracle/ttmpc_oracle.c:forward(), i.e. of mpc_generator.py:155-283.
+``ref_psi`` adds the augmented-Lagrangian terms of the solver's cost psi, and ``ref_psi_grad`` takes
+its gradient by the complex step (no hand derivation, no subtraction).
 """
 from __future__ import annotations
 
@@ -282,19 +284,28 @@ def translate(p, cfg, dx, dy):
 
 
 # ------------------------------------------------------------------ high-precision reference
-def ref_eval(cfg, u, p, terms=False):
+def ref_eval(cfg, u, p, terms=False, dtype=np.longdouble, groups=False):
     """f [n], F1 [n, 2N], F2 [n, Ndyn] in np.longdouble: oracle/ttmpc_oracle.c:forward() restated
     (mpc_generator.py:124-139 path deviation, 203-204 speed and control, 207-211 fleet collision,
     214-220 static, 225-237 dynamic, 242 terminal, 250-264 accelerations; F2_j = S + D_j).
     fmin / fmax where the C code uses them, so NaN inputs behave alike.
 
-    terms=True also returns a dict of per-scene pieces: 'path', 'fleet', 'dyn_soft' [n, Ndyn],
-    'S', 'D' [n, Ndyn], 'contacts' (other-robot contacts), and Lipschitz bounds of f and of F2 with
-    respect to the rolled-out positions: 'lip_f' [n] and 'lip_F2' [n, Ndyn] (sums over the steps of
-    |d term / d position|)."""
+    dtype=np.clongdouble evaluates at complex controls u (the complex step of ref_psi_grad); p stays
+    real.  numpy's fmin / fmax order complex numbers by their real parts first, so every kink takes
+    the branch the real evaluation takes, and fmin.reduce keeps the first of equal minima.
+
+    groups=True also returns a dict of the cost's term groups [n]: 'path', 'speed_control', 'fleet',
+    'dyn_soft', 'terminal', 'acc' (their sum is f up to rounding).
+
+    terms=True (real dtype only) also returns a dict of per-scene pieces: 'path', 'fleet', 'dyn_soft'
+    [n, Ndyn], 'S', 'D' [n, Ndyn], 'contacts' (other-robot contacts), and Lipschitz bounds of f and of
+    F2 with respect to the rolled-out positions: 'lip_f' [n] and 'lip_F2' [n, Ndyn] (sums over the
+    steps of |d term / d position|)."""
     L = np.longdouble
+    if terms and (groups or dtype is not L):
+        raise ValueError("terms=True is real-only and excludes groups=True")
     p = np.asarray(p, np.float64).astype(L)
-    u = np.asarray(u, np.float64).astype(L)
+    u = np.asarray(u, np.float64).astype(L) if dtype is L else np.asarray(u).astype(dtype)
     if p.ndim == 1:
         p, u = p[None], u[None]
     n, N, ns = p.shape[0], cfg.N_hor, cfg.ns
@@ -312,7 +323,7 @@ def ref_eval(cfg, u, p, terms=False):
     v, w = u[:, 0::2], u[:, 1::2]
 
     # rollout: unicycle_model with rk4 (motion_model.py:153-176)
-    X, Y, TH = (np.zeros((n, N), L) for _ in range(3))
+    X, Y, TH = (np.zeros((n, N), dtype) for _ in range(3))
     x, y, th = s[:, 0], s[:, 1], s[:, 2]
     for k in range(N):
         vk, wk = v[:, k], w[:, k]
@@ -354,7 +365,7 @@ def ref_eval(cfg, u, p, terms=False):
         m = np.fmax(L(0), res)                                           # [n, i, k, e]
         S = np.fmax(L(0), (m * m).prod(-1)).sum((1, 2))
     else:
-        S = np.zeros(n, L)
+        S = np.zeros(n, dtype)
 
     # dynamic obstacles
     dx_, dy_ = X[:, None, :] - od[..., 0], Y[:, None, :] - od[..., 1]   # [n, j, k]
@@ -372,13 +383,19 @@ def ref_eval(cfg, u, p, terms=False):
     cost = cost + dyn_soft.sum(1)
 
     # terminal cost and accelerations
-    cost = cost + qN * ((X[:, -1] - s[:, 3]) ** 2 + (Y[:, -1] - s[:, 4]) ** 2) + qthN * (TH[:, -1] - s[:, 5]) ** 2
+    t_xy, t_th = qN * ((X[:, -1] - s[:, 3]) ** 2 + (Y[:, -1] - s[:, 4]) ** 2), qthN * (TH[:, -1] - s[:, 5]) ** 2
+    cost = cost + t_xy + t_th
     vp = np.concatenate([s[:, 6:7], v[:, :-1]], 1)
     wp = np.concatenate([s[:, 7:8], w[:, :-1]], 1)
     a, aw = (v - vp) / ts, (w - wp) / ts
-    cost = cost + (a * a).sum(1) * accp + (aw * aw).sum(1) * waccp
+    a_v, a_w = (a * a).sum(1) * accp, (aw * aw).sum(1) * waccp
+    cost = cost + a_v + a_w
     F1 = np.concatenate([a, aw], 1)
     F2 = S[:, None] + D
+    if groups:
+        speed_control = (qvel[:, None] * (v - vref) ** 2).sum(1) + (rv[:, None] * v * v + rw[:, None] * w * w).sum(1)
+        return cost, F1, F2, dict(path=path, speed_control=speed_control, fleet=fleet,
+                                  dyn_soft=dyn_soft.sum(1), terminal=t_xy + t_th, acc=a_v + a_w)
     if not terms:
         return cost, F1, F2
 
@@ -402,3 +419,48 @@ def ref_eval(cfg, u, p, terms=False):
     parts = dict(path=path, fleet=fleet, dyn_soft=dyn_soft, S=S, D=D, contacts=(fl > 0).sum((1, 2)),
                  robot_contacts=(fl > 0).sum(2), jmin=jmin, lip_f=lip_f, lip_F2=lip_S[:, None] + lip_D)
     return cost, F1, F2, parts
+
+
+def ref_psi(cfg, u, p, c, y=None, dtype=np.longdouble, groups=False):
+    """psi = f + c/2 dist^2_C(F1 + y / max(c, 1)) + c/2 |F2|^2 [n]: oracle/ttmpc_oracle.c:psi_from
+    on ref_eval, with C the box [lin_acc_min, lin_acc_max]^N x [-ang_acc_max, ang_acc_max]^N.
+    c is [n] or a scalar, y [n, 2N] or None (zero).  groups=True returns the term groups instead:
+    ref_eval's, 'alm_F1' (the c/2 dist^2 term) and 'penalty_F2' (the c/2 |F2|^2 term), and with
+    them 'F2' itself (not a term of psi)."""
+    L = np.longdouble
+    f, F1, F2, g = ref_eval(cfg, u, p, dtype=dtype, groups=True)
+    n, N = F1.shape[0], cfg.N_hor
+    c = np.broadcast_to(np.asarray(c, np.float64), (n,)).astype(L)
+    y = np.zeros((n, 2 * N), L) if y is None else np.asarray(y, np.float64).reshape(n, 2 * N).astype(L)
+    lo = np.repeat([L(cfg.lin_acc_min), -L(cfg.ang_acc_max)], N)
+    hi = np.repeat([L(cfg.lin_acc_max), L(cfg.ang_acc_max)], N)
+    z = F1 + y / np.fmax(c, L(1))[:, None]
+    e = z - np.fmin(np.fmax(z, lo), hi)
+    g["alm_F1"] = c * (e * e).sum(1) / 2
+    g["penalty_F2"] = c * (F2 * F2).sum(1) / 2
+    return dict(g, F2=F2) if groups else f + g["alm_F1"] + g["penalty_F2"]
+
+
+def ref_psi_grad(cfg, u, p, c, y=None, groups=False):
+    """grad psi [n, 2N] (np.longdouble) by the complex step: d psi / d u_k = Im psi(u + i h e_k) / h,
+    h = 1e-40, in np.clongdouble.  No difference of nearby values is formed, so the result carries
+    only the rounding of the evaluation itself (~1e-19 relative).  At a kink the branch is the real
+    evaluation's (see ref_eval).  groups=True also returns the gradient of each term group of
+    ref_psi (dict of [n, 2N]; they add up to the total) and the Jacobian of F2 [n, Ndyn, 2N]."""
+    L, Cx = np.longdouble, np.clongdouble
+    h = L(1e-40)
+    u, p = np.asarray(u, np.float64), np.asarray(p, np.float64)
+    if p.ndim == 1:
+        p, u = p[None], u[None]
+    n, m = u.shape
+    parts, jac_F2 = {}, np.zeros((n, cfg.Ndynobs, m), L)
+    for k in range(m):
+        uk = u.astype(Cx)
+        uk[:, k] += 1j * h
+        for name, val in ref_psi(cfg, uk, p, c, y, dtype=Cx, groups=True).items():
+            if name == "F2":
+                jac_F2[:, :, k] = val.imag / h
+            else:
+                parts.setdefault(name, np.zeros((n, m), L))[:, k] = val.imag / h
+    grad = sum(parts.values())
+    return (grad, parts, jac_F2) if groups else grad
