@@ -9,10 +9,11 @@ LIB       := $(PKG)/libttmpc.so
 ORACLE    := oracle/libttmpc_oracle.so
 TASKS_ORACLE := oracle/libttfleet_tasks_oracle.so
 MONITOR_ORACLE := oracle/libttfleet_monitor_oracle.so
+WORLD_ORACLE := oracle/libttfleet_world_oracle.so
 CU        := $(CSRC)/ttmpc_solve.cu $(CSRC)/ttmpc_api.cu $(CSRC)/ttmpc_fleet.cu $(CSRC)/ttdqn.cu
 HDRS      := include/ttmpc.h $(CSRC)/ttmpc_device.cuh $(CSRC)/ttmpc_launch.cuh
 
-all: $(LIB) $(ORACLE) $(TASKS_ORACLE) $(MONITOR_ORACLE)
+all: $(LIB) $(ORACLE) $(TASKS_ORACLE) $(MONITOR_ORACLE) $(WORLD_ORACLE)
 
 $(CSRC)/%.o: $(CSRC)/%.cu $(HDRS)
 	$(NVCC) $(NVFLAGS) -c $< -o $@
@@ -30,7 +31,10 @@ $(TASKS_ORACLE): oracle/ttfleet_tasks_oracle.c
 $(MONITOR_ORACLE): oracle/ttfleet_monitor_oracle.c include/ttmpc.h
 	$(CC) -O2 -fPIC -shared -ffp-contract=off -Wall -o $@ $< -lm
 
+$(WORLD_ORACLE): oracle/ttfleet_world_oracle.c include/ttmpc.h
+	$(CC) -O2 -fPIC -shared -ffp-contract=off -Wall -o $@ $< -lm
+
 clean:
-	rm -f $(CSRC)/*.o $(LIB) $(ORACLE) $(TASKS_ORACLE) $(MONITOR_ORACLE)
+	rm -f $(CSRC)/*.o $(LIB) $(ORACLE) $(TASKS_ORACLE) $(MONITOR_ORACLE) $(WORLD_ORACLE)
 
 .PHONY: all clean

@@ -514,6 +514,71 @@ typedef struct ttmpc_fleet_monitor {
 int ttmpc_fleet_monitor_device(const ttmpc_config *cfg, const ttmpc_fleet *fleet,
                                const ttmpc_fleet_monitor *mon, void *stream);
 
+/* Shared obstacle map of ttmpc_fleet_world_select_device: M >= 0 convex polygons that every robot
+ * shares, of which each robot's K = Nstcobs static slots get the nearest ones before a step.  All
+ * arrays are device pointers.
+ *
+ * The map.  Polygon o has a vertex ring poly_xy[o] (the convex hull the MPC sees), its half-space
+ * row rows[o] of nstcobs doubles b[ne] a0[ne] a1[ne] (what polygon_halfspace_representation gives
+ * for that hull; the kernel copies it and does not read it otherwise) and its axis-aligned bounding
+ * box bbox[o] = (xmin, ymin, xmax, ymax).  reach R (finite, > 0) is the farthest obstacle that
+ * matters; N_hor * ts * max(|lin_vel_min|, lin_vel_max), the farthest a feasible rollout gets, is
+ * the natural choice.
+ *
+ * Selection for robot e, from p = state[e][0:2] (the state the pack kernel packs; a robot that
+ * takes a task does not move, so task queues do not change it):
+ *   - d_o = the distance of p to polygon o: 0 inside (even-odd rule), else the least distance to an
+ *     edge; plain IEEE operations in a fixed order (the ring distance of the monitor's zero-length
+ *     chord).  A polygon with poly_nv < 3 has no distance and is never selected; poly_nv > max_pv
+ *     reads max_pv vertices.
+ *   - eligible: d_o <= R.  n_reach[e] = the number of eligible polygons.
+ *   - the eligible polygons ranked by (d_o, o) ascending (ties to the lower map index); the first
+ *     k = min(K, n_reach) are taken and their rows written in ASCENDING MAP INDEX into slots
+ *     0..k-1 of stc_out[e], zeros into the other slots; slot_poly[e][s] = the map index of slot s,
+ *     -1 for an empty slot.  A map of M <= K polygons all within reach thus gives exactly the rows
+ *     of the same polygons given as one shared block in map order, and a set that stays chosen keeps
+ *     its rows from step to step.  n_reach[e] > K: an obstacle within reach got no slot.
+ *   - every robot is selected, whatever its status (the pack kernel packs every robot).
+ *
+ * The grid.  A uniform grid over the map: cell (cx, cy), 0 <= cx < nx, 0 <= cy < ny, covers
+ * [origin_x + cx cell, origin_x + (cx+1) cell) x [...y...]; its polygons are
+ * cell_items[cell_start[c] .. cell_start[c+1]) with c = cy nx + cx, ascending within a cell.  It
+ * must list polygon o in exactly the cells bx0..bx1 x by0..by1 with
+ * bx0 = clamp(floor((xmin - origin_x) / cell), 0, nx-1), bx1 the same of xmax, by0 / by1 of
+ * ymin / ymax (IEEE subtraction and division), and every polygon must lie inside the grid.  A query
+ * visits cells floor((x - R - origin_x) / cell) - 1 .. floor((x + R - origin_x) / cell) + 1
+ * (likewise in y), clamped to the grid, so no polygon within reach is missed to rounding, and
+ * handles a polygon only in the lowest visited cell of its range, (max(qx0, bx0), max(qy0, by0)).
+ * A robot outside the grid is exact too.  Map indices outside [0, M) in cell_items are skipped and
+ * cell_start is clamped to [0, cell_start[nx ny]]: another grid cannot make the kernel read or write
+ * out of bounds, but only a grid built by the rule above gives the selection above.  The kernel's
+ * work per robot is the visited cells' items, independent of M at a fixed map density.
+ *
+ * Use: before each step call ttmpc_fleet_world_select_device on the step's stream and point
+ * fleet.stc at d_stc_out with stc_shared = 0 (d_stc_out may be the buffer the step reads).     */
+typedef struct ttmpc_fleet_world {
+  int M;                   /* polygons, >= 0                                                  */
+  int max_pv;              /* >= 3: vertex slots per polygon in poly_xy                       */
+  const double *poly_xy;   /* [M][max_pv][2] vertex rings                                     */
+  const int *poly_nv;      /* [M] vertex counts                                               */
+  const double *rows;      /* [M][nstcobs] half-space rows                                    */
+  const double *bbox;      /* [M][4] xmin ymin xmax ymax                                      */
+  double reach;            /* R: finite, > 0                                                  */
+  double origin_x, origin_y;
+  double cell;             /* grid cell size: finite, > 0                                     */
+  int nx, ny;              /* cells, >= 1 each                                                */
+  const int *cell_start;   /* [nx*ny + 1] CSR offsets into cell_items                         */
+  const int *cell_items;   /* [cell_start[nx*ny]] map indices                                 */
+} ttmpc_fleet_world;
+/* Write each robot's nearest map polygons (see ttmpc_fleet_world) on `stream`: d_stc_out
+ * [n][Nstcobs*nstcobs], d_slot_poly [n][Nstcobs] or NULL, d_n_reach [n] or NULL.  Reads fleet->n
+ * and fleet->state only.  world == NULL, M < 0, max_pv < 3, a non-finite or non-positive reach or
+ * cell, nx or ny < 1 (or nx*ny too large for an int), a NULL map or grid array while M > 0, a NULL
+ * d_stc_out or a fleet the step would reject -> TTMPC_ERR_BAD_ARG before any device work. */
+int ttmpc_fleet_world_select_device(const ttmpc_config *cfg, const ttmpc_fleet *fleet,
+                                    const ttmpc_fleet_world *world, double *d_stc_out,
+                                    int *d_slot_poly, int *d_n_reach, void *stream);
+
 /* ------------------------------------------------------------------------
  * DQN side of the hybrid loop (src/main.py:174-193), device-resident.
  *

@@ -5,7 +5,7 @@ tools/r2_single_sweep.sh), profiles/r2_parity_distribution_{gpu,cpu}.json, r2_qn
 r2_hybrid.json, r2_single_latency.txt, profiles/r2_roofline_inputs.json, r2_missions.json (tools/bench_missions.py,
 one line per fleet size), r2_missions_profile.json (its --profile-pack line), r2_monitor.json (tools/bench_monitor.py),
 r2_lidar_moving.json (tools/bench_lidar_moving.py), r2_hybrid_lidar.json (tools/bench_hybrid.py timing runs with and
-without --lidar-moving), r2_hybrid_drive.json (its --monitor drives)."""
+without --lidar-moving), r2_hybrid_drive.json (its --monitor drives), r2_world.json (tools/bench_world.py)."""
 import glob
 import json
 import os
@@ -114,6 +114,40 @@ def monitor_section(mo):
         out.append(f"The same drive with moving_radius = 0, i.e. the rectangles alone: robots with contact {s['robots_with_contact']} "
                    f"({s['contact_steps_total']} robot-steps); min_clearance quantiles "
                    + " / ".join(f"{q[k]:.3f}" for k in ("0.0", "0.01", "0.05", "0.1", "0.5")) + " m.\n")
+    return out
+
+
+def world_section(lines):
+    """Lines of the "Shared obstacle map" section: the lines of tools/bench_world.py."""
+    sel = [r for r in lines if r.get("bench") == "world_select"]
+    drv = [r for r in lines if r.get("bench") == "world_drive"]
+    if not (sel or drv):
+        return []
+    out = ["## Shared obstacle map (`tools/bench_world.py`; `ttmpc_fleet_world_select_device` before every step)\n"]
+    if sel:
+        r0 = sel[0]
+        out += [f"`make_warehouse(n, tasks=1, seed=1000, shelves=M)` (1 m x 4 m shelves, 3 m aisles: the same density at every M), "
+                f"robots at their start crossings, Nstcobs = {r0['nstcobs']}, reach = cell = 6 m; {r0['gpu']}, power limit "
+                f"{r0['power_limit']}. Selection: CUDA events over 200 warm launches; step: the whole step (selection + pack + "
+                "solve + advance, warm start and skip-stopped), mean of 10 steps after 3.\n",
+                "| robots | shelves M | selection ms | step ms | selection / step | world_reach max | mean |",
+                "|---:|---:|---:|---:|---:|---:|---:|"]
+        for r in sel:
+            out.append(f"| {r['robots']} | {r['shelves']:,} | {r['select_ms']:.3f} | {r['step_ms']:.2f} | "
+                       f"{100 * r['select_share_of_step']:.1f} % | {r['world_reach_max']} | {r['world_reach_mean']:.2f} |")
+        out.append("")
+    for d in drv:
+        out += [f"Drive: `make_warehouse({d['robots']}, tasks={d['tasks']}, seed=1000)` ({d['shelves']:,} shelves), up to "
+                f"{d['max_steps']} steps per leg, legs S WS WS S (skip-stopped, WS also warm start), the monitor on the map "
+                f"(robot centre against every shelf); {d['gpu']}, power limit {d['power_limit']}.\n",
+                "| leg | steps | tasks completed | step ms p50 | p90 | robots with contact | world_reach max | robot-steps with world_reach > Nstcobs |",
+                "|---|---:|---:|---:|---:|---:|---:|---:|"]
+        for r in d["legs"]:
+            out.append(f"| {r['leg']} | {r['steps']} | {r['tasks_completed']} | {r['step_ms_p50']:.2f} | {r['step_ms_p90']:.2f} | "
+                       f"{r['robots_with_contact']} | {r['world_reach_max']} | {r['robot_steps_reach_over_nstcobs']:,} |")
+        out.append("")
+        out.append("The drive's step time includes the monitor, which measures every robot against every shelf (O(M) per "
+                   "robot); the selection table's step time has no monitor.\n")
     return out
 
 
@@ -312,6 +346,7 @@ def main():
                    f"{hy.get('mean_inner_iters', 0):.0f} PANOC iterations per solve.\n")
     out += lidar_moving_section(last(os.path.join(G, "r2_lidar_moving.json")), jl(os.path.join(G, "r2_hybrid_lidar.json")),
                                 jl(os.path.join(G, "r2_hybrid_drive.json")))
+    out += world_section(jl(os.path.join(G, "r2_world.json")))
     open(os.path.join(ROOT, "BENCH.md"), "w").write("\n".join(out) + "\n")
     print("\n".join(out))
 

@@ -111,6 +111,18 @@ class TtmpcFleetMonitor(C.Structure):
     ]
 
 
+class TtmpcFleetWorld(C.Structure):
+    """struct ttmpc_fleet_world: shared obstacle map and its grid for ttmpc_fleet_world_select_device
+    (device addresses)."""
+    _fields_ = [
+        ("M", C.c_int), ("max_pv", C.c_int),
+        ("poly_xy", C.c_void_p), ("poly_nv", C.c_void_p), ("rows", C.c_void_p), ("bbox", C.c_void_p),
+        ("reach", C.c_double), ("origin_x", C.c_double), ("origin_y", C.c_double), ("cell", C.c_double),
+        ("nx", C.c_int), ("ny", C.c_int),
+        ("cell_start", C.c_void_p), ("cell_items", C.c_void_p),
+    ]
+
+
 # every symbol include/ttmpc.h declares, with its signature
 _VP, _I, _D = C.c_void_p, C.c_int, C.c_double
 _CFG, _RES = C.POINTER(TtmpcConfig), C.POINTER(TtmpcResult)
@@ -118,6 +130,7 @@ _LAY, _QN, _MOV = C.POINTER(TtdqnLayout), C.POINTER(TtdqnQnet), C.POINTER(TtdqnM
 _FLT = C.POINTER(TtmpcFleet)
 _TSK = C.POINTER(TtmpcFleetTasks)
 _MON = C.POINTER(TtmpcFleetMonitor)
+_WLD = C.POINTER(TtmpcFleetWorld)
 SYMBOLS = {
     "ttmpc_default_config": (None, [_CFG]),
     "ttmpc_num_params": (_I, [_CFG]),
@@ -138,6 +151,7 @@ SYMBOLS = {
     "ttmpc_fleet_step_device": (_I, [_CFG, _FLT, _VP, _I, _RES, _VP]),
     "ttmpc_fleet_step_tasks_device": (_I, [_CFG, _FLT, _TSK, _VP, _I, _RES, _VP]),
     "ttmpc_fleet_monitor_device": (_I, [_CFG, _FLT, _MON, _VP]),
+    "ttmpc_fleet_world_select_device": (_I, [_CFG, _FLT, _WLD, _VP, _VP, _VP, _VP]),
     "ttmpc_read_stats": (_I, [C.POINTER(C.c_ulonglong), _I]),
     "ttmpc_launch_info": (_I, [_CFG, _I] + [C.POINTER(C.c_int)] * 5),
     "ttmpc_measure_fp64_peak": (_I, [C.POINTER(_D), _VP]),

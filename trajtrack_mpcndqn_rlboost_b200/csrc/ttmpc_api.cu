@@ -538,6 +538,27 @@ extern "C" int ttmpc_fleet_monitor_device(const ttmpc_config *cfg, const ttmpc_f
   CUDA_TRY(launch_fleet_monitor(*fleet, *mon, (cudaStream_t)stream));
   return TTMPC_OK;
 }
+extern "C" int ttmpc_fleet_world_select_device(const ttmpc_config *cfg, const ttmpc_fleet *fleet,
+                                               const ttmpc_fleet_world *world, double *d_stc_out,
+                                               int *d_slot_poly, int *d_n_reach, void *stream) {
+  FleetDims d;
+  int rc = fleet_dims(cfg, fleet, &d);
+  if (rc) return rc;
+  if (!world) return fail(TTMPC_ERR_BAD_ARG, "fleet world: null");
+  if (world->M < 0 || world->max_pv < 3) return fail(TTMPC_ERR_BAD_ARG, "fleet world: M < 0 or max_pv < 3");
+  if (!(world->reach > 0.0 && world->reach < INFINITY) || !(world->cell > 0.0 && world->cell < INFINITY))
+    return fail(TTMPC_ERR_BAD_ARG, "fleet world: reach and cell must be finite and > 0");
+  if (world->nx < 1 || world->ny < 1 || (long long)world->nx * world->ny >= 0x7fffffffLL)
+    return fail(TTMPC_ERR_BAD_ARG, "fleet world: nx and ny must be >= 1 and nx*ny + 1 fit in an int");
+  if (world->M > 0 && (!world->poly_xy || !world->poly_nv || !world->rows || !world->bbox || !world->cell_start ||
+                       !world->cell_items))
+    return fail(TTMPC_ERR_BAD_ARG, "fleet world: poly_xy, poly_nv, rows, bbox, cell_start, cell_items are required");
+  if (!d_stc_out) return fail(TTMPC_ERR_BAD_ARG, "fleet world: d_stc_out is required");
+  if (fleet->n == 0) return TTMPC_OK;
+  CUDA_TRY(launch_fleet_world_select(*fleet, *world, cfg->Nstcobs, cfg->nstcobs, d_stc_out, d_slot_poly, d_n_reach,
+                                     (cudaStream_t)stream));
+  return TTMPC_OK;
+}
 
 // Cumulative device-side counters since the last reset:
 // [0] cost-only evaluations [1] cost+gradient evaluations [2] dynamic-obstacle

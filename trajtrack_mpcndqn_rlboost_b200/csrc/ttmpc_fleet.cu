@@ -6,7 +6,8 @@
 //
 // The kernels are copy / scalar work: pack writes the n x np parameter block once, coalesced
 // (HBM-bound, 21 KB per robot), advance touches 5 doubles per robot, the monitor (run after the
-// step, include/ttmpc.h: ttmpc_fleet_monitor) reads a robot's polygons, obstacles and reference rows.
+// step, include/ttmpc.h: ttmpc_fleet_monitor) reads a robot's polygons, obstacles and reference rows,
+// the map selection (run before the step, ttmpc_fleet_world) the map polygons near a robot.
 #include <cuda_runtime.h>
 
 #include "ttmpc_device.cuh"
@@ -451,6 +452,128 @@ __global__ void __launch_bounds__(128) fleet_monitor_kernel(const ttmpc_fleet f,
 
 cudaError_t launch_fleet_monitor(const ttmpc_fleet &f, const ttmpc_fleet_monitor &m, cudaStream_t st) {
   fleet_monitor_kernel<<<(f.n + 127) / 128, 128, 0, st>>>(f, m);
+  return cudaGetLastError();
+}
+
+// ---- shared obstacle map: each robot's nearest map polygons into its static slots
+constexpr int WS_WARPS = 4;     // robots (one warp each) per CTA of fleet_world_select_kernel
+constexpr int WS_CAP = 128;     // candidates a warp buffers; >= K + 32 for every K <= 32 (Nstcobs)
+constexpr int WS_MAX_K = 32;
+
+// grid cell of coordinate v, clamped to 0..n-1 (NaN: 0)
+__device__ __forceinline__ int world_cell(double v, double origin, double cell, int n) {
+  const double a = floor((v - origin) / cell);
+  return a >= 0.0 ? (a <= n - 1 ? (int)a : n - 1) : 0;
+}
+// cells x..y of one axis that the query c +- R visits, widened by one against rounding and
+// clamped to the grid; x > y: none (also for a NaN or infinite coordinate)
+__device__ __forceinline__ int2 world_axis(double c, double R, double origin, double cell, int n) {
+  const double a = floor((c - R - origin) / cell) - 1.0, b = floor((c + R - origin) / cell) + 1.0;
+  if (!(a <= b) || b < 0.0 || a > n - 1) return make_int2(0, -1);
+  return make_int2(a < 0.0 ? 0 : (int)a, b > n - 1 ? n - 1 : (int)b);
+}
+// Keep the K smallest keys (d, o) of the warp's buffer [0, c): each lane ranks its entries against
+// all c (keys are unique: one entry per polygon), the winners land at their rank.  Returns min(c, K).
+__device__ __forceinline__ int world_keep_best(double *bd, int *bo, double *td, int *to, int c, int K, int lane) {
+  if (lane < K) { td[lane] = INFINITY; to[lane] = -1; }
+  __syncwarp();
+  for (int i = lane; i < c; i += 32) {
+    const double di = bd[i];
+    const int oi = bo[i];
+    int r = 0;
+    for (int j = 0; j < c; j++) r += (bd[j] < di || (bd[j] == di && bo[j] < oi)) ? 1 : 0;
+    if (r < K) { td[r] = di; to[r] = oi; }
+  }
+  __syncwarp();
+  const int k = min(c, K);
+  if (lane < k) { bd[lane] = td[lane]; bo[lane] = to[lane]; }
+  __syncwarp();
+  return k;
+}
+
+// One warp per robot (include/ttmpc.h, ttmpc_fleet_world).  The lanes walk the items of the visited
+// cells one row of cells at a time (a row's items are contiguous in cell_items), each lane finds its
+// item's cell, takes the polygon only in its lowest visited cell and computes its distance; eligible
+// (d, o) go to the warp's shared buffer by ballot.  A full buffer is cut to its best K, so any
+// candidate count stays exact.  At the end the best K are ordered by map index and the rows written
+// with consecutive lanes on consecutive doubles.  oracle/ttfleet_world_oracle.c is the brute-force
+// restatement over all M polygons.
+__global__ void __launch_bounds__(32 * WS_WARPS) fleet_world_select_kernel(
+    const double *__restrict__ state, int n, const ttmpc_fleet_world w, int K, int ns,
+    double *__restrict__ stc_out, int *__restrict__ slot_poly, int *__restrict__ n_reach) {
+  __shared__ double s_d[WS_WARPS][WS_CAP], s_td[WS_WARPS][WS_MAX_K];
+  __shared__ int s_o[WS_WARPS][WS_CAP], s_to[WS_WARPS][WS_MAX_K];
+  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+  const int e = blockIdx.x * WS_WARPS + warp;
+  if (e >= n) return;  // the whole warp
+  double *bd = s_d[warp], *td = s_td[warp];
+  int *bo = s_o[warp], *to = s_to[warp];
+  const double x = state[3 * e], y = state[3 * e + 1], R = w.reach;
+  int c = 0, total = 0;
+  if (w.M > 0) {
+    const int2 qx = world_axis(x, R, w.origin_x, w.cell, w.nx), qy = world_axis(y, R, w.origin_y, w.cell, w.ny);
+    const int qx0 = qx.x, qx1 = qx.y, qy0 = qy.x, qy1 = qy.y;
+    const int n_items = max(w.cell_start[w.nx * w.ny], 0);
+    for (int cy = qy0; cy <= qy1; cy++) {
+      const int *cs = w.cell_start + (size_t)cy * w.nx;
+      const int lo = min(max(cs[qx0], 0), n_items), hi = min(max(cs[qx1 + 1], 0), n_items);
+      int cx = qx0;
+      for (int base = lo; base < hi; base += 32) {
+        const int i = base + lane;
+        double d = 0.0;
+        int o = -1;
+        bool take = false;
+        if (i < hi) {
+          while (cx < qx1 && i >= cs[cx + 1]) cx++;
+          o = w.cell_items[i];
+          if (o >= 0 && o < w.M) {
+            const double *bb = w.bbox + 4 * (size_t)o;
+            const int nv = min(w.poly_nv[o], w.max_pv);
+            if (nv >= 3 && cx == max(qx0, world_cell(bb[0], w.origin_x, w.cell, w.nx)) &&
+                cy == max(qy0, world_cell(bb[1], w.origin_y, w.cell, w.ny))) {
+              d = poly_distance(w.poly_xy + (size_t)o * w.max_pv * 2, nv, x, y);
+              take = d <= R;
+            }
+          }
+        }
+        const unsigned bal = __ballot_sync(0xffffffffu, take);
+        if (!bal) continue;
+        const int cnt = __popc(bal);
+        total += cnt;
+        if (c + cnt > WS_CAP) c = world_keep_best(bd, bo, td, to, c, K, lane);
+        if (take) {
+          const int pos = c + __popc(bal & ((1u << lane) - 1u));
+          bd[pos] = d; bo[pos] = o;
+        }
+        c += cnt;
+        __syncwarp();
+      }
+    }
+  }
+  const int k = world_keep_best(bd, bo, td, to, c, K, lane);
+  if (lane < K) to[lane] = -1;
+  __syncwarp();
+  if (lane < k) {  // slot = rank by map index among the taken
+    const int oi = bo[lane];
+    int s = 0;
+    for (int j = 0; j < k; j++) s += bo[j] < oi ? 1 : 0;
+    to[s] = oi;
+  }
+  __syncwarp();
+  const int nrow = K * ns;
+  double *out = stc_out + (size_t)e * nrow;
+  for (int q = lane; q < nrow; q += 32) {
+    const int s = q / ns, o = to[s];
+    out[q] = (o >= 0 && o < w.M) ? w.rows[(size_t)o * ns + (q - s * ns)] : 0.0;
+  }
+  if (slot_poly && lane < K) slot_poly[(size_t)e * K + lane] = to[lane];
+  if (n_reach && lane == 0) n_reach[e] = total;
+}
+
+cudaError_t launch_fleet_world_select(const ttmpc_fleet &f, const ttmpc_fleet_world &w, int K, int ns,
+                                      double *stc_out, int *slot_poly, int *n_reach, cudaStream_t st) {
+  fleet_world_select_kernel<<<(f.n + WS_WARPS - 1) / WS_WARPS, 32 * WS_WARPS, 0, st>>>(
+      f.state, f.n, w, K, ns, stc_out, slot_poly, n_reach);
   return cudaGetLastError();
 }
 

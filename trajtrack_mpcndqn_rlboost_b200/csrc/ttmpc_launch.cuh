@@ -53,6 +53,9 @@ cudaError_t launch_fleet_pack(const ttmpc_fleet &f, const FleetDims &d, double *
 cudaError_t launch_fleet_advance(const ttmpc_fleet &f, const FleetDims &d, const double *u,
                                  const int *exit_status, cudaStream_t st);
 cudaError_t launch_fleet_monitor(const ttmpc_fleet &f, const ttmpc_fleet_monitor &m, cudaStream_t st);
+// K = Nstcobs (<= 32), ns = nstcobs
+cudaError_t launch_fleet_world_select(const ttmpc_fleet &f, const ttmpc_fleet_world &w, int K, int ns,
+                                      double *stc_out, int *slot_poly, int *n_reach, cudaStream_t st);
 cudaError_t launch_fp64_peak(double *out, int blocks, int threads, int iters, cudaStream_t st);
 
 }  // namespace ttmpc

@@ -10,7 +10,9 @@ reference's control loop does per robot per step (src/main.py:155-172, decision_
 through ``ttmpc_fleet_step_device`` (pack -> solve -> advance, include/ttmpc.h).  With
 ``FleetPlanner.enable_monitor`` every step is followed by ``ttmpc_fleet_monitor_device``, which
 records per robot on the device how close it came to its obstacles over the step (swept clearance,
-contacts) and how far it was from its reference path.  The first global
+contacts) and how far it was from its reference path.  With ``FleetPlanner.set_world`` the robots
+share one static map of any size, and every step starts with ``ttmpc_fleet_world_select_device``,
+which writes each robot's nearest map polygons into its static slots.  The first global
 reference trajectories are sampled on the host with the same
 ``TrajectoryGenerator.get_global_ref_traj`` the single-robot mirror uses.  Tasks queued with
 ``FleetPlanner.set_tasks`` are taken on the device (``ttmpc_fleet_step_tasks_device``) and their
@@ -26,13 +28,45 @@ from typing import List, Optional, Sequence
 import numpy as np
 
 from . import _lib
-from .geometry import polygon_halfspace_representation
+from .geometry import convex_hull, polygon_halfspace_representation
 from .mpc_config import Configurator
 from .planner import TrajectoryGenerator
 
 RUNNING, REACHED, FAILED, BAD_TASK, COLLIDED = 0, 1, 2, 3, 4
 GOAL_REACH = 0.08  # a robot that stops at a goal is within its 5 cm box: at most 0.0708 m away
 DYN_OBS_SIZE = 0.8 + 0.8  # main.py:32
+
+
+def world_grid(bbox: np.ndarray, cell: float):
+    """The uniform grid of ``ttmpc_fleet_world`` (include/ttmpc.h) over boxes bbox [M][4] (xmin, ymin,
+    xmax, ymax): origin at the boxes' least corner, ``nx x ny`` cells of size cell, and polygon o
+    listed, ascending within a cell, in every cell its box overlaps.  Returns (origin_x, origin_y, nx,
+    ny, cell_start [nx*ny+1] int32, cell_items int32)."""
+    bbox = np.asarray(bbox, np.float64).reshape(-1, 4)
+    M = len(bbox)
+    if M == 0:
+        return 0.0, 0.0, 1, 1, np.zeros(2, np.int32), np.zeros(0, np.int32)
+    ox, oy = float(bbox[:, 0].min()), float(bbox[:, 1].min())
+    nx = int(np.floor((bbox[:, 2].max() - ox) / cell)) + 1
+    ny = int(np.floor((bbox[:, 3].max() - oy) / cell)) + 1
+    if nx * ny >= 2 ** 31 - 1:
+        raise ValueError(f"world_grid: {nx} x {ny} cells of {cell} m do not fit the grid's int32 offsets")
+
+    def cells(v, o, n):  # floor((v - origin) / cell) in IEEE double, as the kernel computes it
+        return np.clip(np.floor((v - o) / cell), 0, n - 1).astype(np.int64)
+    bx0, bx1 = cells(bbox[:, 0], ox, nx), cells(bbox[:, 2], ox, nx)
+    by0, by1 = cells(bbox[:, 1], oy, ny), cells(bbox[:, 3], oy, ny)
+    wx = bx1 - bx0 + 1
+    cnt = wx * (by1 - by0 + 1)
+    o = np.repeat(np.arange(M), cnt)
+    k = np.arange(int(cnt.sum())) - np.repeat(np.cumsum(cnt) - cnt, cnt)
+    c = (by0[o] + k // wx[o]) * nx + bx0[o] + k % wx[o]
+    order = np.lexsort((o, c))
+    start = np.zeros(nx * ny + 1, np.int64)
+    start[1:] = np.cumsum(np.bincount(c, minlength=nx * ny))
+    if start[-1] >= 2 ** 31:
+        raise ValueError("world_grid: more cell entries than int32 offsets hold")
+    return ox, oy, nx, ny, start.astype(np.int32), o[order].astype(np.int32)
 
 
 def work_mode(config: Configurator, mode: str = "work"):
@@ -106,6 +140,7 @@ class FleetPlanner:
         self.task_next = None  # [n] int32: queued tasks taken so far
         self.static_polys = None  # (polygons, per_robot) of the last update_static_constraints
         self.monitor = None    # _lib.TtmpcFleetMonitor (enable_monitor), None: no monitor
+        self.world = None      # _lib.TtmpcFleetWorld of the shared map (set_world), None: no map
         self.dqn_paths = None  # (path_xy, path_n) the task step keeps current (set_tasks / enable_dqn)
         self._dqn = None       # the DQN side of the step (enable_dqn), None: off
         self.steps = 0
@@ -113,8 +148,10 @@ class FleetPlanner:
     # ------------------------------------------------------------------ obstacles
     def update_static_constraints(self, obstacle_list, per_robot: bool = False):
         """obstacle_list: polygons shared by every robot, or (per_robot=True) one list per robot.
-        Same row layout as InterfaceMpc.update_static_constraints (interface_mpc.py:62-65)."""
+        Same row layout as InterfaceMpc.update_static_constraints (interface_mpc.py:62-65).  Turns a
+        map of ``set_world`` off."""
         cfg = self.config
+        self.world = None
 
         def rows(polys):
             r = [0.0] * cfg.Nstcobs * cfg.nstcobs
@@ -126,6 +163,86 @@ class FleetPlanner:
         self.stc = self.torch.tensor(np.array(data, dtype=np.float64), device=self.state.device)
         self.stc_shared = 0 if per_robot else 1
         self.static_polys = (obstacle_list, per_robot)
+
+    def set_world(self, polygons, reach: Optional[float] = None, cell: Optional[float] = None):
+        """Share one static map of any size among the robots: before every ``step()``, on the step's
+        stream, ``ttmpc_fleet_world_select_device`` (include/ttmpc.h, ``ttmpc_fleet_world``) writes
+        into each robot's Nstcobs static slots the map polygons nearest to it (distance <= reach,
+        ranked by (distance, map index), written in map-index order).  A map of at most Nstcobs
+        polygons, all within reach, gives every robot exactly what
+        ``update_static_constraints(polygons)`` gives.
+
+        polygons: convex obstacles as vertex lists, already processed (inflated) as
+        ``update_static_constraints`` takes them.  Each is replaced by its convex hull, which must
+        have nstcobs / 3 edges (what ``update_static_constraints`` needs to be well defined).
+        reach defaults to N_hor * ts * max(|lin_vel_min|, lin_vel_max), the farthest a feasible
+        rollout gets; cell, the grid's cell size, defaults to reach.  None turns the map off (as
+        ``update_static_constraints`` does) and leaves no static obstacles.
+
+        Per robot, on the device, overwritten by every step: ``stc`` [n][Nstcobs*nstcobs] (the rows
+        the step packs), ``world_slots`` [n][Nstcobs] (map index per slot, -1: empty) and
+        ``world_reach`` [n] (polygons within reach; more than Nstcobs: one of them got no slot)."""
+        t = self.torch
+        cfg = self.config
+        dev = self.state.device
+        K, ns = cfg.Nstcobs, cfg.nstcobs
+        if polygons is None:
+            self.world = None
+            self.stc = t.zeros(1, K * ns, dtype=t.float64, device=dev)
+            self.stc_shared = 1
+            self.static_polys = None
+            return
+        if reach is None:
+            reach = cfg.N_hor * cfg.ts * max(abs(cfg.lin_vel_min), cfg.lin_vel_max)
+        reach = float(reach)
+        cell = reach if cell is None else float(cell)
+        if not (np.isfinite(reach) and reach > 0.0 and np.isfinite(cell) and cell > 0.0):
+            raise ValueError("set_world: reach and cell must be finite and > 0")
+        ne = ns // 3
+        M = len(polygons)
+        xy = np.zeros((M, ne, 2))
+        rows = np.zeros((M, ns))
+        for o, poly in enumerate(polygons):
+            pts = np.asarray(poly, np.float64).reshape(-1, 2)
+            if not np.isfinite(pts).all():
+                raise ValueError(f"set_world: polygon {o} has a non-finite vertex")
+            hull = convex_hull(pts)
+            b, a0, a1 = polygon_halfspace_representation(np.array(poly))
+            if len(hull) != ne or len(b) != ne:
+                raise ValueError(f"set_world: polygon {o} has a hull of {len(hull)} edges, nstcobs = {ns} needs {ne}")
+            xy[o] = hull
+            rows[o] = b + a0 + a1
+        bbox = np.concatenate([xy.min(axis=1), xy.max(axis=1)], axis=1) if M else np.zeros((0, 4))
+        ox, oy, nx, ny, start, items = world_grid(bbox, cell)
+        f64 = dict(dtype=t.float64, device=dev)
+        self.world_poly_xy, self.world_rows, self.world_bbox = (t.tensor(a, **f64) for a in (xy, rows, bbox))
+        self.world_poly_nv = t.full((M,), ne, dtype=t.int32, device=dev)
+        self.world_cell_start = t.tensor(start, device=dev)
+        self.world_cell_items = t.tensor(items, device=dev)
+        w = _lib.TtmpcFleetWorld()
+        w.M, w.max_pv = M, ne
+        if M:
+            w.poly_xy, w.poly_nv = self.world_poly_xy.data_ptr(), self.world_poly_nv.data_ptr()
+            w.rows, w.bbox = self.world_rows.data_ptr(), self.world_bbox.data_ptr()
+            w.cell_start, w.cell_items = self.world_cell_start.data_ptr(), self.world_cell_items.data_ptr()
+        w.reach, w.origin_x, w.origin_y, w.cell, w.nx, w.ny = reach, ox, oy, cell, nx, ny
+        self.stc = t.zeros(self.n, K * ns, **f64)
+        self.stc_shared = 0
+        self.world_slots = t.full((self.n, K), -1, dtype=t.int32, device=dev)
+        self.world_reach = t.zeros(self.n, dtype=t.int32, device=dev)
+        self.static_polys = None
+        self.world = w
+
+    def run_world_select(self, stream=None):
+        """Write each robot's nearest map polygons into ``stc`` from its current state.  ``step()``
+        calls this itself first.  Needs ``set_world``."""
+        if self.world is None:
+            raise RuntimeError("run_world_select: call set_world first")
+        st = stream if stream is not None else self.torch.cuda.current_stream().cuda_stream
+        _lib.check(self.lib.ttmpc_fleet_world_select_device(C.byref(self.cfg), C.byref(self._fleet_struct()),
+                                                            C.byref(self.world), self.stc.data_ptr(),
+                                                            self.world_slots.data_ptr(), self.world_reach.data_ptr(),
+                                                            st), "ttmpc_fleet_world_select_device")
 
     def set_moving_obstacles(self, positions: np.ndarray, displacement_per_step: np.ndarray):
         """positions, displacement_per_step: [n][k][2].  Every step the planner sees
@@ -182,7 +299,9 @@ class FleetPlanner:
         after every ``step()``, on the step's stream.
 
         polygons: static obstacles as vertex rings, shared or (per_robot=True) one list per robot;
-        default: the polygons last given to ``update_static_constraints``, with their per_robot flag.
+        default: the map of ``set_world`` (its hulls, shared) when one is set, else the polygons last
+        given to ``update_static_constraints``, with their per_robot flag.  The monitor measures every
+        robot against every polygon it is given: with a map that is O(M) per robot and step.
         The robot is a disc of robot_radius, a moving obstacle a disc of moving_radius.  The defaults
         monitor the region the MPC's constraints exclude: the robot centre against the polygons the
         MPC sees, and the DYN_OBS_SIZE discs the pack writes for moving obstacles.
@@ -194,6 +313,7 @@ class FleetPlanner:
         which the robot moved ``deviation_max``, ``deviation_sum`` and ``moved_steps``.
         stop_on_contact=True: a RUNNING robot in contact stops with status ``COLLIDED``."""
         t = self.torch
+        use_map = polygons is None and self.world is not None
         if polygons is None and self.static_polys is not None:
             polygons, stored = self.static_polys
             per_robot = stored if per_robot is None else per_robot
@@ -205,7 +325,11 @@ class FleetPlanner:
         dev = self.state.device
         m = _lib.TtmpcFleetMonitor()
         self.mon_poly_xy = self.mon_poly_nv = None
-        if polygons is not None:
+        if use_map and self.world.M > 0:     # the map's own tensors, kept alive here
+            self.mon_poly_xy, self.mon_poly_nv = self.world_poly_xy[None], self.world_poly_nv[None]
+            m.poly_xy, m.poly_nv = self.mon_poly_xy.data_ptr(), self.mon_poly_nv.data_ptr()
+            m.max_poly, m.max_pv, m.poly_shared = self.world.M, self.world.max_pv, 1
+        elif polygons is not None:
             xy, nv = self._polygon_rings(polygons, per_robot)
             self.mon_poly_xy, self.mon_poly_nv = t.tensor(xy, device=dev), t.tensor(nv, device=dev)
             m.poly_xy, m.poly_nv = self.mon_poly_xy.data_ptr(), self.mon_poly_nv.data_ptr()
@@ -512,8 +636,11 @@ class FleetPlanner:
         times the step alone does that).
 
         With the DQN enabled (``enable_dqn``) the step starts with the DQN side of the hybrid loop,
-        which writes ``hint``, on the same stream."""
+        which writes ``hint``, on the same stream.  With a map (``set_world``) the map selection
+        runs before both."""
         st = stream if stream is not None else self.torch.cuda.current_stream().cuda_stream
+        if self.world is not None:
+            self.run_world_select(st)
         if self._dqn is not None:
             self._dqn_step(st, stream)
         f, r = self._fleet_struct(), self._result_struct()

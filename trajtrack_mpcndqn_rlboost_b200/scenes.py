@@ -215,3 +215,64 @@ def make_missions(n: int, tasks: int, seed: int = 0, n_moving: int = 2, max_stat
                 static_polys=polys, task_goals=[g[1:] for g in goals], task_paths=[p[1:] for p in paths],
                 moving_pos=np.stack([ox, oy], axis=-1),
                 moving_disp=np.stack([vmag * np.cos(vdir), vmag * np.sin(vdir)], axis=-1))
+
+
+def make_warehouse(n: int, tasks: int, seed: int = 0, shelves: int = 10_000, shelf=(1.0, 4.0), aisle: float = 3.0,
+                   hops: int = 4):
+    """A warehouse floor for FleetPlanner.set_world: about ``shelves`` rectangular shelves (shelf =
+    width x depth, m) on a lattice with aisles ``aisle`` m wide between them, so the floor's density
+    stays the same at any size.  Robots start at random aisle crossings; every task is a Manhattan
+    route along aisle centre lines (x first or y first, at random) to a random other crossing at most
+    ``hops`` crossings away in each direction, ending 2-20 cm short of it.  A route keeps aisle / 2
+    from every shelf; a robot starts within 5 cm of its first route's first crossing.
+
+    Returns the keys of make_missions with the shared map in place of per-robot obstacles: init,
+    goal, paths (the first task), world_polys (every shelf, CCW rectangles), task_goals / task_paths
+    (the other ``tasks - 1`` tasks), moving_pos / moving_disp ([n][0][2]: no moving obstacles)."""
+    rng = np.random.default_rng(seed)
+    sw, sd = float(shelf[0]), float(shelf[1])
+    gx = int(np.ceil(np.sqrt(shelves)))
+    gy = int(np.ceil(shelves / gx))
+    px, py = sw + aisle, sd + aisle
+    x0 = aisle + px * np.arange(gx)[:, None] + np.zeros(gy)[None]
+    y0 = aisle + py * np.arange(gy)[None, :] + np.zeros(gx)[:, None]
+    x0, y0 = x0.ravel(), y0.ravel()
+    world = [[(a, b), (a + sw, b), (a + sw, b + sd), (a, b + sd)] for a, b in zip(x0.tolist(), y0.tolist())]
+
+    def crossing(i, j):
+        return float(i * px + 0.5 * aisle), float(j * py + 0.5 * aisle)
+
+    ci, cj = rng.integers(0, gx + 1, n), rng.integers(0, gy + 1, n)
+    pos = [crossing(i, j) for i, j in zip(ci, cj)]
+    goals, paths = [[] for _ in range(n)], [[] for _ in range(n)]
+    for _ in range(max(tasks, 1)):
+        di, dj = rng.integers(-hops, hops + 1, n), rng.integers(-hops, hops + 1, n)
+        ni, nj = np.clip(ci + di, 0, gx), np.clip(cj + dj, 0, gy)
+        same = (ni == ci) & (nj == cj)
+        ni = np.where(same, np.where(ci < gx, ci + 1, ci - 1), ni)
+        x_first = rng.random(n) < 0.5
+        short = rng.uniform(0.02, 0.2, n)
+        for e in range(n):
+            # from where the robot stands (on the aisle into its crossing) to the crossing, along one
+            # aisle and the other, and to a stop 2-20 cm short of the target crossing: a sampled
+            # reference never lands on a route's last node, which get_global_ref_traj cannot walk past
+            a, b = crossing(ci[e], cj[e]), crossing(ni[e], nj[e])
+            corner = (b[0], a[1]) if x_first[e] else (a[0], b[1])
+            nodes = [pos[e]]
+            for q in (a, corner, b):
+                if q != nodes[-1]:
+                    nodes.append(q)
+            (px_, py_), (bx, by) = nodes[-2], nodes[-1]
+            L = float(np.hypot(bx - px_, by - py_))
+            nodes[-1] = (bx - (bx - px_) / L * short[e], by - (by - py_) / L * short[e])
+            pos[e] = nodes[-1]
+            paths[e].append(nodes)
+            goals[e].append((nodes[-1][0], nodes[-1][1], 0.0))
+        ci, cj = ni, nj
+    first = [p[0] for p in paths]
+    off = rng.uniform(-0.05, 0.05, (n, 2))  # a parked robot stands a few cm off its spot
+    init = np.array([[p[0][0] + off[e, 0], p[0][1] + off[e, 1], np.arctan2(p[1][1] - p[0][1], p[1][0] - p[0][0])]
+                     for e, p in enumerate(first)])
+    return dict(init=init, goal=np.array([g[0] for g in goals]), paths=first, world_polys=world,
+                task_goals=[g[1:tasks] for g in goals], task_paths=[p[1:tasks] for p in paths],
+                moving_pos=np.zeros((n, 0, 2)), moving_disp=np.zeros((n, 0, 2)))
